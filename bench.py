@@ -10,6 +10,7 @@ A "step" is ONE full reverse chain (T denoiser evaluations + T fused updates) ov
 
   python bench.py --gpus N --steps K --warmup W            (native arm; torchrun for N>1)
   python bench.py --impl reference ...                     (CPU oracle port of the reference path)
+  python bench.py ... --dump-outputs DIR                   (also writes x_0 of the last timed chain to DIR/x0.npy)
 
 Prints ONE JSON line on rank 0.  Besides the contract keys it carries
   roofline      the tcgen05 conv class of one denoiser step: achieved = EXECUTED FLOPs / summed CUDA-event
@@ -32,6 +33,8 @@ import time
 
 import torch
 
+# the benchmark may run from a read-only tree: no bytecode caches next to the project's modules
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -267,18 +270,21 @@ def run_native(args, rank, world, local_rank):
     launches = 0
     graph_launches = 0
     rebuilt = 0
-    barrier()
-    for k in range(args.steps):
-        flush.fill_(k)
-        ev[k][0].record()
-        chain_device(k)
-        ev[k][1].record()
-        launches += net.last_chain_launches(ROWS, COLS, PAST, FUT)
-        gl, rb = net.last_chain_graph_stats(ROWS, COLS, PAST, FUT)
-        graph_launches += gl
-        rebuilt += int(rb)
-    barrier()
-    clk = clocks.stop() if clocks else None
+    x_last = None
+    try:
+        barrier()
+        for k in range(args.steps):
+            flush.fill_(k)
+            ev[k][0].record()
+            x_last = chain_device(k)
+            ev[k][1].record()
+            launches += net.last_chain_launches(ROWS, COLS, PAST, FUT)
+            gl, rb = net.last_chain_graph_stats(ROWS, COLS, PAST, FUT)
+            graph_launches += gl
+            rebuilt += int(rb)
+        barrier()
+    finally:                                      # never leave the nvidia-smi sampler running
+        clk = clocks.stop() if clocks else None
     ms = sum(a.elapsed_time(b) for a, b in ev)
     # ---- timed: end to end through the public call with host buffers ----
     chain_e2e(999)
@@ -345,8 +351,28 @@ def run_native(args, rank, world, local_rank):
                 "sample": f"{args.ref_iters} denoiser+DDPM.step iterations at batch {n} on the host cores "
                           f"(oracle/ restatement of the reference CPU path), extrapolated to {T_STEPS} steps"}
         print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"x0": x_last})
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each output of the last timed step as out_dir/<name>.npy (float32), so that two builds run with the
+    same arguments can be compared output for output.  The files stay within DUMP_MAX_BYTES in all: an array over
+    its share keeps a fixed, seeded subset of its samples (leading dimension)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_MAX_BYTES // len(arrays)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        if a.nbytes > share:
+            keep = share // (a.nbytes // a.shape[0])
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ---- other BASELINE configs / batches: one timed full chain each ------------------------------------------------
@@ -770,7 +796,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-train", action="store_true", help="skip the training-step leg (extra key 'train')")
     ap.add_argument("--no-extras", action="store_true", help="skip the n=1280 / ATC_medium / ETH-UCY chains")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write x_0 of the last timed chain (rank 0's samples) as DIR/x0.npy, float32")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs applies to the native arm")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -1,10 +1,10 @@
 """TEST INFRASTRUCTURE — generates tests/golden/*.npz by running the UNMODIFIED reference
-(imported from /root/reference through oracle/ref_shim.py) on CPU fp32.
+(imported from a checkout of the original project through oracle/ref_shim.py) on CPU fp32.
 
-Run in the build container only:  python -m oracle.make_golden
+Run where such a checkout exists:  python -m oracle.make_golden
 The reference ships no golden vectors of its own (SURVEY.md §4, §8c); these files pin the
-oracle restatement (tests/test_oracle_golden.py) and, on the GPU box where /root/reference
-does not exist, the CUDA path (tests/test_gpu_parity.py).
+oracle restatement (tests/test_oracle_golden.py) and the CUDA path (tests/test_gpu_parity.py)
+without it.
 
 Weights are never stored: every case records the torch seed under which the reference's
 ``UNet(...)`` was constructed plus a SHA-256 of the resulting state_dict; the product ``UNet``

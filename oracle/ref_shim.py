@@ -1,6 +1,7 @@
-"""TEST INFRASTRUCTURE — import shim for the UNMODIFIED reference at /root/reference.
+"""TEST INFRASTRUCTURE — import shim for the UNMODIFIED reference: a checkout of marcemq/crowdmod-ddpm-4D at
+oracle/_ref/ (git-ignored) or wherever $CROWDMOD_REFERENCE points.
 
-Only usable in the build container (the GPU box has no /root/reference).  Used by
+Only usable where such a checkout exists; the repository does not ship one.  Used by
 oracle/make_golden.py to generate tests/golden/* and by the `not gpu` tests that pin the oracle
 restatement against the live reference.  Never imported by the product package.
 
@@ -13,7 +14,8 @@ import os
 import sys
 import types
 
-REF_ROOT = os.environ.get("CROWDMOD_REFERENCE", "/root/reference")
+REF_ROOT = os.environ.get("CROWDMOD_REFERENCE", os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref"))
+MISSING = f"no checkout of the original project at {REF_ROOT} (set CROWDMOD_REFERENCE to its path)"
 
 
 def available() -> bool:

@@ -14,10 +14,11 @@ from crowdmod_ddpm_4d_b200.models.diffusion.forward import ForwardSampler
 from crowdmod_ddpm_4d_b200.utils.checkpoint import get_model_fullname, save_checkpoint
 from crowdmod_ddpm_4d_b200.utils.myparser import getYamlConfig
 from oracle import ddpm_oracle as do
+from oracle import ref_shim
 from tests._util import build_unet, load_golden
 
 CFG = os.path.join(os.path.dirname(__file__), "configs")
-REF_CFG = "/root/reference/config"
+REF_CFG = os.path.join(ref_shim.REF_ROOT, "config")
 
 
 def test_state_dict_contract_atc():
@@ -132,7 +133,7 @@ def test_config_nested_and_legacy_adapter():
     assert sum(p.numel() for p in m.denoiser.parameters() if p.requires_grad) == 28766915
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_CFG), reason="reference configs only exist in the build container")
+@pytest.mark.skipif(not os.path.isdir(REF_CFG), reason=ref_shim.MISSING)
 @pytest.mark.parametrize("name", ["ATC.yml", "ATC_synthetic.yml", "ATC_medium.yml", "HERMES-CR-120.yml",
                                   "ETHUCY_ddpm.yml"])
 def test_all_baseline_configs_load(name):
@@ -142,6 +143,25 @@ def test_all_baseline_configs_load(name):
     rows, cols = cfg.MACROPROPS.ROWS, cfg.MACROPROPS.COLS
     launches, flops = m.denoiser.native_stats(rows, cols, cfg.DATASET.PAST_LEN, cfg.DATASET.FUTURE_LEN)
     assert flops > 0
+
+
+@pytest.mark.parametrize("name,params,gflop", [
+    ("atc_nested.yml", 7200099, 4.323),                    # config/ATC.yml
+    ("atc_synthetic_legacy_flat.yml", 7200099, 4.323),     # config/ATC_synthetic.yml
+    ("atc_legacy_flat.yml", 28766915, 34.44),              # config/ATC_medium.yml
+    ("hermes_nested_model_samples.yml", 7200099, 6.729),   # config/HERMES-CR-120.yml
+    ("ethucy_legacy_flat.yml", 7200099, 0.960),            # config/ETHUCY_ddpm.yml
+])
+def test_baseline_config_schemas_load(name, params, gflop):
+    """The five BASELINE configs' schemas and shapes (stored fixtures): they load, build the denoiser and its
+    native plan, and give the parameter and FLOP counts of BASELINE.md section 2."""
+    cfg = getYamlConfig(os.path.join(CFG, name))
+    m = DDPM_model(cfg, "DDPM-UNet", 3)
+    assert cfg.MODEL.DDPM.CHECKPOINTS_TO_KEEP >= 1
+    assert sum(p.numel() for p in m.denoiser.parameters() if p.requires_grad) == params
+    rows, cols = cfg.MACROPROPS.ROWS, cfg.MACROPROPS.COLS
+    launches, flops = m.denoiser.native_stats(rows, cols, cfg.DATASET.PAST_LEN, cfg.DATASET.FUTURE_LEN)
+    assert launches > 0 and abs(flops / 1e9 - gflop) < 0.01
 
 
 def test_checkpoint_layout(tmp_path):

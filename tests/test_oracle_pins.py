@@ -1,5 +1,9 @@
-"""CPU, build container only: the oracle restatement against the LIVE reference imported from
-/root/reference (skipped where the reference does not exist, e.g. on the GPU box)."""
+"""CPU: the oracle restatement against the LIVE reference imported from a checkout of the original project
+(oracle/ref_shim.py: oracle/_ref/ or $CROWDMOD_REFERENCE; skipped where there is none).  The stored vectors of
+tests/golden/ (tests/test_oracle_golden.py) check the oracle against the reference's outputs on other inputs only:
+UNet forward at the ATC / HERMES / small geometries, seeded init at base 32, the schedule, whole chains (rel-L2,
+not one bit-exact DDPM.step), metrics, DiT at patch 4.  The dataset windows and batch order, the geometries below,
+the base-64 init and the DiT patch-2 case are checked here only."""
 import pytest
 import torch
 
@@ -7,7 +11,7 @@ from oracle import ddpm_oracle as do
 from oracle import ref_shim
 from oracle import unet_oracle as uo
 
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason="/root/reference not present")
+pytestmark = pytest.mark.skipif(not ref_shim.available(), reason=ref_shim.MISSING)
 
 
 @pytest.fixture(scope="module")
