@@ -314,7 +314,26 @@ int cm_op_attn_core(const float* qkv, void* ctx16, int B, int S, int C, int head
 int cm_op_attn_core_backward(const float* qkv, const float* dctx, float* dqkv, int B, int S, int C, int heads,
                              void* stream) {
   if (int e = backward_init()) return e;
-  return attn_core_backward_enqueue(qkv, dctx, dqkv, B, S, C, heads, static_cast<cudaStream_t>(stream));
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (S <= 128) return attn_core_backward_enqueue(qkv, dctx, dqkv, B, S, C, heads, st);
+  // the long-sequence backward reads the forward's row log-sum-exp: rerun the forward into temporaries
+  if (int e = kernels_init()) return e;
+  CM_CHECK(C % heads == 0, "embed dim %d / heads %d unsupported", C, heads);
+  __half* ctx = nullptr;
+  float* lse = nullptr;      // [B][heads][S] log-sum-exp | [B][heads][S] backward row sums
+  CM_CUDA(cudaMalloc(&ctx, (size_t)B * S * C * sizeof(__half)));
+  if (cudaMalloc(&lse, (size_t)2 * B * heads * S * sizeof(float)) != cudaSuccess) {
+    cudaFree(ctx);
+    CM_CHECK(false, "attention backward: out of device memory for the log-sum-exp");
+  }
+  int rc = attn_core_enqueue(qkv, ctx, B, S, C, heads, st, 1, lse);
+  if (!rc) rc = attn_core_backward_enqueue(qkv, dctx, dqkv, B, S, C, heads, st, lse, lse + (size_t)B * heads * S);
+  cudaError_t se = cudaStreamSynchronize(st);
+  cudaFree(ctx);
+  cudaFree(lse);
+  if (rc) return rc;
+  CM_CUDA(se);
+  return 0;
 }
 
 int cm_op_attn_block(const float* x, const float* gamma, const float* beta, const float* w_in, const float* b_in,

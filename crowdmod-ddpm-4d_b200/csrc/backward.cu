@@ -729,7 +729,13 @@ static size_t attn_bwd_smem(int S, int dh) {
 }
 
 int attn_core_backward_enqueue(const float* qkv, const float* dctx, float* dqkv, int B, int S, int C,
-                               int heads, cudaStream_t st) {
+                               int heads, cudaStream_t st, const float* lse, float* dsum) {
+  if (S > 128) {
+    CM_CHECK(C % heads == 0 && (C / heads) % 2 == 0 && C / heads <= 64, "attention: head dim %d / %d unsupported (even, <= 64)",
+             C, heads);
+    CM_CHECK(lse && dsum, "attention backward at S=%d > 128 needs the forward's log-sum-exp and a row-sum workspace", S);
+    return attn_long_backward_enqueue(qkv, dctx, lse, dsum, dqkv, B, S, C, heads, st);
+  }
   CM_CHECK(C % heads == 0 && (C / heads) % 4 == 0 && C % 4 == 0, "embed dim %d / heads %d unsupported", C, heads);
   const size_t smem = attn_bwd_smem(S, C / heads);
   CM_CHECK(smem <= 227 * 1024, "attention backward tile too large for shared memory (S=%d dh=%d)", S, C / heads);

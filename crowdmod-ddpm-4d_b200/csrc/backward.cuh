@@ -77,9 +77,14 @@ int gn_backward_params_all_enqueue(const float* chsum_base, const long long* tab
                                    cudaStream_t st);
 
 // ---- attention core backward (layers.py:16): qkv fp32 [B*S][3C] saved by the forward,
-//      dctx fp32 [B*S][C] -> dqkv fp32 [B*S][3C] (=) ----
+//      dctx fp32 [B*S][C] -> dqkv fp32 [B*S][3C] (=).  S <= 128: one fp32 CTA per (sample, head) with the S x S tile in
+//      shared memory (lse / dsum unused).  S > 128 (attn_long.cu): two deterministic kernels that recompute P from qkv
+//      and lse (fp32 [B][heads][S], the row log-sum-exp attn_core_enqueue wrote); dsum (fp32 [B][heads][S]) is their
+//      workspace for the row sums D_i = sum_j P_ij dP_ij. ----
 int attn_core_backward_enqueue(const float* qkv, const float* dctx, float* dqkv, int B, int S, int C,
-                               int heads, cudaStream_t st);
+                               int heads, cudaStream_t st, const float* lse = nullptr, float* dsum = nullptr);
+int attn_long_backward_enqueue(const float* qkv, const float* dctx, const float* lse, float* dsum, float* dqkv, int B,
+                               int S, int C, int heads, cudaStream_t st);
 
 // ---- final conv backward (unet.py:121,165-167): deps API layout [B][cout][H][W][F], times *scale;
 //      dact (=) fp32 [B][L][H][W][cin]; dw [cout][cin][27] / db [cout] accumulated with atomics ----

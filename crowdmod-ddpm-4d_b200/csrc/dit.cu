@@ -411,7 +411,6 @@ int build(cm_dit* u) {
   u->hp = c.rows / c.patch;
   u->wp = c.cols / c.patch;
   u->Ns = u->hp * u->wp;
-  CM_CHECK(u->Ns <= 128, "more than 128 spatial patches per slot (%d) are not supported by the attention core", u->Ns);
   u->qs = c.past_len / c.t_patch;
   u->nq = u->Tp - u->qs;
   CM_CHECK(u->nq >= 1, "no future temporal slot (past_len %d, t_patch %d)", c.past_len, c.t_patch);

@@ -1446,11 +1446,12 @@ static int attn_dispatch(const float* qkv, __half* ctx, int B, int S, int C, int
 }
 
 int attn_core_enqueue(const float* qkv, __half* ctx, int B, int S, int C, int heads,
-                      cudaStream_t st, int dup) {
+                      cudaStream_t st, int dup, float* lse) {
   CM_CHECK(dup == 1 || dup == 2, "attention: dup must be 1 or 2");
   CM_CHECK(C % heads == 0, "embed dim %d / heads %d unsupported", C, heads);
   const int dh = C / heads;
   CM_CHECK(dh % 2 == 0 && dh <= 64, "attention: head dim %d unsupported (even, <= 64)", dh);
+  if (S > 128) return attn_long_enqueue(qkv, ctx, lse, B, S, C, heads, dup, st);
   if (dh <= 16) return attn_dispatch<16>(qkv, ctx, B, S, C, heads, dup, st);
   if (dh <= 32) return attn_dispatch<32>(qkv, ctx, B, S, C, heads, dup, st);
   return attn_dispatch<64>(qkv, ctx, B, S, C, heads, dup, st);
@@ -1909,6 +1910,7 @@ int kernels_init() {
     CM_CUDA(cudaFuncSetAttribute(attn_block_kernel<8>, cudaFuncAttributePreferredSharedMemoryCarveout, mx));
   }
   if (int rc = attn_init()) return rc;
+  if (int rc = attn_long_init()) return rc;
   if (int rc = conv_init()) return rc;
   done = true;
   return 0;

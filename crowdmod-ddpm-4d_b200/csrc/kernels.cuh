@@ -107,9 +107,16 @@ struct TembParams {
 int temb_enqueue(const TembParams& p, cudaStream_t st);
 
 // ---- attention core softmax(QK^T/sqrt(dh))V per (sample, head) (layers.py:16) ----
-// qkv: fp32 [B*S][3*C] (q | k | v), ctx: fp16 [B*S][dup*C] (dup = 2: hi | lo pair per token)
+// qkv: fp32 [B*S][3*C] (q | k | v), ctx: fp16 [B*S][dup*C] (dup = 2: hi | lo pair per token).  Any S; dh = C / heads
+// even and <= 64.  S <= 128: attn_mma_kernel (whole score row in registers); S > 128: attn_long_kernel (attn_long.cu,
+// keys streamed with the online softmax), which also writes the row log-sum-exp of the scaled scores to lse (fp32
+// [B][heads][S]) when lse is given: the long-sequence backward recomputes P from it.  Capturable (no allocation, no
+// synchronisation).
 int attn_core_enqueue(const float* qkv, __half* ctx, int B, int S, int C, int heads,
-                      cudaStream_t st, int dup = 1);
+                      cudaStream_t st, int dup = 1, float* lse = nullptr);
+int attn_long_enqueue(const float* qkv, __half* ctx, float* lse, int B, int S, int C, int heads, int dup,
+                      cudaStream_t st);
+int attn_long_init();   // attn_long.cu: shared-memory attributes of the long-sequence kernels (called by kernels_init)
 
 // ---- fused AttentionBlock of the sampling path (layers.py:5-18): GroupNorm -> in_proj -> attention core ->
 // out_proj -> + x in one launch (one CTA per sample).  w_in / w_out: packed hi|lo fp16 rows as the 1x1 convs

@@ -180,6 +180,8 @@ struct cm_unet {
   std::vector<size_t> grad_off;         // flat gradient buffer: offset of parameter i
   size_t grad_total = 0;
   int train_reserved = 0, train_prepared = 0;
+  std::vector<float*> attn_lse;         // per op, attention core with S > 128: row log-sum-exp [B][heads][S], then as
+                                        // many floats of backward workspace (reserve_train)
   uint8_t* tarena = nullptr;
   size_t tarena_bytes = 0;
   std::vector<float*> g32;              // per tensor: fp32 gradient [B][pixels][C]
@@ -826,8 +828,9 @@ int run_ops(cm_unet* u, RunCtx& rc, cudaStream_t st, int64_t* launches,
       case OP_ATTN: {
         const Tens& q = u->tens[op.qkv];
         const int S = u->levels[q.level].pps();
+        float* lse = rc.train && oi < u->attn_lse.size() ? u->attn_lse[oi] : nullptr;   // S > 128: kept for the backward
         if (int e = attn_core_enqueue(q.p32, u->tens[op.ctx].p16, rc.batch, S, u->tens[op.ctx].C,
-                                      op.heads, st, rc.dup))
+                                      op.heads, st, rc.dup, lse))
           return e;
       } break;
       case OP_FINAL: {
@@ -928,6 +931,13 @@ int reserve_train(cm_unet* u, int batch) {
   for (int k = 0; k < 8; ++k) o_t[k] = take((size_t)batch * E * 4);
   const size_t o_scale = take(16);
   const size_t o_fd16 = take((size_t)batch * u->levels[0].pps() * 32 * 2);
+  std::vector<size_t> o_lse(u->ops.size(), (size_t)-1);
+  for (size_t i = 0; i < u->ops.size(); ++i) {
+    const Op& op = u->ops[i];
+    if (op.type != OP_ATTN) continue;
+    const size_t S = u->levels[u->tens[op.qkv].level].pps();
+    if (S > 128) o_lse[i] = take((size_t)2 * batch * op.heads * S * 4);   // lse | backward row sums
+  }
   CM_CUDA(cudaMalloc(&u->tarena, off));
   CM_CUDA(cudaMemset(u->tarena, 0, off));
   u->tarena_bytes = off;
@@ -951,6 +961,9 @@ int reserve_train(cm_unet* u, int batch) {
   for (int k = 0; k < 8; ++k) *tp[k] = reinterpret_cast<float*>(u->tarena + o_t[k]);
   u->loss_scale = reinterpret_cast<float*>(u->tarena + o_scale);
   u->final_d16 = reinterpret_cast<__half*>(u->tarena + o_fd16);
+  u->attn_lse.assign(u->ops.size(), nullptr);
+  for (size_t i = 0; i < u->ops.size(); ++i)
+    if (o_lse[i] != (size_t)-1) u->attn_lse[i] = reinterpret_cast<float*>(u->tarena + o_lse[i]);
   u->train_reserved = batch;
   return 0;
 }
@@ -1320,7 +1333,7 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
         const Tens& q = u->tens[op.qkv];
         const int S = u->levels[q.level].pps();
         if (int e = attn_core_backward_enqueue(q.p32, u->g32[op.ctx], u->g32[op.qkv], B, S, u->tens[op.ctx].C,
-                                               op.heads, st))
+                                               op.heads, st, u->attn_lse[oi], u->attn_lse[oi] ? u->attn_lse[oi] + (size_t)B * op.heads * S : nullptr))
           return e;
         written[op.qkv] = 1;
         ++nl;

@@ -175,10 +175,14 @@ CM_API int cm_op_conv3d(int mode, const void* act16, int B, int D, int H, int W,
 CM_API int cm_op_gn_silu(const float* src0, int c0, const float* src1, int c1, const float* gamma,
                   const float* beta, int B, int pixels, float eps, int silu, void* out_norm16,
                   void* out_raw16, void* stream);
+/* attention core softmax(Q K^T / sqrt(dh)) V per (sample, head): qkv fp32 [B][S][3C] (q | k | v), ctx16 fp16 [B][S][C]
+ * out.  Any S (S > 128 streams the keys with the online softmax); dh = C / heads even and <= 64. */
 CM_API int cm_op_attn_core(const float* qkv, void* ctx16, int B, int S, int C, int heads, void* stream);
 /* backward of the attention core (autograd of softmax(Q K^T / sqrt(dh)) V inside nn.MultiheadAttention, reference
  * models/backbones/layers.py:5-18 under loss.backward(), ddpm.py:143): qkv fp32 [B][S][3C] (the in_proj output the
- * training forward saved), dctx fp32 [B][S][C] = gradient of the core's output, dqkv fp32 [B][S][3C] out. */
+ * training forward saved), dctx fp32 [B][S][C] = gradient of the core's output, dqkv fp32 [B][S][3C] out.  Any S;
+ * S <= 128 needs dh % 4 == 0, S > 128 dh even and <= 64 (the forward is rerun into temporaries for its output and
+ * row log-sum-exp).  Deterministic. */
 CM_API int cm_op_attn_core_backward(const float* qkv, const float* dctx, float* dqkv, int B, int S, int C, int heads,
                              void* stream);
 /* whole AttentionBlock of the sampling path (reference models/backbones/layers.py:5-18: GroupNorm(8) ->
