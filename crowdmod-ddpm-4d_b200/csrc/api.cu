@@ -1,11 +1,8 @@
 // Library-level C ABI: error reporting, device error flag, op-level entry points used by the
 // unit tests (each wraps one kernel of the hot path; they allocate temporaries and synchronise,
 // the model-level calls in unet.cu do not).
-#include <stdlib.h>
-
 #include <mutex>
 #include <string>
-#include <vector>
 
 #include "../../include/crowdmod_b200.h"
 #include "backward.cuh"
@@ -21,12 +18,6 @@ namespace cm {
 static thread_local std::string g_err;
 void set_error(const std::string& msg) { g_err = msg; }
 const char* get_error() { return g_err.c_str(); }
-
-bool pdl_enabled() {
-  // measured on B200 (ATC B=64, graph replay): 1.296 ms/step with PDL vs 1.269 without -> opt-in only
-  static const bool on = getenv("CM_PDL") != nullptr;
-  return on;
-}
 
 static int* g_flag = nullptr;
 int* device_error_flag() {
@@ -86,73 +77,6 @@ int cm_op_conv3d(int mode, const void* act16, int B, int D, int H, int W, int ci
       R.p.out32 = out32;
       R.p.out16 = static_cast<__half*>(out16);
       rc = res32_enqueue(R, st);
-      if (const char* e = getenv("CM_DBG_REPS")) {
-        const int reps = atoi(e);
-        cudaEvent_t a, b;
-        cudaEventCreate(&a);
-        cudaEventCreate(&b);
-        cudaStreamSynchronize(st);
-        cudaEventRecord(a, st);
-        for (int i = 0; i < reps && !rc; ++i) rc = res32_enqueue(R, st);
-        cudaEventRecord(b, st);
-        cudaEventSynchronize(b);
-        float ms = 0.f;
-        cudaEventElapsedTime(&ms, a, b);
-        fprintf(stderr, "CM_DBG res32 B=%d D=%d H=%d W=%d cin=%d+%d cout=%d HB=%d units=%d stages=%d grid=%d smem=%zu: %.2f us/launch (%.1f TF/s)\n",
-                B, D, H, W, cin, cin_extra, cout, R.p.HB, R.p.n_units, R.p.stages, R.grid.x, R.smem, ms * 1e3f / reps,
-                R.flops / (ms * 1e-3 / reps) * 1e-12);
-        cudaEventDestroy(a);
-        cudaEventDestroy(b);
-      }
-    }
-    if (!rc && getenv("CM_PLANE_TRACE")) {   // bring-up: event trace of CTA 0 (producer / MMA issuer / drain warp / store warp)
-      const size_t n = (size_t)4 * PL_TRACE_CAP * 2;
-      long long* tr = nullptr;
-      cudaMalloc(&tr, n * 8);
-      cudaMemset(tr, 0, n * 8);
-      R.p.trace = tr;
-      unsigned long long* ct = nullptr;
-      cudaMalloc(&ct, (size_t)R.grid.x * 16);
-      cudaMemset(ct, 0, (size_t)R.grid.x * 16);
-      R.p.cta_times = ct;
-      cudaStreamSynchronize(st);
-      rc = res32_enqueue(R, st);
-      cudaStreamSynchronize(st);
-      {
-        std::vector<unsigned long long> hc((size_t)R.grid.x * 2);
-        cudaMemcpy(hc.data(), ct, hc.size() * 8, cudaMemcpyDeviceToHost);
-        unsigned long long s0 = ~0ull, s1 = 0, e0 = ~0ull, e1 = 0, dmin = ~0ull, dmax = 0;
-        for (unsigned i = 0; i < R.grid.x; ++i) {
-          const unsigned long long a = hc[2 * i], b = hc[2 * i + 1];
-          if (a < s0) s0 = a;
-          if (a > s1) s1 = a;
-          if (b < e0) e0 = b;
-          if (b > e1) e1 = b;
-          if (b - a < dmin) dmin = b - a;
-          if (b - a > dmax) dmax = b - a;
-        }
-        fprintf(stderr, "CTA_TIMES ns: first start 0, last start %llu, first end %llu, last end %llu; CTA duration min %llu max %llu\n",
-                s1 - s0, e0 - s0, e1 - s0, dmin, dmax);
-      }
-      R.p.cta_times = nullptr;
-      cudaFree(ct);
-      std::vector<long long> h(n);
-      cudaMemcpy(h.data(), tr, n * 8, cudaMemcpyDeviceToHost);
-      long long t0 = 0;
-      for (size_t i = 0; i < n; i += 2)
-        if (h[i] && (t0 == 0 || h[i + 1] < t0)) t0 = h[i + 1];
-      static const char* role[4] = {"prod", "mma", "drain", "store"};
-      for (int r = 0; r < 4; ++r) {
-        long long prev = t0;
-        for (int i = 0; i < PL_TRACE_CAP; ++i) {
-          const long long code = h[((size_t)r * PL_TRACE_CAP + i) * 2], t = h[((size_t)r * PL_TRACE_CAP + i) * 2 + 1];
-          if (!code) break;
-          fprintf(stderr, "PL_TRACE %s i=%d code=%lld t=%lld dt=%lld\n", role[r], i, code, t - t0, t - prev);
-          prev = t;
-        }
-      }
-      R.p.trace = nullptr;
-      cudaFree(tr);
     }
     cudaError_t se3 = cudaStreamSynchronize(st);
     cudaFree(wp);
@@ -176,51 +100,6 @@ int cm_op_conv3d(int mode, const void* act16, int B, int D, int H, int W, int ci
       PLn.p.out32 = out32;
       PLn.p.out16 = static_cast<__half*>(out16);
       rc = plane_enqueue(PLn, st);
-      if (const char* e = getenv("CM_DBG_REPS")) {
-        const int reps = atoi(e);
-        cudaEvent_t a, b;
-        cudaEventCreate(&a);
-        cudaEventCreate(&b);
-        cudaStreamSynchronize(st);
-        cudaEventRecord(a, st);
-        for (int i = 0; i < reps && !rc; ++i) rc = plane_enqueue(PLn, st);
-        cudaEventRecord(b, st);
-        cudaEventSynchronize(b);
-        float ms = 0.f;
-        cudaEventElapsedTime(&ms, a, b);
-        fprintf(stderr, "CM_DBG plane B=%d D=%d H=%d W=%d cin=%d+%d cout=%d bn=%d bk=%d R=%d HB=%d tiles=%d units=%d stages=%d grid=%d: %.2f us/launch (%.1f TF/s)\n",
-                B, D, H, W, cin, cin_extra, cout, PLn.bn, PLn.bk, PLn.p.R, PLn.p.HB, PLn.p.ntiles, PLn.p.n_units,
-                PLn.p.stages, PLn.grid.x, ms * 1e3f / reps, PLn.flops / (ms * 1e-3 / reps) * 1e-12);
-        cudaEventDestroy(a);
-        cudaEventDestroy(b);
-      }
-      if (!rc && getenv("CM_PLANE_TRACE")) {   // bring-up: event trace of CTA 0 (producer / MMA issuer / epilogue warp 2)
-        const size_t n = (size_t)3 * PL_TRACE_CAP * 2;
-        long long* tr = nullptr;
-        cudaMalloc(&tr, n * 8);
-        cudaMemset(tr, 0, n * 8);
-        PLn.p.trace = tr;
-        cudaStreamSynchronize(st);
-        rc = plane_enqueue(PLn, st);
-        cudaStreamSynchronize(st);
-        std::vector<long long> h(n);
-        cudaMemcpy(h.data(), tr, n * 8, cudaMemcpyDeviceToHost);
-        long long t0 = 0;
-        for (size_t i = 0; i < n; i += 2)
-          if (h[i] && (t0 == 0 || h[i + 1] < t0)) t0 = h[i + 1];
-        static const char* role[3] = {"prod", "mma", "epi"};
-        for (int r = 0; r < 3; ++r) {
-          long long prev = t0;
-          for (int i = 0; i < PL_TRACE_CAP; ++i) {
-            const long long code = h[((size_t)r * PL_TRACE_CAP + i) * 2], t = h[((size_t)r * PL_TRACE_CAP + i) * 2 + 1];
-            if (!code) break;
-            fprintf(stderr, "PL_TRACE %s i=%d code=%lld t=%lld dt=%lld\n", role[r], i, code, t - t0, t - prev);
-            prev = t;
-          }
-        }
-        PLn.p.trace = nullptr;
-        cudaFree(tr);
-      }
     }
     cudaError_t se2 = cudaStreamSynchronize(st);
     cudaFree(wp);
@@ -235,48 +114,9 @@ int cm_op_conv3d(int mode, const void* act16, int B, int D, int H, int W, int ci
     L.p.resid = resid;
     L.p.out32 = out32;
     L.p.out16 = static_cast<__half*>(out16);
-    if (impl == 0) {
-      rc = conv_enqueue(L, st);
-      if (getenv("CM_DBG_TRACE")) {
-        unsigned long long* tr = nullptr;
-        cudaMalloc(&tr, 512 * 8);
-        cudaMemset(tr, 0, 512 * 8);
-        L.p.trace = tr;
-        cudaStreamSynchronize(st);
-        conv_enqueue(L, st);
-        cudaStreamSynchronize(st);
-        unsigned long long h[512];
-        cudaMemcpy(h, tr, sizeof(h), cudaMemcpyDeviceToHost);
-        const unsigned long long t0 = h[0];
-        fprintf(stderr, "CM_TRACE start=0 setup_done=%lld tmem_full=%lld epi_done=%lld end=%lld\n",
-                (long long)(h[4] - t0), (long long)(h[1] - t0), (long long)(h[2] - t0), (long long)(h[3] - t0));
-        for (int kb = 0; kb < 120 && h[8 + kb * 4]; ++kb)
-          fprintf(stderr, "CM_TRACE kb=%d prod_wait_done=%lld prod_issued=%lld mma_wait_done=%lld mma_committed=%lld\n", kb,
-                  (long long)(h[8 + kb * 4] - t0), (long long)(h[8 + kb * 4 + 1] - t0),
-                  (long long)(h[8 + kb * 4 + 2] - t0), (long long)(h[8 + kb * 4 + 3] - t0));
-        L.p.trace = nullptr;
-        cudaFree(tr);
-      }
-      if (const char* e = getenv("CM_DBG_REPS")) {   // bring-up timing: avg device time of `reps` launches
-        const int reps = atoi(e);
-        cudaEvent_t a, b;
-        cudaEventCreate(&a);
-        cudaEventCreate(&b);
-        cudaStreamSynchronize(st);
-        cudaEventRecord(a, st);
-        for (int i = 0; i < reps && !rc; ++i) rc = conv_enqueue(L, st);
-        cudaEventRecord(b, st);
-        cudaEventSynchronize(b);
-        float ms = 0.f;
-        cudaEventElapsedTime(&ms, a, b);
-        fprintf(stderr, "CM_DBG conv mode=%d M=%d cin=%d cout=%d bn=%d bk=%d stages=%d grid=%d,%d,%d dbg=%d: %.2f us/launch\n",
-                mode, L.p.M, cin, cout, L.bn, L.bk, L.p.stages, L.grid.x, L.grid.y, L.grid.z, L.p.dbg,
-                ms * 1e3f / reps);
-        cudaEventDestroy(a);
-        cudaEventDestroy(b);
-      }
-    } else rc = conv_ref_enqueue(L.p, static_cast<const __half*>(act16),
-                               static_cast<const __half*>(extra16), wp, B, D, H, W, st);
+    if (impl == 0) rc = conv_enqueue(L, st);
+    else rc = conv_ref_enqueue(L.p, static_cast<const __half*>(act16),
+                             static_cast<const __half*>(extra16), wp, B, D, H, W, st);
   }
   cudaError_t se = cudaStreamSynchronize(st);
   cudaFree(wp);
@@ -424,7 +264,7 @@ int cm_op_conv3d_dgrad_f32(int mode, const float* dout32, int B, int D, int H, i
   PlaneLaunch PLn;
   PLn.ok = false;
   if (!rc) rc = conv_prepare(&L, dgrad_mode_of(mode), d16, B, od, oh, ow, dup * cout, nullptr, 0, wp, cin, terms);
-  if (!rc && mode == 0 && getenv("CM_NO_PLANE") == nullptr)
+  if (!rc && mode == 0)
     rc = plane_prepare(&PLn, d16, B, od, oh, ow, dup * cout, nullptr, 0, wp, cin, terms);
   if (!rc) {
     if (PLn.ok) {
@@ -461,28 +301,6 @@ int cm_op_conv3d_wgrad(int mode, const void* act16, int B, int D, int H, int W, 
                        static_cast<const __half*>(extra16), cin_extra, static_cast<const __half*>(dout16),
                        cout, G);
     if (!rc) rc = wgrad_enqueue(L, st);
-    if (!rc) {
-      if (const char* e = getenv("CM_DBG_REPS")) {
-        const int reps = atoi(e);
-        cudaEvent_t a, b;
-        cudaEventCreate(&a);
-        cudaEventCreate(&b);
-        cudaStreamSynchronize(st);
-        cudaEventRecord(a, st);
-        for (int i = 0; i < reps && !rc; ++i) rc = wgrad_enqueue(L, st);
-        cudaEventRecord(b, st);
-        cudaEventSynchronize(b);
-        float ms = 0.f;
-        cudaEventElapsedTime(&ms, a, b);
-        fprintf(stderr, "CM_DBG wgrad mode=%d M=%d cin=%d cout=%d bkc=%d bn=%d splits=%d grid=%d,%d,%d: %.2f us/launch (%.1f TF/s)\n",
-                mode, L.p.M, cin, cout, L.bkc, L.bn, L.p.splits, L.grid.x, L.grid.y, L.grid.z, ms * 1e3f / reps,
-                L.flops / (ms * 1e-3 / reps) * 1e-12);
-        cudaEventDestroy(a);
-        cudaEventDestroy(b);
-        cudaMemsetAsync(G, 0, gel * sizeof(float), st);
-        rc = wgrad_enqueue(L, st);
-      }
-    }
   } else if (impl == 2) {
     // plane / halo scheme (wgrad_plane.cuh): one launch per 32-channel chunk of the main source; the fused 1x1x1 source
     // goes through wgrad_umma_kernel in 1x1x1 mode into its rows of G
@@ -502,35 +320,8 @@ int cm_op_conv3d_wgrad(int mode, const void* act16, int B, int D, int H, int W, 
     if (!rc && cin_extra)
       rc = wgrad_prepare(&XL, 3, static_cast<const __half*>(extra16), B, D, H, W, cin_extra, nullptr, 0,
                          static_cast<const __half*>(dout16), cout, G + (size_t)27 * cin * cout);
-    auto run = [&]() {
-      int e = 0;
-      for (int c = 0; c < nc && !e; ++c) e = wgrad_plane_enqueue(PL[c], st);
-      if (!e && cin_extra) e = wgrad_enqueue(XL, st);
-      return e;
-    };
-    if (!rc) rc = run();
-    if (!rc) {
-      if (const char* e = getenv("CM_DBG_REPS")) {
-        const int reps = atoi(e);
-        cudaEvent_t a, b;
-        cudaEventCreate(&a);
-        cudaEventCreate(&b);
-        cudaStreamSynchronize(st);
-        cudaEventRecord(a, st);
-        for (int i = 0; i < reps && !rc; ++i) rc = run();
-        cudaEventRecord(b, st);
-        cudaEventSynchronize(b);
-        float ms = 0.f;
-        cudaEventElapsedTime(&ms, a, b);
-        fprintf(stderr, "CM_DBG wgrad plane B=%d D=%d H=%d W=%d cin=%d+%d cout=%d HB=%d units=%d stages=%d grid=%d: %.2f us per conv (%.1f TF/s)\n",
-                B, D, H, W, cin, cin_extra, cout, PL[0].p.HB, PL[0].p.n_units, PL[0].p.stages, PL[0].grid.x, ms * 1e3f / reps,
-                2.0 * B * D * H * W * cout * (27.0 * cin + cin_extra) / (ms * 1e-3 / reps) * 1e-12);
-        cudaEventDestroy(a);
-        cudaEventDestroy(b);
-        cudaMemsetAsync(G, 0, gel * sizeof(float), st);
-        rc = run();
-      }
-    }
+    for (int c = 0; c < nc && !rc; ++c) rc = wgrad_plane_enqueue(PL[c], st);
+    if (!rc && cin_extra) rc = wgrad_enqueue(XL, st);
   } else {
     rc = wgrad_ref_enqueue(mode, static_cast<const __half*>(act16), static_cast<const __half*>(extra16),
                            static_cast<const __half*>(dout16), G, B, D, H, W, cin, cin_extra, cout, st);

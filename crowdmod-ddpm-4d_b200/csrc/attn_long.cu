@@ -106,12 +106,10 @@ attn_long_kernel(const float* __restrict__ qkv, __half* __restrict__ ctx, float*
     fence_mbar_init();
   }
   if (warp == 6) tmem_alloc(tmem_slot, AL_TMEM_COLS);
-  pdl_trigger();
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();
 
   if (warp < 4) {
     // ===================== softmax warps =====================
@@ -306,8 +304,9 @@ attn_long_kernel(const float* __restrict__ qkv, __half* __restrict__ ctx, float*
 template <int DHP>
 int al_launch(const float* qkv, __half* ctx, float* lse, int B, int S, int C, int heads, int dup, cudaStream_t st) {
   const dim3 grid((S + 127) / 128, B * heads);
-  return launch_pdl(attn_long_kernel<DHP>, grid, dim3(AL_THREADS), (size_t)AlCfg<DHP>::SMEM, st, qkv, ctx, lse, S, C,
-                    heads, dup, device_error_flag());
+  attn_long_kernel<DHP><<<grid, AL_THREADS, AlCfg<DHP>::SMEM, st>>>(qkv, ctx, lse, S, C, heads, dup, device_error_flag());
+  CM_CUDA(cudaGetLastError());
+  return 0;
 }
 
 // ---------------------------------------------------------------------------------------------

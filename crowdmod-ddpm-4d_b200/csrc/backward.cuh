@@ -45,8 +45,8 @@ int rowsum_enqueue(const float* in, float* out, int B, int C, int ld, int accumu
 int unpack_wgrad_enqueue(int fwd_mode, const float* G, float* dw, float* dwx, int cout, int cin,
                          int cinx, int perm, cudaStream_t st);
 
-// ---- scalar restatement of the weight gradient (test oracle for wgrad_umma_kernel; also the
-//      CM_WGRAD_REF=1 bring-up path).  Same operands, same G layout, G must be zeroed. ----
+// ---- scalar restatement of the weight gradient (test oracle for wgrad_umma_kernel).  Same
+//      operands, same G layout, G must be zeroed. ----
 int wgrad_ref_enqueue(int fwd_mode, const __half* act16, const __half* extra16, const __half* dout16,
                       float* G, int B, int D, int H, int W, int cin, int cinx, int cout,
                       cudaStream_t st);

@@ -47,34 +47,6 @@ const char* get_error();
 int* device_error_flag();                        // api.cu (lazily cudaMalloc'ed, zeroed)
 
 // ------------------------------------------------------------------------------------------
-// programmatic dependent launch (PDL): every kernel of the sampling step lets the NEXT kernel's
-// CTAs be scheduled early (pdl_trigger at its top) and blocks before touching global memory until
-// the PREVIOUS kernel has completed and flushed (pdl_wait).  The launch latency and the prologue
-// (barrier init, TMEM allocation, tensor-map prefetch) of kernel N+1 then overlap the tail of
-// kernel N.  Both instructions are no-ops for launches without the PDL attribute.
-// ------------------------------------------------------------------------------------------
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-
-bool pdl_enabled();   // api.cu: true when CM_PDL is set (measured: no gain inside the CUDA graph, so opt-in)
-
-template <typename... KArgs, typename... Args>
-int launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  CM_CUDA(cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...));
-  return 0;
-}
-
-// ------------------------------------------------------------------------------------------
 // small device helpers
 // ------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {

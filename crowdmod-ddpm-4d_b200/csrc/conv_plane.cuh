@@ -1,6 +1,6 @@
 // "Plane-tile" implicit-GEMM 3-D convolution (k3 s1 p1) on tcgen05 / TMEM, sm_100a.
 //
-// Why a second conv kernel.  Measured on B200 (tools/plane_dbg.py, profiles/), conv_umma_kernel
+// Why a second conv kernel.  Measured on B200 (DESIGN.md 3.1, profiles/), conv_umma_kernel
 // (conv_umma.cuh) is bound by what one SM can pull out of L2 (~32-45 B/clk): it re-fetches its A
 // tile for each of the 27 taps (TMA im2col) and its weight tile for every 128-pixel M tile; and a
 // 128 x 32 tcgen05.mma re-reads its 4 KB A operand from shared memory for only 32 output columns,
@@ -54,7 +54,6 @@ struct PlaneParams {
   int n_ntiles;          // cout / BN
   int a_stage_bytes;     // bytes reserved for the A box per stage (covers ntiles*128 + 2 rows)
   int cin_main, cin_extra, cout, terms, stages;
-  int dbg;               // bring-up knobs (CM_PLANE_DBG): 1 no A loads, 2 no B loads, 4 no MMA, 8 no stores
   const float* bias;
   const float* bias2;
   int lo_from, lo_from_x;   // as ConvParams: k16 slices of lo-half channels skip the lo weight term
@@ -73,17 +72,7 @@ struct PlaneParams {
   // them in a fixed order -> bit-reproducible wherever the sample sits in the batch.
   float* stats_rec;
   int* err_flag;
-  long long* trace;      // bring-up (CM_PLANE_TRACE): CTA 0 records (code, clock64) pairs, 3 regions of PL_TRACE_CAP
 };
-constexpr int PL_TRACE_CAP = 256;
-#define PL_TRACE(region, code)                                                        \
-  do {                                                                                \
-    if (tr_on && tr_n < PL_TRACE_CAP) {                                               \
-      P.trace[((region) * PL_TRACE_CAP + tr_n) * 2] = (code);                         \
-      P.trace[((region) * PL_TRACE_CAP + tr_n) * 2 + 1] = clock64();                  \
-      ++tr_n;                                                                         \
-    }                                                                                 \
-  } while (0)
 
 __device__ __forceinline__ void tma_load_tile_5d(const void* desc, uint64_t* bar, void* smem, int c0,
                                                  int c1, int c2, int c3, int c4) {
@@ -142,8 +131,6 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
   float* sred = ybuf + (P.ntiles * 128 + 2) * TLD;                // [epilogue warps][BN][2] + [BN] shifts
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const bool tr_on = P.trace != nullptr && blockIdx.x == 0 && lane == 0 && warp <= 2;
-  int tr_n = 0;
   const int ncm = P.cin_main / BK;
   const int nks_main = (P.th3 ? 3 : 9) * ncm;         // (td, th, chunk) steps; th3: (td, chunk)
   const int nks = nks_main + P.cin_extra / BK;
@@ -169,12 +156,10 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
     fence_mbar_init();
   }
   if (warp == 2) tmem_alloc(tmem_slot, tmem_cols);
-  pdl_trigger();
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();   // everything above is CTA-local set-up; global memory is touched only from here on
 
   if (warp == 0) {
     // ===================== TMA producer =====================
@@ -187,34 +172,25 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
       int td = 0, th = 0, cc = 0;
       for (int ks = 0; ks < nks; ++ks) {
         if (!mbar_wait(&empty_bar[s], ph ^ 1, P.err_flag, 401)) { alive = false; break; }
-        PL_TRACE(0, 1);
         uint8_t* sa = smem + s * stage_bytes;
         uint8_t* sb = sa + P.a_stage_bytes;
         if (elect_one()) {
           if (ks < nks_main && P.th3) {
-            const uint32_t tx = ((P.dbg & 1) ? 0u : (uint32_t)P.a_box_bytes) + ((P.dbg & 2) ? 0u : (uint32_t)(TERMS * b_term));
-            if (tx) mbar_expect_tx(&full_bar[s], tx); else mbar_arrive(&full_bar[s]);
-            if (!(P.dbg & 1))
-              tma_load_tile_5d(&P.amap, &full_bar[s], sa, cc * BK, -1, U.h0 - 1, U.d0 + td - 1, U.n);
-            if (!(P.dbg & 2)) {
+            mbar_expect_tx(&full_bar[s], (uint32_t)P.a_box_bytes + (uint32_t)(TERMS * b_term));
+            tma_load_tile_5d(&P.amap, &full_bar[s], sa, cc * BK, -1, U.h0 - 1, U.d0 + td - 1, U.n);
 #pragma unroll
-              for (int t = 0; t < TERMS; ++t)
-                tma_load_3d(&P.bmap3, &full_bar[s], sb + t * b_term, cc * BK, U.n_tile * BN + t * P.cout, td * 9);
-            }
+            for (int t = 0; t < TERMS; ++t)
+              tma_load_3d(&P.bmap3, &full_bar[s], sb + t * b_term, cc * BK, U.n_tile * BN + t * P.cout, td * 9);
           } else if (ks < nks_main) {
-            const uint32_t tx = ((P.dbg & 1) ? 0u : a_bytes) + ((P.dbg & 2) ? 0u : (uint32_t)B_STAGE);
-            if (tx) mbar_expect_tx(&full_bar[s], tx); else mbar_arrive(&full_bar[s]);
-            if (!(P.dbg & 1))
-              tma_load_tile_5d(&P.amap, &full_bar[s], sa, cc * BK, -1, U.h0 + th - 1, U.d0 + td - 1, U.n);
+            mbar_expect_tx(&full_bar[s], a_bytes + (uint32_t)B_STAGE);
+            tma_load_tile_5d(&P.amap, &full_bar[s], sa, cc * BK, -1, U.h0 + th - 1, U.d0 + td - 1, U.n);
             const int kcol = ((td * 3 + th) * 3) * P.cin_main + cc * BK;
-            if (!(P.dbg & 2)) {
 #pragma unroll
-              for (int t = 0; t < TERMS; ++t)
+            for (int t = 0; t < TERMS; ++t)
 #pragma unroll
-                for (int tw = 0; tw < 3; ++tw)
-                  tma_load_2d(&P.bmap, &full_bar[s], sb + t * B_TERM + tw * B_TAP, kcol + tw * P.cin_main,
-                              U.n_tile * BN + t * P.cout);
-            }
+              for (int tw = 0; tw < 3; ++tw)
+                tma_load_2d(&P.bmap, &full_bar[s], sb + t * B_TERM + tw * B_TAP, kcol + tw * P.cin_main,
+                            U.n_tile * BN + t * P.cout);
           } else {
             // fused 1x1x1 source: centre tap only (tw = 1 against a box that starts at w = -1)
             const int xc = ks - nks_main;
@@ -226,7 +202,6 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
                           U.n_tile * BN + t * P.cout);
           }
         }
-        PL_TRACE(0, 2);
         if (++cc == ncm) {
           cc = 0;
           if (P.th3) ++td;
@@ -254,11 +229,9 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
       // wait until the epilogue has drained this accumulator buffer (first two units: free)
       if (it >= 2 && !mbar_wait(&tmem_empty[buf], ((it >> 1) - 1) & 1, P.err_flag, 404)) break;
       tc_fence_after();
-      PL_TRACE(1, 3);
       const uint32_t d_base = tmem_base + buf * buf_cols;
       for (int ks = 0; ks < nks; ++ks) {
         if (!mbar_wait(&full_bar[s], ph, P.err_flag, 402)) { alive = false; break; }
-        PL_TRACE(1, 4);
         tc_fence_after();
         const int rel = ks < nks_main ? cc * BK - lo_from : (ks - nks_main) * BK - lo_from_x;
         if (++cc == ncm) cc = 0;
@@ -266,45 +239,43 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
           const uint32_t a_addr = smem_u32(smem + s * stage_bytes);
           const uint32_t a_lo0 = kmajor_desc_lo(a_addr);
           const uint32_t b_lo0 = kmajor_desc_lo(a_addr + P.a_stage_bytes);
-          if (!(P.dbg & 4)) {
-            if (ks < nks_main) {
-              uint32_t first = (ks == 0) ? 0u : 1u;
-              const int nth = P.th3 ? 3 : 1;
-              const uint32_t th_step = (static_cast<uint32_t>(P.Wp) * ROWB) >> 4;   // one grid row of the halo box
-              for (int th = 0; th < nth; ++th) {
-#pragma unroll
-                for (int k = 0; k < BK / 16; ++k) {
-#pragma unroll
-                  for (int t = 0; t < TERMS; ++t) {
-                    if (t == 1 && rel + k * 16 >= 0) continue;          // lo activation half x lo weight term: skipped
-                    const uint32_t b_lo = b_lo0 + ((t * b_term + th * 3 * B_TAP) >> 4) + 2 * k;
-                    uint32_t a_lo = a_lo0 + th * th_step + 2 * k;
-                    uint32_t d = d_base;
-#pragma unroll 2
-                    for (int r = 0; r < P.ntiles; ++r) {
-                      umma_f16_lohi(d, a_lo, b_lo, DESC_HI, IDESC, first);
-                      a_lo += TILE_LO;
-                      d += NST;
-                    }
-                    first = 1u;
-                  }
-                }
-              }
-            } else {
+          if (ks < nks_main) {
+            uint32_t first = (ks == 0) ? 0u : 1u;
+            const int nth = P.th3 ? 3 : 1;
+            const uint32_t th_step = (static_cast<uint32_t>(P.Wp) * ROWB) >> 4;   // one grid row of the halo box
+            for (int th = 0; th < nth; ++th) {
 #pragma unroll
               for (int k = 0; k < BK / 16; ++k) {
 #pragma unroll
                 for (int t = 0; t < TERMS; ++t) {
-                  if (t == 1 && rel + k * 16 >= 0) continue;
-                  const uint32_t b_lo = b_lo0 + ((t * b_term + B_TAP) >> 4) + 2 * k;
-                  uint32_t a_lo = a_lo0 + 2 * k;
-                  uint32_t d = d_base + BN;
+                  if (t == 1 && rel + k * 16 >= 0) continue;          // lo activation half x lo weight term: skipped
+                  const uint32_t b_lo = b_lo0 + ((t * b_term + th * 3 * B_TAP) >> 4) + 2 * k;
+                  uint32_t a_lo = a_lo0 + th * th_step + 2 * k;
+                  uint32_t d = d_base;
 #pragma unroll 2
                   for (int r = 0; r < P.ntiles; ++r) {
-                    umma_f16_lohi(d, a_lo, b_lo, DESC_HI, IDESC_X, 1u);
+                    umma_f16_lohi(d, a_lo, b_lo, DESC_HI, IDESC, first);
                     a_lo += TILE_LO;
                     d += NST;
                   }
+                  first = 1u;
+                }
+              }
+            }
+          } else {
+#pragma unroll
+            for (int k = 0; k < BK / 16; ++k) {
+#pragma unroll
+              for (int t = 0; t < TERMS; ++t) {
+                if (t == 1 && rel + k * 16 >= 0) continue;
+                const uint32_t b_lo = b_lo0 + ((t * b_term + B_TAP) >> 4) + 2 * k;
+                uint32_t a_lo = a_lo0 + 2 * k;
+                uint32_t d = d_base + BN;
+#pragma unroll 2
+                for (int r = 0; r < P.ntiles; ++r) {
+                  umma_f16_lohi(d, a_lo, b_lo, DESC_HI, IDESC_X, 1u);
+                  a_lo += TILE_LO;
+                  d += NST;
                 }
               }
             }
@@ -313,7 +284,6 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
           if (ks == nks - 1) umma_commit(&tmem_full[buf]);     // accumulators of this unit complete
         }
         __syncwarp();
-        PL_TRACE(1, 6);
         if (++s == S) { s = 0; ph ^= 1; }
       }
     }
@@ -331,7 +301,7 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
     constexpr int NG = PL_EPI / 128;                       // warps per TMEM lane quarter
     const int plane = P.HB * P.Wp;
     const int sub_r = et / LPR, sub_c = (et % LPR) * 4;
-    // Unit-independent part of the read-out, computed once per thread (measured, tools/plane_trace.py: the
+    // Unit-independent part of the read-out, computed once per thread (measured, profiles/r2_plane_trace_32to32.txt: the
     // per-unit index divisions and the dependent loads of the column constants were 2100 of the 6800
     // cycles of a unit's epilogue chain): the offset of each of this thread's NJ store rows inside a
     // unit (-1: pad column / beyond the unit), and the per-column constants when they do not depend on
@@ -345,7 +315,7 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
       int w = rem - hl * P.Wp;
 #pragma unroll
       for (int j = 0; j < NJ; ++j) {
-        roff[j] = (q < P.P && w < P.W && !(P.dbg & 8)) ? (dl * P.H + hl) * P.W + w : -1;
+        roff[j] = (q < P.P && w < P.W) ? (dl * P.H + hl) * P.W + w : -1;
         q += RPP;
         w += RPP;
         while (w >= P.Wp) {
@@ -373,7 +343,6 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
     int it = 0;
     bool alive = true;
     for (int u = blockIdx.x; u < P.n_units && alive; u += gridDim.x, ++it) {
-      PL_TRACE(2, 10);
       const PlaneUnit U = plane_unit(P, u);
       const int buf = it & 1;
       const int nn0 = U.n_tile * BN;
@@ -392,16 +361,8 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
             rv[j] = *reinterpret_cast<const float4*>(P.resid + static_cast<size_t>(mi[j]) * P.cout + nn0 + sub_c);
         }
       }
-      PL_TRACE(2, 11);
       if (!mbar_wait(&tmem_full[buf], (it >> 1) & 1, P.err_flag, 403)) { alive = false; break; }
-      PL_TRACE(2, 12);
       tc_fence_after();
-      if (P.dbg & 64) {            // bring-up: no epilogue work at all
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&tmem_empty[buf]);
-        continue;
-      }
       // out[row] = Y0[row] + Y1[row + 1] + Y2[row + 2].  Rows are TMEM lanes: the +1 / +2 shifts are
       // warp shuffles; the two rows a 32-row block needs from the NEXT block travel through `side`
       // (Y1 of its lane 0, Y2 of its lanes 0 and 1) and are added at read-out.  Fixed order -> the
@@ -443,9 +404,7 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&tmem_empty[buf]);
-      PL_TRACE(2, 13);
       asm volatile("bar.sync 1, 512;" ::: "memory");
-      PL_TRACE(2, 14);
       // coalesced read-out: RPP rows per pass, LPR lanes per row
       float4 st1 = make_float4(0.f, 0.f, 0.f, 0.f), st2 = st1;   // GroupNorm partial sums of (v - cv)
 #pragma unroll
@@ -504,9 +463,7 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
         }
         if (et < LPR) *reinterpret_cast<float4*>(sred + (PL_EPI / 32) * BN * 2 + sub_c) = cv;
       }
-      PL_TRACE(2, 15);
       asm volatile("bar.sync 1, 512;" ::: "memory");       // ybuf / side are rewritten by the next unit
-      PL_TRACE(2, 16);
       if (P.stats_rec && et < BN) {
         float a1 = 0.f, a2 = 0.f;
 #pragma unroll
@@ -532,7 +489,6 @@ struct PlaneLaunch {
   dim3 grid;
   int bn, bk;
   size_t smem;
-  double flops;
   bool ok;               // false: geometry not covered, use conv_umma_kernel
 };
 

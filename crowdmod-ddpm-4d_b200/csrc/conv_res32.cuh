@@ -2,7 +2,7 @@
 // the conv_2 of the two finest decoder blocks with their fused 1x1x1 match_input; reference:
 // models/backbones/layers.py:32,43,46, unet.py:32), tcgen05 / TMEM / TMA, sm_100a.
 //
-// Why a third conv kernel (measured on B200, tools/umma_microbench.cu + tools/plane_trace.py, DESIGN.md 3.1):
+// Why a third conv kernel (measured on B200, tools/umma_microbench.cu + profiles/r2_res32_trace_*.txt, DESIGN.md 3.1):
 //   * one thread cannot issue tcgen05.mma faster than one per ~55 cycles, and a 128 x 96 x 16 SS-mode MMA
 //     reads 7 KB of operands from shared memory for 48 cycles of tensor-pipe work: the N = 96 MMAs of
 //     conv_plane_kernel run at 67-73 cycles inside the kernel (shared-memory bandwidth: operand reads +
@@ -19,7 +19,7 @@
 //     (TMEM -> hi+lo sum -> tw row shifts -> shared memory: ~400 cycles per unit) and 8 store warps
 //     (residual, bias / time embedding, GroupNorm records, coalesced fp32 + fp16 stores: ~950 cycles), so
 //     neither adds to the unit period (3 600 cycles, set by the MMA issuer: 6 MMAs in ~700 cycles, then
-//     ~330 cycles of commit / barrier wait per stage -- tools/plane_trace.py with TRACE_IMPL=3).
+//     ~330 cycles of commit / barrier wait per stage -- profiles/r2_res32_trace_32to32.txt).
 // Measured (B200, ATC level 0, B = 64): 31.3 us against 37.2 us for conv_plane_kernel; B = 1280: 517 us against 815 us.
 // Operand / epilogue semantics are those of conv_plane_kernel (mode 0 + optional 1x1x1 K-slab); hi and lo
 // products are accumulated separately in fp32 and added in the epilogue (deterministic, fixed order).
@@ -61,8 +61,6 @@ struct Res32Params {
   __half* out16;
   float* stats_rec;      // GroupNorm records, as PlaneParams::stats_rec (units_per_sample records of HB*W rows)
   int* err_flag;
-  long long* trace;      // bring-up (CM_PLANE_TRACE): CTA 0 records (code, clock64) pairs, 4 regions of PL_TRACE_CAP
-  unsigned long long* cta_times;   // bring-up: per CTA {start, end} %globaltimer
 };
 
 template <int TERMS>   // always 2 (a template keeps the definition in this header; instantiated in conv_umma.cu only)
@@ -96,9 +94,6 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
   float* ybuf = side + 2 * 5 * 3 * C;                        // [2][128][TLD]
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const bool tr_on = P.trace != nullptr && blockIdx.x == 0 && lane == 0 &&
-                     (warp <= 1 || warp == R32_DRAIN_W0 || warp == R32_STORE_W0);
-  int tr_n = 0;
   const int nks = 3 + P.nx;                                  // ring stages per unit: td = 0..2, then the 1x1x1 chunks
   const int hblocks = P.H / P.HB;
 
@@ -125,17 +120,10 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
     fence_mbar_init();
   }
   if (warp == 2) tmem_alloc(tmem_slot, 512);
-  pdl_trigger();
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();   // everything above is CTA-local set-up; global memory is touched only from here on
-  if (P.cta_times && threadIdx.x == 0) {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    P.cta_times[2 * blockIdx.x] = t;
-  }
 
   if (warp == 0) {
     // ===================== TMA producer =====================
@@ -158,7 +146,6 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
       const int h0 = (v - d * hblocks) * P.HB;
       for (int ks = 0; ks < nks; ++ks) {
         if (!mbar_wait(&empty_bar[s], ph ^ 1, P.err_flag, 501)) { alive = false; break; }
-        PL_TRACE(0, 1);
         if (elect_one()) {
           uint8_t* sa = ring + s * P.stage_bytes;
           if (ks < 3) {
@@ -178,7 +165,7 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
     // tcgen05.mma issue is effectively synchronous (the issuing thread is held while the tensor pipe works off its one
     // queued MMA), so every instruction the issuer executes between two MMAs of different stages is tensor-pipe idle
     // time: the per-stage wait / commit / descriptor code of the first version cost ~330 cycles per stage, 3 600 cycles
-    // per unit against 1 728 of MMA work (tools/plane_trace.py).  This version keeps the issuer's instruction stream
+    // per unit against 1 728 of MMA work (profiles/r2_res32_trace_32to32.txt).  This version keeps the issuer's instruction stream
     // minimal: ONE thread (no elect / warp-sync per stage), the four barriers a unit depends on (accumulator buffer free,
     // the three td planes loaded) polled TOGETHER up front with independent try_waits (64 cycles for three against 158 for
     // one bounded wait loop, tools/umma_microbench.cu), then the 18 MMAs of the unit straight-line with compile-time
@@ -232,7 +219,6 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
           }
         }
         tc_fence_after();
-        PL_TRACE(1, 4);
         const uint32_t d_base = tmem_base + buf * R32_NST;
 #pragma unroll
         for (int ks = 0; ks < 3; ++ks) {
@@ -259,7 +245,6 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
         }
         if (!alive) break;
         umma_commit(&tmem_full[buf]);                          // accumulator of this unit complete
-        PL_TRACE(1, 6);
       }
     }
   } else if (warp >= R32_DRAIN_W0 && warp < R32_STORE_W0) {
@@ -272,12 +257,9 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
     int it = 0;
     for (int u = blockIdx.x; u < P.n_units; u += gridDim.x, ++it) {
       const int buf = it & 1;
-      PL_TRACE(2, 20);
       if (!mbar_wait(&tmem_full[buf], (it >> 1) & 1, P.err_flag, 503)) break;
-      PL_TRACE(2, 21);
       tc_fence_after();
       if (it >= 2 && !mbar_wait(&ybuf_empty[buf], ((it >> 1) - 1) & 1, P.err_flag, 506)) break;
-      PL_TRACE(2, 22);
       const uint32_t t_lane = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) + buf * R32_NST + c * 16;
       float* yb = ybuf + static_cast<size_t>(buf) * 128 * TLD;
       float* sd = side + (static_cast<size_t>(buf) * 5 + quarter) * 3 * C;
@@ -304,7 +286,6 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&tmem_empty[buf]);
-      PL_TRACE(2, 23);
       if (lane < 2) {
         float4* s1v = reinterpret_cast<float4*>(sd + c * 16);
         float4* s2v = reinterpret_cast<float4*>(sd + (lane == 0 ? C : 2 * C) + c * 16);
@@ -325,7 +306,6 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
       for (int i = 0; i < 4; ++i) dst[i] = make_float4(y0[4 * i], y0[4 * i + 1], y0[4 * i + 2], y0[4 * i + 3]);
       __syncwarp();
       if (lane == 0) mbar_arrive(&ybuf_full[buf]);            // release: this warp's rows / side rows are written
-      PL_TRACE(2, 24);
     }
   } else if (warp >= R32_STORE_W0) {
     // ===================== store warps: transpose buffer -> residual / constants / records -> global =====================
@@ -380,9 +360,7 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
             rv[j] = *reinterpret_cast<const float4*>(P.resid + static_cast<size_t>(mi[j]) * C + sub_c);
         }
       }
-      PL_TRACE(3, 30);
       if (!mbar_wait(&ybuf_full[buf], (it >> 1) & 1, P.err_flag, 507)) break;
-      PL_TRACE(3, 31);
       const float* yb = ybuf + static_cast<size_t>(buf) * 128 * TLD;
       const float* sdb = side + static_cast<size_t>(buf) * 5 * 3 * C;
       float4 st1 = make_float4(0.f, 0.f, 0.f, 0.f), st2 = st1;   // GroupNorm partial sums of (v - cv)
@@ -421,7 +399,6 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
       // this warp has read its rows of the transpose buffer: hand it back to the drain warps
       __syncwarp();
       if (lane == 0) mbar_arrive(&ybuf_empty[buf]);
-      PL_TRACE(3, 32);
       if (P.stats_rec) {
         // lanes that share a channel quad (same lane % LPR) hold different rows: butterfly over them
 #pragma unroll
@@ -450,24 +427,17 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
           *rec = make_float4(cvs[buf * C + st], a1, a2, 0.f);
         }
       }
-      PL_TRACE(3, 33);
     }
   }
   tc_fence_before();
   __syncthreads();
   if (warp == 2) tmem_dealloc(tmem_base, 512);
-  if (P.cta_times && threadIdx.x == 0) {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    P.cta_times[2 * blockIdx.x + 1] = t;
-  }
 }
 
 struct Res32Launch {
   Res32Params p;
   dim3 grid;
   size_t smem;
-  double flops;
   bool ok;               // false: shape not covered, use conv_plane_kernel / conv_umma_kernel
 };
 

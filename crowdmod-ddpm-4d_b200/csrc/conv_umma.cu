@@ -7,7 +7,6 @@
 #include "wgrad_plane.cuh"
 
 #include <cudaTypedefs.h>
-#include <stdlib.h>
 #include <string.h>
 
 namespace cm {
@@ -91,21 +90,21 @@ int launch_t(const ConvLaunch& L, cudaStream_t st) {
     cfg.blockDim = dim3(CONV_THREADS);
     cfg.dynamicSmemBytes = L.smem;
     cfg.stream = st;
-    cudaLaunchAttribute attr[2];
+    cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
     attr[0].val.clusterDim.x = 1;
     attr[0].val.clusterDim.y = 1;
     attr[0].val.clusterDim.z = L.p.ksplit;
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[1].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 2 : 1;
+    cfg.numAttrs = 1;
     if (L.p.terms == 2) CM_CUDA(cudaLaunchKernelEx(&cfg, conv_umma_kernel<BN, BK, 2>, L.p));
     else CM_CUDA(cudaLaunchKernelEx(&cfg, conv_umma_kernel<BN, BK, 1>, L.p));
     return 0;
   }
-  if (L.p.terms == 2) return launch_pdl(conv_umma_kernel<BN, BK, 2>, L.grid, dim3(CONV_THREADS), L.smem, st, L.p);
-  return launch_pdl(conv_umma_kernel<BN, BK, 1>, L.grid, dim3(CONV_THREADS), L.smem, st, L.p);
+  if (L.p.terms == 2) conv_umma_kernel<BN, BK, 2><<<L.grid, CONV_THREADS, L.smem, st>>>(L.p);
+  else conv_umma_kernel<BN, BK, 1><<<L.grid, CONV_THREADS, L.smem, st>>>(L.p);
+  CM_CUDA(cudaGetLastError());
+  return 0;
 }
 
 template <int BN, int BK>
@@ -183,8 +182,7 @@ int conv_prepare(ConvLaunch* L, int mode, const __half* act, int B, int D, int H
     // M-starved deep-K layers (coarsest level: a few dozen M tiles, K in the thousands): keep the
     // widest N tile (A and the weights are fetched once per tile) and split K across a cluster.
     const long nkb_all = (long)(k * k * k) * (cin / bk) + cin_extra / bk;
-    static const bool no_split = getenv("CM_NO_SPLITK") != nullptr;
-    if (!no_split && allow_splitk && p.nphase == 1 && m_tiles * (cout / bn) < 100) {
+    if (allow_splitk && p.nphase == 1 && m_tiles * (cout / bn) < 100) {
       long sk = 2 * 148 / (m_tiles * (cout / bn));   // two CTAs per SM (see the stage budget below)
       if (sk > 8) sk = 8;
       while (sk > 1 && nkb_all / sk < 4) --sk;
@@ -248,8 +246,6 @@ int conv_prepare(ConvLaunch* L, int mode, const __half* act, int B, int D, int H
   // UpSample phase convs have only 8 k-blocks per phase: co-residency (>= 3 CTAs per SM hiding each
   // other's set-up and epilogue) beats pipeline depth (measured: 51.6 us with 2 stages vs 63.7 with 4)
   if (p.nphase == 8) stages = 2;
-  if (const char* e = getenv("CM_DBG_STAGES")) stages = atoi(e);
-  if (const char* e = getenv("CM_DBG_SKIP")) p.dbg = atoi(e);
   if (stages > CONV_MAX_STAGES) stages = CONV_MAX_STAGES;
   while (stages > 2 && (size_t)stages * stage_bytes + 2048 > 200 * 1024) --stages;
   p.stages = stages;
@@ -273,14 +269,12 @@ int conv_prepare(ConvLaunch* L, int mode, const __half* act, int B, int D, int H
   L->smem = (size_t)stages * stage_bytes + 1024 /*align slack*/ + 256 /*barriers*/ + 512 /*colv*/;
   // scatter convs: 4 phases per CTA when that still leaves >= 2 CTAs per SM, else 2, else 1
   p.ppc = 1;
-  if (p.nphase == 8 && getenv("CM_NO_PPC") == nullptr) {
+  if (p.nphase == 8) {
     const long tiles = (long)((p.M + CONV_BM - 1) / CONV_BM) * (cout / bn);
     if (tiles * 2 >= 296) p.ppc = 4;
     else if (tiles * 4 >= 296) p.ppc = 2;
-    if (const char* e = getenv("CM_PPC")) p.ppc = atoi(e);
   }
   L->grid = dim3((p.M + CONV_BM - 1) / CONV_BM, cout / bn, p.ksplit > 1 ? p.ksplit : p.nphase / p.ppc);
-  L->flops = 2.0 * p.M * cout * (double)(k * k * k * cin + cin_extra) * p.nphase;
   return 0;
 }
 
@@ -335,8 +329,10 @@ int make_plane_map(CUtensorMap* map, const __half* base, int B, int D, int H, in
 
 template <int BN, int BK>
 int plane_launch_t(const PlaneLaunch& L, cudaStream_t st) {
-  if (L.p.terms == 2) return launch_pdl(conv_plane_kernel<BN, BK, 2>, L.grid, dim3(PL_THREADS), L.smem, st, L.p);
-  return launch_pdl(conv_plane_kernel<BN, BK, 1>, L.grid, dim3(PL_THREADS), L.smem, st, L.p);
+  if (L.p.terms == 2) conv_plane_kernel<BN, BK, 2><<<L.grid, PL_THREADS, L.smem, st>>>(L.p);
+  else conv_plane_kernel<BN, BK, 1><<<L.grid, PL_THREADS, L.smem, st>>>(L.p);
+  CM_CUDA(cudaGetLastError());
+  return 0;
 }
 template <int BN, int BK>
 int plane_attr_t() {
@@ -376,7 +372,6 @@ int plane_prepare(PlaneLaunch* L, const __half* act, int B, int D, int H, int W,
     CM_CUDA(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev));
   }
   int bk = (cin % 64 == 0 && cin_extra % 64 == 0) ? 64 : 32;
-  if (getenv("CM_PLANE_BK32")) bk = 32;                 // experiment (tools/plane_knock5.py): twice the stages, same MMAs and bytes
   int bn = (cout % 128 == 0) ? 128 : (cout % 64 == 0 ? 64 : 32);
   while (bn > 32 && 3 * bn > 256) bn >>= 1;             // tw-stacked MMA: N = 3*BN <= 256
   const int nst = 3 * bn;
@@ -405,14 +400,12 @@ int plane_prepare(PlaneLaunch* L, const __half* act, int B, int D, int H, int W,
     const double eff = (double)R * HB * W / (ntiles * 128.0);
     if (eff < 0.6) return;                               // mostly padding: leave it to conv_umma
     // useful rows per modelled CTA time: a unit costs its MMAs (~55 cycles each, tw taps stacked along N) plus a fixed
-    // ~2 600 cycles and ~310 cycles per pipeline stage whatever it computes (knock-out skeleton runs, DESIGN.md 3.1.5 and
-    // tools/dgrad_knock.py: 2.3 us per unit on the HERMES grid) -- fewer, fatter units win when the rows-per-tile efficiency
-    // is close.  unit_cost = 0 (CM_PLANE_OLD_SCORE) is the round-1 score eff x fill.
-    static const bool old_score = getenv("CM_PLANE_OLD_SCORE") != nullptr;
+    // ~2 600 cycles and ~310 cycles per pipeline stage whatever it computes (knock-out skeleton runs, DESIGN.md 3.1.5:
+    // 2.3 us per unit on the HERMES grid) -- fewer, fatter units win when the rows-per-tile efficiency is close.
     const double bk_model = R == 1 ? 32.0 : (double)bk;   // th3 stages (single-plane units) use BK = 32
     const double mma_tile = 55.0 * (9.0 * (cin / 16) + (cin_extra / 16)) * terms;
     const double stages = (R == 1 ? 3.0 : 9.0) * (cin / bk_model) + cin_extra / bk_model;
-    const double unit_cost = old_score ? 0.0 : 2600.0 + 310.0 * stages;
+    const double unit_cost = 2600.0 + 310.0 * stages;
     const double score = eff * ((double)units / (waves * n_sm)) * (ntiles * mma_tile) / (ntiles * mma_tile + unit_cost);
     if (score > best * 1.0001 || (score > best * 0.9999 && R * HB > bestR * bestHB)) {
       best = score;
@@ -430,8 +423,7 @@ int plane_prepare(PlaneLaunch* L, const __half* act, int B, int D, int H, int W,
   const int ntiles = (P + 127) / 128;
   PlaneParams& p = L->p;
   // th3 mode (see PlaneParams::th3): single-plane units only; BK = 32 keeps the nine-slab weight stage small
-  static const bool no_th3 = getenv("CM_PLANE_NO_TH3") != nullptr;
-  bool th3 = !no_th3 && R == 1;
+  bool th3 = R == 1;
   if (th3) {
     // needs two stages of {A halo box, nine weight slabs per term} next to the epilogue buffers
     const long a3 = ((long)(ntiles * 128 + 2 * Wp) * 64 + 1023) / 1024 * 1024;
@@ -461,19 +453,16 @@ int plane_prepare(PlaneLaunch* L, const __half* act, int B, int D, int H, int W,
   p.cin_main = cin; p.cin_extra = cin_extra; p.cout = cout; p.terms = terms;
   p.out_ld = cout;
   p.err_flag = device_error_flag();
-  if (const char* e = getenv("CM_PLANE_DBG")) p.dbg = atoi(e);
   const long stage = p.a_stage_bytes + (long)terms * (th3 ? 3 : 1) * nst * rowb;
   const long tail = tail_fixed + ybuf_bytes(ntiles);
   int stages = (int)((smem_cap - tail) / stage);
   if (stages > PL_MAX_STAGES) stages = PL_MAX_STAGES;
-  if (const char* e = getenv("CM_PLANE_STAGES")) stages = atoi(e);
   if (stages < 2) return 0;
   p.stages = stages;
   L->bn = bn;
   L->bk = bk;
   L->smem = (size_t)stages * stage + tail;
   L->grid = dim3(p.n_units < n_sm ? p.n_units : n_sm, 1, 1);
-  L->flops = 2.0 * B * D * H * W * cout * (27.0 * cin + cin_extra);
   L->ok = true;
   return 0;
 }
@@ -504,8 +493,7 @@ int res32_prepare(Res32Launch* L, const __half* act, int B, int D, int H, int W,
   if (int rc = res32_init()) return rc;
   memset(L, 0, sizeof(*L));
   L->ok = false;
-  static const bool off = getenv("CM_NO_RES32") != nullptr;
-  if (off || cin != R32_C || cout != R32_C || terms != 2 || cin_extra % R32_C || cin_extra > 3 * R32_C) return 0;
+  if (cin != R32_C || cout != R32_C || terms != 2 || cin_extra % R32_C || cin_extra > 3 * R32_C) return 0;
   const int Wp = W + 2;
   if (Wp > 128) return 0;
   int HB = 0;
@@ -526,8 +514,7 @@ int res32_prepare(Res32Launch* L, const __half* act, int B, int D, int H, int W,
   const long fixed = 9L * R32_WBLK + (long)nx * R32_WX + tail + 1024;
   int stages = (int)((227L * 1024 - fixed) / stage_bytes);
   if (stages > R32_MAX_STAGES) stages = R32_MAX_STAGES;
-  if (const char* e = getenv("CM_RES32_STAGES")) stages = atoi(e);
-  if (stages < 3 || stages > R32_MAX_STAGES) return 0;
+  if (stages < 3) return 0;
   if (int rc = make_plane_map(&p.amap, act, B, D, H, W, R32_C, 32, 1, HB + 2)) return rc;
   if (nx) {
     CM_CHECK(extra != nullptr, "extra source pointer missing");
@@ -557,13 +544,14 @@ int res32_prepare(Res32Launch* L, const __half* act, int B, int D, int H, int W,
   p.err_flag = device_error_flag();
   L->smem = (size_t)fixed + (size_t)stages * stage_bytes;
   L->grid = dim3(p.n_units < n_sm ? p.n_units : n_sm, 1, 1);
-  L->flops = 2.0 * B * D * H * W * cout * (27.0 * cin + cin_extra);
   L->ok = true;
   return 0;
 }
 
 int res32_enqueue(const Res32Launch& L, cudaStream_t st) {
-  return launch_pdl(conv_res32_kernel<2>, L.grid, dim3(R32_THREADS), L.smem, st, L.p);
+  conv_res32_kernel<2><<<L.grid, R32_THREADS, L.smem, st>>>(L.p);
+  CM_CUDA(cudaGetLastError());
+  return 0;
 }
 
 // ================================ weight gradient (wgrad_umma.cuh) ================================
@@ -706,7 +694,6 @@ int wgrad_prepare(WgradLaunch* L, int mode, const __half* act, int B, int D, int
   L->bn = bn;
   L->smem = (size_t)stages * stage_bytes + 1024 + 256;
   L->grid = dim3(m_tiles, p.n_tiles * splits, p.nphase);
-  L->flops = 2.0 * p.M * cout * (double)p.krows * p.nphase;
   return 0;
 }
 
@@ -732,7 +719,6 @@ int wgrad_plane_prepare(WgradPlaneLaunch* L, const __half* act, int B, int D, in
   if (int rc = load_driver_syms()) return rc;
   memset(L, 0, sizeof(*L));
   L->ok = false;
-  if (getenv("CM_NO_WGRAD_PLANE") != nullptr) return 0;
   if (cout != 32 || cin % 32 != 0 || c0 % 32 != 0 || c0 + 32 > cin) return 0;
   const int Wp = W + 2;
   const int HB = (Wp % 2 == 0) ? 6 : 14;                     // (HB + 2) * Wp must be a multiple of 16 (pixels per MMA)
@@ -759,7 +745,6 @@ int wgrad_plane_prepare(WgradPlaneLaunch* L, const __half* act, int B, int D, in
   p.cin = cin;
   p.G = G;
   p.err_flag = device_error_flag();
-  if (const char* e = getenv("CM_WGP_DBG")) p.dbg = atoi(e);
   if (int rc = make_plane_box_map(&p.amap, act, B, D, H, W, cin, act_ld, Wp, HB + 3)) return rc;
   if (int rc = make_plane_box_map(&p.gmap, dout, B, D, H, W, cout, dout_ld, Wp, HB)) return rc;
   int n_sm = 148;

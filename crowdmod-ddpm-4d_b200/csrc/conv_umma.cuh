@@ -18,12 +18,6 @@
 
 namespace cm {
 
-__device__ __forceinline__ unsigned long long gtime_ns() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-
 constexpr int CONV_BM = 128;        // UMMA M (cta_group::1)
 constexpr int CONV_THREADS = 192;   // warp0 TMA, warp1 MMA, warps2-5 epilogue
 constexpr int CONV_MAX_STAGES = 8;
@@ -73,12 +67,12 @@ struct ConvParams {
   // set up once; measured: the per-CTA set-up was more than half of the 8-tap phase convs' time)
   int ppc;
   int* err_flag;
-  unsigned long long* trace;   // bring-up: per-k-block timestamps of CTA (0,0,0) (CM_DBG_TRACE)
-  int dbg;               // bring-up knobs (CM_DBG_SKIP): 1 no A loads, 2 no B loads, 4 no MMA, 8 no stores
 };
 
+// at most 112 registers: three CTAs of CONV_THREADS per SM, the co-residency conv_prepare's stage budget and the UpSample
+// phase convs are planned for
 template <int BN, int BK, int TERMS>
-__global__ void __launch_bounds__(CONV_THREADS, 1)
+__global__ void __maxnreg__(112)
 conv_umma_kernel(const __grid_constant__ ConvParams P) {
   constexpr int ROWB = BK * 2;                  // bytes per smem row (swizzle span)
   constexpr int A_BYTES = CONV_BM * ROWB;
@@ -135,15 +129,11 @@ conv_umma_kernel(const __grid_constant__ ConvParams P) {
     fence_mbar_init();
   }
   if (warp == 2) tmem_alloc(tmem_slot, TMEM_COLS);
-  pdl_trigger();
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();   // everything above is CTA-local set-up; global memory is touched only from here on
 
-  const bool tr = P.trace != nullptr && blockIdx.x == gridDim.x / 2 && blockIdx.y == 0 && blockIdx.z == 0;
-  if (tr && threadIdx.x == 0) P.trace[0] = gtime_ns();
   if (warp == 0) {
     // ===================== TMA producer (whole warp runs the loop; one elected lane issues) ====
     {
@@ -154,7 +144,7 @@ conv_umma_kernel(const __grid_constant__ ConvParams P) {
       r -= z0 * P.oh * P.ow;
       const int p0 = r / P.ow;
       const int q0 = r - p0 * P.ow;
-      const uint32_t tx = ((P.dbg & 1) ? 0 : A_BYTES) + ((P.dbg & 2) ? 0 : terms * B_BYTES);
+      const uint32_t tx = A_BYTES + terms * B_BYTES;
       int s = 0, git = 0;
       uint32_t ph = 0;
       bool alive = true;
@@ -176,22 +166,17 @@ conv_umma_kernel(const __grid_constant__ ConvParams P) {
         if (git >= S && !mbar_wait(&empty_bar[s], ph ^ 1, P.err_flag, 101)) { alive = false; break; }   // first S slots: free
         uint8_t* sa = smem + s * stage_bytes;
         if (elect_one()) {
-          if (tr && kb < 120) P.trace[8 + kb * 4 + 0] = gtime_ns();
-          if (tx) mbar_expect_tx(&full_bar[s], tx); else mbar_arrive(&full_bar[s]);
-          if (P.dbg & 1) {
-          } else if (kb < nkb_main) {
+          mbar_expect_tx(&full_bar[s], tx);
+          if (kb < nkb_main) {
             tma_load_im2col_5d(&P.amap[phase], &full_bar[s], sa, cc * BK, w0, h0, d0, n0,
                                (uint16_t)tw, (uint16_t)th, (uint16_t)td);
           } else {
             tma_load_im2col_5d(&P.xmap, &full_bar[s], sa, (kb - nkb_main) * BK, q0, p0, z0, n0, 0, 0, 0);
           }
-          if (!(P.dbg & 2)) {
 #pragma unroll
-            for (int t = 0; t < terms; ++t)
-              tma_load_2d(&P.bmap, &full_bar[s], sa + A_BYTES + t * B_BYTES, kbase + kb * BK,
-                          n_tile * BN + t * P.cout);
-          }
-          if (tr && kb < 120) P.trace[8 + kb * 4 + 1] = gtime_ns();
+          for (int t = 0; t < terms; ++t)
+            tma_load_2d(&P.bmap, &full_bar[s], sa + A_BYTES + t * B_BYTES, kbase + kb * BK,
+                        n_tile * BN + t * P.cout);
         }
         // advance (channel chunk, tap) counters and the stage ring without div/mod
         if (++cc == ncm) {
@@ -229,19 +214,14 @@ conv_umma_kernel(const __grid_constant__ ConvParams P) {
         // first channel of this k-block relative to where the lo halves of the operand pairs start
         const int rel = kb < nkb_main ? cc * BK - lo_from : (kb - nkb_main) * BK - lo_from_x;
         if (elect_one()) {
-          if (tr && kb < 120) P.trace[8 + kb * 4 + 2] = gtime_ns();
           const uint32_t a_lo = lo0 + s * lo_stage;
-          if (!(P.dbg & 4)) {
 #pragma unroll
-            for (int k = 0; k < BK / 16; ++k) {
-              const uint32_t idesc = (TERMS == 2 && acc && rel + k * 16 >= 0) ? IDESC_HI : IDESC;
-              umma_f16_lohi(tmem_base, a_lo + 2 * k, a_lo + (A_BYTES >> 4) + 2 * k, DESC_HI, idesc, acc);
-              acc = 1;
-            }
+          for (int k = 0; k < BK / 16; ++k) {
+            const uint32_t idesc = (TERMS == 2 && acc && rel + k * 16 >= 0) ? IDESC_HI : IDESC;
+            umma_f16_lohi(tmem_base, a_lo + 2 * k, a_lo + (A_BYTES >> 4) + 2 * k, DESC_HI, idesc, acc);
+            acc = 1;
           }
-          if (P.dbg & 64) mbar_arrive(&empty_bar[s]);
-          else umma_commit(&empty_bar[s]);   // frees the smem slot once these MMAs retire
-          if (tr && kb < 120) P.trace[8 + kb * 4 + 3] = gtime_ns();
+          umma_commit(&empty_bar[s]);   // frees the smem slot once these MMAs retire
         }
         if (++cc == ncm) cc = 0;
         if (++s == S) { s = 0; ph ^= 1; }
@@ -309,7 +289,6 @@ conv_umma_kernel(const __grid_constant__ ConvParams P) {
     }
     if (!mbar_wait(tmem_full, pi & 1, P.err_flag, 103)) break;
     tc_fence_after();
-    if (tr && warp == 2 && lane == 0) P.trace[1] = gtime_ns();
 
     if (P.ksplit > 1) {
       // split-K: raw partial accumulators -> this CTA's shared memory (the pipeline stages are idle:
@@ -350,7 +329,7 @@ conv_umma_kernel(const __grid_constant__ ConvParams P) {
 #pragma unroll
         for (int i = 0; i < 16; ++i) v[i] += v2[i];
       }
-      if (!valid || (P.dbg & 8)) continue;
+      if (!valid) continue;
 #pragma unroll
       for (int i = 0; i < 16; i += 4) {
         const float4 t4 = *reinterpret_cast<const float4*>(colv + c * 16 + i);
@@ -476,11 +455,9 @@ conv_umma_kernel(const __grid_constant__ ConvParams P) {
     // peers may still be reading this CTA's partial tile
     asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
   }
-  if (tr && warp == 2 && lane == 0) P.trace[2] = gtime_ns();
   tc_fence_before();
   __syncthreads();
   if (warp == 2) tmem_dealloc(tmem_base, TMEM_COLS);
-  if (tr && threadIdx.x == 0) P.trace[3] = gtime_ns();
 }
 
 // -------------------------------- host side --------------------------------
@@ -495,7 +472,6 @@ struct ConvLaunch {
   dim3 grid;
   int bn, bk;
   size_t smem;
-  double flops;         // algorithmic 2*M*N*K of this launch (all phases)
 };
 
 // Fill amap/xmap/bmap + geometry.  `mode`: 0 = k3 s1 p1 ("same"), 1 = k3 s2 p1 (DownSample),

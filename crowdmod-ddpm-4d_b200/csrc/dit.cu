@@ -3,12 +3,12 @@
 // behind the same C ABI style as the UNet plan: forward(future, t, past) and the fused reverse chain.
 //
 // Every nn.Linear / the patch-embedding Conv3d (kernel = stride: a per-patch linear map) runs on the tcgen05 implicit-GEMM
-// kernel of conv_umma.cuh in its 1x1x1 mode (fp16 activations, hi + lo fp16 weights, fp32 accumulation in TMEM, bias
-// fused); spatial self-attention is the attention core of kernels.cu (mma.sync, S = 27 tokens); what is new here are the
-// bandwidth kernels between them: LayerNorm + AdaLN modulate -> fp16 operand, gated residual add, exact GELU, the
-// temporal cross-attention (future slots query the T_p <= 8 slots of their spatial patch), patch gather / scatter, and
-// the DDPM / DDIM update fused into the un-patch kernel.  Sampling (eval) only: training this backbone still raises.
-#include <stdlib.h>
+// kernel of conv_umma.cuh in its 1x1x1 mode (fp16 activations, hi + lo fp16 weights, fp32 accumulation in TMEM; bias, exact
+// GELU and the gated residual adds fused into its epilogue); spatial self-attention is the attention core of kernels.cu
+// (mma.sync, S = 27 tokens); what is new here are the bandwidth kernels between them: LayerNorm + AdaLN modulate -> fp16
+// operand, the temporal cross-attention (future slots query the T_p <= 8 slots of their spatial patch), patch gather /
+// scatter, and the DDPM / DDIM update fused into the un-patch kernel.  Sampling (eval) only: training this backbone still
+// raises.
 #include <string.h>
 
 #include <map>
@@ -46,8 +46,7 @@ __global__ void dit_gather_emb_kernel(const float* __restrict__ table, const lon
   for (int d = threadIdx.x; d < D; d += blockDim.x) out[(size_t)b * D + d] = __float2half_rn(table[(size_t)ti * D + d]);
 }
 
-// out16 = fp16(act(in32)); act: 0 identity, 1 SiLU, 2 SiLU(SiLU(.)) (c = SiLU(time_proj), AdaLN applies SiLU again),
-// 3 exact GELU (nn.GELU default: 0.5 x (1 + erf(x / sqrt 2)))
+// out16 = fp16(act(in32)); act: 0 identity, 1 SiLU, 2 SiLU(SiLU(.)) (c = SiLU(time_proj), AdaLN applies SiLU again)
 __device__ __forceinline__ float silu_exact(float x) { return x / (1.0f + expf(-x)); }
 __global__ void dit_act16_kernel(const float* __restrict__ in, __half* __restrict__ out, size_t n4, int act) {
   for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n4; i += (size_t)gridDim.x * blockDim.x) {
@@ -58,7 +57,6 @@ __global__ void dit_act16_kernel(const float* __restrict__ in, __half* __restric
       float x = r[k];
       if (act == 1) x = silu_exact(x);
       else if (act == 2) x = silu_exact(silu_exact(x));
-      else if (act == 3) x = 0.5f * x * (1.0f + erff(x * 0.70710678118654752f));
       r[k] = x;
     }
     __half2 h0 = __floats2half2_rn(r[0], r[1]), h1 = __floats2half2_rn(r[2], r[3]);
@@ -151,23 +149,6 @@ __global__ void __launch_bounds__(256) dit_ln_mod_kernel(const float* __restrict
     u.x = *reinterpret_cast<uint32_t*>(&h0);
     u.y = *reinterpret_cast<uint32_t*>(&h1);
     *reinterpret_cast<uint2*>(out + (size_t)warp * D + d) = u;
-  }
-}
-
-// x[xrow][:] += gate[b][:] * y[yrow][:], yrow = b*y_rps + j (j < y_rps), xrow = b*x_rps + x_off + j
-// (the gated residuals of DiT4D_V4.py:166, :193, :208; the temporal one touches the future slots only)
-__global__ void dit_gate_add_kernel(float* __restrict__ x, const float* __restrict__ y, const float* __restrict__ mods, int ld_mods,
-                                    int off_gate, int y_rows, int y_rps, int x_rps, int x_off, int D) {
-  const size_t total = (size_t)y_rows * D / 4;
-  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
-    const int yrow = (int)(i / (D / 4)), d = (int)(i - (size_t)yrow * (D / 4)) * 4;
-    const int b = yrow / y_rps, j = yrow - b * y_rps;
-    const size_t xo = ((size_t)b * x_rps + x_off + j) * D + d;
-    const float4 g = *reinterpret_cast<const float4*>(mods + (size_t)b * ld_mods + off_gate + d);
-    const float4 yv = reinterpret_cast<const float4*>(y)[i];
-    float4 xv = *reinterpret_cast<float4*>(x + xo);
-    xv.x += g.x * yv.x; xv.y += g.y * yv.y; xv.z += g.z * yv.z; xv.w += g.w * yv.w;
-    *reinterpret_cast<float4*>(x + xo) = xv;
   }
 }
 
@@ -351,10 +332,9 @@ struct cm_dit {
   // workspace pointers
   long long* t_dev = nullptr;
   __half *e16 = nullptr, *h16 = nullptr, *a16 = nullptr, *xm16 = nullptr, *ctx16 = nullptr, *g16 = nullptr;
-  float *h32 = nullptr, *h2_32 = nullptr, *c32 = nullptr, *mods = nullptr, *x32 = nullptr, *qkv32 = nullptr, *tmp32 = nullptr,
-        *mlp32 = nullptr, *out32 = nullptr, *chain_x = nullptr, *chain_past = nullptr, *d_coef = nullptr;
+  float *h32 = nullptr, *h2_32 = nullptr, *c32 = nullptr, *mods = nullptr, *x32 = nullptr, *qkv32 = nullptr, *out32 = nullptr,
+        *chain_x = nullptr, *chain_past = nullptr, *d_coef = nullptr;
   int coef_cap = 0;
-  bool fused = true;                   // epilogue fusions on (CM_DIT_NOFUSE=1 keeps the separate bandwidth kernels)
   float* mods_table = nullptr;         // [table_steps][Jtot]: AdaLN vectors of every timestep (sampling, batch-uniform t)
   bool table_ready = false;
   int* d_step = nullptr;
@@ -557,8 +537,8 @@ int reserve(cm_dit* u, int batch) {
   const size_t o_h32 = take(Bp * u->E * 4), o_h2 = take(Bp * u->E * 4), o_c32 = take(Bp * u->D * 4);
   const size_t o_mods = take(Bp * u->Jtot * 4);
   const size_t o_a16 = take(R * u->Kpad * 2), o_x32 = take(R * u->D * 4), o_xm = take(R * u->D * 2);
-  const size_t o_qkv = take(R * 3 * u->D * 4), o_ctx = take(R * u->D * 2), o_tmp = take(R * u->D * 4);
-  const size_t o_mlp = take(R * u->Dm * 4), o_g16 = take(R * u->Dm * 2), o_out = take(R * u->Nout * 4);
+  const size_t o_qkv = take(R * 3 * u->D * 4), o_ctx = take(R * u->D * 2);
+  const size_t o_g16 = take(R * u->Dm * 2), o_out = take(R * u->Nout * 4);
   const size_t xel = (size_t)batch * c.out_channels * c.rows * c.cols * c.future_len;
   const size_t pel = (size_t)batch * c.in_channels * c.rows * c.cols * (c.past_len > 0 ? c.past_len : 1);
   const size_t o_cx = take(xel * 4), o_cp = take(pel * 4);
@@ -578,8 +558,6 @@ int reserve(cm_dit* u, int batch) {
   u->xm16 = reinterpret_cast<__half*>(a + o_xm);
   u->qkv32 = reinterpret_cast<float*>(a + o_qkv);
   u->ctx16 = reinterpret_cast<__half*>(a + o_ctx);
-  u->tmp32 = reinterpret_cast<float*>(a + o_tmp);
-  u->mlp32 = reinterpret_cast<float*>(a + o_mlp);
   u->g16 = reinterpret_cast<__half*>(a + o_g16);
   u->out32 = reinterpret_cast<float*>(a + o_out);
   u->chain_x = reinterpret_cast<float*>(a + o_cx);
@@ -592,9 +570,9 @@ int reserve(cm_dit* u, int batch) {
 
 // GEMM out32[rows][cout] = act16[rows][cin] . W^T + bias  (conv_umma 1x1x1 mode; rows = nb * d * h * w)
 int prep_gemm(cm_dit* u, DitLinear& l, const __half* act, int nb, int d, int h, int w, float* out32) {
-  // K <= 1024 here: narrower N tiles fill the SMs without the cluster split-K reduction (CM_DIT_SPLITK=1 to compare)
-  static const bool splitk = getenv("CM_DIT_SPLITK") != nullptr && !u->fused;   // the epilogue fusions live in the non-split path
-  if (int rc = conv_prepare(&l.launch, 3, act, nb, d, h, w, l.cin, nullptr, 0, u->wpack + l.pack_off, l.cout, 2, splitk)) return rc;
+  // no split-K: the epilogue fusions (act / gate / rmap) live in the non-split path, and with K <= 1024 narrower N tiles
+  // fill the SMs without the cluster reduction
+  if (int rc = conv_prepare(&l.launch, 3, act, nb, d, h, w, l.cin, nullptr, 0, u->wpack + l.pack_off, l.cout, 2, false)) return rc;
   l.launch.p.bias = l.b >= 0 ? u->params[l.b].ptr : l.b_dev;
   l.launch.p.out32 = out32;
   l.launch.p.out16 = nullptr;
@@ -611,25 +589,21 @@ int prepare(cm_dit* u, int batch) {
   if (int e = prep_gemm(u, u->patch, u->a16, batch, 1, Tp, Ns, u->x32)) return e;
   for (auto& b : u->blocks) {
     if (int e = prep_gemm(u, b.s_in, u->xm16, batch, 1, Tp, Ns, u->qkv32)) return e;
-    if (int e = prep_gemm(u, b.s_out, u->ctx16, batch, 1, Tp, Ns, u->tmp32)) return e;
+    if (int e = prep_gemm(u, b.s_out, u->ctx16, batch, 1, Tp, Ns, u->x32)) return e;
     if (int e = prep_gemm(u, b.t_in, u->xm16, batch, 1, Tp, Ns, u->qkv32)) return e;
-    if (int e = prep_gemm(u, b.t_out, u->ctx16, batch, 1, u->nq, Ns, u->tmp32)) return e;
-    if (int e = prep_gemm(u, b.fc1, u->xm16, batch, 1, Tp, Ns, u->mlp32)) return e;
-    if (int e = prep_gemm(u, b.fc2, u->g16, batch, 1, Tp, Ns, u->tmp32)) return e;
-    if (u->fused) {
-      // epilogue fusions (ConvParams::act / gate / rmap): GELU + fp16 operand out of fc1; the three gated residuals
-      // x += gate * (GEMM + bias) written in place into the token stream (the temporal one into the future slots)
-      b.fc1.launch.p.act = 1;
-      b.fc1.launch.p.out32 = nullptr;
-      b.fc1.launch.p.out16 = u->g16;
-      for (DitLinear* l : {&b.s_out, &b.t_out, &b.fc2}) {
-        l->launch.p.resid = u->x32;
-        l->launch.p.out32 = u->x32;
-        l->launch.p.gate = u->mods;           // + the block's gate offset, set per launch in run_forward
-      }
-      b.t_out.launch.p.rmap_out = u->tokens;
-      b.t_out.launch.p.rmap_off = u->qs * Ns;
+    if (int e = prep_gemm(u, b.t_out, u->ctx16, batch, 1, u->nq, Ns, u->x32)) return e;
+    if (int e = prep_gemm(u, b.fc1, u->xm16, batch, 1, Tp, Ns, nullptr)) return e;
+    if (int e = prep_gemm(u, b.fc2, u->g16, batch, 1, Tp, Ns, u->x32)) return e;
+    // epilogue fusions (ConvParams::act / gate / rmap): GELU + fp16 operand out of fc1; the three gated residuals
+    // x += gate * (GEMM + bias) written in place into the token stream (the temporal one into the future slots)
+    b.fc1.launch.p.act = 1;
+    b.fc1.launch.p.out16 = u->g16;
+    for (DitLinear* l : {&b.s_out, &b.t_out, &b.fc2}) {
+      l->launch.p.resid = u->x32;
+      l->launch.p.gate = u->mods;           // + the block's gate offset, set per launch in run_forward
     }
+    b.t_out.launch.p.rmap_out = u->tokens;
+    b.t_out.launch.p.rmap_off = u->qs * Ns;
   }
   if (int e = prep_gemm(u, u->final_lin, u->xm16, batch, 1, Tp, Ns, u->out32)) return e;
   if (u->graph_exec) {            // the captured step bakes the launches of the previous batch
@@ -666,7 +640,7 @@ int run_conditioning(cm_dit* u, int rows, DitLinear& t1, DitLinear& t2, DitLinea
 int run_forward(cm_dit* u, int B, const float* future, const float* past, UnpatchParams up, int ld_mods, cudaStream_t st,
                 int64_t* launches) {
   const cm_dit_config& c = u->cfg;
-  const int D = u->D, Tp = u->Tp, Ns = u->Ns, R = B * u->tokens, Rq = B * u->nq * Ns;
+  const int D = u->D, Tp = u->Tp, Ns = u->Ns, R = B * u->tokens;
   int64_t n = 0;
   if (ld_mods != 0) {
     if (int e = run_conditioning(u, B, u->t1, u->t2, u->tproj, u->adaln, st)) return e;
@@ -690,16 +664,11 @@ int run_forward(cm_dit* u, int B, const float* future, const float* past, Unpatc
     DIT_LAUNCH_CHECK();
     if (int e = conv_enqueue(b.s_in.launch, st)) return e;
     if (int e = attn_core_enqueue(u->qkv32, u->ctx16, B * Tp, Ns, D, c.heads, st, 1)) return e;
-    if (u->fused) {
+    {
       ConvLaunch L = b.s_out.launch;
       L.p.gate = u->mods + mo + 2 * D;
       L.p.gate_ld = ld_mods;
       if (int e = conv_enqueue(L, st)) return e;
-    } else {
-      if (int e = conv_enqueue(b.s_out.launch, st)) return e;
-      dit_gate_add_kernel<<<grid_for((size_t)R * D / 4), 256, 0, st>>>(u->x32, u->tmp32, u->mods, ld_mods, mo + 2 * D, R, u->tokens,
-                                                                       u->tokens, 0, D);
-      DIT_LAUNCH_CHECK();
     }
     // 2. temporal cross-attention (future slots of every spatial patch query all of its slots)
     dit_ln_mod_kernel<<<ln_blocks, 256, 0, st>>>(u->x32, u->mods, ld_mods, mo + 3 * D, mo + 4 * D, u->tokens, R, D, u->xm16);
@@ -710,36 +679,23 @@ int run_forward(cm_dit* u, int B, const float* future, const float* past, Unpatc
       dit_tattn_kernel<<<(warps * 32 + 255) / 256, 256, 0, st>>>(u->qkv32, u->ctx16, B, Tp, Ns, D, c.heads, u->qs);
       DIT_LAUNCH_CHECK();
     }
-    if (u->fused) {
+    {
       ConvLaunch L = b.t_out.launch;
       L.p.gate = u->mods + mo + 5 * D;
       L.p.gate_ld = ld_mods;
       if (int e = conv_enqueue(L, st)) return e;
-    } else {
-      if (int e = conv_enqueue(b.t_out.launch, st)) return e;
-      dit_gate_add_kernel<<<grid_for((size_t)Rq * D / 4), 256, 0, st>>>(u->x32, u->tmp32, u->mods, ld_mods, mo + 5 * D, Rq, u->nq * Ns,
-                                                                        u->tokens, u->qs * Ns, D);
-      DIT_LAUNCH_CHECK();
     }
     // 3. MLP
     dit_ln_mod_kernel<<<ln_blocks, 256, 0, st>>>(u->x32, u->mods, ld_mods, mo + 6 * D, mo + 7 * D, u->tokens, R, D, u->xm16);
     DIT_LAUNCH_CHECK();
     if (int e = conv_enqueue(b.fc1.launch, st)) return e;
-    if (u->fused) {
+    {
       ConvLaunch L = b.fc2.launch;
       L.p.gate = u->mods + mo + 8 * D;
       L.p.gate_ld = ld_mods;
       if (int e = conv_enqueue(L, st)) return e;
-      n += 11;
-    } else {
-      dit_act16_kernel<<<grid_for((size_t)R * u->Dm / 4), 256, 0, st>>>(u->mlp32, u->g16, (size_t)R * u->Dm / 4, 3);
-      DIT_LAUNCH_CHECK();
-      if (int e = conv_enqueue(b.fc2.launch, st)) return e;
-      dit_gate_add_kernel<<<grid_for((size_t)R * D / 4), 256, 0, st>>>(u->x32, u->tmp32, u->mods, ld_mods, mo + 8 * D, R, u->tokens,
-                                                                       u->tokens, 0, D);
-      DIT_LAUNCH_CHECK();
-      n += 15;
     }
+    n += 11;
   }
   // ---- final layer (chunk(2): shift, scale) + un-patch (+ reverse-step update)
   const int mo = c.depth * 9 * D;
@@ -795,7 +751,6 @@ int cm_dit_create(const cm_dit_config* cfg, cm_dit** out) {
   CM_CHECK(cfg && out, "null argument");
   cm_dit* u = new cm_dit();
   u->cfg = *cfg;
-  u->fused = getenv("CM_DIT_NOFUSE") == nullptr;
   if (int e = build(u)) {
     delete u;
     return e;

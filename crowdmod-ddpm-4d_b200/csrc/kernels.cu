@@ -5,7 +5,6 @@
 #include "pack.cuh"
 
 #include <cooperative_groups.h>
-#include <stdlib.h>
 
 
 namespace cm {
@@ -322,8 +321,8 @@ __global__ void __launch_bounds__(384) gn_fused_kernel(const GnParams p) {
 
 
 // =============================================================================================
-// GroupNorm as two fully parallel streaming kernels (default path; the cluster kernel above is
-// kept behind CM_GN_CLUSTER=1 for A/B measurements):
+// GroupNorm as two fully parallel streaming kernels (the cluster kernel above serves calls without a
+// partial-statistics buffer and tensors of more than 4 * GN2_T channels):
 //   gn_stats2_kernel : CTA = (pixel slice, sample).  Every thread accumulates shifted sums of its
 //                      (fixed) channel quad, converts them to (n, mean, M2) and the CTA merges
 //                      the triples per group with Chan's formula in a fixed tree -> partial[b][slice][g].
@@ -392,7 +391,6 @@ struct GnRing {
 };
 
 __global__ void __launch_bounds__(GN2_T) gn_stats2_kernel(const GnParams p, int slices, float* __restrict__ partial) {
-  pdl_trigger();
   extern __shared__ __align__(128) unsigned char gn_dyn[];
   __shared__ uint64_t full_bar[GN3_NS];
   __shared__ float tri[GN2_T][3];
@@ -420,7 +418,6 @@ __global__ void __launch_bounds__(GN2_T) gn_stats2_kernel(const GnParams p, int 
     fence_mbar_init();
   }
   __syncthreads();
-  pdl_wait();
   if (tid == 0)
     for (int s = 0; s < GN3_NS && s < rg.total; ++s) rg.issue(s);
   const bool from0 = c < p.c0;
@@ -489,7 +486,6 @@ __global__ void __launch_bounds__(GN2_T) gn_stats2_kernel(const GnParams p, int 
 
 __global__ void __launch_bounds__(GN2_T) gn_apply2_kernel(const GnParams p, int slices, int stat_slices,
                                                           const float* __restrict__ partial) {
-  pdl_trigger();
   extern __shared__ __align__(128) unsigned char gn_dyn[];
   __shared__ uint64_t full_bar[GN3_NS];
   __shared__ float stat[2][8];
@@ -516,7 +512,6 @@ __global__ void __launch_bounds__(GN2_T) gn_apply2_kernel(const GnParams p, int 
     fence_mbar_init();
   }
   __syncthreads();
-  pdl_wait();
   // the data stream starts before the statistics prologue; the last ring slot doubles as the
   // staging buffer of the producers' records and joins the ring after the prologue
   if (tid == 0)
@@ -683,8 +678,6 @@ __global__ void __launch_bounds__(GN2_T) gn_apply2_kernel(const GnParams p, int 
 constexpr int GNS_CACHE = 8;
 
 __global__ void __launch_bounds__(1024) gn_small_kernel(const GnParams p) {
-  pdl_trigger();
-  pdl_wait();
   __shared__ float tri[1024][3];
   __shared__ float stat[2][8];
   const int C = p.c0 + p.c1, cg_ch = C >> 3, Q = C >> 2, vpp = Q >> 3;
@@ -794,8 +787,7 @@ int gn_silu_enqueue(const GnParams& p, float* partial, cudaStream_t st, int* lau
   if (launches) *launches = 1;
   const int C = p.c0 + p.c1;
   CM_CHECK(C % 32 == 0 && p.c0 % 4 == 0, "GroupNorm channels must be a multiple of 32 (C=%d)", C);
-  static const bool use_cluster = getenv("CM_GN_CLUSTER") != nullptr;
-  if (partial && !use_cluster && C / 4 <= GN2_T && C <= 512 && p.rec0.rec && (p.c1 == 0 || p.rec1.rec)) {
+  if (partial && C / 4 <= GN2_T && C <= 512 && p.rec0.rec && (p.c1 == 0 || p.rec1.rec)) {
     // statistics come from the producing convs: one streaming apply kernel, no statistics pass
     const int Q = C / 4;
     const long nvec = (long)p.pixels * Q;
@@ -804,10 +796,11 @@ int gn_silu_enqueue(const GnParams& p, float* partial, cudaStream_t st, int* lau
     if (slices > max_slices) slices = max_slices;
     if (slices > GN2_MAX_SLICES) slices = GN2_MAX_SLICES;
     if (slices < 1) slices = 1;
-    return launch_pdl(gn_apply2_kernel, dim3(slices, p.B), dim3(GN2_T), GN3_SMEM, st, p, slices, 0,
-                      static_cast<const float*>(partial));
+    gn_apply2_kernel<<<dim3(slices, p.B), GN2_T, GN3_SMEM, st>>>(p, slices, 0, partial);
+    CM_CUDA(cudaGetLastError());
+    return 0;
   }
-  if (partial && !use_cluster && C / 4 <= GN2_T) {
+  if (partial && C / 4 <= GN2_T) {
     const int Q = C / 4;
     const long nvec = (long)p.pixels * Q;                       // float4 per sample
     if (nvec <= 1024L * GNS_CACHE) {
@@ -818,7 +811,8 @@ int gn_silu_enqueue(const GnParams& p, float* partial, cudaStream_t st, int* lau
       if (T < 256) T = 256;
       while ((long)(T / Q) * Q * GNS_CACHE < nvec) T += 32;      // sweeping threads are floor(T/Q)*Q
       if (T <= 1024) {
-        if (int e = launch_pdl(gn_small_kernel, dim3(p.B), dim3(T), 0, st, p)) return e;
+        gn_small_kernel<<<p.B, T, 0, st>>>(p);
+        CM_CUDA(cudaGetLastError());
         return 0;
       }
     }
@@ -828,12 +822,11 @@ int gn_silu_enqueue(const GnParams& p, float* partial, cudaStream_t st, int* lau
     if (slices > max_slices) slices = max_slices;
     if (slices > GN2_MAX_SLICES) slices = GN2_MAX_SLICES;
     if (slices < 1) slices = 1;
-    if (int e = launch_pdl(gn_stats2_kernel, dim3(slices, p.B), dim3(GN2_T), GN3_SMEM, st, p, slices, partial)) return e;
-    if (int e = launch_pdl(gn_apply2_kernel, dim3(slices, p.B), dim3(GN2_T), GN3_SMEM, st, p, slices, slices,
-                           static_cast<const float*>(partial)))
-      return e;
-    if (launches) *launches = 2;
+    gn_stats2_kernel<<<dim3(slices, p.B), GN2_T, GN3_SMEM, st>>>(p, slices, partial);
     CM_CUDA(cudaGetLastError());
+    gn_apply2_kernel<<<dim3(slices, p.B), GN2_T, GN3_SMEM, st>>>(p, slices, slices, partial);
+    CM_CUDA(cudaGetLastError());
+    if (launches) *launches = 2;
     return 0;
   }
   const int Q = C / 4;
@@ -875,8 +868,6 @@ __global__ void __launch_bounds__(256)
 first_conv_kernel(const float* __restrict__ x, const float* __restrict__ past,
                   const float* __restrict__ w, const float* __restrict__ bias,
                   float* __restrict__ out, int B, int H, int W, int P, int F, int cout) {
-  pdl_trigger();
-  pdl_wait();
   extern __shared__ float sm[];
   constexpr int K = 27 * CIN;
   const int L = P + F;
@@ -966,7 +957,7 @@ int first_conv_enqueue(const float* x, const float* past, const float* w, const 
   const size_t smem = ((size_t)27 * cin * cout + (size_t)cin * (FC_TS + 2) * (FC_TS + 2) * (L + 2)) * sizeof(float);
 #define CM_FIRST(CI)                                                                           \
   case CI:                                                                                     \
-    if (int e = launch_pdl(first_conv_kernel<CI>, dim3(blocks), dim3(threads), smem, st, x, past, w, bias, out, B, H, W, P, F, cout)) return e; \
+    first_conv_kernel<CI><<<blocks, threads, smem, st>>>(x, past, w, bias, out, B, H, W, P, F, cout); \
     break;
   switch (cin) {
     CM_FIRST(1) CM_FIRST(2) CM_FIRST(3) CM_FIRST(4)
@@ -984,8 +975,6 @@ constexpr int FIN_FC = 3;   // output frames per 4-lane group: taps along time s
 
 template <int COUT>
 __global__ void __launch_bounds__(256) final_conv_kernel(const FinalParams p) {
-  pdl_trigger();
-  pdl_wait();
   // weights as [h tap][w tap][ci][time tap][co]: the 8 channels x 3 time taps x COUT outputs a lane needs
   // for one spatial tap are contiguous (vector loads, broadcast across the warp's sites)
   extern __shared__ __align__(16) float ws[];
@@ -1157,9 +1146,9 @@ int final_conv_enqueue(const FinalParams& p, cudaStream_t st) {
   if (blocks > 148 * 4) blocks = 148 * 4;          // at most one resident wave; the kernel grid-strides
   const size_t smem = (size_t)27 * p.cin * p.cout * sizeof(float);
 #define CM_FINAL(CO)                                                                           \
-  case CO: {                                                                                   \
-    if (int e = launch_pdl(final_conv_kernel<CO>, dim3(blocks), dim3(256), smem, st, p)) return e; \
-  } break;
+  case CO:                                                                                     \
+    final_conv_kernel<CO><<<blocks, 256, smem, st>>>(p);                                       \
+    break;
   switch (p.cout) {
     CM_FINAL(1) CM_FINAL(2) CM_FINAL(3) CM_FINAL(4)
   }
@@ -1277,8 +1266,6 @@ __device__ __forceinline__ void split_h2(float x, float y, uint32_t* hi, uint32_
 template <int DH, int NT>
 __global__ void __launch_bounds__(NT * 16) attn_mma_kernel(const float* __restrict__ qkv, __half* __restrict__ ctx,
                                                           int S, int C, int heads, int dup) {
-  pdl_trigger();
-  pdl_wait();
   const int dh = C / heads;
   constexpr int SP = NT * 8;            // padded sequence length
   constexpr int KLD = DH + 8;           // smem row stride (halfs) of K  [SP][KLD]
@@ -1423,7 +1410,8 @@ template <int DH, int NT>
 static int attn_launch(const float* qkv, __half* ctx, int B, int S, int C, int heads, int dup, cudaStream_t st) {
   constexpr int SP = NT * 8;
   const size_t smem = ((size_t)2 * SP * (DH + 8) + (size_t)DH * (SP + 8)) * sizeof(__half);
-  if (int e = launch_pdl(attn_mma_kernel<DH, NT>, dim3(B * heads), dim3(NT * 16), smem, st, qkv, ctx, S, C, heads, dup)) return e;
+  attn_mma_kernel<DH, NT><<<B * heads, NT * 16, smem, st>>>(qkv, ctx, S, C, heads, dup);
+  CM_CUDA(cudaGetLastError());
   return 0;
 }
 
@@ -1541,8 +1529,6 @@ template <int NT>   // NT = padded tokens / 8 (even): SP = 16, 32, ... 128
 __global__ void __launch_bounds__(AB_THREADS, 1) attn_block_kernel(const AttnBlockParams p) {
   namespace cgr = cooperative_groups;
   cgr::cluster_group cluster = cgr::this_cluster();
-  pdl_trigger();
-  pdl_wait();
   constexpr int SP = NT * 8, MTILES = SP / 16;
   constexpr int VLD = SP + 8;
   constexpr int MH = (MTILES + 1) / 2;                   // M tiles per half (phase 1 splits M over warp halves)
@@ -1827,15 +1813,13 @@ static int attn_block_launch(const AttnBlockParams& p, int B, cudaStream_t st) {
   cfg.blockDim = dim3(AB_THREADS);
   cfg.dynamicSmemBytes = attn_block_smem<NT>();
   cfg.stream = st;
-  cudaLaunchAttribute at[2];
+  cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeClusterDimension;
   at[0].val.clusterDim.x = 2;
   at[0].val.clusterDim.y = 1;
   at[0].val.clusterDim.z = 1;
-  at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = at;
-  cfg.numAttrs = pdl_enabled() ? 2 : 1;
+  cfg.numAttrs = 1;
   CM_CUDA(cudaLaunchKernelEx(&cfg, attn_block_kernel<NT>, p));
   return 0;
 }
@@ -1898,17 +1882,6 @@ int kernels_init() {
   CM_CUDA(cudaFuncSetAttribute(final_conv_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
   CM_CUDA(cudaFuncSetAttribute(gn_stats2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GN3_SMEM));
   CM_CUDA(cudaFuncSetAttribute(gn_apply2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GN3_SMEM));
-  if (getenv("CM_CARVEOUT")) {
-    // experiment: the conv kernels use 227 KB of shared memory; give the bandwidth kernels between them the same
-    // L1 / shared-memory carve-out so that consecutive launches do not reconfigure the SMs
-    const int mx = cudaSharedmemCarveoutMaxShared;
-    CM_CUDA(cudaFuncSetAttribute(gn_stats2_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, mx));
-    CM_CUDA(cudaFuncSetAttribute(gn_apply2_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, mx));
-    CM_CUDA(cudaFuncSetAttribute(gn_small_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, mx));
-    CM_CUDA(cudaFuncSetAttribute(final_conv_kernel<3>, cudaFuncAttributePreferredSharedMemoryCarveout, mx));
-    CM_CUDA(cudaFuncSetAttribute(pack_first_input_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, mx));
-    CM_CUDA(cudaFuncSetAttribute(attn_block_kernel<8>, cudaFuncAttributePreferredSharedMemoryCarveout, mx));
-  }
   if (int rc = attn_init()) return rc;
   if (int rc = attn_long_init()) return rc;
   if (int rc = conv_init()) return rc;
@@ -1920,14 +1893,13 @@ int kernels_init() {
 // chain bookkeeping
 // =============================================================================================
 __global__ void advance_step_kernel(int* step_dev, int* t_dev, const int* tsteps, int nsteps) {
-  pdl_trigger();
-  pdl_wait();
   const int s = *step_dev + 1;
   *step_dev = s;
   *t_dev = tsteps[s < nsteps ? s : nsteps - 1];
 }
 int advance_step_enqueue(int* step_dev, int* t_dev, const int* tsteps, int nsteps, cudaStream_t st) {
-  if (int e = launch_pdl(advance_step_kernel, dim3(1), dim3(1), 0, st, step_dev, t_dev, tsteps, nsteps)) return e;
+  advance_step_kernel<<<1, 1, 0, st>>>(step_dev, t_dev, tsteps, nsteps);
+  CM_CUDA(cudaGetLastError());
   return 0;
 }
 __global__ void advance_step_cond_kernel(int* step_dev, int* t_dev, const int* tsteps, int nsteps,

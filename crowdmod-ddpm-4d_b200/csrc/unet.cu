@@ -61,7 +61,6 @@ struct Op {
       resid = -1, out = -1, cin = 0, cin_extra = 0, cout = 0, in_level = 0;
   size_t wpack_off = 0;   // element offset into the packed-weight buffer
   size_t wpack2_off = 0;  // same in the training forward's cache (hi|lo pair activation operands, K doubled)
-  int terms = 0;            // weight terms of THIS conv's forward (0 = cfg.weight_terms)
   ConvLaunch launch;
   PlaneLaunch plaunch;      // plane-tile kernel (conv_plane.cuh) when it covers the geometry
   Res32Launch rlaunch;      // weights-resident 32 -> 32 kernel (conv_res32.cuh) when it covers the shape (sampling / eval)
@@ -108,7 +107,6 @@ struct cm_unet {
   // first conv on the tensor cores: the 3(+)-channel input is packed into a zero-padded 32-channel fp16
   // operand and run through the plane-tile kernel (falls back to first_conv_kernel when not covered)
   int first_in = -1;
-  int fullres_terms = 0;    // CROWDMOD_FULLRES_TERMS (0 = same as cfg.weight_terms)
   size_t first_wpack_off = 0;
   PlaneLaunch first_plane;
   Res32Launch first_res;
@@ -292,7 +290,6 @@ int add_conv(cm_unet* u, const std::string& tag, int mode, int in, int extra, in
   u->g_elems += wgrad_g_elems(mode, op.cin, op.cin_extra, cout);
   op.colsum_off = u->colsum_per_sample;
   u->colsum_per_sample += cout;
-  if (mode == 0 && op.in_level == 0 && u->fullres_terms > 0) op.terms = u->fullres_terms;
   u->ops.push_back(op);
   return op.out;
 }
@@ -479,13 +476,6 @@ int build_plan(cm_unet* u) {
   return 0;
 }
 
-// Forward weight precision per conv.  Policy knob CROWDMOD_FULLRES_TERMS (default: cfg.weight_terms):
-// the full-resolution k3 s1 convs -- where the tensor pipe is bound by the number of MMA
-// instructions -- may run with single fp16 weights while every other layer keeps the hi+lo split.
-int fwd_terms(const cm_unet* u, const Op& op) {
-  return op.terms > 0 ? op.terms : u->cfg.weight_terms;
-}
-
 int check_params_bound(cm_unet* u) {
   for (auto& p : u->params)
     CM_CHECK(p.ptr != nullptr, "parameter '%s' not bound (cm_unet_set_param)", p.name.c_str());
@@ -548,12 +538,6 @@ int reserve(cm_unet* u, int batch) {
   return 0;
 }
 
-// hi|lo operand pairs against hi+lo weight terms: the lo x lo product (2^-22 of the result) is skipped unless CM_KEEP_LOLO is set
-static bool keep_lolo() {
-  static const bool k = getenv("CM_KEEP_LOLO") != nullptr;
-  return k;
-}
-
 // conv launches depend on the live batch (grid, tensor-map extents): (re)built per call batch
 // dup = 1: single fp16 activation operands (sampling / eval); dup = 2: hi|lo pair rows (training forward)
 int prepare_convs(cm_unet* u, int batch, int dup) {
@@ -562,40 +546,35 @@ int prepare_convs(cm_unet* u, int batch, int dup) {
     const Level& l0 = u->levels[0];
     u->first_plane.ok = false;
     u->first_res.ok = false;
-    static const bool no_tc_first = getenv("CM_NO_PLANE") != nullptr || getenv("CM_FIRST_SIMT") != nullptr;
-    if (!no_tc_first) {
-      if (int rc = plane_prepare(&u->first_plane, u->tens[u->first_in].p16, batch, l0.D, l0.H, l0.W, 32 * dup, nullptr, 0,
-                                 wbase + (dup == 2 ? u->first_wpack2_off : u->first_wpack_off), u->cfg.base_channels,
-                                 (u->fullres_terms > 0 && dup == 1) ? u->fullres_terms : u->cfg.weight_terms))
+    if (int rc = plane_prepare(&u->first_plane, u->tens[u->first_in].p16, batch, l0.D, l0.H, l0.W, 32 * dup, nullptr, 0,
+                               wbase + (dup == 2 ? u->first_wpack2_off : u->first_wpack_off), u->cfg.base_channels,
+                               u->cfg.weight_terms))
+      return rc;
+    if (u->first_plane.ok) {
+      u->first_plane.p.lo_from = dup == 2 ? 32 : 0;
+      u->first_plane.p.bias = u->params[u->p_first_b].ptr;
+      u->first_plane.p.out32 = nullptr;   // set per run (tensor of the OP_FIRST op)
+    }
+    if (u->first_plane.ok && dup == 1) {
+      if (int rc = res32_prepare(&u->first_res, u->tens[u->first_in].p16, batch, l0.D, l0.H, l0.W, 32, nullptr, 0,
+                                 wbase + u->first_wpack_off, u->cfg.base_channels, u->cfg.weight_terms))
         return rc;
-      if (u->first_plane.ok) {
-        u->first_plane.p.lo_from = (dup == 2 && !keep_lolo()) ? 32 : 0;
-        u->first_plane.p.bias = u->params[u->p_first_b].ptr;
-        u->first_plane.p.out32 = nullptr;   // set per run (tensor of the OP_FIRST op)
-      }
-      const int first_terms = (u->fullres_terms > 0 && dup == 1) ? u->fullres_terms : u->cfg.weight_terms;
-      if (u->first_plane.ok && dup == 1) {
-        if (int rc = res32_prepare(&u->first_res, u->tens[u->first_in].p16, batch, l0.D, l0.H, l0.W, 32, nullptr, 0,
-                                   wbase + u->first_wpack_off, u->cfg.base_channels, first_terms))
-          return rc;
-        if (u->first_res.ok) u->first_res.p.bias = u->params[u->p_first_b].ptr;
-      }
-      for (Op& fo : u->ops) {
-        if (fo.type != OP_FIRST) continue;
-        Tens& t = u->tens[fo.out];
-        t.rec_units = 0;
-        static const bool no_rec = getenv("CM_NO_GNREC") != nullptr;
-        if (u->first_res.ok && t.rec && !no_rec) {
-          Res32Params& q = u->first_res.p;
-          q.stats_rec = t.rec;
-          t.rec_units = q.units_per_sample;
-          t.rec_nvalid = q.HB * q.W;
-        } else if (u->first_plane.ok && t.rec && !no_rec) {
-          PlaneParams& q = u->first_plane.p;
-          q.stats_rec = t.rec;
-          t.rec_units = q.units_per_sample;
-          t.rec_nvalid = q.R * q.HB * q.W;
-        }
+      if (u->first_res.ok) u->first_res.p.bias = u->params[u->p_first_b].ptr;
+    }
+    for (Op& fo : u->ops) {
+      if (fo.type != OP_FIRST) continue;
+      Tens& t = u->tens[fo.out];
+      t.rec_units = 0;
+      if (u->first_res.ok && t.rec) {
+        Res32Params& q = u->first_res.p;
+        q.stats_rec = t.rec;
+        t.rec_units = q.units_per_sample;
+        t.rec_nvalid = q.HB * q.W;
+      } else if (u->first_plane.ok && t.rec) {
+        PlaneParams& q = u->first_plane.p;
+        q.stats_rec = t.rec;
+        t.rec_units = q.units_per_sample;
+        t.rec_nvalid = q.R * q.HB * q.W;
       }
     }
   }
@@ -605,16 +584,16 @@ int prepare_convs(cm_unet* u, int batch, int dup) {
     const Tens& tin = u->tens[op.in];
     const __half* extra = op.extra >= 0 ? u->tens[op.extra].p16 : nullptr;
     const __half* wp = wbase + (dup == 2 ? op.wpack2_off : op.wpack_off);
-    const int terms = dup == 2 ? u->cfg.weight_terms : fwd_terms(u, op);
+    const int terms = u->cfg.weight_terms;
     if (int rc = conv_prepare(&op.launch, op.mode, tin.p16, batch, li.D, li.H, li.W, op.cin * dup, extra,
                               op.cin_extra * dup, wp, op.cout, terms))
       return rc;
-    const bool skip_lolo = dup == 2 && !keep_lolo();
+    // hi|lo operand pairs against hi+lo weight terms: the lo x lo product (2^-22 of the result) is skipped
+    const bool skip_lolo = dup == 2;
     op.launch.p.lo_from = skip_lolo ? op.cin : 0;
     op.launch.p.lo_from_x = skip_lolo ? op.cin_extra : 0;
     op.plaunch.ok = false;
-    static const bool no_plane = getenv("CM_NO_PLANE") != nullptr;
-    if (op.mode == 0 && !no_plane) {
+    if (op.mode == 0) {
       if (int rc = plane_prepare(&op.plaunch, tin.p16, batch, li.D, li.H, li.W, op.cin * dup, extra, op.cin_extra * dup,
                                  wp, op.cout, terms))
         return rc;
@@ -647,13 +626,12 @@ int prepare_convs(cm_unet* u, int batch, int dup) {
     {
       Tens& t = u->tens[op.out];
       t.rec_units = 0;
-      static const bool no_rec = getenv("CM_NO_GNREC") != nullptr;
-      if (op.rlaunch.ok && t.rec && !no_rec) {
+      if (op.rlaunch.ok && t.rec) {
         Res32Params& q = op.rlaunch.p;
         q.stats_rec = t.rec;
         t.rec_units = q.units_per_sample;
         t.rec_nvalid = q.HB * q.W;
-      } else if (op.plaunch.ok && t.rec && !no_rec) {
+      } else if (op.plaunch.ok && t.rec) {
         PlaneParams& q = op.plaunch.p;
         q.stats_rec = t.rec;
         t.rec_units = q.units_per_sample;
@@ -702,14 +680,13 @@ int run_ops(cm_unet* u, RunCtx& rc, cudaStream_t st, int64_t* launches,
   const cm_unet_config& c = u->cfg;
   int op_index = 0;
   int skip = 0;            // ops already covered by a fused launch (their profile events still tick)
-  static const bool no_attn_fuse = getenv("CM_NO_ATTN_FUSE") != nullptr;
   for (size_t oi = 0; oi < u->ops.size(); ++oi) {
     Op& op = u->ops[oi];
     if (events) CM_CUDA(cudaEventRecord(events[op_index], st));
     ++op_index;
     if (skip > 0) { --skip; continue; }
     // sampling path: the whole AttentionBlock (GroupNorm, in_proj, core, out_proj + residual) is one launch
-    if (op.type == OP_GN && !rc.train && !no_attn_fuse && oi + 3 < u->ops.size() &&
+    if (op.type == OP_GN && !rc.train && oi + 3 < u->ops.size() &&
         u->ops[oi + 2].type == OP_ATTN && u->ops[oi + 1].type == OP_CONV && u->ops[oi + 3].type == OP_CONV &&
         u->ops[oi + 1].in == op.out_norm && op.src1 < 0) {
       const Op& ip = u->ops[oi + 1];
@@ -717,8 +694,7 @@ int run_ops(cm_unet* u, RunCtx& rc, cudaStream_t st, int64_t* launches,
       const Op& po = u->ops[oi + 3];
       const int Cc = u->tens[op.src0].C;
       const int S = u->levels[u->tens[op.src0].level].pps();
-      const int terms = ip.terms ? ip.terms : c.weight_terms;
-      if (attn_block_supported(S, Cc, at.heads) && terms == 2 && ip.mode == 3 && po.mode == 3 && po.resid == op.src0 &&
+      if (attn_block_supported(S, Cc, at.heads) && c.weight_terms == 2 && ip.mode == 3 && po.mode == 3 && po.resid == op.src0 &&
           ip.extra < 0 && po.extra < 0 && ip.cout == 3 * Cc && po.cout == Cc) {
         if (int e = attn_block_enqueue(u->tens[op.src0].p32, u->params[op.gamma].ptr, u->params[op.beta].ptr,
                                        u->wpack + ip.wpack_off, u->params[ip.bias].ptr, u->wpack + po.wpack_off,
@@ -983,7 +959,7 @@ int build_jobs(cm_unet* u) {
     j.dst = u->wpack + op.wpack_off;
     j.kind = op.mode == 2 ? 1 : 0;
     j.cout = op.cout; j.cin = op.cin; j.cinx = op.cin_extra; j.taps = op.mode == 3 ? 1 : 27;
-    j.terms = op.mode == 2 ? terms : fwd_terms(u, op);
+    j.terms = terms;
     j.perm = 1; j.cin_src = op.cin; j.dup = 1;
     jobs.push_back(j);
   }
@@ -993,7 +969,7 @@ int build_jobs(cm_unet* u) {
     j.dst = u->wpack + u->first_wpack_off;
     j.kind = 0;
     j.cout = u->cfg.base_channels; j.cin = 32; j.cinx = 0; j.taps = 27;
-    j.terms = u->fullres_terms > 0 ? u->fullres_terms : terms;
+    j.terms = terms;
     j.perm = 1; j.cin_src = u->cfg.in_channels; j.dup = 1;
     jobs.push_back(j);
   }
@@ -1004,7 +980,6 @@ int build_jobs(cm_unet* u) {
     for (int k = 0; k < u->n_jobs_fwd; ++k) {
       PackJob j = jobs[k];
       j.dup = 2;
-      j.terms = terms;
       jobs.push_back(j);
     }
     int k = u->n_jobs_fwd;
@@ -1093,15 +1068,15 @@ int prepare_train(cm_unet* u, int batch) {
                               dup * op.cout, nullptr, 0, u->dpack + op.dpack_off, op.cin, u->cfg.weight_terms))
       return rc;
     op.dlaunch.p.out32 = u->g32[op.in];
-    op.dlaunch.p.lo_from = (dup == 2 && !keep_lolo()) ? op.cout : 0;
+    op.dlaunch.p.lo_from = dup == 2 ? op.cout : 0;
     op.dplaunch.ok = false;
-    if (op.mode == 0 && getenv("CM_NO_PLANE") == nullptr) {
+    if (op.mode == 0) {
       if (int rc = plane_prepare(&op.dplaunch, u->g16[op.out], batch, lo.D, lo.H, lo.W, dup * op.cout, nullptr, 0,
                                  u->dpack + op.dpack_off, op.cin, u->cfg.weight_terms))
         return rc;
       if (op.dplaunch.ok) {
         op.dplaunch.p.out32 = u->g32[op.in];
-        op.dplaunch.p.lo_from = (dup == 2 && !keep_lolo()) ? op.cout : 0;
+        op.dplaunch.p.lo_from = dup == 2 ? op.cout : 0;
       }
     }
     if (op.cin_extra) {
@@ -1109,7 +1084,7 @@ int prepare_train(cm_unet* u, int batch) {
                                 u->dpack + op.dxpack_off, op.cin_extra, u->cfg.weight_terms))
         return rc;
       op.dxlaunch.p.out32 = u->g32[op.extra];
-      op.dxlaunch.p.lo_from = (dup == 2 && !keep_lolo()) ? op.cout : 0;
+      op.dxlaunch.p.lo_from = dup == 2 ? op.cout : 0;
     }
     const __half* extra = op.extra >= 0 ? u->tens[op.extra].p16 : nullptr;
     // activations / the 1x1 source: the hi halves of the forward's (hi|lo pair) rows
@@ -1139,7 +1114,7 @@ int prepare_train(cm_unet* u, int batch) {
   // first conv: its operand is the packed fp16 input [pixels][32 (x live_dup)] of the forward (channels >= in_channels are
   // zero), so its weight gradient is one plane launch over the hi halves like any other 32 -> 32 layer
   u->first_wpl.ok = false;
-  if (u->first_plane.ok && u->cfg.base_channels == 32 && getenv("CM_FIRST_WGRAD_SIMT") == nullptr) {
+  if (u->first_plane.ok && u->cfg.base_channels == 32) {
     const Level& l0 = u->levels[0];
     const int out = u->ops[0].out;
     if (int rc = wgrad_plane_prepare(&u->first_wpl, u->tens[u->first_in].p16, batch, l0.D, l0.H, l0.W, 32, u->live_dup * 32, 0,
@@ -1147,7 +1122,7 @@ int prepare_train(cm_unet* u, int batch) {
       return rc;
   }
   u->final_wpl.ok = false;
-  if (u->ops.back().type == OP_FINAL && u->ops.back().cin == 32 && getenv("CM_FINAL_WGRAD_SIMT") == nullptr) {
+  if (u->ops.back().type == OP_FINAL && u->ops.back().cin == 32) {
     const Level& l0 = u->levels[0];
     const Op& fo = u->ops.back();
     if (int rc = wgrad_plane_prepare(&u->final_wpl, u->tens[fo.in].p16, batch, l0.D, l0.H, l0.W, 32, u->live_dup * 32, 0,
@@ -1196,17 +1171,6 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
   std::vector<long long> gn_tab;        // {chsum offset, C, dgamma offset, dbeta offset} per GroupNorm, plan order
   std::vector<long long> up_tab;        // {mode, G offset, dw offset, dwx offset | -1, cout, cin, cinx, perm} per conv
   std::vector<long long> rs_tab;        // {channel-sum offset in the training arena, row stride, cout, bias-grad offset}
-  // bring-up: CM_BWD_TRACE=1 brackets every backward stage with CUDA events and prints a table
-  static const bool trace = getenv("CM_BWD_TRACE") != nullptr;
-  std::vector<std::pair<std::string, cudaEvent_t>> marks;
-  auto mark = [&](const std::string& what) {
-    if (!trace) return;
-    cudaEvent_t ev;
-    cudaEventCreate(&ev);
-    cudaEventRecord(ev, st);
-    marks.emplace_back(what, ev);
-  };
-  mark("begin");
   for (int oi = (int)u->ops.size() - 1; oi >= 0; --oi) {
     Op& op = u->ops[oi];
     switch (op.type) {
@@ -1226,7 +1190,6 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
         }
         written[op.in] = 1;
         nl += 2;
-        mark("final_bwd " + op.tag);
       } break;
       case OP_GN: {
         GnBwdParams g{};
@@ -1266,7 +1229,6 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
         gn_tab.push_back((long long)u->grad_off[op.beta]);
         if (int e = gn_backward_enqueue(g, u->gn_bwd_partial, st)) return e;
         nl += 2;
-        mark("gn_bwd " + op.tag);
       } break;
       case OP_CONV: {
         CM_CHECK(written[op.out], "backward: gradient of '%s' output missing", op.tag.c_str());
@@ -1291,7 +1253,6 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
           rs_tab.push_back((long long)op.cout);
           rs_tab.push_back((long long)u->grad_off[bidx]);
         }
-        mark("cast_colsum " + op.tag);
         if (op.dplaunch.ok) {
           PlaneLaunch L = op.dplaunch;
           L.p.resid = written[op.in] ? u->g32[op.in] : nullptr;   // accumulate in place
@@ -1310,7 +1271,6 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
           if (int e = conv_enqueue(L, st)) return e;
           ++nl;
         }
-        mark("dgrad " + op.tag);
         if (op.n_wpl > 0) {
           for (int c = 0; c < op.n_wpl; ++c)
             if (int e = wgrad_plane_enqueue(op.wpl[c], st)) return e;
@@ -1320,7 +1280,6 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
         } else if (int e = wgrad_enqueue(op.wlaunch, st)) {
           return e;
         }
-        mark("wgrad " + op.tag);
         // packed-K scratch -> nn.Conv3d weight layout: all convs in one launch after the op loop
         for (long long v : {(long long)op.mode, (long long)op.g_off, (long long)u->grad_off[op.w],
                             op.wx >= 0 ? (long long)u->grad_off[op.wx] : -1LL, (long long)op.cout, (long long)op.cin,
@@ -1337,7 +1296,6 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
           return e;
         written[op.qkv] = 1;
         ++nl;
-        mark("attn_bwd " + op.tag);
       } break;
       case OP_FIRST: {
         CM_CHECK(written[op.out], "backward: gradient of the first conv output missing");
@@ -1362,7 +1320,6 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
           return e;
         }
         ++nl;
-        mark("first_wgrad " + op.tag);
       } break;
     }
   }
@@ -1380,7 +1337,6 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
     }
     if (int e = unpack_wgrad_all_enqueue(u->d_up_tab, (int)(up_tab.size() / 8), u->G, grads, st)) return e;
     ++nl;
-    mark("unpack all");
   }
   // ---- conv bias gradients: one launch ----
   if (!rs_tab.empty()) {
@@ -1398,7 +1354,6 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
                                    grads, st))
       return e;
     ++nl;
-    mark("bias_sums all");
   }
   // ---- dgamma / dbeta of every GroupNorm: one launch ----
   if (!gn_tab.empty()) {
@@ -1412,7 +1367,6 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
     if (int e = gn_backward_params_all_enqueue(u->gn_chsum, u->d_gn_tab, (int)(gn_tab.size() / 4), B, grads, st))
       return e;
     ++nl;
-    mark("gn_params all");
   }
   // ---- time-embedding MLP (embeddings.py:22-34) and the per-block dense_1 (layers.py:35,62) ----
   const size_t nE = (size_t)B * E;
@@ -1449,22 +1403,6 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
     return e;
   if (int e = scale_inplace_enqueue(grads, u->grad_total, u->loss_scale + 1, st)) return e;
   nl += 8;
-  mark("temb_mlp + unscale");
-  if (trace) {
-    cudaStreamSynchronize(st);
-    std::map<std::string, float> agg;
-    float total = 0.f;
-    for (size_t i = 1; i < marks.size(); ++i) {
-      float ms = 0.f;
-      cudaEventElapsedTime(&ms, marks[i - 1].second, marks[i].second);
-      fprintf(stderr, "CM_BWD %-60s %8.1f us\n", marks[i].first.c_str(), ms * 1e3f);
-      agg[marks[i].first.substr(0, marks[i].first.find(' '))] += ms;
-      total += ms;
-    }
-    for (auto& kv : agg) fprintf(stderr, "CM_BWD_SUM %-14s %8.3f ms\n", kv.first.c_str(), kv.second);
-    fprintf(stderr, "CM_BWD_SUM %-14s %8.3f ms\n", "total", total);
-    for (auto& m : marks) cudaEventDestroy(m.second);
-  }
   if (launches) *launches = nl;
   return 0;
 }
@@ -1488,10 +1426,6 @@ int cm_unet_create(const cm_unet_config* cfg, cm_unet** out) {
   CM_CHECK(u->cfg.train_act_terms >= 0 && u->cfg.train_act_terms <= 2, "train_act_terms must be 0 (default), 1 or 2");
   u->act_dup_train = u->cfg.train_act_terms == 1 ? 1 : 2;
   u->cfg.train_act_terms = u->act_dup_train;
-  if (const char* e = getenv("CROWDMOD_FULLRES_TERMS")) {
-    const int ft = atoi(e);
-    if (ft == 1 || ft == 2) u->fullres_terms = ft < u->cfg.weight_terms ? ft : 0;
-  }
   if (int e = build_plan(u.get())) return e;
   *out = u.release();
   return 0;

@@ -45,7 +45,6 @@ struct WgradPlaneParams {
   int g_slot_bytes;      // guard + box + guard
   int cin;               // channels of the whole main source: G row = tap * cin + c0 + ci
   float* G;              // [27 * cin (+ extra rows)][32] fp32, zeroed by the caller
-  int dbg;               // bring-up knobs (CM_WGP_DBG): 1 no TMA loads, 4 no MMA
   int* err_flag;
 };
 
@@ -104,15 +103,11 @@ __global__ void __launch_bounds__(WP_THREADS, 1) wgrad_plane_kernel(const __grid
         const int d = v / P.hblocks;
         const int h0 = (v - d * P.hblocks) * P.HB;
         uint8_t* sa = smem + s * P.stage_bytes;
-        if (P.dbg & 1) {
-          mbar_arrive(&full_bar[s]);
-        } else {
-          mbar_expect_tx(&full_bar[s], tx);
+        mbar_expect_tx(&full_bar[s], tx);
 #pragma unroll
-          for (int td = 0; td < 3; ++td)
-            tma_load_tile_5d(&P.amap, &full_bar[s], sa + td * P.a_slot_bytes, P.c0, -1, h0 - 1, d + td - 1, n);
-          tma_load_tile_5d(&P.gmap, &full_bar[s], sa + 3 * P.a_slot_bytes + P.g_data_off, 0, 0, h0, d, n);
-        }
+        for (int td = 0; td < 3; ++td)
+          tma_load_tile_5d(&P.amap, &full_bar[s], sa + td * P.a_slot_bytes, P.c0, -1, h0 - 1, d + td - 1, n);
+        tma_load_tile_5d(&P.gmap, &full_bar[s], sa + 3 * P.a_slot_bytes + P.g_data_off, 0, 0, h0, d, n);
       }
       __syncwarp();
       if (++s == S) { s = 0; ph ^= 1; }
@@ -130,7 +125,7 @@ __global__ void __launch_bounds__(WP_THREADS, 1) wgrad_plane_kernel(const __grid
         // N chunks (th = 2, 1, 0) one grid row apart, starting two grid rows above the dOut box
         const uint32_t g_lo0 = mnmajor_desc_lo(base + 3 * P.a_slot_bytes + P.g_data_off - 2 * P.Wp * 64, P.Wp * 64);
 #pragma unroll
-        for (int td = 0; td < 3 && !(P.dbg & 4); ++td) {
+        for (int td = 0; td < 3; ++td) {
           // M chunks (tw = 0..3) one box row (64 B) apart
           const uint32_t a_lo = mnmajor_desc_lo(base + td * P.a_slot_bytes, 64);
           const uint32_t d_tmem = tmem_base + td * 96;

@@ -221,7 +221,6 @@ struct WgradLaunch {
   dim3 grid;
   int bkc, bnc, bn;
   size_t smem;
-  double flops;
 };
 
 // `mode` = forward conv mode (0 k3 s1, 1 k3 s2, 2 nearest-x2 + k3 as 8 phases, 3 1x1x1).

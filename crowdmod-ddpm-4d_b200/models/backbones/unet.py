@@ -42,15 +42,13 @@ _PLANS: "weakref.WeakKeyDictionary[nn.Module, Dict[Tuple[int, int, int, int], _N
 
 def _graph_mode(use_graph) -> int:
     """cm_chain_args.use_graph: False/0 eager, 1 / "step" per-step graph replay, True / 2 / "chain" the whole
-    chain as ONE graph (conditional WHILE node).  CROWDMOD_CHAIN_GRAPH={eager,step,chain} overrides True."""
+    chain as ONE graph (conditional WHILE node)."""
     if use_graph is False or use_graph == 0:
         return 0
-    if use_graph is True:
-        use_graph = os.environ.get("CROWDMOD_CHAIN_GRAPH", "chain")
+    if use_graph is True or use_graph in (2, "chain"):   # before the 1 test: True == 1
+        return 2
     if use_graph in (1, "step"):
         return 1
-    if use_graph in (2, "chain"):
-        return 2
     if use_graph == "eager":
         return 0
     raise ValueError(f"use_graph={use_graph!r}: expected False, True, 'eager', 'step' or 'chain'")

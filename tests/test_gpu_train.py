@@ -11,7 +11,6 @@ took the worst tensor from 2.6e-3 (round 1, single fp16 operands: the error was 
 rounding propagating into every deep-layer gradient -- shown by the CPU emulation in
 profiles/r2_train_grad_parity.txt) to 5.8e-4 / 3.4e-4 / 3.2e-4 on the three cases below (measured on B200).
 """
-import os
 import pytest
 import torch
 import torch.nn.functional as F
@@ -27,7 +26,6 @@ GRAD_TOL = 1e-3
 TENSOR_TOL = 1e-3
 # name (regex) -> (bound, why): empty -- every tensor meets TENSOR_TOL (see the module docstring)
 TENSOR_EXCEPTIONS = {}
-REPORT_ONLY = os.environ.get("CM_TEST_REPORT_ONLY") == "1"     # bring-up: print every tensor, assert the global gate only
 
 
 @pytest.fixture(scope="module", autouse=True)
@@ -68,10 +66,6 @@ def _compare(lo, go, ln, gn):
     worst = sorted(((rel_l2(gn[k], go[k]), k) for k in go), reverse=True)
     print("global grad rel-L2 = %.3e; worst tensors: %s" % ((num / den) ** 0.5,
           ", ".join("%s %.2e" % (k, e) for e, k in worst[:6])))
-    if REPORT_ONLY:
-        for e, k in worst:
-            if e > 0.5 * TENSOR_TOL:
-                print("TENSOR %-60s rel-L2 %.3e  numel %d  |g| %.3e" % (k, e, go[k].numel(), go[k].double().norm().item()))
     assert (num / den) ** 0.5 <= GRAD_TOL
     import re
     for e, k in worst:
@@ -84,8 +78,7 @@ def _compare(lo, go, ln, gn):
         for pat, (b, _why) in TENSOR_EXCEPTIONS.items():
             if re.fullmatch(pat, k):
                 bound = b
-        if not REPORT_ONLY:
-            assert e <= bound, f"{k}: rel-L2 {e:.3e} > {bound:.1e}"
+        assert e <= bound, f"{k}: rel-L2 {e:.3e} > {bound:.1e}"
 
 
 @pytest.mark.parametrize("name", ["train_small", "train_atc_b2"])
@@ -104,8 +97,6 @@ def test_train_step_vs_oracle_and_reference_golden(name):
         r = torch.randn(gn[k].shape, generator=g)
         n_ref, p_ref = float(a["grad_norms"][i]), float(a["grad_proj"][i])
         if n_ref < 1e-12:
-            continue
-        if REPORT_ONLY:
             continue
         assert abs(gn[k].double().norm().item() - n_ref) <= TENSOR_TOL * n_ref, k
         assert abs((gn[k].double() * r.double()).sum().item() - p_ref) <= TENSOR_TOL * n_ref * r.norm().item(), k

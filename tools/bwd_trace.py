@@ -1,6 +1,6 @@
-"""Per-stage device times of one native backward (HERMES-CR-120 shape, batch 64): CM_BWD_TRACE=1."""
+"""One native training step (forward + backward) at the HERMES-CR-120 shape, batch 64, run three times: the workload of
+gpu_ll_train.sh (launch list) and, with PROFILE_API=1, of ll_split.py (third step only)."""
 import os, sys
-os.environ["CM_BWD_TRACE"] = "1"
 import torch
 import torch.nn.functional as F
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
