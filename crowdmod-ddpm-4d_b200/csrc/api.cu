@@ -6,12 +6,8 @@
 
 #include "../../include/crowdmod_b200.h"
 #include "backward.cuh"
-#include "wgrad_plane.cuh"
-#include "conv_plane.cuh"
-#include "conv_res32.cuh"
-#include "conv_umma.cuh"
+#include "conv_run.cuh"
 #include "kernels.cuh"
-#include "wgrad_umma.cuh"
 
 namespace cm {
 
@@ -60,63 +56,27 @@ int cm_op_conv3d(int mode, const void* act16, int B, int D, int H, int W, int ci
   int rc = 0;
   if (mode == 2) rc = pack_upsample_weights(w, wp, cout, cin, terms, 0, st);
   else rc = pack_conv_weights(w, wx, wp, cout, cin, cin_extra, mode == 3 ? 1 : 27, terms, 0, st);
-  ConvLaunch L;
-  if (!rc && impl == 3) {
-    // weights-resident 32 -> 32 kernel (conv_res32.cuh).  Fails if the shape is not covered.
-    Res32Launch R;
-    rc = (mode == 0) ? res32_prepare(&R, static_cast<const __half*>(act16), B, D, H, W, cin,
-                                     static_cast<const __half*>(extra16), cin_extra, wp, cout, terms)
-                     : 2;
-    if (!rc && !R.ok) {
-      set_error("weights-resident conv does not cover this shape");
+  ConvEpilogue e{};
+  e.bias = bias;
+  e.resid = resid;
+  e.out32 = out32;
+  e.out16 = static_cast<__half*>(out16);
+  const __half* a16 = static_cast<const __half*>(act16);
+  const __half* x16 = static_cast<const __half*>(extra16);
+  // impl: 0 conv_umma, 2 conv_plane, 3 conv_res32 (each fails if it does not cover the conv), else the scalar reference
+  const unsigned kind = impl == 0 ? CONV_UMMA : impl == 2 ? CONV_PLANE : impl == 3 ? CONV_RES32 : 0;
+  if (!rc && kind) {
+    ConvRun R;
+    rc = conv_run_prepare(&R, kind, mode, a16, B, D, H, W, cin, x16, cin_extra, wp, cout, terms, e);
+    if (!rc && !R.covered()) {
+      set_error("the requested conv kernel does not cover this shape");
       rc = 2;
     }
-    if (!rc) {
-      R.p.bias = bias;
-      R.p.resid = resid;
-      R.p.out32 = out32;
-      R.p.out16 = static_cast<__half*>(out16);
-      rc = res32_enqueue(R, st);
-    }
-    cudaError_t se3 = cudaStreamSynchronize(st);
-    cudaFree(wp);
-    if (rc) return rc;
-    CM_CUDA(se3);
-    return 0;
-  }
-  if (!rc && impl == 2) {
-    // plane-tile kernel (conv_plane.cuh); mode 0 only.  Fails if the geometry is not covered.
-    PlaneLaunch PLn;
-    rc = (mode == 0) ? plane_prepare(&PLn, static_cast<const __half*>(act16), B, D, H, W, cin,
-                                     static_cast<const __half*>(extra16), cin_extra, wp, cout, terms)
-                     : 2;
-    if (!rc && !PLn.ok) {
-      set_error("plane-tile conv does not cover this geometry");
-      rc = 2;
-    }
-    if (!rc) {
-      PLn.p.bias = bias;
-      PLn.p.resid = resid;
-      PLn.p.out32 = out32;
-      PLn.p.out16 = static_cast<__half*>(out16);
-      rc = plane_enqueue(PLn, st);
-    }
-    cudaError_t se2 = cudaStreamSynchronize(st);
-    cudaFree(wp);
-    if (rc) return rc;
-    CM_CUDA(se2);
-    return 0;
-  }
-  if (!rc) rc = conv_prepare(&L, mode, static_cast<const __half*>(act16), B, D, H, W, cin,
-                             static_cast<const __half*>(extra16), cin_extra, wp, cout, terms);
-  if (!rc) {
-    L.p.bias = bias;
-    L.p.resid = resid;
-    L.p.out32 = out32;
-    L.p.out16 = static_cast<__half*>(out16);
-    if (impl == 0) rc = conv_enqueue(L, st);
-    else rc = conv_ref_enqueue(L.p, static_cast<const __half*>(act16),
-                             static_cast<const __half*>(extra16), wp, B, D, H, W, st);
+    if (!rc) rc = conv_run_enqueue(R, st);
+  } else if (!rc) {
+    ConvLaunch L;
+    rc = conv_prepare(&L, mode, a16, B, D, H, W, cin, x16, cin_extra, wp, cout, terms, e);
+    if (!rc) rc = conv_ref_enqueue(L.p, a16, x16, wp, B, D, H, W, st);
   }
   cudaError_t se = cudaStreamSynchronize(st);
   cudaFree(wp);
@@ -228,13 +188,12 @@ int cm_op_conv3d_dgrad(int mode, const void* dout16, int B, int D, int H, int W,
   __half* wp = nullptr;
   CM_CUDA(cudaMalloc(&wp, (size_t)terms * cin * ktot * sizeof(__half) + 16));
   int rc = pack_dgrad_weights(mode, w, wp, cout, cin, terms, 0, 1, st);
-  ConvLaunch L;
-  if (!rc) rc = conv_prepare(&L, dgrad_mode_of(mode), static_cast<const __half*>(dout16), B, od, oh, ow, cout,
-                             nullptr, 0, wp, cin, terms);
-  if (!rc) {
-    L.p.out32 = dx32;
-    rc = conv_enqueue(L, st);
-  }
+  ConvEpilogue e{};
+  e.out32 = dx32;
+  ConvRun R;
+  if (!rc) rc = conv_run_prepare(&R, CONV_UMMA, dgrad_mode_of(mode), static_cast<const __half*>(dout16), B, od, oh, ow,
+                                 cout, nullptr, 0, wp, cin, terms, e);
+  if (!rc) rc = conv_run_enqueue(R, st);
   cudaError_t se = cudaStreamSynchronize(st);
   cudaFree(wp);
   if (rc) return rc;
@@ -260,21 +219,13 @@ int cm_op_conv3d_dgrad_f32(int mode, const float* dout32, int B, int D, int H, i
   CM_CUDA(cudaMalloc(&d16, npix * cout * dup * sizeof(__half) + 16));
   int rc = pack_dgrad_weights(mode, w, wp, cout, cin, terms, 0, dup, st);
   if (!rc) rc = cast_colsum_enqueue(dout32, d16, dup, nullptr, 0, nullptr, 0, B, od * oh * ow, cout, st);
-  ConvLaunch L;
-  PlaneLaunch PLn;
-  PLn.ok = false;
-  if (!rc) rc = conv_prepare(&L, dgrad_mode_of(mode), d16, B, od, oh, ow, dup * cout, nullptr, 0, wp, cin, terms);
-  if (!rc && mode == 0)
-    rc = plane_prepare(&PLn, d16, B, od, oh, ow, dup * cout, nullptr, 0, wp, cin, terms);
-  if (!rc) {
-    if (PLn.ok) {
-      PLn.p.out32 = dx32;
-      rc = plane_enqueue(PLn, st);
-    } else {
-      L.p.out32 = dx32;
-      rc = conv_enqueue(L, st);
-    }
-  }
+  ConvEpilogue e{};
+  e.out32 = dx32;
+  ConvRun R;
+  if (!rc)
+    rc = conv_run_prepare(&R, CONV_UMMA | CONV_PLANE, dgrad_mode_of(mode), d16, B, od, oh, ow, dup * cout, nullptr, 0,
+                          wp, cin, terms, e);
+  if (!rc) rc = conv_run_enqueue(R, st);
   cudaError_t se = cudaStreamSynchronize(st);
   cudaFree(wp);
   cudaFree(d16);
@@ -295,33 +246,17 @@ int cm_op_conv3d_wgrad(int mode, const void* act16, int B, int D, int H, int W, 
   CM_CUDA(cudaMalloc(&G, gel * sizeof(float)));
   CM_CUDA(cudaMemsetAsync(G, 0, gel * sizeof(float), st));
   int rc = 0;
-  if (impl == 0) {
-    WgradLaunch L;
-    rc = wgrad_prepare(&L, mode, static_cast<const __half*>(act16), B, D, H, W, cin,
-                       static_cast<const __half*>(extra16), cin_extra, static_cast<const __half*>(dout16),
-                       cout, G);
-    if (!rc) rc = wgrad_enqueue(L, st);
-  } else if (impl == 2) {
-    // plane / halo scheme (wgrad_plane.cuh): one launch per 32-channel chunk of the main source; the fused 1x1x1 source
-    // goes through wgrad_umma_kernel in 1x1x1 mode into its rows of G
-    CM_CHECK(mode == 0, "plane wgrad covers k3 s1 p1 convs (mode 0), got mode %d", mode);
-    WgradPlaneLaunch PL[8];
-    const int nc = cin / 32;
-    CM_CHECK(nc >= 1 && nc <= 8, "plane wgrad: cin %d not covered", cin);
-    for (int c = 0; c < nc && !rc; ++c) {
-      rc = wgrad_plane_prepare(&PL[c], static_cast<const __half*>(act16), B, D, H, W, cin, 0, c * 32,
-                               static_cast<const __half*>(dout16), 0, cout, G);
-      if (!rc && !PL[c].ok) {
-        cm::set_error("plane wgrad does not cover this shape");
-        rc = 1;
-      }
+  if (impl == 0 || impl == 2) {
+    // impl 2: the plane / halo scheme (wgrad_plane.cuh), mode 0 with 32 output channels only
+    WgradRun R;
+    rc = wgrad_run_prepare(&R, impl == 0 ? CONV_UMMA : CONV_PLANE, mode, static_cast<const __half*>(act16), B, D, H, W,
+                           cin, static_cast<const __half*>(extra16), cin_extra, static_cast<const __half*>(dout16),
+                           cout, G);
+    if (!rc && R.launches() == 0) {
+      cm::set_error("plane wgrad does not cover this shape");
+      rc = 1;
     }
-    WgradLaunch XL;
-    if (!rc && cin_extra)
-      rc = wgrad_prepare(&XL, 3, static_cast<const __half*>(extra16), B, D, H, W, cin_extra, nullptr, 0,
-                         static_cast<const __half*>(dout16), cout, G + (size_t)27 * cin * cout);
-    for (int c = 0; c < nc && !rc; ++c) rc = wgrad_plane_enqueue(PL[c], st);
-    if (!rc && cin_extra) rc = wgrad_enqueue(XL, st);
+    if (!rc) rc = wgrad_run_enqueue(R, st);
   } else {
     rc = wgrad_ref_enqueue(mode, static_cast<const __half*>(act16), static_cast<const __half*>(extra16),
                            static_cast<const __half*>(dout16), G, B, D, H, W, cin, cin_extra, cout, st);

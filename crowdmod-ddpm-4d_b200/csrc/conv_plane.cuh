@@ -26,6 +26,7 @@
 // the optional fused 1x1x1 match_input K-slab).
 #pragma once
 #include "common.cuh"
+#include "conv_umma.cuh"
 
 namespace cm {
 
@@ -54,23 +55,7 @@ struct PlaneParams {
   int n_ntiles;          // cout / BN
   int a_stage_bytes;     // bytes reserved for the A box per stage (covers ntiles*128 + 2 rows)
   int cin_main, cin_extra, cout, terms, stages;
-  const float* bias;
-  const float* bias2;
-  int lo_from, lo_from_x;   // as ConvParams: k16 slices of lo-half channels skip the lo weight term
-  const float* temb;
-  const int* t_dev;
-  int temb_ld, temb_bstride;
-  const float* resid;
-  float* out32;
-  __half* out16;
-  int out_ld;
-  int out16_ld, out16_lo;   // fp16 copy: row stride in elements (0 -> out_ld); out16_lo > 0: also write the lo half
-                            // fp16(v - hi) out16_lo elements further (hi|lo pair operand of the training forward)
-  // GroupNorm statistics records of the values this launch writes (nullptr = none): per (sample, unit
-  // of the sample, output channel) a float4 {shift, sum(v - shift), sum((v - shift)^2), 0} over the
-  // unit's R*HB*W valid rows; units belong to ONE sample, so the consumer (gn_apply2_kernel) merges
-  // them in a fixed order -> bit-reproducible wherever the sample sits in the batch.
-  float* stats_rec;
+  ConvEpilogue epi;      // GroupNorm records over the unit's R*HB*W valid rows
   int* err_flag;
 };
 
@@ -221,8 +206,8 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
     uint32_t ph = 0;
     int it = 0;
     bool alive = true;
-    const int lo_from = P.lo_from > 0 ? P.lo_from : 0x40000000;
-    const int lo_from_x = P.lo_from_x > 0 ? P.lo_from_x : 0x40000000;
+    const int lo_from = P.epi.lo_from > 0 ? P.epi.lo_from : 0x40000000;
+    const int lo_from_x = P.epi.lo_from_x > 0 ? P.epi.lo_from_x : 0x40000000;
     for (int u = blockIdx.x; u < P.n_units && alive; u += gridDim.x, ++it) {
       const int buf = it & 1;
       int cc = 0;
@@ -293,7 +278,7 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
     const int quarter = warp & 3;
     const int group = (warp - 2) >> 2;                     // 0..3
     const int et = threadIdx.x - 64;
-    const bool temb_uniform = P.temb != nullptr && P.temb_bstride == 0;
+    const bool temb_uniform = P.epi.temb != nullptr && P.epi.temb_bstride == 0;
     constexpr int LPR = BN / 4;                            // lanes per row in the store phase
     constexpr int RPP = PL_EPI / LPR;                      // rows per store pass of the epilogue threads
     constexpr int NJ = PL_NJ;                              // store rows per thread (host: ntiles*128 <= NJ*RPP)
@@ -324,20 +309,20 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
         }
       }
     }
-    const int trow_u = (temb_uniform && P.t_dev) ? *P.t_dev : 0;
+    const int trow_u = (temb_uniform && P.epi.t_dev) ? *P.epi.t_dev : 0;
     auto load_cv = [&](int nn, int n) {
       float4 c = make_float4(0.f, 0.f, 0.f, 0.f), b2 = c, t4 = c;
-      if (P.bias) c = *reinterpret_cast<const float4*>(P.bias + nn);
-      if (P.bias2) b2 = *reinterpret_cast<const float4*>(P.bias2 + nn);
-      if (P.temb) {
-        const size_t trow = temb_uniform ? static_cast<size_t>(trow_u) * P.temb_ld : static_cast<size_t>(n) * P.temb_bstride;
-        t4 = *reinterpret_cast<const float4*>(P.temb + trow + nn);
+      if (P.epi.bias) c = *reinterpret_cast<const float4*>(P.epi.bias + nn);
+      if (P.epi.bias2) b2 = *reinterpret_cast<const float4*>(P.epi.bias2 + nn);
+      if (P.epi.temb) {
+        const size_t trow = temb_uniform ? static_cast<size_t>(trow_u) * P.epi.temb_ld : static_cast<size_t>(n) * P.epi.temb_bstride;
+        t4 = *reinterpret_cast<const float4*>(P.epi.temb + trow + nn);
       }
       c.x += b2.x; c.y += b2.y; c.z += b2.z; c.w += b2.w;      // same order as before: (bias + bias2) + temb
       c.x += t4.x; c.y += t4.y; c.z += t4.z; c.w += t4.w;
       return c;
     };
-    const bool cv_const = P.n_ntiles == 1 && (P.temb == nullptr || temb_uniform);
+    const bool cv_const = P.n_ntiles == 1 && (P.epi.temb == nullptr || temb_uniform);
     float4 cv = make_float4(0.f, 0.f, 0.f, 0.f);
     if (cv_const) cv = load_cv(sub_c, 0);
     int it = 0;
@@ -357,8 +342,8 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
         for (int j = 0; j < NJ; ++j) {
           mi[j] = roff[j] < 0 ? -1 : base + roff[j];
           rv[j] = make_float4(0.f, 0.f, 0.f, 0.f);
-          if (mi[j] >= 0 && P.resid)
-            rv[j] = *reinterpret_cast<const float4*>(P.resid + static_cast<size_t>(mi[j]) * P.cout + nn0 + sub_c);
+          if (mi[j] >= 0 && P.epi.resid)
+            rv[j] = *reinterpret_cast<const float4*>(P.epi.resid + static_cast<size_t>(mi[j]) * P.cout + nn0 + sub_c);
         }
       }
       if (!mbar_wait(&tmem_full[buf], (it >> 1) & 1, P.err_flag, 403)) { alive = false; break; }
@@ -430,24 +415,24 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
         st2.z = fmaf(v.z, v.z, st2.z); st2.w = fmaf(v.w, v.w, st2.w);
         v.x += cv.x; v.y += cv.y; v.z += cv.z; v.w += cv.w;
         const size_t m = static_cast<size_t>(mi[j]);
-        if (P.out32) *reinterpret_cast<float4*>(P.out32 + m * P.out_ld + nn0 + sub_c) = v;
-        if (P.out16) {
+        if (P.epi.out32) *reinterpret_cast<float4*>(P.epi.out32 + m * P.epi.out_ld + nn0 + sub_c) = v;
+        if (P.epi.out16) {
           __half2 h0 = __floats2half2_rn(v.x, v.y), h1 = __floats2half2_rn(v.z, v.w);
           uint2 uu;
           uu.x = *reinterpret_cast<uint32_t*>(&h0);
           uu.y = *reinterpret_cast<uint32_t*>(&h1);
-          __half* o16 = P.out16 + m * (P.out16_ld > 0 ? P.out16_ld : P.out_ld) + nn0 + sub_c;
+          __half* o16 = P.epi.out16 + m * (P.epi.out16_ld > 0 ? P.epi.out16_ld : P.epi.out_ld) + nn0 + sub_c;
           *reinterpret_cast<uint2*>(o16) = uu;
-          if (P.out16_lo > 0) {
+          if (P.epi.out16_lo > 0) {
             const float2 f0 = __half22float2(h0), f1 = __half22float2(h1);
             __half2 l0 = __floats2half2_rn(v.x - f0.x, v.y - f0.y), l1 = __floats2half2_rn(v.z - f1.x, v.w - f1.y);
             uu.x = *reinterpret_cast<uint32_t*>(&l0);
             uu.y = *reinterpret_cast<uint32_t*>(&l1);
-            *reinterpret_cast<uint2*>(o16 + P.out16_lo) = uu;
+            *reinterpret_cast<uint2*>(o16 + P.epi.out16_lo) = uu;
           }
         }
       }
-      if (P.stats_rec) {
+      if (P.epi.stats_rec) {
         // lanes that share a channel quad (same lane % LPR) hold different rows: butterfly over them
 #pragma unroll
         for (int w = LPR; w < 32; w <<= 1) {
@@ -464,7 +449,7 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
         if (et < LPR) *reinterpret_cast<float4*>(sred + (PL_EPI / 32) * BN * 2 + sub_c) = cv;
       }
       asm volatile("bar.sync 1, 512;" ::: "memory");       // ybuf / side are rewritten by the next unit
-      if (P.stats_rec && et < BN) {
+      if (P.epi.stats_rec && et < BN) {
         float a1 = 0.f, a2 = 0.f;
 #pragma unroll
         for (int wv = 0; wv < PL_EPI / 32; ++wv) {             // fixed order over the epilogue warps
@@ -473,7 +458,7 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
         }
         const int hblocks = P.H / P.HB;
         const int uis = (U.d0 / P.R) * hblocks + U.h0 / P.HB;
-        float4* rec = reinterpret_cast<float4*>(P.stats_rec) +
+        float4* rec = reinterpret_cast<float4*>(P.epi.stats_rec) +
                       (static_cast<size_t>(U.n) * P.units_per_sample + uis) * P.cout + nn0 + et;
         *rec = make_float4(sred[(PL_EPI / 32) * BN * 2 + et], a1, a2, 0.f);
       }
@@ -489,13 +474,13 @@ struct PlaneLaunch {
   dim3 grid;
   int bn, bk;
   size_t smem;
-  bool ok;               // false: geometry not covered, use conv_umma_kernel
+  bool ok;               // false: geometry not covered
 };
 
 // Fills L for a k3 s1 p1 conv (+ optional 1x1x1 extra source).  Returns 0 with L->ok = false when
-// the geometry is outside what this kernel covers (caller falls back to conv_umma).
+// the geometry is outside what this kernel covers.
 int plane_prepare(PlaneLaunch* L, const __half* act, int B, int D, int H, int W, int cin,
-                  const __half* extra, int cin_extra, const __half* wpacked, int cout, int terms);
+                  const __half* extra, int cin_extra, const __half* wpacked, int cout, int terms, const ConvEpilogue& epi);
 int plane_enqueue(const PlaneLaunch& L, cudaStream_t st);
 int plane_init();
 

@@ -51,15 +51,7 @@ struct Res32Params {
   int n_units;           // B * units_per_sample
   int nx;                // 1x1x1 chunks of 32 channels (0..3)
   int stages, stage_bytes;
-  const float* bias;
-  const float* bias2;
-  const float* temb;
-  const int* t_dev;
-  int temb_ld, temb_bstride;
-  const float* resid;
-  float* out32;
-  __half* out16;
-  float* stats_rec;      // GroupNorm records, as PlaneParams::stats_rec (units_per_sample records of HB*W rows)
+  ConvEpilogue epi;      // rows of 32 channels, no hi|lo operand pairs; GroupNorm records over HB*W rows
   int* err_flag;
 };
 
@@ -315,7 +307,7 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
     const int st = threadIdx.x - R32_STORE_W0 * 32;          // 0..255
     const int sw = st >> 5;                                  // store warp 0..7
     const int sub_r = st / LPR, sub_c = (st % LPR) * 4;
-    const bool temb_uniform = P.temb != nullptr && P.temb_bstride == 0;
+    const bool temb_uniform = P.epi.temb != nullptr && P.epi.temb_bstride == 0;
     // unit-independent: offset of each of this thread's store rows inside a unit (-1: pad column / beyond the unit)
     int roff[NJ];
 #pragma unroll
@@ -324,20 +316,20 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
       const int hl = q / P.Wp, w = q - hl * P.Wp;
       roff[j] = (q < P.P && w < P.W) ? hl * P.W + w : -1;
     }
-    const int trow_u = (temb_uniform && P.t_dev) ? *P.t_dev : 0;
+    const int trow_u = (temb_uniform && P.epi.t_dev) ? *P.epi.t_dev : 0;
     auto load_cv = [&](int n) {
       float4 cc = make_float4(0.f, 0.f, 0.f, 0.f), b2 = cc, t4 = cc;
-      if (P.bias) cc = *reinterpret_cast<const float4*>(P.bias + sub_c);
-      if (P.bias2) b2 = *reinterpret_cast<const float4*>(P.bias2 + sub_c);
-      if (P.temb) {
-        const size_t trow = temb_uniform ? static_cast<size_t>(trow_u) * P.temb_ld : static_cast<size_t>(n) * P.temb_bstride;
-        t4 = *reinterpret_cast<const float4*>(P.temb + trow + sub_c);
+      if (P.epi.bias) cc = *reinterpret_cast<const float4*>(P.epi.bias + sub_c);
+      if (P.epi.bias2) b2 = *reinterpret_cast<const float4*>(P.epi.bias2 + sub_c);
+      if (P.epi.temb) {
+        const size_t trow = temb_uniform ? static_cast<size_t>(trow_u) * P.epi.temb_ld : static_cast<size_t>(n) * P.epi.temb_bstride;
+        t4 = *reinterpret_cast<const float4*>(P.epi.temb + trow + sub_c);
       }
       cc.x += b2.x; cc.y += b2.y; cc.z += b2.z; cc.w += b2.w;
       cc.x += t4.x; cc.y += t4.y; cc.z += t4.z; cc.w += t4.w;
       return cc;
     };
-    const bool cv_const = P.temb == nullptr || temb_uniform;
+    const bool cv_const = P.epi.temb == nullptr || temb_uniform;
     float4 cv = make_float4(0.f, 0.f, 0.f, 0.f);
     if (cv_const) cv = load_cv(0);
     int it = 0;
@@ -356,8 +348,8 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
         for (int j = 0; j < NJ; ++j) {
           mi[j] = roff[j] < 0 ? -1 : base + roff[j];
           rv[j] = make_float4(0.f, 0.f, 0.f, 0.f);
-          if (mi[j] >= 0 && P.resid)
-            rv[j] = *reinterpret_cast<const float4*>(P.resid + static_cast<size_t>(mi[j]) * C + sub_c);
+          if (mi[j] >= 0 && P.epi.resid)
+            rv[j] = *reinterpret_cast<const float4*>(P.epi.resid + static_cast<size_t>(mi[j]) * C + sub_c);
         }
       }
       if (!mbar_wait(&ybuf_full[buf], (it >> 1) & 1, P.err_flag, 507)) break;
@@ -387,19 +379,19 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
         st2.z = fmaf(vv.z, vv.z, st2.z); st2.w = fmaf(vv.w, vv.w, st2.w);
         vv.x += cv.x; vv.y += cv.y; vv.z += cv.z; vv.w += cv.w;
         const size_t m = static_cast<size_t>(mi[j]);
-        if (P.out32) *reinterpret_cast<float4*>(P.out32 + m * C + sub_c) = vv;
-        if (P.out16) {
+        if (P.epi.out32) *reinterpret_cast<float4*>(P.epi.out32 + m * C + sub_c) = vv;
+        if (P.epi.out16) {
           __half2 h0v = __floats2half2_rn(vv.x, vv.y), h1v = __floats2half2_rn(vv.z, vv.w);
           uint2 uu;
           uu.x = *reinterpret_cast<uint32_t*>(&h0v);
           uu.y = *reinterpret_cast<uint32_t*>(&h1v);
-          *reinterpret_cast<uint2*>(P.out16 + m * C + sub_c) = uu;
+          *reinterpret_cast<uint2*>(P.epi.out16 + m * C + sub_c) = uu;
         }
       }
       // this warp has read its rows of the transpose buffer: hand it back to the drain warps
       __syncwarp();
       if (lane == 0) mbar_arrive(&ybuf_empty[buf]);
-      if (P.stats_rec) {
+      if (P.epi.stats_rec) {
         // lanes that share a channel quad (same lane % LPR) hold different rows: butterfly over them
 #pragma unroll
         for (int wd = LPR; wd < 32; wd <<= 1) {
@@ -423,7 +415,7 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
             a1 += sr[(wv * C + st) * 2];
             a2 += sr[(wv * C + st) * 2 + 1];
           }
-          float4* rec = reinterpret_cast<float4*>(P.stats_rec) + (static_cast<size_t>(n) * P.units_per_sample + v) * C + st;
+          float4* rec = reinterpret_cast<float4*>(P.epi.stats_rec) + (static_cast<size_t>(n) * P.units_per_sample + v) * C + st;
           *rec = make_float4(cvs[buf * C + st], a1, a2, 0.f);
         }
       }
@@ -438,13 +430,14 @@ struct Res32Launch {
   Res32Params p;
   dim3 grid;
   size_t smem;
-  bool ok;               // false: shape not covered, use conv_plane_kernel / conv_umma_kernel
+  bool ok;               // false: shape not covered
 };
 
 // Fills L for a k3 s1 p1 conv with cin = cout = 32, two weight terms (+ optional 1x1x1 source of 32/64/96
-// channels).  Returns 0 with L->ok = false when the shape is outside what this kernel covers.
+// channels).  Returns 0 with L->ok = false when the shape is outside what this kernel covers; refuses an
+// epilogue with hi|lo operand pairs or fp16 rows wider than 32 channels.
 int res32_prepare(Res32Launch* L, const __half* act, int B, int D, int H, int W, int cin, const __half* extra,
-                  int cin_extra, const __half* wpacked, int cout, int terms);
+                  int cin_extra, const __half* wpacked, int cout, int terms, const ConvEpilogue& epi);
 int res32_enqueue(const Res32Launch& L, cudaStream_t st);
 int res32_init();
 

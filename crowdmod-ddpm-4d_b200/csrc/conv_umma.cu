@@ -1,10 +1,5 @@
 // Host side of the tcgen05 implicit-GEMM conv: tensor-map construction and launch.
-#include "conv_umma.cuh"
-#include "kernels.cuh"
-#include "wgrad_umma.cuh"
-#include "conv_plane.cuh"
-#include "conv_res32.cuh"
-#include "wgrad_plane.cuh"
+#include "conv_run.cuh"
 
 #include <cudaTypedefs.h>
 #include <string.h>
@@ -144,7 +139,8 @@ size_t conv_packed_k(int mode, int cin, int cin_extra) {
 }
 
 int conv_prepare(ConvLaunch* L, int mode, const __half* act, int B, int D, int H, int W, int cin,
-                 const __half* extra, int cin_extra, const __half* wpacked, int cout, int terms, bool allow_splitk) {
+                 const __half* extra, int cin_extra, const __half* wpacked, int cout, int terms, const ConvEpilogue& epi,
+                 bool allow_splitk) {
   if (int rc = load_driver_syms()) return rc;
   CM_CHECK(mode >= 0 && mode <= 4, "bad conv mode %d", mode);
   CM_CHECK(cin % 32 == 0 && cin_extra % 32 == 0, "channels must be multiples of 32 (cin=%d extra=%d)",
@@ -228,7 +224,9 @@ int conv_prepare(ConvLaunch* L, int mode, const __half* act, int B, int D, int H
   p.kphase = (mode == 2) ? 8 * cin : 0;
   p.terms = terms;
   p.cout = cout;
-  p.out_ld = cout;
+  p.epi = epi;
+  p.epi.stats_rec = nullptr;   // a request: this kernel writes no GroupNorm records
+  p.epi.out_ld = cout;
   p.scatter = (mode == 2) ? 1 : 0;
   p.err_flag = device_error_flag();
 
@@ -358,7 +356,7 @@ int plane_init() {
 }
 
 int plane_prepare(PlaneLaunch* L, const __half* act, int B, int D, int H, int W, int cin,
-                  const __half* extra, int cin_extra, const __half* wpacked, int cout, int terms) {
+                  const __half* extra, int cin_extra, const __half* wpacked, int cout, int terms, const ConvEpilogue& epi) {
   if (int rc = load_driver_syms()) return rc;
   memset(L, 0, sizeof(*L));
   L->ok = false;
@@ -451,7 +449,8 @@ int plane_prepare(PlaneLaunch* L, const __half* act, int B, int D, int H, int W,
   p.n_units = B * p.units_per_sample * p.n_ntiles;
   p.a_stage_bytes = (int)(((long)(ntiles * 128 + (th3 ? 2 * Wp : 8)) * rowb + 1023) / 1024 * 1024);
   p.cin_main = cin; p.cin_extra = cin_extra; p.cout = cout; p.terms = terms;
-  p.out_ld = cout;
+  p.epi = epi;
+  p.epi.out_ld = cout;
   p.err_flag = device_error_flag();
   const long stage = p.a_stage_bytes + (long)terms * (th3 ? 3 : 1) * nst * rowb;
   const long tail = tail_fixed + ybuf_bytes(ntiles);
@@ -489,13 +488,13 @@ int res32_init() {
 }
 
 int res32_prepare(Res32Launch* L, const __half* act, int B, int D, int H, int W, int cin, const __half* extra,
-                  int cin_extra, const __half* wpacked, int cout, int terms) {
+                  int cin_extra, const __half* wpacked, int cout, int terms, const ConvEpilogue& epi) {
   if (int rc = res32_init()) return rc;
   memset(L, 0, sizeof(*L));
   L->ok = false;
   if (cin != R32_C || cout != R32_C || terms != 2 || cin_extra % R32_C || cin_extra > 3 * R32_C) return 0;
   const int Wp = W + 2;
-  if (Wp > 128) return 0;
+  if (Wp > 128 || H > 256) return 0;   // H: conv_plane's limit; res32 stands in for conv_plane, never for conv_umma alone
   int HB = 0;
   for (int hb = 1; hb <= H; ++hb)
     if (H % hb == 0 && hb * Wp <= 128) HB = hb;
@@ -515,6 +514,9 @@ int res32_prepare(Res32Launch* L, const __half* act, int B, int D, int H, int W,
   int stages = (int)((227L * 1024 - fixed) / stage_bytes);
   if (stages > R32_MAX_STAGES) stages = R32_MAX_STAGES;
   if (stages < 3) return 0;
+  CM_CHECK(epi.lo_from == 0 && epi.lo_from_x == 0 && epi.out16_lo == 0,
+           "weights-resident conv: hi|lo operand pairs are not supported");
+  CM_CHECK(epi.out16_ld == 0 || epi.out16_ld == R32_C, "weights-resident conv: fp16 rows of %d channels", epi.out16_ld);
   if (int rc = make_plane_map(&p.amap, act, B, D, H, W, R32_C, 32, 1, HB + 2)) return rc;
   if (nx) {
     CM_CHECK(extra != nullptr, "extra source pointer missing");
@@ -541,6 +543,8 @@ int res32_prepare(Res32Launch* L, const __half* act, int B, int D, int H, int W,
   p.nx = nx;
   p.stages = stages;
   p.stage_bytes = stage_bytes;
+  p.epi = epi;
+  p.epi.out_ld = R32_C;
   p.err_flag = device_error_flag();
   L->smem = (size_t)fixed + (size_t)stages * stage_bytes;
   L->grid = dim3(p.n_units < n_sm ? p.n_units : n_sm, 1, 1);
@@ -772,6 +776,86 @@ int wgrad_plane_init() {
 int wgrad_enqueue(const WgradLaunch& L, cudaStream_t st) {
   if (L.bkc == 64) return wg_dispatch<64>(L, st);
   return wg_dispatch<32>(L, st);
+}
+
+// ================================ kernel choice (conv_run.cuh) ================================
+int conv_run_prepare(ConvRun* R, unsigned kinds, int mode, const __half* act, int B, int D, int H, int W, int cin,
+                     const __half* extra, int cin_extra, const __half* wpacked, int cout, int terms,
+                     const ConvEpilogue& epi) {
+  if (mode == 0 && (kinds & CONV_RES32)) {
+    Res32Launch& L = R->l.emplace<Res32Launch>();
+    if (int rc = res32_prepare(&L, act, B, D, H, W, cin, extra, cin_extra, wpacked, cout, terms, epi)) return rc;
+    if (L.ok) return 0;
+  }
+  if (mode == 0 && (kinds & CONV_PLANE)) {
+    PlaneLaunch& L = R->l.emplace<PlaneLaunch>();
+    if (int rc = plane_prepare(&L, act, B, D, H, W, cin, extra, cin_extra, wpacked, cout, terms, epi)) return rc;
+    if (L.ok) return 0;
+  }
+  R->l = std::monostate{};
+  if (kinds & CONV_UMMA)
+    return conv_prepare(&R->l.emplace<ConvLaunch>(), mode, act, B, D, H, W, cin, extra, cin_extra, wpacked, cout, terms, epi);
+  return 0;
+}
+
+int conv_run_enqueue(const ConvRun& R, cudaStream_t st) {
+  if (const auto* L = std::get_if<Res32Launch>(&R.l)) return res32_enqueue(*L, st);
+  if (const auto* L = std::get_if<PlaneLaunch>(&R.l)) return plane_enqueue(*L, st);
+  CM_CHECK(R.covered(), "conv launch not prepared");
+  return conv_enqueue(std::get<ConvLaunch>(R.l), st);
+}
+
+ConvEpilogue& conv_run_epi(ConvRun& R) {
+  if (auto* L = std::get_if<Res32Launch>(&R.l)) return L->p.epi;
+  if (auto* L = std::get_if<PlaneLaunch>(&R.l)) return L->p.epi;
+  return std::get<ConvLaunch>(R.l).p.epi;
+}
+
+GnRec conv_run_records(const ConvRun& R) {
+  if (const auto* L = std::get_if<Res32Launch>(&R.l))
+    if (L->p.epi.stats_rec) return GnRec{L->p.epi.stats_rec, L->p.units_per_sample, L->p.HB * L->p.W};
+  if (const auto* L = std::get_if<PlaneLaunch>(&R.l))
+    if (L->p.epi.stats_rec) return GnRec{L->p.epi.stats_rec, L->p.units_per_sample, L->p.R * L->p.HB * L->p.W};
+  return GnRec{};
+}
+
+int wgrad_run_prepare(WgradRun* R, unsigned kinds, int mode, const __half* act, int B, int D, int H, int W, int cin,
+                      const __half* extra, int cin_extra, const __half* dout, int cout, float* G, int dout_ld,
+                      int act_ld, int extra_ld) {
+  R->n_plane = 0;
+  R->has_umma = false;
+  // next to the umma scheme the plane chunks are used up to 4 (measured); forced, up to the 8 of the array
+  const int nc = cin / 32, max_nc = (kinds & CONV_UMMA) ? 4 : 8;
+  if ((kinds & CONV_PLANE) && mode == 0 && cout == 32 && cin % 32 == 0 && nc >= 1 && nc <= max_nc) {
+    bool ok = true;
+    for (int c = 0; c < nc && ok; ++c) {
+      if (int rc = wgrad_plane_prepare(&R->plane[c], act, B, D, H, W, cin, act_ld, c * 32, dout, dout_ld, cout, G))
+        return rc;
+      ok = R->plane[c].ok;
+    }
+    if (ok) {
+      if (cin_extra) {
+        if (int rc = wgrad_prepare(&R->umma, 3, extra, B, D, H, W, cin_extra, nullptr, 0, dout, cout,
+                                   G + (size_t)27 * cin * cout, dout_ld, extra_ld, 0))
+          return rc;
+        R->has_umma = true;
+      }
+      R->n_plane = nc;
+      return 0;
+    }
+  }
+  if (!(kinds & CONV_UMMA)) return 0;
+  if (int rc = wgrad_prepare(&R->umma, mode, act, B, D, H, W, cin, extra, cin_extra, dout, cout, G, dout_ld, act_ld,
+                             extra_ld))
+    return rc;
+  R->has_umma = true;
+  return 0;
+}
+
+int wgrad_run_enqueue(const WgradRun& R, cudaStream_t st) {
+  for (int c = 0; c < R.n_plane; ++c)
+    if (int e = wgrad_plane_enqueue(R.plane[c], st)) return e;
+  return R.has_umma ? wgrad_enqueue(R.umma, st) : 0;
 }
 
 }  // namespace cm

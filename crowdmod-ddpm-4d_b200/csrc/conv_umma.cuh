@@ -22,6 +22,33 @@ constexpr int CONV_BM = 128;        // UMMA M (cta_group::1)
 constexpr int CONV_THREADS = 192;   // warp0 TMA, warp1 MMA, warps2-5 epilogue
 constexpr int CONV_MAX_STAGES = 8;
 
+// Epilogue of the three forward conv kernels (conv_umma, conv_plane, conv_res32):
+// out = acc + bias + bias2 + temb row + resid, stored fp32 and / or fp16.
+// Field order: the int pairs (lo_from, lo_from_x), (temb_ld, temb_bstride), (out_ld, out16_ld) start at 8-byte
+// boundaries, as in the parameter structs before this one existed; ptxas then emits the same code (apart, it
+// loads them separately and conv_umma_kernel<., ., 1> takes up to 3 more registers).
+struct ConvEpilogue {
+  int lo_from, lo_from_x;   // > 0: channels >= lo_from of the main (lo_from_x: the 1x1x1) source are the lo halves of hi|lo
+                            // operand pairs (training): their k16 slices skip the lo weight term (a_lo * w_lo ~ 2^-22)
+  const float* bias;
+  const float* bias2;
+  const float* temb;     // [rows][temb_ld] projection table, nullptr = none
+  const int* t_dev;      // device int: row of `temb` for the whole batch (sampling); nullptr = 0
+  int temb_ld;
+  int temb_bstride;      // per-sample row stride (training: temb_ld, sampling: 0)
+  const float* resid;    // fp32 [M][cout] or nullptr
+  float* out32;          // fp32 [rows][out_ld] or nullptr
+  __half* out16;         // fp16 [rows][out16_ld] or nullptr
+  int out_ld;            // set by the prepare functions (cout)
+  int out16_ld, out16_lo;   // fp16 copy: row stride in elements (0 -> out_ld); out16_lo > 0: also write the lo half
+                            // fp16(v - hi) out16_lo elements further (hi|lo pair operand of the training forward)
+  // GroupNorm statistics records of the values the launch writes (nullptr = none), plane and res32 kernels only: per
+  // (sample, unit of the sample, output channel) a float4 {shift, sum(v - shift), sum((v - shift)^2), 0} over the unit's
+  // valid rows; units belong to ONE sample, so the consumer (gn_apply2_kernel) merges them in a fixed order ->
+  // bit-reproducible wherever the sample sits in the batch.
+  float* stats_rec;
+};
+
 struct ConvParams {
   CUtensorMap amap[8];   // main source, one map per output phase (1 normally, 8 for upsample)
   CUtensorMap xmap;      // optional extra 1x1x1 source (match_input fused as a K-slab)
@@ -36,22 +63,9 @@ struct ConvParams {
   int cin_main, cin_extra;
   int kphase;            // packed-K elements per phase
   int terms;             // 1 = fp16 weights, 2 = hi+lo split weights
-  int lo_from, lo_from_x;   // > 0: channels >= lo_from of the main (lo_from_x: the 1x1x1) source are the lo halves of hi|lo
-                            // operand pairs (training): their k16 slices skip the lo weight term (a_lo * w_lo ~ 2^-22)
   int cout;
   int stages;
-  const float* bias;
-  const float* bias2;
-  const float* temb;     // [rows][temb_ld] projection table, nullptr = none
-  const int* t_dev;      // device int: row of `temb` for the whole batch (sampling); nullptr = 0
-  int temb_ld;
-  int temb_bstride;      // per-sample row stride (training: temb_ld, sampling: 0)
-  const float* resid;    // fp32 [M][cout] or nullptr
-  float* out32;          // fp32 [rows][out_ld] or nullptr
-  __half* out16;         // fp16 [rows][out16_ld] or nullptr
-  int out_ld;
-  int out16_ld, out16_lo;   // fp16 copy: row stride in elements (0 -> out_ld); out16_lo > 0: also write the lo half
-                            // fp16(v - hi) out16_lo elements further (hi|lo pair operand of the training forward)
+  ConvEpilogue epi;      // stats_rec unused
   // optional epilogue extras of the non-split path (the DiT plan, dit.cu): v = act(acc + bias); v *= gate[sample][n];
   // v += resid; rows of sample b land at output row b*rmap_out + rmap_off + (m - b*pps) (resid is read there too)
   int act;               // 0 none, 1 exact GELU
@@ -194,8 +208,8 @@ conv_umma_kernel(const __grid_constant__ ConvParams P) {
     // ===================== MMA issuer (whole warp runs the loop; one elected lane issues) =====
     {
       constexpr uint32_t DESC_HI = kmajor_desc_hi(ROWB);
-      const int lo_from = P.lo_from > 0 ? P.lo_from : 0x40000000;
-      const int lo_from_x = P.lo_from_x > 0 ? P.lo_from_x : 0x40000000;
+      const int lo_from = P.epi.lo_from > 0 ? P.epi.lo_from : 0x40000000;
+      const int lo_from_x = P.epi.lo_from_x > 0 ? P.epi.lo_from_x : 0x40000000;
       const uint32_t lo0 = kmajor_desc_lo(smem_u32(smem));
       const uint32_t lo_stage = static_cast<uint32_t>(stage_bytes) >> 4;
       int s = 0;
@@ -240,14 +254,14 @@ conv_umma_kernel(const __grid_constant__ ConvParams P) {
     const int m = m_tile * CONV_BM + row;
     const bool valid = m < P.M;
     const int et = threadIdx.x - 64;  // 0..127 within the epilogue warps
-    const bool temb_uniform = P.temb != nullptr && P.temb_bstride == 0;
+    const bool temb_uniform = P.epi.temb != nullptr && P.epi.temb_bstride == 0;
     {
-      const int trow = (P.temb && P.t_dev) ? *P.t_dev : 0;
+      const int trow = (P.epi.temb && P.epi.t_dev) ? *P.epi.t_dev : 0;
       for (int c = et; c < BN; c += 128) {
         const int n = n_tile * BN + c;
-        float v = P.bias ? P.bias[n] : 0.f;
-        if (P.bias2) v += P.bias2[n];
-        if (temb_uniform) v += P.temb[static_cast<size_t>(trow) * P.temb_ld + n];
+        float v = P.epi.bias ? P.epi.bias[n] : 0.f;
+        if (P.epi.bias2) v += P.epi.bias2[n];
+        if (temb_uniform) v += P.epi.temb[static_cast<size_t>(trow) * P.epi.temb_ld + n];
         colv[c] = v;
       }
     }
@@ -269,8 +283,8 @@ conv_umma_kernel(const __grid_constant__ ConvParams P) {
     }
     const float* gate_row = (P.gate && valid) ? P.gate + static_cast<size_t>(b) * P.gate_ld + n_tile * BN : nullptr;
     const float* temb_row = nullptr;     // per-sample rows (training): added per element
-    if (P.temb && !temb_uniform)
-      temb_row = P.temb + static_cast<size_t>(b) * P.temb_bstride + n_tile * BN;
+    if (P.epi.temb && !temb_uniform)
+      temb_row = P.epi.temb + static_cast<size_t>(b) * P.epi.temb_bstride + n_tile * BN;
     asm volatile("bar.sync 1, 128;" ::: "memory");   // colv visible to the 4 epilogue warps
 
     const uint32_t t_lane = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16);
@@ -281,7 +295,7 @@ conv_umma_kernel(const __grid_constant__ ConvParams P) {
       orow = ((static_cast<size_t>(b) * (2 * P.od) + (2 * sz + pz)) * (2 * P.oh) + (2 * sp + pp)) *
                  (2 * P.ow) + (2 * sq + pq);
     }
-    const float* rp = (P.resid && valid && P.ksplit <= 1) ? P.resid + orow * P.cout + n_tile * BN : nullptr;   // orow == m unless scattering
+    const float* rp = (P.epi.resid && valid && P.ksplit <= 1) ? P.epi.resid + orow * P.cout + n_tile * BN : nullptr;   // orow == m unless scattering
     float4 rnext[4];
     if (rp) {                      // first residual chunk in flight while the main loop finishes
 #pragma unroll
@@ -362,13 +376,13 @@ conv_umma_kernel(const __grid_constant__ ConvParams P) {
       const int n = n_tile * BN + c * 16;
       // row-per-thread stores: 32 bytes (one sector) per instruction (256-bit stores; every row start and n are multiples
       // of 16 elements, so fp32 chunks are 64-byte and fp16 chunks 32-byte aligned)
-      if (P.out32) {
-        float* op = P.out32 + orow * P.out_ld + n;
+      if (P.epi.out32) {
+        float* op = P.epi.out32 + orow * P.epi.out_ld + n;
         st_global_v8(op, v);
         st_global_v8(op + 8, v + 8);
       }
-      if (P.out16) {
-        __half* op = P.out16 + orow * (P.out16_ld > 0 ? P.out16_ld : P.out_ld) + n;
+      if (P.epi.out16) {
+        __half* op = P.epi.out16 + orow * (P.epi.out16_ld > 0 ? P.epi.out16_ld : P.epi.out_ld) + n;
         uint32_t uh[8], ul[8];
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
@@ -379,7 +393,7 @@ conv_umma_kernel(const __grid_constant__ ConvParams P) {
           ul[i] = *reinterpret_cast<const uint32_t*>(&l);
         }
         st_global_v8(op, uh);
-        if (P.out16_lo > 0) st_global_v8(op + P.out16_lo, ul);
+        if (P.epi.out16_lo > 0) st_global_v8(op + P.epi.out16_lo, ul);
       }
     }
     if (pi + 1 < ppc) {          // hand the accumulator back to the MMA warp for the next phase
@@ -413,7 +427,7 @@ conv_umma_kernel(const __grid_constant__ ConvParams P) {
         // all peer loads (and the residual) in flight together, then a fixed-order sum
         float4 pv[8];
         float4 r4 = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (P.resid) r4 = *reinterpret_cast<const float4*>(P.resid + static_cast<size_t>(m) * P.cout + n);
+        if (P.epi.resid) r4 = *reinterpret_cast<const float4*>(P.epi.resid + static_cast<size_t>(m) * P.cout + n);
 #pragma unroll
         for (int sidx = 0; sidx < 8; ++sidx) {
           pv[sidx] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -429,25 +443,25 @@ conv_umma_kernel(const __grid_constant__ ConvParams P) {
         for (int sidx = 0; sidx < 8; ++sidx) {
           acc.x += pv[sidx].x; acc.y += pv[sidx].y; acc.z += pv[sidx].z; acc.w += pv[sidx].w;
         }
-        if (P.temb && P.temb_bstride != 0) {
-          const float4 t4 = *reinterpret_cast<const float4*>(P.temb + static_cast<size_t>(m / P.pps) * P.temb_bstride + n);
+        if (P.epi.temb && P.epi.temb_bstride != 0) {
+          const float4 t4 = *reinterpret_cast<const float4*>(P.epi.temb + static_cast<size_t>(m / P.pps) * P.epi.temb_bstride + n);
           acc.x += t4.x; acc.y += t4.y; acc.z += t4.z; acc.w += t4.w;
         }
         acc.x += r4.x; acc.y += r4.y; acc.z += r4.z; acc.w += r4.w;
-        if (P.out32) *reinterpret_cast<float4*>(P.out32 + static_cast<size_t>(m) * P.out_ld + n) = acc;
-        if (P.out16) {
+        if (P.epi.out32) *reinterpret_cast<float4*>(P.epi.out32 + static_cast<size_t>(m) * P.epi.out_ld + n) = acc;
+        if (P.epi.out16) {
           __half2 h0 = __floats2half2_rn(acc.x, acc.y), h1 = __floats2half2_rn(acc.z, acc.w);
           uint2 u;
           u.x = *reinterpret_cast<uint32_t*>(&h0);
           u.y = *reinterpret_cast<uint32_t*>(&h1);
-          __half* o16 = P.out16 + static_cast<size_t>(m) * (P.out16_ld > 0 ? P.out16_ld : P.out_ld) + n;
+          __half* o16 = P.epi.out16 + static_cast<size_t>(m) * (P.epi.out16_ld > 0 ? P.epi.out16_ld : P.epi.out_ld) + n;
           *reinterpret_cast<uint2*>(o16) = u;
-          if (P.out16_lo > 0) {
+          if (P.epi.out16_lo > 0) {
             const float2 f0 = __half22float2(h0), f1 = __half22float2(h1);
             __half2 l0 = __floats2half2_rn(acc.x - f0.x, acc.y - f0.y), l1 = __floats2half2_rn(acc.z - f1.x, acc.w - f1.y);
             u.x = *reinterpret_cast<uint32_t*>(&l0);
             u.y = *reinterpret_cast<uint32_t*>(&l1);
-            *reinterpret_cast<uint2*>(o16 + P.out16_lo) = u;
+            *reinterpret_cast<uint2*>(o16 + P.epi.out16_lo) = u;
           }
         }
       }
@@ -461,12 +475,6 @@ conv_umma_kernel(const __grid_constant__ ConvParams P) {
 }
 
 // -------------------------------- host side --------------------------------
-struct ConvGeom {
-  // source activation tensor (fp16, channels-last)
-  int B, D, H, W;       // D=grid rows, H=grid cols, W=time frames (fastest spatial)
-  int C;                // channels of the main source
-};
-
 struct ConvLaunch {
   ConvParams p;
   dim3 grid;
@@ -476,9 +484,10 @@ struct ConvLaunch {
 
 // Fill amap/xmap/bmap + geometry.  `mode`: 0 = k3 s1 p1 ("same"), 1 = k3 s2 p1 (DownSample),
 // 2 = nearest-x2 + k3 p1 decomposed into 8 phase convs with 2x2x2 combined taps (UpSample),
-// 3 = 1x1x1.  Extra source: 1x1x1 over the OUTPUT grid with cin_extra channels.
+// 3 = 1x1x1.  Extra source: 1x1x1 over the OUTPUT grid with cin_extra channels.  epi.stats_rec is dropped.
 int conv_prepare(ConvLaunch* L, int mode, const __half* act, int B, int D, int H, int W, int cin,
-                 const __half* extra, int cin_extra, const __half* wpacked, int cout, int terms, bool allow_splitk = true);
+                 const __half* extra, int cin_extra, const __half* wpacked, int cout, int terms, const ConvEpilogue& epi,
+                 bool allow_splitk = true);
 int conv_enqueue(const ConvLaunch& L, cudaStream_t st);
 size_t conv_packed_k(int mode, int cin, int cin_extra);   // K elements of the packed weight rows
 

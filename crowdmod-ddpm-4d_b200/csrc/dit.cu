@@ -572,11 +572,10 @@ int reserve(cm_dit* u, int batch) {
 int prep_gemm(cm_dit* u, DitLinear& l, const __half* act, int nb, int d, int h, int w, float* out32) {
   // no split-K: the epilogue fusions (act / gate / rmap) live in the non-split path, and with K <= 1024 narrower N tiles
   // fill the SMs without the cluster reduction
-  if (int rc = conv_prepare(&l.launch, 3, act, nb, d, h, w, l.cin, nullptr, 0, u->wpack + l.pack_off, l.cout, 2, false)) return rc;
-  l.launch.p.bias = l.b >= 0 ? u->params[l.b].ptr : l.b_dev;
-  l.launch.p.out32 = out32;
-  l.launch.p.out16 = nullptr;
-  return 0;
+  ConvEpilogue e{};
+  e.bias = l.b >= 0 ? u->params[l.b].ptr : l.b_dev;
+  e.out32 = out32;
+  return conv_prepare(&l.launch, 3, act, nb, d, h, w, l.cin, nullptr, 0, u->wpack + l.pack_off, l.cout, 2, e, false);
 }
 
 int prepare(cm_dit* u, int batch) {
@@ -597,9 +596,9 @@ int prepare(cm_dit* u, int batch) {
     // epilogue fusions (ConvParams::act / gate / rmap): GELU + fp16 operand out of fc1; the three gated residuals
     // x += gate * (GEMM + bias) written in place into the token stream (the temporal one into the future slots)
     b.fc1.launch.p.act = 1;
-    b.fc1.launch.p.out16 = u->g16;
+    b.fc1.launch.p.epi.out16 = u->g16;
     for (DitLinear* l : {&b.s_out, &b.t_out, &b.fc2}) {
-      l->launch.p.resid = u->x32;
+      l->launch.p.epi.resid = u->x32;
       l->launch.p.gate = u->mods;           // + the block's gate offset, set per launch in run_forward
     }
     b.t_out.launch.p.rmap_out = u->tokens;

@@ -1970,11 +1970,11 @@ __global__ void conv_ref_kernel(const ConvParams p, const __half* __restrict__ a
         for (int c = 0; c < p.cin_extra; ++c) acc = fmaf(__half2float(ap[c]), __half2float(wk[c]), acc);
       }
     }
-    if (p.bias) acc += p.bias[n];
-    if (p.bias2) acc += p.bias2[n];
-    if (p.temb) {
-      const int trow = p.t_dev ? *p.t_dev : 0;
-      acc += p.temb[(size_t)trow * p.temb_ld + (size_t)b * p.temb_bstride + n];
+    if (p.epi.bias) acc += p.epi.bias[n];
+    if (p.epi.bias2) acc += p.epi.bias2[n];
+    if (p.epi.temb) {
+      const int trow = p.epi.t_dev ? *p.epi.t_dev : 0;
+      acc += p.epi.temb[(size_t)trow * p.epi.temb_ld + (size_t)b * p.epi.temb_bstride + n];
     }
     size_t orow = m;
     if (p.scatter) {
@@ -1982,9 +1982,9 @@ __global__ void conv_ref_kernel(const ConvParams p, const __half* __restrict__ a
       orow = (((size_t)b * (2 * p.od) + (2 * z + pz)) * (2 * p.oh) + (2 * pp_ + pp)) * (2 * p.ow) +
              (2 * q + pq);
     }
-    if (p.resid) acc += p.resid[orow * p.cout + n];
-    if (p.out32) p.out32[orow * p.out_ld + n] = acc;
-    if (p.out16) p.out16[orow * p.out_ld + n] = __float2half_rn(acc);
+    if (p.epi.resid) acc += p.epi.resid[orow * p.cout + n];
+    if (p.epi.out32) p.epi.out32[orow * p.epi.out_ld + n] = acc;
+    if (p.epi.out16) p.epi.out16[orow * p.epi.out_ld + n] = __float2half_rn(acc);
   }
 }
 

@@ -25,7 +25,7 @@ int pack_upsample_weights(const float* w, __half* dst, int cout, int cin, int te
                           cudaStream_t st, int dup = 1);
 
 // ---- GroupNorm(8) [+SiLU] [+Dropout3d scale] -> fp16 operand (layers.py:30,41,57,70; :9,14) ----
-// GroupNorm statistics records written by a producing plane-tile conv (PlaneParams::stats_rec)
+// GroupNorm statistics records written by a producing plane-tile or res32 conv (ConvEpilogue::stats_rec)
 struct GnRec {
   const float* rec;   // [B][units][C_src] float4 {shift, sum, sumsq, 0}; nullptr = none
   int units;          // units per sample

@@ -16,13 +16,9 @@
 
 #include "../../include/crowdmod_b200.h"
 #include "backward.cuh"
-#include "conv_plane.cuh"
-#include "conv_res32.cuh"
-#include "wgrad_plane.cuh"
-#include "conv_umma.cuh"
+#include "conv_run.cuh"
 #include "kernels.cuh"
 #include "pack.cuh"
-#include "wgrad_umma.cuh"
 
 namespace cm {
 
@@ -46,7 +42,7 @@ struct Tens {
   // GroupNorm statistics records emitted by the plane-tile conv that produces this tensor
   bool gn_src = false;      // consumed by a GroupNorm
   float* rec = nullptr;     // [batch][D*H][C] float4 (sized for the finest unit split)
-  int rec_units = 0, rec_nvalid = 0;   // set when the producing launch emits records, else 0
+  GnRec gn_rec{};           // what the producing launch writes there (units == 0: no records)
 };
 
 enum OpType { OP_FIRST, OP_GN, OP_CONV, OP_ATTN, OP_FINAL };
@@ -61,9 +57,7 @@ struct Op {
       resid = -1, out = -1, cin = 0, cin_extra = 0, cout = 0, in_level = 0;
   size_t wpack_off = 0;   // element offset into the packed-weight buffer
   size_t wpack2_off = 0;  // same in the training forward's cache (hi|lo pair activation operands, K doubled)
-  ConvLaunch launch;
-  PlaneLaunch plaunch;      // plane-tile kernel (conv_plane.cuh) when it covers the geometry
-  Res32Launch rlaunch;      // weights-resident 32 -> 32 kernel (conv_res32.cuh) when it covers the shape (sampling / eval)
+  ConvRun fwd;
   // ATTN
   int qkv = -1, ctx = -1, heads = 4;
   // training (backward) bookkeeping
@@ -72,14 +66,8 @@ struct Op {
   size_t dpack_off = 0, dxpack_off = 0;   // CONV: dgrad weight caches (main / fused 1x1 source)
   size_t g_off = 0;         // CONV: offset of the packed-K weight-gradient scratch
   size_t colsum_off = 0;    // CONV: per-sample channel sums of dOut ([B][cout])
-  ConvLaunch dlaunch, dxlaunch;
-  PlaneLaunch dplaunch;     // dgrad of a k3 s1 conv is a k3 s1 conv: plane-tile kernel when it fits
-  WgradLaunch wlaunch;
-  // full-resolution convs with 32 output channels: plane / halo weight gradient (wgrad_plane.cuh), one launch per
-  // 32-channel chunk of the main source, the fused 1x1x1 source through wgrad_umma_kernel in 1x1x1 mode (n_wpl = 0: off)
-  WgradPlaneLaunch wpl[4];
-  int n_wpl = 0;
-  WgradLaunch wxlaunch;
+  ConvRun dgrad, dgrad_x;   // data gradients of the main and the fused 1x1x1 source
+  WgradRun wgrad;
 };
 
 struct Level {
@@ -105,11 +93,10 @@ struct cm_unet {
   int p_table = -1, p_w1 = -1, p_b1 = -1, p_w2 = -1, p_b2 = -1;
   int p_first_w = -1, p_first_b = -1, p_final_w = -1, p_final_b = -1;
   // first conv on the tensor cores: the 3(+)-channel input is packed into a zero-padded 32-channel fp16
-  // operand and run through the plane-tile kernel (falls back to first_conv_kernel when not covered)
+  // operand and run through the plane-tile or res32 kernel (falls back to first_conv_kernel when neither covers it)
   int first_in = -1;
   size_t first_wpack_off = 0;
-  PlaneLaunch first_plane;
-  Res32Launch first_res;
+  ConvRun first;
   WgradPlaneLaunch first_wpl;          // first conv's weight gradient through the plane / halo kernel (base_channels == 32)
   size_t first_g_off = 0;              // its packed-K scratch (27 taps x 32 packed channels x 32) and channel-sum slot
   int first_colsum_off = 0;
@@ -144,7 +131,8 @@ struct cm_unet {
   __half* wpack2 = nullptr;             // forward weights packed against hi|lo activation rows (training)
   size_t wpack2_elems = 0, first_wpack2_off = 0;
   bool packed2 = false;
-  int live_dup = 1;                     // activation-operand layout the conv launches are currently prepared for
+  int live_batch = 0;                   // batch the conv launches are prepared for (0: none)
+  int live_dup = 1;                     // and activation-operand layout
   // workspace (per reserved batch)
   int reserved_batch = 0;
   uint8_t* arena = nullptr;
@@ -526,7 +514,7 @@ int reserve(cm_unet* u, int batch) {
     t.p32 = t.need32 ? reinterpret_cast<float*>(u->arena + o32[i]) : nullptr;
     t.p16 = t.need16 ? reinterpret_cast<__half*>(u->arena + o16[i]) : nullptr;
     t.rec = t.gn_src ? reinterpret_cast<float*>(u->arena + orec[i]) : nullptr;
-    t.rec_units = 0;
+    t.gn_rec = GnRec{};
   }
   u->temb_batch = reinterpret_cast<float*>(u->arena + temb_off);
   u->gn_partial = reinterpret_cast<float*>(u->arena + gnp_off);
@@ -542,120 +530,47 @@ int reserve(cm_unet* u, int batch) {
 // dup = 1: single fp16 activation operands (sampling / eval); dup = 2: hi|lo pair rows (training forward)
 int prepare_convs(cm_unet* u, int batch, int dup) {
   const __half* wbase = dup == 2 ? u->wpack2 : u->wpack;
+  // res32 only for single fp16 operands: it has no hi|lo operand pairs
+  const unsigned fast = dup == 1 ? CONV_PLANE | CONV_RES32 : CONV_PLANE;
   {
     const Level& l0 = u->levels[0];
-    u->first_plane.ok = false;
-    u->first_res.ok = false;
-    if (int rc = plane_prepare(&u->first_plane, u->tens[u->first_in].p16, batch, l0.D, l0.H, l0.W, 32 * dup, nullptr, 0,
-                               wbase + (dup == 2 ? u->first_wpack2_off : u->first_wpack_off), u->cfg.base_channels,
-                               u->cfg.weight_terms))
+    Tens& t = u->tens[u->ops[0].out];
+    ConvEpilogue e{};
+    e.bias = u->params[u->p_first_b].ptr;
+    e.out32 = t.p32;
+    e.lo_from = dup == 2 ? 32 : 0;
+    e.stats_rec = t.rec;
+    if (int rc = conv_run_prepare(&u->first, fast, 0, u->tens[u->first_in].p16, batch, l0.D, l0.H, l0.W, 32 * dup,
+                                  nullptr, 0, wbase + (dup == 2 ? u->first_wpack2_off : u->first_wpack_off),
+                                  u->cfg.base_channels, u->cfg.weight_terms, e))
       return rc;
-    if (u->first_plane.ok) {
-      u->first_plane.p.lo_from = dup == 2 ? 32 : 0;
-      u->first_plane.p.bias = u->params[u->p_first_b].ptr;
-      u->first_plane.p.out32 = nullptr;   // set per run (tensor of the OP_FIRST op)
-    }
-    if (u->first_plane.ok && dup == 1) {
-      if (int rc = res32_prepare(&u->first_res, u->tens[u->first_in].p16, batch, l0.D, l0.H, l0.W, 32, nullptr, 0,
-                                 wbase + u->first_wpack_off, u->cfg.base_channels, u->cfg.weight_terms))
-        return rc;
-      if (u->first_res.ok) u->first_res.p.bias = u->params[u->p_first_b].ptr;
-    }
-    for (Op& fo : u->ops) {
-      if (fo.type != OP_FIRST) continue;
-      Tens& t = u->tens[fo.out];
-      t.rec_units = 0;
-      if (u->first_res.ok && t.rec) {
-        Res32Params& q = u->first_res.p;
-        q.stats_rec = t.rec;
-        t.rec_units = q.units_per_sample;
-        t.rec_nvalid = q.HB * q.W;
-      } else if (u->first_plane.ok && t.rec) {
-        PlaneParams& q = u->first_plane.p;
-        q.stats_rec = t.rec;
-        t.rec_units = q.units_per_sample;
-        t.rec_nvalid = q.R * q.HB * q.W;
-      }
-    }
+    t.gn_rec = conv_run_records(u->first);
   }
   for (Op& op : u->ops) {
     if (op.type != OP_CONV) continue;
     const Level& li = u->levels[op.in_level];
-    const Tens& tin = u->tens[op.in];
-    const __half* extra = op.extra >= 0 ? u->tens[op.extra].p16 : nullptr;
-    const __half* wp = wbase + (dup == 2 ? op.wpack2_off : op.wpack_off);
-    const int terms = u->cfg.weight_terms;
-    if (int rc = conv_prepare(&op.launch, op.mode, tin.p16, batch, li.D, li.H, li.W, op.cin * dup, extra,
-                              op.cin_extra * dup, wp, op.cout, terms))
-      return rc;
+    Tens& t = u->tens[op.out];
+    ConvEpilogue e{};
+    e.bias = op.bias >= 0 ? u->params[op.bias].ptr : nullptr;
+    e.bias2 = op.bias2 >= 0 ? u->params[op.bias2].ptr : nullptr;
+    e.resid = op.resid >= 0 ? u->tens[op.resid].p32 : nullptr;
+    e.out32 = t.p32;
+    e.out16 = t.p16;
+    e.out16_ld = op.cout * dup;
+    e.out16_lo = dup == 2 ? op.cout : 0;
     // hi|lo operand pairs against hi+lo weight terms: the lo x lo product (2^-22 of the result) is skipped
-    const bool skip_lolo = dup == 2;
-    op.launch.p.lo_from = skip_lolo ? op.cin : 0;
-    op.launch.p.lo_from_x = skip_lolo ? op.cin_extra : 0;
-    op.plaunch.ok = false;
-    if (op.mode == 0) {
-      if (int rc = plane_prepare(&op.plaunch, tin.p16, batch, li.D, li.H, li.W, op.cin * dup, extra, op.cin_extra * dup,
-                                 wp, op.cout, terms))
-        return rc;
-      if (op.plaunch.ok) {
-        PlaneParams& q = op.plaunch.p;
-        q.lo_from = skip_lolo ? op.cin : 0;
-        q.lo_from_x = skip_lolo ? op.cin_extra : 0;
-        q.bias = op.bias >= 0 ? u->params[op.bias].ptr : nullptr;
-        q.bias2 = op.bias2 >= 0 ? u->params[op.bias2].ptr : nullptr;
-        q.resid = op.resid >= 0 ? u->tens[op.resid].p32 : nullptr;
-        q.out32 = u->tens[op.out].p32;
-        q.out16 = u->tens[op.out].p16;
-        q.out16_ld = op.cout * dup;
-        q.out16_lo = dup == 2 ? op.cout : 0;
-      }
-    }
-    op.rlaunch.ok = false;
-    if (op.mode == 0 && dup == 1 && op.plaunch.ok) {
-      if (int rc = res32_prepare(&op.rlaunch, tin.p16, batch, li.D, li.H, li.W, op.cin, extra, op.cin_extra, wp, op.cout, terms))
-        return rc;
-      if (op.rlaunch.ok) {
-        Res32Params& q = op.rlaunch.p;
-        q.bias = op.bias >= 0 ? u->params[op.bias].ptr : nullptr;
-        q.bias2 = op.bias2 >= 0 ? u->params[op.bias2].ptr : nullptr;
-        q.resid = op.resid >= 0 ? u->tens[op.resid].p32 : nullptr;
-        q.out32 = u->tens[op.out].p32;
-        q.out16 = u->tens[op.out].p16;
-      }
-    }
-    {
-      Tens& t = u->tens[op.out];
-      t.rec_units = 0;
-      if (op.rlaunch.ok && t.rec) {
-        Res32Params& q = op.rlaunch.p;
-        q.stats_rec = t.rec;
-        t.rec_units = q.units_per_sample;
-        t.rec_nvalid = q.HB * q.W;
-      } else if (op.plaunch.ok && t.rec) {
-        PlaneParams& q = op.plaunch.p;
-        q.stats_rec = t.rec;
-        t.rec_units = q.units_per_sample;
-        t.rec_nvalid = q.R * q.HB * q.W;
-      }
-    }
-    ConvParams& p = op.launch.p;
-    p.bias = op.bias >= 0 ? u->params[op.bias].ptr : nullptr;
-    p.bias2 = op.bias2 >= 0 ? u->params[op.bias2].ptr : nullptr;
-    p.resid = op.resid >= 0 ? u->tens[op.resid].p32 : nullptr;
-    p.out32 = u->tens[op.out].p32;
-    p.out16 = u->tens[op.out].p16;
-    p.out16_ld = op.cout * dup;
-    p.out16_lo = dup == 2 ? op.cout : 0;
-    CM_CHECK(p.out32 || p.out16, "conv '%s' has no consumer", op.tag.c_str());
+    e.lo_from = dup == 2 ? op.cin : 0;
+    e.lo_from_x = dup == 2 ? op.cin_extra : 0;
+    e.stats_rec = t.rec;
+    CM_CHECK(e.out32 || e.out16, "conv '%s' has no consumer", op.tag.c_str());
+    if (int rc = conv_run_prepare(&op.fwd, CONV_UMMA | fast, op.mode, u->tens[op.in].p16, batch, li.D, li.H, li.W,
+                                  op.cin * dup, op.extra >= 0 ? u->tens[op.extra].p16 : nullptr, op.cin_extra * dup,
+                                  wbase + (dup == 2 ? op.wpack2_off : op.wpack_off), op.cout, u->cfg.weight_terms, e))
+      return rc;
+    t.gn_rec = conv_run_records(op.fwd);
   }
+  u->live_batch = batch;
   u->live_dup = dup;
-  return 0;
-}
-
-// batch * dup the conv launches are prepared for (0 = none): a change of either rebuilds them
-int live_batch_of(const cm_unet* u) {
-  for (const Op& op : u->ops)
-    if (op.type == OP_CONV) return op.launch.p.pps ? (op.launch.p.M / op.launch.p.pps) * u->live_dup : 0;
   return 0;
 }
 
@@ -709,19 +624,11 @@ int run_ops(cm_unet* u, RunCtx& rc, cudaStream_t st, int64_t* launches,
     switch (op.type) {
       case OP_FIRST: {
         const Level& l0 = u->levels[0];
-        if (u->first_plane.ok) {
+        if (u->first.covered()) {
           if (int e = pack_first_input_enqueue(rc.future, rc.past, u->tens[u->first_in].p16, rc.batch, l0.H, l0.W,
                                                c.past_len, c.future_len, c.in_channels, rc.dup, st))
             return e;
-          if (u->first_res.ok) {
-            Res32Launch R = u->first_res;
-            R.p.out32 = u->tens[op.out].p32;
-            if (int e = res32_enqueue(R, st)) return e;
-          } else {
-            PlaneLaunch L = u->first_plane;
-            L.p.out32 = u->tens[op.out].p32;
-            if (int e = plane_enqueue(L, st)) return e;
-          }
+          if (int e = conv_run_enqueue(u->first, st)) return e;
           if (launches) ++*launches;
           break;
         }
@@ -747,15 +654,11 @@ int run_ops(cm_unet* u, RunCtx& rc, cudaStream_t st, int64_t* launches,
         g.out_raw = op.out_raw >= 0 ? u->tens[op.out_raw].p16 : nullptr;
         g.dup = rc.dup;
         {
-          const Tens& t0 = u->tens[op.src0];
-          const bool ok0 = t0.rec_units > 0;
-          const bool ok1 = op.src1 < 0 || u->tens[op.src1].rec_units > 0;
-          if (ok0 && ok1) {
-            g.rec0 = GnRec{t0.rec, t0.rec_units, t0.rec_nvalid};
-            if (op.src1 >= 0) {
-              const Tens& t1 = u->tens[op.src1];
-              g.rec1 = GnRec{t1.rec, t1.rec_units, t1.rec_nvalid};
-            }
+          const GnRec r0 = u->tens[op.src0].gn_rec;
+          const GnRec r1 = op.src1 >= 0 ? u->tens[op.src1].gn_rec : GnRec{};
+          if (r0.units > 0 && (op.src1 < 0 || r1.units > 0)) {
+            g.rec0 = r0;
+            g.rec1 = r1;
           }
         }
         if (rc.train) {
@@ -770,36 +673,15 @@ int run_ops(cm_unet* u, RunCtx& rc, cudaStream_t st, int64_t* launches,
         if (launches) *launches += nl - 1;
       } break;
       case OP_CONV: {
-        if (op.rlaunch.ok) {
-          Res32Launch R = op.rlaunch;
-          if (op.temb_off >= 0) {
-            R.p.temb = rc.temb + op.temb_off;
-            R.p.t_dev = rc.t_dev;
-            R.p.temb_ld = u->temb_ld;
-            R.p.temb_bstride = rc.temb_bstride;
-          }
-          if (int e = res32_enqueue(R, st)) return e;
-          break;
-        }
-        if (op.plaunch.ok) {
-          PlaneLaunch L = op.plaunch;
-          if (op.temb_off >= 0) {
-            L.p.temb = rc.temb + op.temb_off;
-            L.p.t_dev = rc.t_dev;
-            L.p.temb_ld = u->temb_ld;
-            L.p.temb_bstride = rc.temb_bstride;
-          }
-          if (int e = plane_enqueue(L, st)) return e;
-          break;
-        }
-        ConvLaunch L = op.launch;
+        ConvRun r = op.fwd;
         if (op.temb_off >= 0) {
-          L.p.temb = rc.temb + op.temb_off;
-          L.p.t_dev = rc.t_dev;
-          L.p.temb_ld = u->temb_ld;
-          L.p.temb_bstride = rc.temb_bstride;
+          ConvEpilogue& ep = conv_run_epi(r);
+          ep.temb = rc.temb + op.temb_off;
+          ep.t_dev = rc.t_dev;
+          ep.temb_ld = u->temb_ld;
+          ep.temb_bstride = rc.temb_bstride;
         }
-        if (int e = conv_enqueue(L, st)) return e;
+        if (int e = conv_run_enqueue(r, st)) return e;
       } break;
       case OP_ATTN: {
         const Tens& q = u->tens[op.qkv];
@@ -856,7 +738,7 @@ int ensure_ready(cm_unet* u, int batch, int dup, cudaStream_t st) {
     u->packed2 = true;
   }
   if (int e = reserve(u, batch)) return e;
-  if (live_batch_of(u) != batch * dup || u->live_dup != dup) {
+  if (u->live_batch != batch || u->live_dup != dup) {
     if (u->graph_exec) {
       cudaGraphExecDestroy(u->graph_exec);
       u->graph_exec = nullptr;
@@ -1062,59 +944,32 @@ int prepare_train(cm_unet* u, int batch) {
     if (op.type != OP_CONV) continue;
     const Level& li = u->levels[op.in_level];
     const Level& lo = u->levels[u->tens[op.out].level];
-    // data gradient of the main source: a conv over dOut (geometry of the OUTPUT grid)
+    // data gradients: convs over dOut (geometry of the OUTPUT grid) into the fp32 gradients of the sources
     const int dup = u->dgrad_dup;
-    if (int rc = conv_prepare(&op.dlaunch, dgrad_mode_of(op.mode), u->g16[op.out], batch, lo.D, lo.H, lo.W,
-                              dup * op.cout, nullptr, 0, u->dpack + op.dpack_off, op.cin, u->cfg.weight_terms))
+    ConvEpilogue e{};
+    e.out32 = u->g32[op.in];
+    e.lo_from = dup == 2 ? op.cout : 0;
+    if (int rc = conv_run_prepare(&op.dgrad, CONV_UMMA | CONV_PLANE, dgrad_mode_of(op.mode), u->g16[op.out], batch, lo.D,
+                                  lo.H, lo.W, dup * op.cout, nullptr, 0, u->dpack + op.dpack_off, op.cin,
+                                  u->cfg.weight_terms, e))
       return rc;
-    op.dlaunch.p.out32 = u->g32[op.in];
-    op.dlaunch.p.lo_from = dup == 2 ? op.cout : 0;
-    op.dplaunch.ok = false;
-    if (op.mode == 0) {
-      if (int rc = plane_prepare(&op.dplaunch, u->g16[op.out], batch, lo.D, lo.H, lo.W, dup * op.cout, nullptr, 0,
-                                 u->dpack + op.dpack_off, op.cin, u->cfg.weight_terms))
-        return rc;
-      if (op.dplaunch.ok) {
-        op.dplaunch.p.out32 = u->g32[op.in];
-        op.dplaunch.p.lo_from = dup == 2 ? op.cout : 0;
-      }
-    }
     if (op.cin_extra) {
-      if (int rc = conv_prepare(&op.dxlaunch, 3, u->g16[op.out], batch, lo.D, lo.H, lo.W, dup * op.cout, nullptr, 0,
-                                u->dpack + op.dxpack_off, op.cin_extra, u->cfg.weight_terms))
+      e.out32 = u->g32[op.extra];
+      if (int rc = conv_run_prepare(&op.dgrad_x, CONV_UMMA, 3, u->g16[op.out], batch, lo.D, lo.H, lo.W, dup * op.cout,
+                                    nullptr, 0, u->dpack + op.dxpack_off, op.cin_extra, u->cfg.weight_terms, e))
         return rc;
-      op.dxlaunch.p.out32 = u->g32[op.extra];
-      op.dxlaunch.p.lo_from = dup == 2 ? op.cout : 0;
     }
-    const __half* extra = op.extra >= 0 ? u->tens[op.extra].p16 : nullptr;
     // activations / the 1x1 source: the hi halves of the forward's (hi|lo pair) rows
-    if (int rc = wgrad_prepare(&op.wlaunch, op.mode, u->tens[op.in].p16, batch, li.D, li.H, li.W, op.cin, extra,
-                               op.cin_extra, u->g16[op.out], op.cout, u->G + op.g_off, dup * op.cout,
-                               u->live_dup * op.cin, u->live_dup * op.cin_extra))
+    if (int rc = wgrad_run_prepare(&op.wgrad, CONV_UMMA | CONV_PLANE, op.mode, u->tens[op.in].p16, batch, li.D, li.H,
+                                   li.W, op.cin, op.extra >= 0 ? u->tens[op.extra].p16 : nullptr, op.cin_extra,
+                                   u->g16[op.out], op.cout, u->G + op.g_off, dup * op.cout, u->live_dup * op.cin,
+                                   u->live_dup * op.cin_extra))
       return rc;
-    op.n_wpl = 0;
-    if (op.mode == 0 && op.cout == 32 && op.cin % 32 == 0 && op.cin / 32 <= 4) {
-      const int nc = op.cin / 32;
-      bool ok = true;
-      for (int c = 0; c < nc && ok; ++c) {
-        if (int rc = wgrad_plane_prepare(&op.wpl[c], u->tens[op.in].p16, batch, li.D, li.H, li.W, op.cin, u->live_dup * op.cin,
-                                         c * 32, u->g16[op.out], dup * op.cout, op.cout, u->G + op.g_off))
-          return rc;
-        ok = op.wpl[c].ok;
-      }
-      if (ok && op.cin_extra) {
-        if (int rc = wgrad_prepare(&op.wxlaunch, 3, extra, batch, li.D, li.H, li.W, op.cin_extra, nullptr, 0, u->g16[op.out],
-                                   op.cout, u->G + op.g_off + (size_t)27 * op.cin * op.cout, dup * op.cout,
-                                   u->live_dup * op.cin_extra, 0))
-          return rc;
-      }
-      if (ok) op.n_wpl = nc;
-    }
   }
   // first conv: its operand is the packed fp16 input [pixels][32 (x live_dup)] of the forward (channels >= in_channels are
   // zero), so its weight gradient is one plane launch over the hi halves like any other 32 -> 32 layer
   u->first_wpl.ok = false;
-  if (u->first_plane.ok && u->cfg.base_channels == 32) {
+  if (u->first.covered() && u->cfg.base_channels == 32) {
     const Level& l0 = u->levels[0];
     const int out = u->ops[0].out;
     if (int rc = wgrad_plane_prepare(&u->first_wpl, u->tens[u->first_in].p16, batch, l0.D, l0.H, l0.W, 32, u->live_dup * 32, 0,
@@ -1253,33 +1108,21 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
           rs_tab.push_back((long long)op.cout);
           rs_tab.push_back((long long)u->grad_off[bidx]);
         }
-        if (op.dplaunch.ok) {
-          PlaneLaunch L = op.dplaunch;
-          L.p.resid = written[op.in] ? u->g32[op.in] : nullptr;   // accumulate in place
+        {
+          ConvRun r = op.dgrad;
+          conv_run_epi(r).resid = written[op.in] ? u->g32[op.in] : nullptr;   // accumulate in place
           written[op.in] = 1;
-          if (int e = plane_enqueue(L, st)) return e;
-        } else {
-          ConvLaunch L = op.dlaunch;
-          L.p.resid = written[op.in] ? u->g32[op.in] : nullptr;   // accumulate in place
-          written[op.in] = 1;
-          if (int e = conv_enqueue(L, st)) return e;
+          if (int e = conv_run_enqueue(r, st)) return e;
         }
         if (op.cin_extra) {
-          ConvLaunch L = op.dxlaunch;
-          L.p.resid = written[op.extra] ? u->g32[op.extra] : nullptr;
+          ConvRun r = op.dgrad_x;
+          conv_run_epi(r).resid = written[op.extra] ? u->g32[op.extra] : nullptr;
           written[op.extra] = 1;
-          if (int e = conv_enqueue(L, st)) return e;
+          if (int e = conv_run_enqueue(r, st)) return e;
           ++nl;
         }
-        if (op.n_wpl > 0) {
-          for (int c = 0; c < op.n_wpl; ++c)
-            if (int e = wgrad_plane_enqueue(op.wpl[c], st)) return e;
-          if (op.cin_extra)
-            if (int e = wgrad_enqueue(op.wxlaunch, st)) return e;
-          nl += op.n_wpl - 1 + (op.cin_extra ? 1 : 0);
-        } else if (int e = wgrad_enqueue(op.wlaunch, st)) {
-          return e;
-        }
+        if (int e = wgrad_run_enqueue(op.wgrad, st)) return e;
+        nl += op.wgrad.launches() - 1;
         // packed-K scratch -> nn.Conv3d weight layout: all convs in one launch after the op loop
         for (long long v : {(long long)op.mode, (long long)op.g_off, (long long)u->grad_off[op.w],
                             op.wx >= 0 ? (long long)u->grad_off[op.wx] : -1LL, (long long)op.cout, (long long)op.cin,
@@ -1487,8 +1330,7 @@ static int bind_one(cm_unet* u, int idx, const float* dev_ptr) {
       cudaGraphExecDestroy(u->graph_exec);
       u->graph_exec = nullptr;
     }
-    for (Op& op : u->ops)
-      if (op.type == OP_CONV) op.launch.p.M = 0;   // force prepare_convs (bias pointers)
+    u->live_batch = 0;   // force prepare_convs (bias pointers)
   }
   return 0;
 }
