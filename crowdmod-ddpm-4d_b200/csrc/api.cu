@@ -115,10 +115,10 @@ int cm_op_attn_core_backward(const float* qkv, const float* dctx, float* dqkv, i
                              void* stream) {
   if (int e = backward_init()) return e;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (S <= 128) return attn_core_backward_enqueue(qkv, dctx, dqkv, B, S, C, heads, st);
-  // the long-sequence backward reads the forward's row log-sum-exp: rerun the forward into temporaries
+  CM_CHECK(heads > 0 && C % heads == 0, "embed dim %d / heads %d unsupported", C, heads);
+  if (!attn_uses_long(S, C / heads)) return attn_core_backward_enqueue(qkv, dctx, dqkv, B, S, C, heads, st);
+  // the streaming backward reads the forward's row log-sum-exp: rerun the forward into temporaries
   if (int e = kernels_init()) return e;
-  CM_CHECK(C % heads == 0, "embed dim %d / heads %d unsupported", C, heads);
   __half* ctx = nullptr;
   float* lse = nullptr;      // [B][heads][S] log-sum-exp | [B][heads][S] backward row sums
   CM_CUDA(cudaMalloc(&ctx, (size_t)B * S * C * sizeof(__half)));

@@ -1,5 +1,6 @@
-// Attention core for sequences longer than 128 tokens (any S > 128; S <= 128 stays on attn_mma_kernel and
-// attn_core_backward_kernel).  Contracts in kernels.cuh (forward) and backward.cuh (backward).
+// Attention core for sequences longer than 128 tokens and for head dims above 64 (attn_uses_long in kernels.cuh; the
+// rest stays on attn_mma_kernel and attn_core_backward_kernel).  Contracts in kernels.cuh (forward) and backward.cuh
+// (backward).
 //
 // Forward (attn_long_kernel): one CTA per (128-query tile, sample * head); keys stream in tiles of 128 with the
 // online softmax (running max m and sum l per query row).  Numerics follow attn_mma_kernel:
@@ -8,15 +9,18 @@
 //           so the scores are in the log2 domain and each exponential is one ex2.approx.
 //   P . V   P = 2^(s - m) in [0, 1] and V as single fp16 operands, a second tcgen05 product with N = DHP.
 // Only the hi and lo halves are stored; the concatenation is three descriptor streams over them.  DHP is the head
-// dim padded to 16 / 32 / 64.
+// dim padded to 16 / 32 / 64 / 128.
 //   warps 0-3  softmax: thread t owns query row t (TMEM lane t); per key tile it reads the scores from TMEM twice
 //              (row max, then exponentials), writes P to shared memory, and folds the previous tile's P.V product
 //              into O (registers) as O = O * alpha + PV.  The Q tile is staged by these warps once.
 //   warps 4-5  producer: K and V rows (fp32) -> fp16 hi / lo K rows and V^T, 128-byte swizzled K-major, 2 stages.
+//              At DHP = 128 two K stages do not fit next to Q (227 KB): K has one buffer, refilled once S(j-1) is done
+//              (the s_full commit), and only V has two.
 //   warp  6    MMA issuer (one elected thread).
 // Per key tile j the issuer runs PV(j-1) then S(j) and commits once: that commit tells the softmax warps both that
 // S(j) is in TMEM and that PV(j-1) has finished reading P, so P and the PV columns are single-buffered.  256 TMEM
 // columns (S: 128, PV: DHP) let two CTAs share an SM at DHP <= 32, so one CTA's softmax overlaps the other's MMAs.
+// At DHP = 128 S and PV fill all 256 columns, and O (128 floats a row) stays in the softmax threads' registers.
 //
 // Backward: two deterministic fp32 SIMT kernels (no atomics) that recompute P = exp(s - lse) from qkv and the
 // forward's row log-sum-exp.  attn_long_dq_kernel walks one 64-query tile per CTA over all key tiles (twice: first the
@@ -41,7 +45,12 @@ struct AlCfg {
   static constexpr uint32_t V_BYTES = 2u * DHP * 128u;                      // V^T: 2 chunks of 64 keys x DHP rows
   static constexpr uint32_t P_BYTES = 2u * 128u * 128u;                     // 128 rows x 2 chunks of 64 keys
   static constexpr uint32_t STAGE_BYTES = K_BYTES + V_BYTES;
-  static constexpr uint32_t SMEM = 1024 + Q_BYTES + AL_STAGES * STAGE_BYTES + P_BYTES + 256;
+  static constexpr bool K_SOLO = DHP > 64;                                  // one K buffer, two V buffers
+  static constexpr uint32_t KV_BYTES = K_SOLO ? K_BYTES + AL_STAGES * V_BYTES : AL_STAGES * STAGE_BYTES;
+  static constexpr uint32_t SMEM = 1024 + Q_BYTES + KV_BYTES + P_BYTES + 256;
+  // stage s: K rows at s * K_STRIDE, V^T at s * V_STRIDE + K_BYTES in the K / V region
+  static constexpr uint32_t K_STRIDE = K_SOLO ? 0u : STAGE_BYTES;
+  static constexpr uint32_t V_STRIDE = K_SOLO ? V_BYTES : STAGE_BYTES;
 };
 
 // byte offset of element (row, col) in a K-major operand of `rows` rows stored as 64-column chunks with the 128-byte
@@ -79,7 +88,7 @@ attn_long_kernel(const float* __restrict__ qkv, __half* __restrict__ ctx, float*
   const uint32_t raw_addr = smem_u32(smem_raw);
   uint8_t* Qs = smem_raw + (((raw_addr + 1023u) & ~1023u) - raw_addr);
   uint8_t* KVs = Qs + Cfg::Q_BYTES;
-  uint8_t* Ps = KVs + AL_STAGES * Cfg::STAGE_BYTES;
+  uint8_t* Ps = KVs + Cfg::KV_BYTES;
   uint64_t* bars = reinterpret_cast<uint64_t*>(Ps + Cfg::P_BYTES);
   uint64_t* q_full = bars;                  // count 128: Q tile staged
   uint64_t* kv_full = bars + 1;             // [2] count 64: K / V stage written
@@ -229,8 +238,9 @@ attn_long_kernel(const float* __restrict__ qkv, __half* __restrict__ ctx, float*
     for (int j = 0; j < nkt; ++j) {
       const int s = j & 1;
       if (j >= AL_STAGES && !mbar_wait(&kv_empty[s], ((j >> 1) - 1) & 1, err, 603)) break;
-      uint8_t* Ks = KVs + s * Cfg::STAGE_BYTES;
-      uint8_t* Vt = Ks + Cfg::K_BYTES;
+      if (Cfg::K_SOLO && j > 0 && !mbar_wait(s_full, (j - 1) & 1, err, 608)) break;   // S(j-1) has read K
+      uint8_t* Ks = KVs + s * Cfg::K_STRIDE;
+      uint8_t* Vt = KVs + s * Cfg::V_STRIDE + Cfg::K_BYTES;
 #pragma unroll 4
       for (int idx = pt; idx < 128 * PAIRS; idx += 64) {
         const int key = idx / PAIRS, d = (idx - key * PAIRS) * 2;
@@ -260,7 +270,7 @@ attn_long_kernel(const float* __restrict__ qkv, __half* __restrict__ ctx, float*
     // descriptor offset (16-byte units) of column `col` in a 128-row [hi | lo] operand
     auto col_lo = [](int col) -> uint32_t { return ((static_cast<uint32_t>(col >> 6) * 128u * 128u) >> 4) + 2u * ((col & 63) >> 4); };
     auto issue_pv = [&](int jj) {                    // O(TMEM) = P . V(jj): 8 k16 steps over 128 keys
-      const uint32_t v_lo = kv_lo + (((jj & 1) * Cfg::STAGE_BYTES + Cfg::K_BYTES) >> 4);
+      const uint32_t v_lo = kv_lo + (((jj & 1) * Cfg::V_STRIDE + Cfg::K_BYTES) >> 4);
 #pragma unroll
       for (int k = 0; k < 8; ++k)
         umma_f16_lohi(t_o, p_lo + (((k >> 2) * 128u * 128u) >> 4) + 2 * (k & 3),
@@ -275,7 +285,7 @@ attn_long_kernel(const float* __restrict__ qkv, __half* __restrict__ ctx, float*
       tc_fence_after();
       if (elect_one()) {
         if (j > 0) issue_pv(j - 1);
-        const uint32_t k_lo = kv_lo + (((j & 1) * Cfg::STAGE_BYTES) >> 4);
+        const uint32_t k_lo = kv_lo + (((j & 1) * Cfg::K_STRIDE) >> 4);
 #pragma unroll
         for (int seg = 0; seg < 3; ++seg)            // [Qh | Ql | Qh] . [Kh | Kh | Kl]
 #pragma unroll
@@ -580,6 +590,7 @@ int attn_long_init() {
   if (int rc = al_attr<16>()) return rc;
   if (int rc = al_attr<32>()) return rc;
   if (int rc = al_attr<64>()) return rc;
+  if (int rc = al_attr<128>()) return rc;
   CM_CHECK(device_error_flag() != nullptr, "device error flag allocation failed");
   done = true;
   return 0;
@@ -590,7 +601,8 @@ int attn_long_enqueue(const float* qkv, __half* ctx, float* lse, int B, int S, i
   const int dh = C / heads;
   if (dh <= 16) return al_launch<16>(qkv, ctx, lse, B, S, C, heads, dup, st);
   if (dh <= 32) return al_launch<32>(qkv, ctx, lse, B, S, C, heads, dup, st);
-  return al_launch<64>(qkv, ctx, lse, B, S, C, heads, dup, st);
+  if (dh <= 64) return al_launch<64>(qkv, ctx, lse, B, S, C, heads, dup, st);
+  return al_launch<128>(qkv, ctx, lse, B, S, C, heads, dup, st);
 }
 
 int attn_long_backward_enqueue(const float* qkv, const float* dctx, const float* lse, float* dsum, float* dqkv, int B,
@@ -599,7 +611,8 @@ int attn_long_backward_enqueue(const float* qkv, const float* dctx, const float*
   const int dh = C / heads;
   if (dh <= 16) return al_bwd_launch<16>(a, B, st);
   if (dh <= 32) return al_bwd_launch<32>(a, B, st);
-  return al_bwd_launch<64>(a, B, st);
+  if (dh <= 64) return al_bwd_launch<64>(a, B, st);
+  return al_bwd_launch<128>(a, B, st);
 }
 
 }  // namespace cm

@@ -730,10 +730,11 @@ static size_t attn_bwd_smem(int S, int dh) {
 
 int attn_core_backward_enqueue(const float* qkv, const float* dctx, float* dqkv, int B, int S, int C,
                                int heads, cudaStream_t st, const float* lse, float* dsum) {
-  if (S > 128) {
-    CM_CHECK(C % heads == 0 && (C / heads) % 2 == 0 && C / heads <= 64, "attention: head dim %d / %d unsupported (even, <= 64)",
+  if (attn_uses_long(S, C / heads)) {
+    CM_CHECK(C % heads == 0 && (C / heads) % 2 == 0 && C / heads <= 128, "attention: head dim %d / %d unsupported (even, <= 128)",
              C, heads);
-    CM_CHECK(lse && dsum, "attention backward at S=%d > 128 needs the forward's log-sum-exp and a row-sum workspace", S);
+    CM_CHECK(lse && dsum, "attention backward at S=%d, dh=%d needs the forward's log-sum-exp and a row-sum workspace", S,
+             C / heads);
     return attn_long_backward_enqueue(qkv, dctx, lse, dsum, dqkv, B, S, C, heads, st);
   }
   CM_CHECK(C % heads == 0 && (C / heads) % 4 == 0 && C % 4 == 0, "embed dim %d / heads %d unsupported", C, heads);
@@ -941,14 +942,18 @@ pack_final_dout_kernel(const float* __restrict__ deps, const float* __restrict__
   }
 }
 
-// dout16 != nullptr: the weight gradient is left to the caller's plane launch over dout16 (filled here, with the bias
-// gradient); nullptr: the SIMT weight-gradient kernel
+constexpr int FCB_MAX_CIN = 256;   // the data-gradient kernel keeps all 27 * cin * cout weights in shared memory
+
+// dout16 != nullptr: the weight gradient is left to the caller's launch over dout16 (filled here, with the bias
+// gradient); nullptr: the SIMT weight-gradient kernel (cin <= 64)
 int final_conv_backward_enqueue(const float* deps, const float* scale_dev, const __half* act, int act_ld, int act_lo,
                                 const float* w, float* dact, float* dw, float* db, int B, int H, int W,
                                 int L, int P, int cin, int cout, __half* dout16, cudaStream_t st) {
   const int ald = act_ld > 0 ? act_ld : cin;
   CM_CHECK(cout >= 1 && cout <= 4, "final conv supports 1..4 output channels (got %d)", cout);
-  CM_CHECK(cin % 32 == 0 && 27 * cin <= 2048, "final conv backward: cin must be a multiple of 32, <= 64");
+  CM_CHECK(cin % 32 == 0 && cin <= FCB_MAX_CIN && (dout16 || 27 * cin <= 2048),
+           "final conv backward: cin %d must be a multiple of 32, <= 64 (<= %d with the packed weight gradient)", cin,
+           FCB_MAX_CIN);
   const size_t total = (size_t)B * L * H * W * (cin / 8);
   const int blocks = grid_for(total, 256, 148 * 16);
   const size_t smem = (size_t)27 * cin * cout * sizeof(float);
@@ -1246,10 +1251,11 @@ int backward_init() {
   if (done) return 0;
   CM_CUDA(cudaFuncSetAttribute(attn_core_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                227 * 1024));
-  CM_CUDA(cudaFuncSetAttribute(final_conv_dact_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
-  CM_CUDA(cudaFuncSetAttribute(final_conv_dact_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
-  CM_CUDA(cudaFuncSetAttribute(final_conv_dact_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
-  CM_CUDA(cudaFuncSetAttribute(final_conv_dact_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+  constexpr int fcb_smem = 27 * FCB_MAX_CIN * 4 * sizeof(float);
+  CM_CUDA(cudaFuncSetAttribute(final_conv_dact_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, fcb_smem));
+  CM_CUDA(cudaFuncSetAttribute(final_conv_dact_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, fcb_smem));
+  CM_CUDA(cudaFuncSetAttribute(final_conv_dact_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, fcb_smem));
+  CM_CUDA(cudaFuncSetAttribute(final_conv_dact_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, fcb_smem));
   if (int rc = wgrad_init()) return rc;
   done = true;
   return 0;

@@ -77,8 +77,8 @@ int gn_backward_params_all_enqueue(const float* chsum_base, const long long* tab
                                    cudaStream_t st);
 
 // ---- attention core backward (layers.py:16): qkv fp32 [B*S][3C] saved by the forward,
-//      dctx fp32 [B*S][C] -> dqkv fp32 [B*S][3C] (=).  S <= 128: one fp32 CTA per (sample, head) with the S x S tile in
-//      shared memory (lse / dsum unused).  S > 128 (attn_long.cu): two deterministic kernels that recompute P from qkv
+//      dctx fp32 [B*S][C] -> dqkv fp32 [B*S][3C] (=).  One fp32 CTA per (sample, head) with the S x S tile in shared
+//      memory (lse / dsum unused), unless attn_uses_long(S, dh) (attn_long.cu): two deterministic kernels that recompute P from qkv
 //      and lse (fp32 [B][heads][S], the row log-sum-exp attn_core_enqueue wrote); dsum (fp32 [B][heads][S]) is their
 //      workspace for the row sums D_i = sum_j P_ij dP_ij. ----
 int attn_core_backward_enqueue(const float* qkv, const float* dctx, float* dqkv, int B, int S, int C,
@@ -89,6 +89,8 @@ int attn_long_backward_enqueue(const float* qkv, const float* dctx, const float*
 // ---- final conv backward (unet.py:121,165-167): deps API layout [B][cout][H][W][F], times *scale;
 //      dact (=) fp32 [B][L][H][W][cin]; dw [cout][cin][27] / db [cout] accumulated with atomics ----
 // act: fp16 [B][L][H][W][act_ld] (act_ld 0 -> cin); act_lo > 0: hi|lo pair rows, the lo half is added
+// dout16 != nullptr: dw is left to the caller, which runs a conv weight gradient over dout16 (fp16 [B][L][H][W][32],
+// d_eps * scale in columns 0 .. cout-1); cin <= 64 without it, <= 256 with it
 int final_conv_backward_enqueue(const float* deps, const float* scale_dev, const __half* act, int act_ld, int act_lo,
                                 const float* w, float* dact, float* dw, float* db, int B, int H, int W,
                                 int L, int P, int cin, int cout, __half* dout16, cudaStream_t st);

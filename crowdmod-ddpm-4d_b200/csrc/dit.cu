@@ -376,8 +376,8 @@ void reserve_pack(cm_dit* u, DitLinear& l, int cin_packed) {
 int build(cm_dit* u) {
   const cm_dit_config& c = u->cfg;
   CM_CHECK(c.in_channels >= 1 && c.in_channels <= 4 && c.out_channels >= 1 && c.out_channels <= 4, "in/out channels must be in 1..4");
-  CM_CHECK(c.hidden % 32 == 0 && c.hidden % c.heads == 0 && c.hidden / c.heads <= 64 && (c.hidden / c.heads) % 2 == 0,
-           "hidden size %d / heads %d unsupported (hidden %% 32 == 0, head dim even and <= 64)", c.hidden, c.heads);
+  CM_CHECK(c.hidden % 32 == 0 && c.hidden % c.heads == 0 && c.hidden / c.heads <= 128 && (c.hidden / c.heads) % 2 == 0,
+           "hidden size %d / heads %d unsupported (hidden %% 32 == 0, head dim even and <= 128)", c.hidden, c.heads);
   CM_CHECK(c.rows % c.patch == 0 && c.cols % c.patch == 0, "grid %dx%d not divisible by the patch size %d (DiT4D_V4.py:26-29)", c.rows,
            c.cols, c.patch);
   const int T = c.past_len + c.future_len;

@@ -1438,8 +1438,8 @@ int attn_core_enqueue(const float* qkv, __half* ctx, int B, int S, int C, int he
   CM_CHECK(dup == 1 || dup == 2, "attention: dup must be 1 or 2");
   CM_CHECK(C % heads == 0, "embed dim %d / heads %d unsupported", C, heads);
   const int dh = C / heads;
-  CM_CHECK(dh % 2 == 0 && dh <= 64, "attention: head dim %d unsupported (even, <= 64)", dh);
-  if (S > 128) return attn_long_enqueue(qkv, ctx, lse, B, S, C, heads, dup, st);
+  CM_CHECK(dh % 2 == 0 && dh <= 128, "attention: head dim %d unsupported (even, <= 128)", dh);
+  if (attn_uses_long(S, dh)) return attn_long_enqueue(qkv, ctx, lse, B, S, C, heads, dup, st);
   if (dh <= 16) return attn_dispatch<16>(qkv, ctx, B, S, C, heads, dup, st);
   if (dh <= 32) return attn_dispatch<32>(qkv, ctx, B, S, C, heads, dup, st);
   return attn_dispatch<64>(qkv, ctx, B, S, C, heads, dup, st);

@@ -108,10 +108,12 @@ int temb_enqueue(const TembParams& p, cudaStream_t st);
 
 // ---- attention core softmax(QK^T/sqrt(dh))V per (sample, head) (layers.py:16) ----
 // qkv: fp32 [B*S][3*C] (q | k | v), ctx: fp16 [B*S][dup*C] (dup = 2: hi | lo pair per token).  Any S; dh = C / heads
-// even and <= 64.  S <= 128: attn_mma_kernel (whole score row in registers); S > 128: attn_long_kernel (attn_long.cu,
-// keys streamed with the online softmax), which also writes the row log-sum-exp of the scaled scores to lse (fp32
-// [B][heads][S]) when lse is given: the long-sequence backward recomputes P from it.  Capturable (no allocation, no
-// synchronisation).
+// even and <= 128.  attn_uses_long(S, dh): attn_long_kernel (attn_long.cu, keys streamed with the online softmax), which
+// also writes the row log-sum-exp of the scaled scores to lse (fp32 [B][heads][S]) when lse is given: the streaming
+// backward recomputes P from it.  Otherwise attn_mma_kernel (whole score row in registers).  Capturable (no
+// allocation, no synchronisation).
+// The one test of which kernels an attention core uses; the training plans size their lse slices by it.
+inline bool attn_uses_long(int S, int dh) { return S > 128 || dh > 64; }
 int attn_core_enqueue(const float* qkv, __half* ctx, int B, int S, int C, int heads,
                       cudaStream_t st, int dup = 1, float* lse = nullptr);
 int attn_long_enqueue(const float* qkv, __half* ctx, float* lse, int B, int S, int C, int heads, int dup,

@@ -97,11 +97,11 @@ struct cm_unet {
   int first_in = -1;
   size_t first_wpack_off = 0;
   ConvRun first;
-  WgradPlaneLaunch first_wpl;          // first conv's weight gradient through the plane / halo kernel (base_channels == 32)
-  size_t first_g_off = 0;              // its packed-K scratch (27 taps x 32 packed channels x 32) and channel-sum slot
+  WgradRun first_wg;                   // first conv's weight gradient over the packed operand (edge_wgrad_kinds)
+  size_t first_g_off = 0;              // its packed-K scratch (27 taps x 32 packed channels x base) and channel-sum slot
   int first_colsum_off = 0;
-  WgradPlaneLaunch final_wpl;          // final conv's weight gradient the same way: d_eps packed into 32 fp16 columns
-  size_t final_g_off = 0;
+  WgradRun final_wg;                   // final conv's weight gradient the same way: d_eps packed into 32 fp16 columns
+  size_t final_g_off = 0;              // its packed-K scratch (27 taps x cin x 32)
   __half* final_d16 = nullptr;         // [B * L * H * W][32]: columns >= out_channels and past frames stay zero
   // device state
   __half* wpack = nullptr;
@@ -166,7 +166,7 @@ struct cm_unet {
   std::vector<size_t> grad_off;         // flat gradient buffer: offset of parameter i
   size_t grad_total = 0;
   int train_reserved = 0, train_prepared = 0;
-  std::vector<float*> attn_lse;         // per op, attention core with S > 128: row log-sum-exp [B][heads][S], then as
+  std::vector<float*> attn_lse;         // per op, attention core with attn_uses_long: row log-sum-exp [B][heads][S], then as
                                         // many floats of backward workspace (reserve_train)
   uint8_t* tarena = nullptr;
   size_t tarena_bytes = 0;
@@ -340,6 +340,11 @@ int add_resblock(cm_unet* u, const std::string& prefix, int src0, int src1, int 
   return o;
 }
 
+// Which kernels may take the weight gradient of the first conv (c = its cout) or the final conv (c = its cin) as a conv
+// weight gradient over the packed fp16 operands (wgrad_run).  0: the SIMT kernels of backward.cu, which cover 32 and 64
+// channels; 64 keeps them, 32 takes the plane kernel, wider layers the plane chunks or wgrad_umma.
+unsigned edge_wgrad_kinds(int c) { return c == 32 ? CONV_PLANE : c == 64 ? 0u : CONV_UMMA | CONV_PLANE; }
+
 int build_plan(cm_unet* u) {
   const cm_unet_config& c = u->cfg;
   CM_CHECK(c.num_levels >= 1 && c.num_levels <= CM_MAX_LEVELS, "num_levels out of range");
@@ -432,7 +437,7 @@ int build_plan(cm_unet* u) {
   fin.cin = in_ch;
   u->ops.push_back(fin);
   u->final_g_off = u->g_elems;
-  u->g_elems += (size_t)27 * 32 * 32;
+  u->g_elems += (size_t)27 * (edge_wgrad_kinds(in_ch) ? in_ch : 32) * 32;
 
   // algorithmic FLOPs per sample of the reference graph (dense formulation: 27-tap upsample
   // convs, separate 1x1 match_input, attention), SURVEY.md §8(d)
@@ -686,7 +691,7 @@ int run_ops(cm_unet* u, RunCtx& rc, cudaStream_t st, int64_t* launches,
       case OP_ATTN: {
         const Tens& q = u->tens[op.qkv];
         const int S = u->levels[q.level].pps();
-        float* lse = rc.train && oi < u->attn_lse.size() ? u->attn_lse[oi] : nullptr;   // S > 128: kept for the backward
+        float* lse = rc.train && oi < u->attn_lse.size() ? u->attn_lse[oi] : nullptr;   // streaming path: kept for the backward
         if (int e = attn_core_enqueue(q.p32, u->tens[op.ctx].p16, rc.batch, S, u->tens[op.ctx].C,
                                       op.heads, st, rc.dup, lse))
           return e;
@@ -794,7 +799,8 @@ int reserve_train(cm_unet* u, int batch) {
     const Op& op = u->ops[i];
     if (op.type != OP_ATTN) continue;
     const size_t S = u->levels[u->tens[op.qkv].level].pps();
-    if (S > 128) o_lse[i] = take((size_t)2 * batch * op.heads * S * 4);   // lse | backward row sums
+    if (attn_uses_long((int)S, u->tens[op.ctx].C / op.heads))
+      o_lse[i] = take((size_t)2 * batch * op.heads * S * 4);   // lse | backward row sums
   }
   CM_CUDA(cudaMalloc(&u->tarena, off));
   CM_CUDA(cudaMemset(u->tarena, 0, off));
@@ -967,21 +973,23 @@ int prepare_train(cm_unet* u, int batch) {
       return rc;
   }
   // first conv: its operand is the packed fp16 input [pixels][32 (x live_dup)] of the forward (channels >= in_channels are
-  // zero), so its weight gradient is one plane launch over the hi halves like any other 32 -> 32 layer
-  u->first_wpl.ok = false;
-  if (u->first.covered() && u->cfg.base_channels == 32) {
+  // zero), so its weight gradient is a conv weight gradient over the hi halves like any other layer with cin = 32
+  const int base = u->cfg.base_channels;
+  u->first_wg = WgradRun{};
+  if (u->first.covered() && edge_wgrad_kinds(base)) {
     const Level& l0 = u->levels[0];
     const int out = u->ops[0].out;
-    if (int rc = wgrad_plane_prepare(&u->first_wpl, u->tens[u->first_in].p16, batch, l0.D, l0.H, l0.W, 32, u->live_dup * 32, 0,
-                                     u->g16[out], u->dgrad_dup * 32, 32, u->G + u->first_g_off))
+    if (int rc = wgrad_run_prepare(&u->first_wg, edge_wgrad_kinds(base), 0, u->tens[u->first_in].p16, batch, l0.D, l0.H,
+                                   l0.W, 32, nullptr, 0, u->g16[out], base, u->G + u->first_g_off, u->dgrad_dup * base,
+                                   u->live_dup * 32))
       return rc;
   }
-  u->final_wpl.ok = false;
-  if (u->ops.back().type == OP_FINAL && u->ops.back().cin == 32) {
+  u->final_wg = WgradRun{};
+  if (u->ops.back().type == OP_FINAL && edge_wgrad_kinds(u->ops.back().cin)) {
     const Level& l0 = u->levels[0];
     const Op& fo = u->ops.back();
-    if (int rc = wgrad_plane_prepare(&u->final_wpl, u->tens[fo.in].p16, batch, l0.D, l0.H, l0.W, 32, u->live_dup * 32, 0,
-                                     u->final_d16, 32, 32, u->G + u->final_g_off))
+    if (int rc = wgrad_run_prepare(&u->final_wg, edge_wgrad_kinds(fo.cin), 0, u->tens[fo.in].p16, batch, l0.D, l0.H, l0.W,
+                                   fo.cin, nullptr, 0, u->final_d16, 32, u->G + u->final_g_off, 32, u->live_dup * fo.cin))
       return rc;
   }
   u->train_prepared = batch;
@@ -1033,15 +1041,15 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
         if (int e = final_conv_backward_enqueue(d_eps, u->loss_scale, u->tens[op.in].p16, u->live_dup * op.cin,
                                                 u->live_dup == 2 ? op.cin : 0, u->params[u->p_final_w].ptr, u->g32[op.in], gp(u->p_final_w),
                                                 gp(u->p_final_b), B, l0.H, l0.W, l0.D, c.past_len, op.cin,
-                                                c.out_channels, u->final_wpl.ok ? u->final_d16 : nullptr, st))
+                                                c.out_channels, u->final_wg.launches() ? u->final_d16 : nullptr, st))
           return e;
-        if (u->final_wpl.ok) {
-          if (int e = wgrad_plane_enqueue(u->final_wpl, st)) return e;
-          // G is (tap, 32 channels) x 32 packed columns: G's cout in the upper half of the cout entry
+        if (u->final_wg.launches()) {
+          if (int e = wgrad_run_enqueue(u->final_wg, st)) return e;
+          // G is (tap, cin) x 32 packed columns: G's cout in the upper half of the cout entry
           for (long long v : {0LL, (long long)u->final_g_off, (long long)u->grad_off[u->p_final_w], -1LL,
                               (long long)c.out_channels | (32LL << 16), (long long)op.cin, 0LL, 1LL})
             up_tab.push_back(v);
-          ++nl;
+          nl += u->final_wg.launches();
         }
         written[op.in] = 1;
         nl += 2;
@@ -1142,7 +1150,7 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
       } break;
       case OP_FIRST: {
         CM_CHECK(written[op.out], "backward: gradient of the first conv output missing");
-        if (u->first_wpl.ok) {
+        if (u->first_wg.launches()) {
           float* cs = u->colsum + (size_t)B * u->first_colsum_off;
           if (int e = cast_colsum_enqueue(u->g32[op.out], u->g16[op.out], u->dgrad_dup, nullptr, 0, cs, c.base_channels, B,
                                           l0.pps(), c.base_channels, st))
@@ -1151,12 +1159,12 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
           rs_tab.push_back((long long)c.base_channels);
           rs_tab.push_back((long long)c.base_channels);
           rs_tab.push_back((long long)u->grad_off[u->p_first_b]);
-          if (int e = wgrad_plane_enqueue(u->first_wpl, st)) return e;
+          if (int e = wgrad_run_enqueue(u->first_wg, st)) return e;
           // G rows are (tap, 32 packed channels): cin of G in the upper half of the cin entry
           for (long long v : {0LL, (long long)u->first_g_off, (long long)u->grad_off[u->p_first_w], -1LL,
                               (long long)c.base_channels, (long long)c.in_channels | (32LL << 16), 0LL, 1LL})
             up_tab.push_back(v);
-          ++nl;
+          nl += u->first_wg.launches();
         } else if (int e = first_conv_wgrad_enqueue(u->live_future, u->live_past, u->g32[op.out], gp(u->p_first_w),
                                                     gp(u->p_first_b), B, l0.H, l0.W, c.past_len, c.future_len,
                                                     c.in_channels, c.base_channels, st)) {
