@@ -165,7 +165,14 @@ class DDPM_model:
         """One process per GPU, global batch split over the ranks: broadcasts rank 0's parameters so every
         replica starts from the same model, then averages the flat gradient buffer with ONE all-reduce per
         step.  The epoch loss is averaged over ranks before ReduceLROnPlateau / best-checkpoint decisions, the
-        random extra-checkpoint epochs are drawn on rank 0, and only rank 0 writes checkpoints."""
+        random extra-checkpoint epochs are drawn on rank 0, and only rank 0 writes checkpoints.
+
+        Sampling is sharded too: every reverse chain (``_generate_ddpm`` / ``_generate_ddim``, hence ``sampling``
+        and ``generate_metrics``) takes x_T, ``past``, the noise seed (or the ``noise_source`` noise) from rank 0,
+        runs this rank's contiguous slice of the samples (``shard_samples``) and all-gathers x_0 (and the history)
+        back to every rank.  The Philox noise is keyed by the global sample index, so x_0 is the single-GPU chain
+        that rank 0's inputs give, up to the fp32 summation order of a smaller batch, whatever the other ranks'
+        RNG state or data order.  Only rank 0 plots, computes metrics and writes files."""
         import torch.distributed as dist
         from ..backbones.unet_autograd import enable_data_parallel
         if not (dist.is_available() and dist.is_initialized()):
@@ -291,16 +298,74 @@ class DDPM_model:
             noise = self.noise_source(nsteps, tuple(x.shape), x.device).contiguous()
         else:
             seed = int(torch.randint(0, 2 ** 62, (1,)).item())   # consumes torch's generator once
+        if self._sharded():
+            hist = self._sharded_chain(past, x, tsteps, coef, mode, history, noise, seed)
+        else:
+            hist = None
+            if history:
+                hist = torch.empty((nsteps + 1,) + tuple(x.shape), device=x.device, dtype=torch.float32)
+                hist[0].copy_(x)
+            self.denoiser.sample_chain(past, x, tsteps, coef, mode=mode, noise=noise, seed=seed,
+                                       sample_offset=self.sample_offset, history=hist,
+                                       use_graph=self.use_cuda_graph)
+        if self.device.type == "cuda":
+            from ..backbones.unet import _native
+            _native().check_device_error("the reverse chain")     # synchronises: x_0 is about to be read anyway
+        return hist
+
+    # ------------------------------------------------------------------ sharded sampling (enable_data_parallel)
+    def _sharded(self):
+        return self.data_parallel and self.world > 1
+
+    def _from_rank0(self, t):
+        """The group's rank 0's value of ``t`` on every rank: a contiguous copy on the receiving ranks, so that the
+        caller's tensor is never overwritten."""
+        import torch.distributed as dist
+        buf = t.contiguous() if self.rank == 0 else torch.empty(t.shape, dtype=t.dtype, device=t.device)
+        src = dist.get_global_rank(self.dp_group, 0) if self.dp_group is not None else 0
+        dist.broadcast(buf, src=src, group=self.dp_group)
+        return buf
+
+    def _gather_samples(self, part, n, dim):
+        """Every rank's ``shard_samples`` slice of a sample axis (``dim``) concatenated in rank order, on every rank.
+        The shards can differ by one sample: each is padded to the largest so that ONE all_gather_into_tensor
+        moves them all, and the padding is trimmed afterwards."""
+        import torch.distributed as dist
+        sizes = [hi - lo for lo, hi in (shard_samples(n, r, self.world) for r in range(self.world))]
+        shape = list(part.shape)
+        shape[dim] = sizes[0]
+        buf = part
+        if part.shape[dim] != sizes[0]:
+            buf = part.new_zeros(shape)
+            buf.narrow(dim, 0, part.shape[dim]).copy_(part)
+        out = part.new_empty([self.world * shape[0]] + shape[1:])     # gloo accepts only the concatenated form
+        dist.all_gather_into_tensor(out, buf, group=self.dp_group)
+        out = out.view([self.world] + shape)
+        return torch.cat([out[r].narrow(dim, 0, s) for r, s in enumerate(sizes)], dim)
+
+    def _sharded_chain(self, past, x, tsteps, coef, mode, history, noise, seed):
+        """``_chain`` over the data-parallel group.  ``x`` (x_T) already holds rank 0's draw; ``past``, the seed and
+        the injected noise are taken from rank 0 too, so the result does not depend on the other ranks' RNG state
+        or data order.  This rank runs its slice [lo, hi) of the samples with Philox offset ``sample_offset + lo``,
+        then x_0 (in place in ``x``) and the history are gathered back to the full batch."""
+        past = self._from_rank0(past)
+        seed = int(self._from_rank0(torch.tensor([seed], dtype=torch.int64, device=x.device)).item())
+        if noise is not None:
+            noise = self._from_rank0(noise)
+        n = x.shape[0]
+        lo, hi = shard_samples(n, self.rank, self.world)
+        mine = x[lo:hi]                  # a contiguous view: the chain runs in place on the caller's x
         hist = None
         if history:
-            hist = torch.empty((nsteps + 1,) + tuple(x.shape), device=x.device, dtype=torch.float32)
-            hist[0].copy_(x)
-        self.denoiser.sample_chain(past, x, tsteps, coef, mode=mode, noise=noise, seed=seed,
-                                   sample_offset=self.sample_offset, history=hist,
-                                   use_graph=self.use_cuda_graph)
-        from ..backbones.unet import _native
-        _native().check_device_error("the reverse chain")     # synchronises: x_0 is about to be read anyway
-        return hist
+            hist = torch.empty((tsteps.numel() + 1,) + tuple(mine.shape), device=x.device, dtype=torch.float32)
+            hist[0].copy_(mine)
+        if hi > lo:                      # with n < world some ranks hold no sample (cm_dit_sample rejects n = 0)
+            self.denoiser.sample_chain(past[lo:hi], mine, tsteps, coef, mode=mode,
+                                       noise=noise[:, lo:hi].contiguous() if noise is not None else None, seed=seed,
+                                       sample_offset=self.sample_offset + lo, history=hist,
+                                       use_graph=self.use_cuda_graph)
+        x.copy_(self._gather_samples(mine, n, 0))
+        return self._gather_samples(hist, n, 1) if history else None
 
     def _guidance(self):
         g = self.cfg.MODEL.DDPM.GUIDANCE
@@ -309,11 +374,15 @@ class DDPM_model:
                                       "(SURVEY.md §2 #6)")
         return g, (self.cfg.MODEL.DDPM.LAMBDA_GUIDANCE if g == "Sparsity" else 0.0)
 
+    def _x_T(self, nsamples):
+        x = torch.randn((nsamples, self.mprops_count, self.cfg.MACROPROPS.ROWS,
+                         self.cfg.MACROPROPS.COLS, self.cfg.DATASET.FUTURE_LEN), device=self.device)
+        return self._from_rank0(x) if self._sharded() else x
+
     @torch.inference_mode()
     def _generate_ddpm(self, past: torch.Tensor, backward_sampler: DDPM, nsamples, history=False):
         self.denoiser.eval()
-        xnoisy = torch.randn((nsamples, self.mprops_count, self.cfg.MACROPROPS.ROWS,
-                              self.cfg.MACROPROPS.COLS, self.cfg.DATASET.FUTURE_LEN), device=self.device)
+        xnoisy = self._x_T(nsamples)
         x_T = xnoisy.clone()
         guidance, lam = self._guidance()
         tsteps, coef = ddpm_coefficients(backward_sampler, guidance, lam)
@@ -325,8 +394,7 @@ class DDPM_model:
     def _generate_ddim(self, past: torch.Tensor, taus, backward_sampler: DDPM, nsamples, history=False):
         self.denoiser.eval()
         sigma_t = self.cfg.MODEL.DDPM.SIGMA
-        xnoisy = torch.randn((nsamples, self.mprops_count, self.cfg.MACROPROPS.ROWS,
-                              self.cfg.MACROPROPS.COLS, self.cfg.DATASET.FUTURE_LEN), device=self.device)
+        xnoisy = self._x_T(nsamples)
         x_T = xnoisy.clone()
         guidance, lam = self._guidance()
         tsteps, coef = ddim_coefficients(backward_sampler, taus, sigma_t, guidance, lam)
@@ -357,7 +425,9 @@ class DDPM_model:
     def sampling(self, batched_test_data, plotType, model_fullname, plotMprop, plotPast, samePastSeq,
                  macropropPlotter):
         logging.info(f'model full name:{model_fullname}')
-        create_directory(self.output_dir)
+        writer = (not self.data_parallel) or self.rank == 0
+        if writer:
+            create_directory(self.output_dir)
         self._load(model_fullname)
         backward_sampler = DDPM(timesteps=self.cfg.MODEL.DDPM.TIMESTEPS, scale=self.cfg.MODEL.DDPM.SCALE)
         backward_sampler.to(self.device)
@@ -380,6 +450,8 @@ class DDPM_model:
             random_past_samples = past_test[random_past_idx]
             random_future_samples = future_test[random_past_idx]
             predictions = self._predict(random_past_samples, backward_sampler, nsamples)
+            if not writer:
+                return predictions
             try:
                 from utils.plot.plot_sampled_mprops import setup_predictions_plot
                 setup_predictions_plot(predictions, random_past_idx, random_past_samples,
@@ -393,7 +465,9 @@ class DDPM_model:
     def generate_metrics(self, batched_test_data, chunkRepdPastSeq, metric, batches_to_use,
                          samples_per_batch, model_fullname, output_dir):
         logging.info(f'model full name:{model_fullname}')
-        create_directory(self.output_dir)
+        writer = (not self.data_parallel) or self.rank == 0
+        if writer:
+            create_directory(self.output_dir)
         self._load(model_fullname)
         match = re.search(r'TE\d+_PL\d+_FL\d+_CE\d+_NA', model_fullname)
         backward_sampler = DDPM(timesteps=self.cfg.MODEL.DDPM.TIMESTEPS, scale=self.cfg.MODEL.DDPM.SCALE)
@@ -413,6 +487,8 @@ class DDPM_model:
             random_past_idx = torch.repeat_interleave(random_past_idx, chunkRepdPastSeq)[:samples_per_batch]
             random_past_samples = past_test[random_past_idx]
             random_future_samples = future_test[random_past_idx]
+            if self._sharded():          # every rank returns the (prediction, ground truth) pairs rank 0 scores
+                random_future_samples = self._from_rank0(random_future_samples)
             x = self._predict(random_past_samples, backward_sampler, samples_per_batch)
             for i in range(len(random_past_idx)):
                 pred_seq_list.append(x[i])
@@ -420,6 +496,8 @@ class DDPM_model:
             count_batch += 1
             if count_batch == batches_to_use:
                 break
+        if not writer:
+            return pred_seq_list, gt_seq_list
         logging.info("===" * 20)
         logging.info(f'Computing metrics on predicted mprops sequences with {self.arch} model.')
         # reduction metrics (PSNR / MASK_PSNR / RE_DENSITY / TV) on the device in one launch; SSIM, the motion-feature
