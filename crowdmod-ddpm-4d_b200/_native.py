@@ -127,6 +127,19 @@ SIGNATURES = {
     "cm_op_final_conv": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
                                    C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                    C.c_void_p]),
+    "cm_op_gn_backward": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int] + [C.c_void_p] * 6
+                          + [C.c_int] * 4 + [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
+                                             C.c_int, C.c_void_p]),
+    "cm_op_cast_colsum": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p,
+                                    C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "cm_op_rowsum_all": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64), C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "cm_op_final_conv_backward": (C.c_int, [C.c_void_p, C.c_float, C.c_void_p, C.c_int, C.c_int] + [C.c_void_p] * 4
+                                  + [C.c_int] * 7 + [C.c_void_p, C.c_void_p]),
+    "cm_op_first_conv_wgrad": (C.c_int, [C.c_void_p] * 5 + [C.c_int] * 7 + [C.c_void_p]),
+    "cm_op_temb_backward": (C.c_int, [C.c_void_p] * 4 + [C.c_int] * 4
+                            + [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_int,
+                               C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64)] + [C.c_void_p] * 7),
+    "cm_op_loss_scale": (C.c_int, [C.c_void_p, C.c_int64, C.c_float, C.c_void_p, C.c_void_p]),
     "cm_dit_create": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p)]),
     "cm_dit_destroy": (C.c_int, [C.c_void_p]),
     "cm_dit_param_count": (C.c_int, [C.c_void_p]),

@@ -1203,9 +1203,9 @@ __global__ void temb_dense_dgrad_kernel(const float* __restrict__ dtemb, int ld,
 int temb_dense_backward_enqueue(const float* dtemb, int ld, int B, const float* s2, int E, const float* const* wd,
                                 const int* couts, const int* offs, int nblocks, float* grads,
                                 const long long* goff_w, const long long* goff_b, float* ds2, cudaStream_t st) {
+  CM_CHECK(E <= 1024, "time-embedding width %d > 1024 unsupported", E);
   temb_dense_wgrad_kernel<<<dim3((E + 127) / 128, ld), 128, 0, st>>>(dtemb, ld, B, s2, E, couts, offs, nblocks, grads,
                                                                     goff_w, goff_b);
-  CM_CHECK(E <= 1024, "time-embedding width %d > 1024 unsupported", E);
   int G = 1024 / E;
   if (G > 8) G = 8;
   if (G > nblocks) G = nblocks;
@@ -1244,6 +1244,24 @@ int scale_inplace_enqueue(float* x, size_t n, const float* factor_dev, cudaStrea
   scale_inplace_kernel<<<grid_for(n, 256, 2048), 256, 0, st>>>(x, n, factor_dev);
   CM_CUDA(cudaGetLastError());
   return 0;
+}
+
+int temb_backward_enqueue(const TembBwdParams& p, float* grads, cudaStream_t st) {
+  const int B = p.B, E = p.E;
+  const size_t nE = (size_t)B * E;
+  if (int e = silu_forward_enqueue(p.h1, p.s1, nE, st)) return e;
+  if (int e = silu_forward_enqueue(p.h2, p.s2, nE, st)) return e;
+  // (dense_1.bias gradient == the batch sum of dtemb; the conv_1 bias gradient is the same sum)
+  if (int e = temb_dense_backward_enqueue(p.dtemb, p.ld, B, p.s2, E, p.wd, p.couts, p.offs, p.nblocks, grads, p.goff_w,
+                                          p.goff_b, p.ds2, st))
+    return e;
+  if (int e = silu_backward_enqueue(p.h2, p.ds2, p.dh2, nE, st)) return e;
+  if (int e = rowsum_enqueue(p.dh2, p.db2, B, E, E, 0, st)) return e;
+  if (int e = small_gemm_enqueue(E, E, B, p.dh2, 1, E, p.s1, E, 1, p.dw2, E, 0, st)) return e;
+  if (int e = small_gemm_enqueue(B, E, E, p.dh2, E, 1, p.w2, E, 1, p.ds1, E, 0, st)) return e;
+  if (int e = silu_backward_enqueue(p.h1, p.ds1, p.dh1, nE, st)) return e;
+  if (int e = rowsum_enqueue(p.dh1, p.db1, B, E, E, 0, st)) return e;
+  return small_gemm_enqueue(E, p.base, B, p.dh1, 1, E, p.e, p.base, 1, p.dw1, p.base, 0, st);
 }
 
 int backward_init() {

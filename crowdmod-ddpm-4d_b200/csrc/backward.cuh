@@ -112,6 +112,22 @@ int silu_backward_enqueue(const float* pre, const float* dpost, float* dpre, siz
 // y = silu(x)
 int silu_forward_enqueue(const float* x, float* y, size_t n, cudaStream_t st);
 int scale_inplace_enqueue(float* x, size_t n, const float* factor_dev, cudaStream_t st);
+// The whole time-embedding MLP backward (embeddings.py:22-34 and every block's dense_1): e [B][base] = table rows,
+// h1 = e W1^T + b1, h2 = SiLU(h1) W2^T + b2 (the forward's saves), dtemb [B][ld] = gradient of the dense_1 outputs
+// (block k: columns offs[k] .. offs[k] + couts[k]); s1, s2, ds1, ds2, dh1, dh2 are [B][E] scratch, left holding
+// SiLU(h1), SiLU(h2) and the gradients w.r.t. those and h1, h2.  Parameter gradients (=): dense_1 into grads at
+// goff_w / goff_b, the MLP's into dw1, db1, dw2, db2.  11 launches.
+struct TembBwdParams {
+  const float* e; const float* h1; const float* h2;
+  const float* dtemb; int ld;
+  const float* const* wd; const int* couts; const int* offs; int nblocks;   // device tables
+  const long long* goff_w; const long long* goff_b;                         // device tables
+  const float* w2;
+  float* dw1; float* db1; float* dw2; float* db2;
+  float* s1; float* s2; float* ds1; float* ds2; float* dh1; float* dh2;
+  int B, E, base;
+};
+int temb_backward_enqueue(const TembBwdParams& p, float* grads, cudaStream_t st);
 
 // one-time cudaFuncSetAttribute calls (kept out of stream capture)
 int backward_init();

@@ -46,4 +46,9 @@ int wgrad_run_prepare(WgradRun* R, unsigned kinds, int mode, const __half* act, 
                       int act_ld = 0, int extra_ld = 0);
 int wgrad_run_enqueue(const WgradRun& R, cudaStream_t st);
 
+// Which kernels may take the weight gradient of the first conv (c = its cout) or the final conv (c = its cin) as a conv
+// weight gradient over the packed fp16 operands (wgrad_run).  0: the SIMT kernels of backward.cu, which cover 32 and 64
+// channels; 64 keeps them, 32 takes the plane kernel, wider layers the plane chunks or wgrad_umma.
+inline unsigned edge_wgrad_kinds(int c) { return c == 32 ? CONV_PLANE : c == 64 ? 0u : CONV_UMMA | CONV_PLANE; }
+
 }  // namespace cm

@@ -340,11 +340,6 @@ int add_resblock(cm_unet* u, const std::string& prefix, int src0, int src1, int 
   return o;
 }
 
-// Which kernels may take the weight gradient of the first conv (c = its cout) or the final conv (c = its cin) as a conv
-// weight gradient over the packed fp16 operands (wgrad_run).  0: the SIMT kernels of backward.cu, which cover 32 and 64
-// channels; 64 keeps them, 32 takes the plane kernel, wider layers the plane chunks or wgrad_umma.
-unsigned edge_wgrad_kinds(int c) { return c == 32 ? CONV_PLANE : c == 64 ? 0u : CONV_UMMA | CONV_PLANE; }
-
 int build_plan(cm_unet* u) {
   const cm_unet_config& c = u->cfg;
   CM_CHECK(c.num_levels >= 1 && c.num_levels <= CM_MAX_LEVELS, "num_levels out of range");
@@ -1220,10 +1215,6 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
     ++nl;
   }
   // ---- time-embedding MLP (embeddings.py:22-34) and the per-block dense_1 (layers.py:35,62) ----
-  const size_t nE = (size_t)B * E;
-  if (int e = silu_forward_enqueue(u->tsave_h1, u->ts1, nE, st)) return e;
-  if (int e = silu_forward_enqueue(u->tsave_h2, u->ts2, nE, st)) return e;
-  nl += 2;
   {
     const int nb = (int)u->temb_couts.size();
     if (!u->d_goff_w) {
@@ -1237,23 +1228,20 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
       CM_CUDA(cudaMemcpy(u->d_goff_w, gw.data(), nb * sizeof(long long), cudaMemcpyHostToDevice));
       CM_CUDA(cudaMemcpy(u->d_goff_b, gb.data(), nb * sizeof(long long), cudaMemcpyHostToDevice));
     }
-    // (dense_1.bias gradient == the batch sum of dtemb; the conv_1 bias gradient is the same sum)
-    if (int e = temb_dense_backward_enqueue(u->dtemb, u->temb_ld, B, u->ts2, E, u->d_wd, u->d_couts, u->d_offs, nb,
-                                            grads, u->d_goff_w, u->d_goff_b, u->tds2, st))
-      return e;
-    nl += 2;
+    TembBwdParams tb{};
+    tb.e = u->tsave_e; tb.h1 = u->tsave_h1; tb.h2 = u->tsave_h2;
+    tb.dtemb = u->dtemb; tb.ld = u->temb_ld;
+    tb.wd = u->d_wd; tb.couts = u->d_couts; tb.offs = u->d_offs; tb.nblocks = nb;
+    tb.goff_w = u->d_goff_w; tb.goff_b = u->d_goff_b;
+    tb.w2 = u->params[u->p_w2].ptr;
+    tb.dw1 = gp(u->p_w1); tb.db1 = gp(u->p_b1); tb.dw2 = gp(u->p_w2); tb.db2 = gp(u->p_b2);
+    tb.s1 = u->ts1; tb.s2 = u->ts2; tb.ds1 = u->tds1; tb.ds2 = u->tds2; tb.dh1 = u->tdh1; tb.dh2 = u->tdh2;
+    tb.B = B; tb.E = E; tb.base = c.base_channels;
+    if (int e = temb_backward_enqueue(tb, grads, st)) return e;
+    nl += 11;
   }
-  if (int e = silu_backward_enqueue(u->tsave_h2, u->tds2, u->tdh2, nE, st)) return e;
-  if (int e = rowsum_enqueue(u->tdh2, gp(u->p_b2), B, E, E, 0, st)) return e;
-  if (int e = small_gemm_enqueue(E, E, B, u->tdh2, 1, E, u->ts1, E, 1, gp(u->p_w2), E, 0, st)) return e;
-  if (int e = small_gemm_enqueue(B, E, E, u->tdh2, E, 1, u->params[u->p_w2].ptr, E, 1, u->tds1, E, 0, st)) return e;
-  if (int e = silu_backward_enqueue(u->tsave_h1, u->tds1, u->tdh1, nE, st)) return e;
-  if (int e = rowsum_enqueue(u->tdh1, gp(u->p_b1), B, E, E, 0, st)) return e;
-  if (int e = small_gemm_enqueue(E, c.base_channels, B, u->tdh1, 1, E, u->tsave_e, c.base_channels, 1,
-                                 gp(u->p_w1), c.base_channels, 0, st))
-    return e;
   if (int e = scale_inplace_enqueue(grads, u->grad_total, u->loss_scale + 1, st)) return e;
-  nl += 8;
+  ++nl;
   if (launches) *launches = nl;
   return 0;
 }

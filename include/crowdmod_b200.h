@@ -213,6 +213,52 @@ CM_API int cm_op_conv3d_wgrad(int mode, const void* act16, int B, int D, int H, 
                               const void* extra16, int cin_extra, const void* dout16, int cout,
                               float* dw, float* dwx, int impl, void* stream);
 
+/* fp32 kernels of the training backward, one enqueue function each (tests compare them with float64 autograd).
+ * Channels-last fp32 tensors [B][pixels][C] unless stated.
+ *
+ * GroupNorm(8) (+SiLU) (+Dropout3d scale) backward over the channel concat of src0 [.][c0] and src1 [.][c1] (c1 = 0:
+ * one source; C = c0 + c1 a multiple of 32, c0 of 4): stats [B][8][2] = the forward's (mean, rstd) per group; dnorm
+ * [B][pixels][C] = gradient of the (scaled) output; draw: optional gradient added to dx unchanged; drop_scale:
+ * optional [B][drop_ld] scale per (sample, channel).  dsrc0 / dsrc1 (=) when init0 / init1, else (+=).  dgamma /
+ * dbeta [C] (=): params_all = 0 through the per-GroupNorm kernel, 1 through the table kernel the model uses. */
+CM_API int cm_op_gn_backward(const float* src0, int c0, const float* src1, int c1, const float* gamma, const float* beta,
+                             const float* stats, const float* dnorm, const float* draw, const float* drop_scale,
+                             int drop_ld, int B, int pixels, int silu, float* dsrc0, int init0, float* dsrc1, int init1,
+                             float* dgamma, float* dbeta, int params_all, void* stream);
+/* dOut preparation of a conv: src fp32 [B][pixels][C] -> dst16 fp16 [B][pixels][C] (dup 1) or the hi|lo pair
+ * [B][pixels][2C] (dup 2; NULL: no cast); acc_dst (=) src when acc_init, else (+=) (NULL: none); colsum[b * colsum_ld
+ * + c] += per-sample channel sums (NULL: none).  A value beyond the fp16 range is clamped and sets device error 301. */
+CM_API int cm_op_cast_colsum(const float* src, void* dst16, int dup, float* acc_dst, int acc_init, float* colsum,
+                             int colsum_ld, int B, int pixels, int C, void* stream);
+/* Bias gradients of n convs in one launch: tab (HOST) [n][4] = {source offset (floats from base), row stride,
+ * channels, output offset (floats into grads)}; grads[out + c] = sum_b base[src + b * ld + c]. */
+CM_API int cm_op_rowsum_all(const float* base, const int64_t* tab, int n, int B, float* grads, void* stream);
+/* Final conv backward (unet.py:121,165-167): deps fp32 [B][cout][H][W][L-P] (API layout, future frames) times the
+ * loss scale `scale`; act16 fp16 [B][L][H][W][act_ld] (act_ld 0 -> cin; act_lo > 0: hi|lo pair rows, lo at +act_lo);
+ * w [cout][cin][27].  dact fp32 [B][L][H][W][cin], dw [cout][cin][27], db [cout], all (=) and scaled by `scale`.
+ * dout16 NULL: the SIMT weight gradient (cin 32 or 64); else a caller-owned fp16 [B][L][H][W][32] buffer that
+ * receives the packed d_eps * scale, and dw comes from the conv weight gradient over it, as in the training backward. */
+CM_API int cm_op_final_conv_backward(const float* deps, float scale, const void* act16, int act_ld, int act_lo,
+                                     const float* w, float* dact, float* dw, float* db, int B, int H, int W, int L,
+                                     int P, int cin, int cout, void* dout16, void* stream);
+/* First conv weight / bias gradient (unet.py:32): x [B][cin][H][W][F], past [B][cin][H][W][P] (API layout), dout fp32
+ * [B][L][H][W][cout]; dw [cout][cin][27], db [cout] (=). */
+CM_API int cm_op_first_conv_wgrad(const float* x, const float* past, const float* dout, float* dw, float* db, int B,
+                                  int H, int W, int P, int F, int cin, int cout, void* stream);
+/* Time-embedding MLP backward as the training backward runs it (embeddings.py:22-34, layers.py:35,62): e [B][base],
+ * h1 / h2 [B][E] the pre-activations, dtemb [B][ld] the gradient of every block's dense_1 output (block k: columns
+ * offs[k] .. + couts[k], weight wd[k] [couts[k]][E]); wd / couts / offs / goff_w / goff_b are HOST arrays [nblocks]
+ * (wd: device pointers).  Outputs (=): dense_1 weight / bias gradients into dense_grads at goff_w / goff_b, dw1
+ * [E][base], db1 [E], dw2 [E][E], db2 [E], and ds1 / ds2 [B][E], the gradients w.r.t. SiLU(h1) and SiLU(h2). */
+CM_API int cm_op_temb_backward(const float* e, const float* h1, const float* h2, const float* dtemb, int ld, int B,
+                               int base, int E, const float* w2, const void* const* wd, const int32_t* couts,
+                               const int32_t* offs, int nblocks, float* dense_grads, const int64_t* goff_w,
+                               const int64_t* goff_b, float* dw1, float* db1, float* dw2, float* db2, float* ds1,
+                               float* ds2, void* stream);
+/* Loss scale of the training backward: scale_out[0] = S = 2^e with e = floor(log2(target / max|x|)) clamped to
+ * [-60, 60] (1 when max|x| is 0 or not finite), scale_out[1] = 1/S (device float[2]). */
+CM_API int cm_op_loss_scale(const float* x, int64_t n, float target, float* scale_out, void* stream);
+
 /* ---- second backbone: DiT4D_V4 (SURVEY.md section 8 f2) ------------------------------------------------------
  * Replaces /root/reference/models/backbones/DiT4D_V4.py:228-375 (selected by --arch DDPM-DiT at
  * models/diffusion/ddpm.py:88-104) for inference / sampling: same forward(future, t, past) contract and the same
