@@ -150,6 +150,15 @@ SIGNATURES = {
     "cm_dit_sample": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "cm_dit_flops_per_sample": (C.c_double, [C.c_void_p]),
     "cm_dit_last_launches": (C.c_int64, [C.c_void_p]),
+    "cm_op_dit_patchify": (C.c_int, [C.c_void_p, C.c_void_p] + [C.c_int] * 9 + [C.c_void_p, C.c_void_p]),
+    "cm_op_dit_add_pos": (C.c_int, [C.c_void_p] * 3 + [C.c_int] * 4 + [C.c_void_p]),
+    "cm_op_dit_ln_mod": (C.c_int, [C.c_void_p, C.c_void_p] + [C.c_int] * 6 + [C.c_void_p, C.c_void_p]),
+    "cm_op_dit_tattn": (C.c_int, [C.c_void_p, C.c_void_p] + [C.c_int] * 6 + [C.c_void_p]),
+    "cm_op_dit_linear": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
+                                   C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "cm_op_dit_unpatch_step": (C.c_int, [C.c_void_p, C.c_int] + [C.c_int] * 8 + [C.c_void_p] * 3
+                               + [C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_uint64, C.c_int64, C.c_void_p,
+                                  C.c_void_p]),
     "cm_window_gather": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
                                    C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "cm_metrics_reduce": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,

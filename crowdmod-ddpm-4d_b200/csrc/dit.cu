@@ -296,6 +296,85 @@ int grid_for(size_t work_items, int block = 256) {
 
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
+#define DIT_LAUNCH_CHECK() CM_CUDA(cudaGetLastError())
+
+// One enqueue function per bandwidth kernel: run_forward and the op-level entry points (cm_op_dit_*) both launch
+// through these, with the limits build() enforces checked before the launch.
+int patchify_enqueue(const float* future, const float* past, const PatchGeom& g, __half* out, cudaStream_t st) {
+  CM_CHECK(g.B >= 1 && g.C >= 1 && g.C <= 4 && g.p >= 1 && g.pt >= 1 && g.H == g.hp * g.p && g.W == g.wp * g.p &&
+               g.P + g.F == g.Tp * g.pt && g.Kpad % 32 == 0 && g.Kpad >= g.C * g.pt * g.p * g.p,
+           "patchify: bad geometry (C %d, %dx%d, P %d F %d, p %d, pt %d, Kpad %d)", g.C, g.H, g.W, g.P, g.F, g.p, g.pt,
+           g.Kpad);
+  const size_t rows = (size_t)g.B * g.Tp * g.hp * g.wp;
+  dit_patchify_kernel<<<grid_for(rows * g.Kpad), 256, 0, st>>>(future, past, g, out);
+  DIT_LAUNCH_CHECK();
+  return 0;
+}
+
+int add_pos_enqueue(float* x, const float* spatial, const float* temporal, int rows, int Tp, int Ns, int D, cudaStream_t st) {
+  CM_CHECK(rows >= 1 && Tp >= 1 && Ns >= 1 && D % 32 == 0 && D > 0, "add_pos: rows %d Tp %d Ns %d D %d", rows, Tp, Ns, D);
+  dit_add_pos_kernel<<<grid_for((size_t)rows * D / 4), 256, 0, st>>>(x, spatial, temporal, rows, Tp, Ns, D);
+  DIT_LAUNCH_CHECK();
+  return 0;
+}
+
+int ln_mod_enqueue(const float* x, const float* mods, int ld_mods, int off_shift, int off_scale, int rows_per_sample,
+                   int rows, int D, __half* out16, cudaStream_t st) {
+  CM_CHECK(rows >= 1 && rows_per_sample >= 1 && D % 32 == 0 && D > 0 && ld_mods >= 0 && ld_mods % 4 == 0 &&
+               off_shift >= 0 && off_shift % 4 == 0 && off_scale >= 0 && off_scale % 4 == 0,
+           "ln_mod: rows %d per sample %d D %d ld_mods %d offsets %d %d", rows, rows_per_sample, D, ld_mods, off_shift,
+           off_scale);
+  dit_ln_mod_kernel<<<(rows * 32 + 255) / 256, 256, 0, st>>>(x, mods, ld_mods, off_shift, off_scale, rows_per_sample,
+                                                               rows, D, out16);
+  DIT_LAUNCH_CHECK();
+  return 0;
+}
+
+int tattn_enqueue(const float* qkv, __half* ctx16, int B, int Tp, int Ns, int D, int heads, int qs, cudaStream_t st) {
+  // the kernel keeps the Tp scores of a query in sc[8]
+  CM_CHECK(B >= 1 && Ns >= 1 && Tp >= 1 && Tp <= 8 && qs >= 0 && qs < Tp, "temporal attention: B %d Tp %d qs %d Ns %d", B,
+           Tp, qs, Ns);
+  CM_CHECK(D % 32 == 0 && heads >= 1 && D % heads == 0 && D / heads <= 128 && (D / heads) % 2 == 0,
+           "temporal attention: D %d / heads %d unsupported (D %% 32 == 0, head dim even and <= 128)", D, heads);
+  const int warps = B * (Tp - qs) * Ns * heads;
+  dit_tattn_kernel<<<(warps * 32 + 255) / 256, 256, 0, st>>>(qkv, ctx16, B, Tp, Ns, D, heads, qs);
+  DIT_LAUNCH_CHECK();
+  return 0;
+}
+
+int unpatch_step_enqueue(const UnpatchParams& up, cudaStream_t st) {
+  CM_CHECK(up.B >= 1 && up.C >= 1 && up.C <= 4 && up.H == up.hp * up.p && up.W == up.wp * up.p &&
+               up.P + up.F == up.Tp * up.pt && up.F >= 1 && up.ld >= up.pt * up.C * up.p * up.p,
+           "un-patch: bad geometry (C %d, %dx%d, P %d F %d, p %d, pt %d, ld %d)", up.C, up.H, up.W, up.P, up.F, up.p,
+           up.pt, up.ld);
+  CM_CHECK(!up.x || (up.coef && (up.mode == 0 || up.mode == 1)), "un-patch: the update needs coefficients and mode 0 or 1");
+  dit_unpatch_step_kernel<<<grid_for((size_t)up.B * up.H * up.W * up.F), 256, 0, st>>>(up);
+  DIT_LAUNCH_CHECK();
+  return 0;
+}
+
+// Epilogue fusions of a DiT GEMM (ConvParams::act / gate / rmap), on a launch conv_prepare made in 1x1x1 mode without
+// split-K: v = act(acc + bias) (act 1: exact GELU), written to epi.out32 and / or out16; gate != nullptr: the gated
+// residual out32[orow] += gate[sample * gate_ld + n] * v in place (resid aliases out32); rmap_out > 0: GEMM row m of
+// sample b = m / pps lands at orow = b * rmap_out + rmap_off + (m - b * pps), else orow = m.
+void dit_epilogue(ConvParams& p, int act, __half* out16, const float* gate, int gate_ld, int rmap_out, int rmap_off) {
+  p.act = act;
+  p.epi.out16 = out16;
+  p.gate = gate;
+  p.gate_ld = gate_ld;
+  p.epi.resid = gate ? p.epi.out32 : nullptr;
+  p.rmap_out = rmap_out;
+  p.rmap_off = rmap_off;
+}
+
+// a prepared gated-residual GEMM with this launch's gate rows (the block's offset into mods, ld_mods per sample)
+int gated_enqueue(const ConvLaunch& prepared, const float* gate, int gate_ld, cudaStream_t st) {
+  ConvLaunch L = prepared;
+  L.p.gate = gate;
+  L.p.gate_ld = gate_ld;
+  return conv_enqueue(L, st);
+}
+
 }  // namespace
 }  // namespace cm
 
@@ -566,8 +645,6 @@ int reserve(cm_dit* u, int batch) {
   return 0;
 }
 
-#define DIT_LAUNCH_CHECK() CM_CUDA(cudaGetLastError())
-
 // GEMM out32[rows][cout] = act16[rows][cin] . W^T + bias  (conv_umma 1x1x1 mode; rows = nb * d * h * w)
 int prep_gemm(cm_dit* u, DitLinear& l, const __half* act, int nb, int d, int h, int w, float* out32) {
   // no split-K: the epilogue fusions (act / gate / rmap) live in the non-split path, and with K <= 1024 narrower N tiles
@@ -593,16 +670,13 @@ int prepare(cm_dit* u, int batch) {
     if (int e = prep_gemm(u, b.t_out, u->ctx16, batch, 1, u->nq, Ns, u->x32)) return e;
     if (int e = prep_gemm(u, b.fc1, u->xm16, batch, 1, Tp, Ns, nullptr)) return e;
     if (int e = prep_gemm(u, b.fc2, u->g16, batch, 1, Tp, Ns, u->x32)) return e;
-    // epilogue fusions (ConvParams::act / gate / rmap): GELU + fp16 operand out of fc1; the three gated residuals
-    // x += gate * (GEMM + bias) written in place into the token stream (the temporal one into the future slots)
-    b.fc1.launch.p.act = 1;
-    b.fc1.launch.p.epi.out16 = u->g16;
-    for (DitLinear* l : {&b.s_out, &b.t_out, &b.fc2}) {
-      l->launch.p.epi.resid = u->x32;
-      l->launch.p.gate = u->mods;           // + the block's gate offset, set per launch in run_forward
-    }
-    b.t_out.launch.p.rmap_out = u->tokens;
-    b.t_out.launch.p.rmap_off = u->qs * Ns;
+    // epilogue fusions: GELU + fp16 operand out of fc1; the three gated residuals x += gate * (GEMM + bias) written in
+    // place into the token stream (the temporal one into the future slots).  The gate rows (the block's offset into
+    // mods) are set per launch in run_forward.
+    dit_epilogue(b.fc1.launch.p, 1, u->g16, nullptr, 0, 0, 0);
+    dit_epilogue(b.s_out.launch.p, 0, nullptr, u->mods, 0, 0, 0);
+    dit_epilogue(b.t_out.launch.p, 0, nullptr, u->mods, 0, u->tokens, u->qs * Ns);
+    dit_epilogue(b.fc2.launch.p, 0, nullptr, u->mods, 0, 0, 0);
   }
   if (int e = prep_gemm(u, u->final_lin, u->xm16, batch, 1, Tp, Ns, u->out32)) return e;
   if (u->graph_exec) {            // the captured step bakes the launches of the previous batch
@@ -647,66 +721,38 @@ int run_forward(cm_dit* u, int B, const float* future, const float* past, Unpatc
   }
   // ---- patchify + positional embeddings
   PatchGeom g{B, c.in_channels, c.rows, c.cols, c.past_len, c.future_len, c.patch, c.t_patch, u->hp, u->wp, Tp, u->Kpad};
-  dit_patchify_kernel<<<grid_for((size_t)R * u->Kpad), 256, 0, st>>>(future, past, g, u->a16);
-  DIT_LAUNCH_CHECK();
+  if (int e = patchify_enqueue(future, past, g, u->a16, st)) return e;
   if (int e = conv_enqueue(u->patch.launch, st)) return e;
-  dit_add_pos_kernel<<<grid_for((size_t)R * D / 4), 256, 0, st>>>(u->x32, u->params[u->p_spatial].ptr, u->params[u->p_temporal].ptr, R, Tp,
-                                                                  Ns, D);
-  DIT_LAUNCH_CHECK();
+  if (int e = add_pos_enqueue(u->x32, u->params[u->p_spatial].ptr, u->params[u->p_temporal].ptr, R, Tp, Ns, D, st)) return e;
   n += 3;
-  const int ln_blocks = (R * 32 + 255) / 256;
   for (int i = 0; i < c.depth; ++i) {
     cm_dit::Block& b = u->blocks[i];
     const int mo = i * 9 * D;     // chunk(9): shift1, scale1, gate1, shift2, scale2, gate2, shift3, scale3, gate3
     // 1. spatial self-attention (every temporal slot is its own sequence of Ns tokens)
-    dit_ln_mod_kernel<<<ln_blocks, 256, 0, st>>>(u->x32, u->mods, ld_mods, mo, mo + D, u->tokens, R, D, u->xm16);
-    DIT_LAUNCH_CHECK();
+    if (int e = ln_mod_enqueue(u->x32, u->mods, ld_mods, mo, mo + D, u->tokens, R, D, u->xm16, st)) return e;
     if (int e = conv_enqueue(b.s_in.launch, st)) return e;
     if (int e = attn_core_enqueue(u->qkv32, u->ctx16, B * Tp, Ns, D, c.heads, st, 1)) return e;
-    {
-      ConvLaunch L = b.s_out.launch;
-      L.p.gate = u->mods + mo + 2 * D;
-      L.p.gate_ld = ld_mods;
-      if (int e = conv_enqueue(L, st)) return e;
-    }
+    if (int e = gated_enqueue(b.s_out.launch, u->mods + mo + 2 * D, ld_mods, st)) return e;
     // 2. temporal cross-attention (future slots of every spatial patch query all of its slots)
-    dit_ln_mod_kernel<<<ln_blocks, 256, 0, st>>>(u->x32, u->mods, ld_mods, mo + 3 * D, mo + 4 * D, u->tokens, R, D, u->xm16);
-    DIT_LAUNCH_CHECK();
+    if (int e = ln_mod_enqueue(u->x32, u->mods, ld_mods, mo + 3 * D, mo + 4 * D, u->tokens, R, D, u->xm16, st)) return e;
     if (int e = conv_enqueue(b.t_in.launch, st)) return e;
-    {
-      const int warps = B * u->nq * Ns * c.heads;
-      dit_tattn_kernel<<<(warps * 32 + 255) / 256, 256, 0, st>>>(u->qkv32, u->ctx16, B, Tp, Ns, D, c.heads, u->qs);
-      DIT_LAUNCH_CHECK();
-    }
-    {
-      ConvLaunch L = b.t_out.launch;
-      L.p.gate = u->mods + mo + 5 * D;
-      L.p.gate_ld = ld_mods;
-      if (int e = conv_enqueue(L, st)) return e;
-    }
+    if (int e = tattn_enqueue(u->qkv32, u->ctx16, B, Tp, Ns, D, c.heads, u->qs, st)) return e;
+    if (int e = gated_enqueue(b.t_out.launch, u->mods + mo + 5 * D, ld_mods, st)) return e;
     // 3. MLP
-    dit_ln_mod_kernel<<<ln_blocks, 256, 0, st>>>(u->x32, u->mods, ld_mods, mo + 6 * D, mo + 7 * D, u->tokens, R, D, u->xm16);
-    DIT_LAUNCH_CHECK();
+    if (int e = ln_mod_enqueue(u->x32, u->mods, ld_mods, mo + 6 * D, mo + 7 * D, u->tokens, R, D, u->xm16, st)) return e;
     if (int e = conv_enqueue(b.fc1.launch, st)) return e;
-    {
-      ConvLaunch L = b.fc2.launch;
-      L.p.gate = u->mods + mo + 8 * D;
-      L.p.gate_ld = ld_mods;
-      if (int e = conv_enqueue(L, st)) return e;
-    }
+    if (int e = gated_enqueue(b.fc2.launch, u->mods + mo + 8 * D, ld_mods, st)) return e;
     n += 11;
   }
   // ---- final layer (chunk(2): shift, scale) + un-patch (+ reverse-step update)
   const int mo = c.depth * 9 * D;
-  dit_ln_mod_kernel<<<ln_blocks, 256, 0, st>>>(u->x32, u->mods, ld_mods, mo, mo + D, u->tokens, R, D, u->xm16);
-  DIT_LAUNCH_CHECK();
+  if (int e = ln_mod_enqueue(u->x32, u->mods, ld_mods, mo, mo + D, u->tokens, R, D, u->xm16, st)) return e;
   if (int e = conv_enqueue(u->final_lin.launch, st)) return e;
   up.out = u->out32;
   up.ld = u->Nout;
   up.B = B; up.C = c.out_channels; up.H = c.rows; up.W = c.cols; up.P = c.past_len; up.F = c.future_len;
   up.p = c.patch; up.pt = c.t_patch; up.hp = u->hp; up.wp = u->wp; up.Tp = Tp;
-  dit_unpatch_step_kernel<<<grid_for((size_t)B * c.rows * c.cols * c.future_len), 256, 0, st>>>(up);
-  DIT_LAUNCH_CHECK();
+  if (int e = unpatch_step_enqueue(up, st)) return e;
   n += 3;
   if (launches) *launches += n;
   return 0;
@@ -910,6 +956,100 @@ int cm_dit_sample(cm_dit* u, const cm_chain_args* a, void* stream) {
   }
   CM_CUDA(cudaMemcpyAsync(a->x, u->chain_x, xel * sizeof(float), cudaMemcpyDeviceToDevice, st));
   return 0;
+}
+
+// ---- op-level entry points: each launches through the enqueue function run_forward uses, then synchronises ----
+
+static int dit_op_sync(int rc, cudaStream_t st) {
+  const cudaError_t se = cudaStreamSynchronize(st);
+  if (rc) return rc;
+  CM_CUDA(se);
+  return 0;
+}
+
+int cm_op_dit_patchify(const float* future, const float* past, int B, int C, int H, int W, int P, int F, int p, int pt,
+                       int kpad, void* a16, void* stream) {
+  CM_CHECK(p >= 1 && pt >= 1 && H % p == 0 && W % p == 0 && (P + F) % pt == 0 && (P + F) / pt <= 8,
+           "patchify: %dx%d, P %d F %d not divisible by patch %d / t_patch %d (or more than 8 slots)", H, W, P, F, p, pt);
+  const PatchGeom g{B, C, H, W, P, F, p, pt, H / p, W / p, (P + F) / pt, kpad};
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  return dit_op_sync(patchify_enqueue(future, past, g, static_cast<__half*>(a16), st), st);
+}
+
+int cm_op_dit_add_pos(float* x, const float* spatial, const float* temporal, int rows, int Tp, int Ns, int D, void* stream) {
+  CM_CHECK(Tp <= 8, "more than 8 temporal slots (%d)", Tp);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  return dit_op_sync(add_pos_enqueue(x, spatial, temporal, rows, Tp, Ns, D, st), st);
+}
+
+int cm_op_dit_ln_mod(const float* x, const float* mods, int ld_mods, int off_shift, int off_scale, int rows_per_sample,
+                     int rows, int D, void* out16, void* stream) {
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  return dit_op_sync(ln_mod_enqueue(x, mods, ld_mods, off_shift, off_scale, rows_per_sample, rows, D,
+                                    static_cast<__half*>(out16), st), st);
+}
+
+int cm_op_dit_tattn(const float* qkv, void* ctx16, int B, int Tp, int Ns, int D, int heads, int qs, void* stream) {
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  return dit_op_sync(tattn_enqueue(qkv, static_cast<__half*>(ctx16), B, Tp, Ns, D, heads, qs, st), st);
+}
+
+int cm_op_dit_linear(const void* act16, int nb, int pps, int cin, const float* w, const float* bias, int cout, int act,
+                     const float* gate, int gate_ld, int rmap_out, int rmap_off, float* out32, void* out16, void* stream) {
+  CM_CHECK(nb >= 1 && pps >= 1 && cin >= 32 && cin <= 1024 && act >= 0 && act <= 1 && gate_ld >= 0,
+           "DiT linear: nb %d pps %d cin %d act %d gate_ld %d", nb, pps, cin, act, gate_ld);
+  CM_CHECK(!gate || out32, "DiT linear: the gated residual updates out32 in place");
+  CM_CHECK(rmap_out == 0 || (gate && rmap_out >= pps && rmap_off >= 0 && rmap_off + pps <= rmap_out),
+           "DiT linear: rmap_out %d / rmap_off %d must place the %d rows of a sample inside its row block", rmap_out,
+           rmap_off, pps);
+  if (int e = kernels_init()) return e;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  __half* wp = nullptr;   // hi|lo packed rows [2 * cout][cin], as pack_linear caches them
+  CM_CUDA(cudaMalloc(&wp, (size_t)2 * cout * cin * sizeof(__half)));
+  int rc = pack_conv_weights(w, nullptr, wp, cout, cin, 0, 1, 2, 0, st);
+  ConvEpilogue e{};
+  e.bias = bias;
+  e.out32 = out32;
+  ConvLaunch L;
+  if (!rc) rc = conv_prepare(&L, 3, static_cast<const __half*>(act16), nb, 1, 1, pps, cin, nullptr, 0, wp, cout, 2, e, false);
+  if (!rc) {
+    dit_epilogue(L.p, act, static_cast<__half*>(out16), gate, gate_ld, rmap_out, rmap_off);
+    rc = conv_enqueue(L, st);
+  }
+  rc = dit_op_sync(rc, st);
+  cudaFree(wp);
+  return rc;
+}
+
+int cm_op_dit_unpatch_step(const float* out, int ld, int B, int C, int H, int W, int P, int F, int p, int pt,
+                           float* eps_out, float* x, const float* coef, int nsteps, int step, int mode, const float* noise,
+                           uint64_t seed, int64_t sample_offset, float* history, void* stream) {
+  CM_CHECK(p >= 1 && pt >= 1 && H % p == 0 && W % p == 0 && (P + F) % pt == 0 && (P + F) / pt <= 8,
+           "un-patch: %dx%d, P %d F %d not divisible by patch %d / t_patch %d (or more than 8 slots)", H, W, P, F, p, pt);
+  CM_CHECK(!x || (nsteps >= 1 && step >= 0 && step < nsteps), "un-patch: step %d outside [0, %d)", step, nsteps);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  // the step index and {seed, sample_offset} travel through device memory, as in cm_dit_sample
+  unsigned long long* dev = nullptr;
+  CM_CUDA(cudaMalloc(&dev, 3 * sizeof(unsigned long long)));
+  const unsigned long long h[3] = {seed, static_cast<unsigned long long>(sample_offset), static_cast<unsigned long long>(step)};
+  int rc = cudaMemcpyAsync(dev, h, sizeof(h), cudaMemcpyHostToDevice, st) == cudaSuccess ? 0 : 1;
+  UnpatchParams up{};
+  up.out = out;
+  up.ld = ld;
+  up.B = B; up.C = C; up.H = H; up.W = W; up.P = P; up.F = F;
+  up.p = p; up.pt = pt; up.hp = H / p; up.wp = W / p; up.Tp = (P + F) / pt;
+  up.eps_out = eps_out;
+  up.x = x;
+  up.coef = coef;
+  up.step_dev = reinterpret_cast<const int*>(dev + 2);       // low word of a little-endian 64-bit slot
+  up.mode = mode;
+  up.noise = noise;
+  up.chain_dev = dev;
+  up.history = history;
+  if (!rc) rc = unpatch_step_enqueue(up, st);
+  rc = dit_op_sync(rc, st);
+  cudaFree(dev);
+  return rc;
 }
 
 }  // extern "C"

@@ -291,6 +291,45 @@ CM_API int cm_dit_sample(cm_dit* d, const cm_chain_args* args, void* stream);
 CM_API double cm_dit_flops_per_sample(const cm_dit* d);
 CM_API int64_t cm_dit_last_launches(const cm_dit* d);
 
+/* Op-level entry points of the DiT plan (unit tests; allocate temporaries, synchronise).  Each launches through the
+ * same enqueue function as cm_dit_forward / cm_dit_sample, with the limits cm_dit_create enforces: C <= 4, at most 8
+ * temporal slots Tp = (P + F) / pt, D % 32 == 0, head dim D / heads even and <= 128.
+ *
+ * Patch embedding operand (DiT4D_V4.py:47-63, :356-359): future [B][C][H][W][F], past [B][C][H][W][P] fp32 (API layout)
+ * -> a16 fp16 [B][Tp][H/p][W/p][kpad], column ((c*pt + dt)*p + dy)*p + dx of x = cat(past, future) along time; columns
+ * K = C*pt*p*p .. kpad-1 are written as 0 (kpad a multiple of 32, >= K). */
+CM_API int cm_op_dit_patchify(const float* future, const float* past, int B, int C, int H, int W, int P, int F, int p,
+                              int pt, int kpad, void* a16, void* stream);
+/* x fp32 [rows][D] (row = (b*Tp + slot)*Ns + s) += spatial [Ns][D] then + temporal [>= Tp][D], in place. */
+CM_API int cm_op_dit_add_pos(float* x, const float* spatial, const float* temporal, int rows, int Tp, int Ns, int D,
+                             void* stream);
+/* out16 fp16 [rows][D] = LayerNorm(x [rows][D], eps 1e-6, no affine) * (1 + scale) + shift, with shift / scale the D
+ * floats at mods + b*ld_mods + off_shift / off_scale, b = row / rows_per_sample (ld_mods 0: one vector for every row;
+ * ld_mods and the offsets multiples of 4). */
+CM_API int cm_op_dit_ln_mod(const float* x, const float* mods, int ld_mods, int off_shift, int off_scale,
+                            int rows_per_sample, int rows, int D, void* out16, void* stream);
+/* Temporal cross-attention core (DiT4D_V4.py:168-190): qkv fp32 [B][Tp][Ns][3D] (q | k | v, heads split each D) ->
+ * ctx16 fp16 [B][Tp-qs][Ns][D]: slots qs .. Tp-1 of every (sample, spatial patch) query all Tp slots, per head. */
+CM_API int cm_op_dit_tattn(const float* qkv, void* ctx16, int B, int Tp, int Ns, int D, int heads, int qs, void* stream);
+/* One DiT Linear on the tcgen05 GEMM in 1x1x1 mode with the plan's epilogue fusions: act16 fp16 [nb*pps][cin]
+ * (cin % 32 == 0, <= 1024), w fp32 [cout][cin] (packed hi|lo), bias [cout], cout % 32 == 0; v = act(A.W^T + bias)
+ * (act 1: exact GELU).  gate NULL: out32 [nb*pps][cout] = v (NULL: none), out16 fp16 [nb*pps][cout] = fp16(v) (NULL:
+ * none).  gate != NULL: out32 += gate[b*gate_ld + n] * v in place for the rows of sample b = m / pps, at row m, or at
+ * row b*rmap_out + rmap_off + (m - b*pps) when rmap_out > 0 (the temporal out-projection into the future slots). */
+CM_API int cm_op_dit_linear(const void* act16, int nb, int pps, int cin, const float* w, const float* bias, int cout,
+                            int act, const float* gate, int gate_ld, int rmap_out, int rmap_off, float* out32,
+                            void* out16, void* stream);
+/* Un-patch + reverse-step update (DiT4D_V4.py:80-102, ddpm.py:25-38, :262-265, guidance.py:4-8): out fp32
+ * [B*Tp*(H/p)*(W/p)][ld] FinalLayer rows, column ((dt*C + c)*p + dy)*p + dx.  eps_out [B][C][H][W][F] (NULL: none)
+ * = the future frames.  x [B][C][H][W][F] (NULL: no update) takes step `step` of the chain in place with coef (device
+ * [nsteps][8], cm_chain_args), mode 0 / 1, noise (device [nsteps][B*C*H*W*F]) or Philox(seed, sample_offset); history
+ * (device [nsteps+1][B*C*H*W*F], NULL: none) receives x in slot step+1.  The step and {seed, sample_offset} are read
+ * from device memory, as in a captured chain step. */
+CM_API int cm_op_dit_unpatch_step(const float* out, int ld, int B, int C, int H, int W, int P, int F, int p, int pt,
+                                  float* eps_out, float* x, const float* coef, int nsteps, int step, int mode,
+                                  const float* noise, uint64_t seed, int64_t sample_offset, float* history,
+                                  void* stream);
+
 /* ---- callers either side of the hot path (SURVEY.md section 8 f3 / f4) -------------------------------------- */
 
 /* Data feed: one batch of (past, future) windows gathered ON the device from HBM-resident raw sequences.
