@@ -64,6 +64,56 @@ class ChainArgs(C.Structure):
     ]
 
 
+class ConvEpilogue(C.Structure):
+    """struct cm_conv_epilogue (include/crowdmod_b200.h)."""
+
+    _fields_ = [
+        ("bias", C.c_void_p),
+        ("bias2", C.c_void_p),
+        ("temb", C.c_void_p),
+        ("t_dev", C.c_void_p),
+        ("temb_ld", C.c_int32),
+        ("temb_bstride", C.c_int32),
+        ("resid", C.c_void_p),
+        ("out32", C.c_void_p),
+        ("out16", C.c_void_p),
+        ("out16_ld", C.c_int32),
+        ("out16_lo", C.c_int32),
+        ("lo_from", C.c_int32),
+        ("lo_from_x", C.c_int32),
+        ("stats_rec", C.c_void_p),
+    ]
+
+
+class GnArgs(C.Structure):
+    """struct cm_gn_args (include/crowdmod_b200.h)."""
+
+    _fields_ = [
+        ("src0", C.c_void_p),
+        ("src1", C.c_void_p),
+        ("c0", C.c_int32),
+        ("c1", C.c_int32),
+        ("gamma", C.c_void_p),
+        ("beta", C.c_void_p),
+        ("B", C.c_int32),
+        ("pixels", C.c_int32),
+        ("eps", C.c_float),
+        ("silu", C.c_int32),
+        ("drop_scale", C.c_void_p),
+        ("drop_ld", C.c_int32),
+        ("out_norm16", C.c_void_p),
+        ("out_raw16", C.c_void_p),
+        ("dup", C.c_int32),
+        ("stats", C.c_void_p),
+        ("rec0", C.c_void_p),
+        ("rec0_units", C.c_int32),
+        ("rec0_nvalid", C.c_int32),
+        ("rec1", C.c_void_p),
+        ("rec1_units", C.c_int32),
+        ("rec1_nvalid", C.c_int32),
+    ]
+
+
 # name -> (restype, argtypes); must list EVERY function include/crowdmod_b200.h declares
 # (tests/test_abi.py checks the two against each other).
 SIGNATURES = {
@@ -116,6 +166,15 @@ SIGNATURES = {
     "cm_op_gn_silu": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                 C.c_int, C.c_int, C.c_float, C.c_int, C.c_void_p, C.c_void_p,
                                 C.c_void_p]),
+    "cm_op_conv3d_epi": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                   C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
+                                   C.POINTER(ConvEpilogue), C.c_int, C.POINTER(C.c_int32), C.c_void_p]),
+    "cm_op_gn": (C.c_int, [C.POINTER(GnArgs), C.POINTER(C.c_int32), C.c_void_p]),
+    "cm_op_first_conv_packed": (C.c_int, [C.c_void_p] * 4 + [C.c_int] * 8
+                                + [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_int32), C.c_void_p]),
+    "cm_op_temb": (C.c_int, [C.c_void_p] * 5 + [C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_int32),
+                                                C.POINTER(C.c_int32), C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int,
+                                                C.c_void_p, C.c_int] + [C.c_void_p] * 4),
     "cm_op_attn_core": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
                                   C.c_void_p]),
     "cm_op_attn_core_backward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
@@ -127,6 +186,9 @@ SIGNATURES = {
     "cm_op_final_conv": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
                                    C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                    C.c_void_p]),
+    "cm_op_final_conv_step": (C.c_int, [C.c_void_p, C.c_int, C.c_int] + [C.c_void_p] * 3 + [C.c_int] * 7
+                         + [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_uint64, C.c_int64,
+                            C.c_void_p, C.c_void_p]),
     "cm_op_gn_backward": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int] + [C.c_void_p] * 6
                           + [C.c_int] * 4 + [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                              C.c_int, C.c_void_p]),

@@ -107,6 +107,171 @@ int cm_op_gn_silu(const float* src0, int c0, const float* src1, int c1, const fl
   return 0;
 }
 
+// ---- the UNet forward's fused epilogues (conv_run_* / gn_silu_enqueue / pack_first_input_enqueue, as unet.cu) ----
+static ConvEpilogue conv_epi_of(const cm_conv_epilogue* x) {
+  ConvEpilogue e{};
+  if (!x) return e;
+  e.bias = x->bias; e.bias2 = x->bias2;
+  e.temb = x->temb; e.t_dev = x->t_dev; e.temb_ld = x->temb_ld; e.temb_bstride = x->temb_bstride;
+  e.resid = x->resid;
+  e.out32 = x->out32;
+  e.out16 = static_cast<__half*>(x->out16);
+  e.out16_ld = x->out16_ld; e.out16_lo = x->out16_lo;
+  e.lo_from = x->lo_from; e.lo_from_x = x->lo_from_x;
+  e.stats_rec = x->stats_rec;
+  return e;
+}
+
+// {units per sample, rows per unit, planes per unit, grid rows per unit} of the records a prepared launch writes
+static void conv_rec_geom(const ConvRun& R, int32_t* g) {
+  if (!g) return;
+  g[0] = g[1] = g[2] = g[3] = 0;
+  const GnRec r = conv_run_records(R);
+  if (r.units == 0) return;
+  g[0] = r.units;
+  g[1] = r.nvalid;
+  if (const auto* L = std::get_if<Res32Launch>(&R.l)) { g[2] = 1; g[3] = L->p.HB; }
+  if (const auto* L = std::get_if<PlaneLaunch>(&R.l)) { g[2] = L->p.R; g[3] = L->p.HB; }
+}
+
+int cm_op_conv3d_epi(int mode, const void* act16, int B, int D, int H, int W, int cin, const void* extra16,
+                     int cin_extra, int dup, const float* w, const float* wx, int cout, int terms,
+                     const cm_conv_epilogue* epi, int impl, int32_t* rec_geom, void* stream) {
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (int e = kernels_init()) return e;
+  CM_CHECK(dup == 1 || dup == 2, "dup must be 1 or 2");
+  CM_CHECK(impl == 0 || impl == 2 || impl == 3, "impl must be 0 (conv_umma), 2 (conv_plane) or 3 (conv_res32)");
+  const size_t ktot = conv_packed_k(mode, dup * cin, dup * cin_extra);
+  __half* wp = nullptr;
+  CM_CUDA(cudaMalloc(&wp, (size_t)terms * cout * ktot * sizeof(__half)));
+  int rc = 0;
+  if (mode == 2) rc = pack_upsample_weights(w, wp, cout, cin, terms, 0, st, dup);
+  else rc = pack_conv_weights(w, wx, wp, cout, cin, cin_extra, mode == 3 ? 1 : 27, terms, 0, st, dup);
+  const unsigned kind = impl == 0 ? CONV_UMMA : impl == 2 ? CONV_PLANE : CONV_RES32;
+  ConvRun R;
+  if (!rc)
+    rc = conv_run_prepare(&R, kind, mode, static_cast<const __half*>(act16), B, D, H, W, dup * cin,
+                          static_cast<const __half*>(extra16), dup * cin_extra, wp, cout, terms, conv_epi_of(epi));
+  if (!rc && !R.covered()) {
+    set_error("the requested conv kernel does not cover this shape");
+    rc = 2;
+  }
+  if (!rc) conv_rec_geom(R, rec_geom);
+  if (!rc) rc = conv_run_enqueue(R, st);
+  cudaError_t se = cudaStreamSynchronize(st);
+  cudaFree(wp);
+  if (rc) return rc;
+  CM_CUDA(se);
+  return 0;
+}
+
+int cm_op_gn(const cm_gn_args* a, int32_t* launches, void* stream) {
+  CM_CHECK(a && a->B > 0 && a->pixels > 0, "GroupNorm: empty input");
+  if (int e = kernels_init()) return e;
+  GnParams g{};
+  g.src0 = a->src0; g.c0 = a->c0; g.src1 = a->src1; g.c1 = a->c1;
+  g.gamma = a->gamma; g.beta = a->beta; g.B = a->B; g.pixels = a->pixels; g.eps = a->eps; g.silu = a->silu;
+  g.drop_scale = a->drop_scale; g.drop_ld = a->drop_ld;
+  g.out_norm = static_cast<__half*>(a->out_norm16);
+  g.out_raw = static_cast<__half*>(a->out_raw16);
+  g.dup = a->dup;
+  g.stats = a->stats;
+  g.rec0 = GnRec{a->rec0, a->rec0 ? a->rec0_units : 0, a->rec0 ? a->rec0_nvalid : 0};
+  g.rec1 = GnRec{a->rec1, a->rec1 ? a->rec1_units : 0, a->rec1 ? a->rec1_nvalid : 0};
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  float* partial = nullptr;   // the plan's gn_partial: [B][GN2_MAX_SLICES = 32][8][3]
+  CM_CUDA(cudaMalloc(&partial, (size_t)a->B * 32 * 8 * 3 * sizeof(float)));
+  int nl = 0;
+  const int rc = gn_silu_enqueue(g, partial, st, &nl);
+  cudaError_t se = cudaStreamSynchronize(st);
+  cudaFree(partial);
+  if (launches) *launches = nl;
+  if (rc) return rc;
+  CM_CUDA(se);
+  return 0;
+}
+
+int cm_op_first_conv_packed(const float* x, const float* past, const float* w, const float* bias, int B, int H, int W,
+                            int P, int F, int cin, int cout, int dup, float* out32, void* in16, float* stats_rec,
+                            int32_t* rec_geom, void* stream) {
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (int e = kernels_init()) return e;
+  CM_CHECK(dup == 1 || dup == 2, "dup must be 1 or 2");
+  const int L = P + F;
+  const size_t n16 = (size_t)B * L * H * W * 32 * dup;
+  __half* wp = nullptr;
+  __half* a16 = nullptr;
+  CM_CUDA(cudaMalloc(&wp, (size_t)2 * cout * 27 * 32 * dup * sizeof(__half)));
+  if (cudaMalloc(&a16, n16 * sizeof(__half)) != cudaSuccess) {
+    cudaFree(wp);
+    CM_CHECK(false, "first conv: out of device memory for the packed operand");
+  }
+  // channels cin..31 stay zero (the plan's arena is zero-initialised)
+  int rc = cudaMemsetAsync(a16, 0, n16 * sizeof(__half), st) == cudaSuccess ? 0 : 1;
+  if (!rc) rc = pack_conv_weights_padded(w, wp, cout, cin, 32, 2, 1, st, dup);
+  if (!rc) rc = pack_first_input_enqueue(x, past, a16, B, H, W, P, F, cin, dup, st);
+  ConvEpilogue e{};
+  e.bias = bias;
+  e.out32 = out32;
+  e.lo_from = dup == 2 ? 32 : 0;
+  e.stats_rec = stats_rec;
+  // as prepare_convs: res32 for single fp16 operands, the plane kernel for hi|lo pairs
+  ConvRun R;
+  if (!rc)
+    rc = conv_run_prepare(&R, dup == 1 ? CONV_PLANE | CONV_RES32 : CONV_PLANE, 0, a16, B, L, H, W, 32 * dup, nullptr, 0,
+                          wp, cout, 2, e);
+  if (!rc && !R.covered()) {
+    set_error("first conv: neither the plane nor the res32 kernel covers this grid");
+    rc = 2;
+  }
+  if (!rc) conv_rec_geom(R, rec_geom);
+  if (!rc) rc = conv_run_enqueue(R, st);
+  if (!rc && in16)
+    rc = cudaMemcpyAsync(in16, a16, n16 * sizeof(__half), cudaMemcpyDeviceToDevice, st) == cudaSuccess ? 0 : 1;
+  cudaError_t se = cudaStreamSynchronize(st);
+  cudaFree(wp);
+  cudaFree(a16);
+  if (rc) return rc;
+  CM_CUDA(se);
+  return 0;
+}
+
+int cm_op_temb(const float* table, const float* w1, const float* b1, const float* w2, const float* b2,
+               const void* const* wd, const void* const* bd, const int32_t* couts, const int32_t* offs, int nblocks,
+               int base, int E, const int64_t* t, int rows, float* out, int ld, float* save_e, float* save_h1,
+               float* save_h2, void* stream) {
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  CM_CHECK(nblocks > 0 && rows > 0, "time embedding: empty input");
+  // device tables: wd[nblocks] | bd[nblocks] (8-byte entries), couts | offs (int)
+  const size_t tab_bytes = (size_t)nblocks * (2 * 8 + 2 * 4);
+  char* tmp = nullptr;
+  CM_CUDA(cudaMalloc(&tmp, tab_bytes));
+  std::vector<char> h(tab_bytes);
+  memcpy(h.data(), wd, (size_t)nblocks * 8);
+  memcpy(h.data() + (size_t)nblocks * 8, bd, (size_t)nblocks * 8);
+  memcpy(h.data() + (size_t)nblocks * 16, couts, (size_t)nblocks * 4);
+  memcpy(h.data() + (size_t)nblocks * 20, offs, (size_t)nblocks * 4);
+  TembParams p{};
+  p.table = table; p.w1 = w1; p.b1 = b1; p.w2 = w2; p.b2 = b2;
+  p.wd = reinterpret_cast<const float* const*>(tmp);
+  p.bd = reinterpret_cast<const float* const*>(tmp + (size_t)nblocks * 8);
+  p.couts = reinterpret_cast<const int*>(tmp + (size_t)nblocks * 16);
+  p.offs = reinterpret_cast<const int*>(tmp + (size_t)nblocks * 20);
+  p.nblocks = nblocks;
+  p.base = base; p.E = E;
+  p.t = reinterpret_cast<const long long*>(t);
+  p.rows = rows;
+  p.out = out; p.ld = ld;
+  p.save_e = save_e; p.save_h1 = save_h1; p.save_h2 = save_h2;
+  int rc = cudaMemcpyAsync(tmp, h.data(), tab_bytes, cudaMemcpyHostToDevice, st) == cudaSuccess ? 0 : 1;
+  if (!rc) rc = temb_enqueue(p, st);
+  cudaError_t se = cudaStreamSynchronize(st);
+  cudaFree(tmp);
+  if (rc) return rc;
+  CM_CUDA(se);
+  return 0;
+}
+
 int cm_op_attn_core(const float* qkv, void* ctx16, int B, int S, int C, int heads, void* stream) {
   if (int e = kernels_init()) return e;
   return attn_core_enqueue(qkv, static_cast<__half*>(ctx16), B, S, C, heads,
@@ -174,6 +339,38 @@ int cm_op_final_conv(const void* act16, const float* w, const float* bias, float
   f.w = w; f.bias = bias; f.B = B; f.H = H; f.W = W; f.L = L; f.P = P; f.cin = cin; f.cout = cout;
   f.eps_out = eps_out;
   return final_conv_enqueue(f, static_cast<cudaStream_t>(stream));
+}
+
+int cm_op_final_conv_step(const void* act16, int act_ld, int act_lo, const float* w, const float* bias, float* eps_out,
+                          int B, int H, int W, int L, int P, int cin, int cout, float* x, const float* coef, int nsteps,
+                          int step, int mode, const float* noise, uint64_t seed, int64_t sample_offset, float* history,
+                          void* stream) {
+  if (int e = kernels_init()) return e;
+  CM_CHECK(!x || (nsteps >= 1 && step >= 0 && step < nsteps), "final conv: step %d outside [0, %d)", step, nsteps);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  // the step index and {seed, sample_offset} travel through device memory, as in cm_ddpm_sample
+  unsigned long long* dev = nullptr;
+  CM_CUDA(cudaMalloc(&dev, 3 * sizeof(unsigned long long)));
+  const unsigned long long h[3] = {seed, static_cast<unsigned long long>(sample_offset), static_cast<unsigned long long>(step)};
+  int rc = cudaMemcpyAsync(dev, h, sizeof(h), cudaMemcpyHostToDevice, st) == cudaSuccess ? 0 : 1;
+  FinalParams f{};
+  f.act = static_cast<const __half*>(act16);
+  f.act_ld = act_ld; f.act_lo = act_lo;
+  f.w = w; f.bias = bias; f.B = B; f.H = H; f.W = W; f.L = L; f.P = P; f.cin = cin; f.cout = cout;
+  f.eps_out = eps_out;
+  f.x = x;
+  f.coef = coef;
+  f.step_dev = reinterpret_cast<const int*>(dev + 2);        // low word of a little-endian 64-bit slot
+  f.mode = mode;
+  f.noise = noise;
+  f.chain_dev = dev;
+  f.history = history;
+  if (!rc) rc = final_conv_enqueue(f, st);
+  cudaError_t se = cudaStreamSynchronize(st);
+  cudaFree(dev);
+  if (rc) return rc;
+  CM_CUDA(se);
+  return 0;
 }
 
 

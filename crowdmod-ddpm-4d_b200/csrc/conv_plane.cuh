@@ -110,7 +110,7 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
   uint64_t* tmem_full = empty_bar + PL_MAX_STAGES;         // [2]
   uint64_t* tmem_empty = tmem_full + 2;                    // [2]
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_empty + 2);
-  float* colv = reinterpret_cast<float*>(tail + 256);      // [BN]
+  float* rrow0 = reinterpret_cast<float*>(tail + 256);     // [BN] residual of the unit's first row (GroupNorm records)
   float* side = reinterpret_cast<float*>(tail + 256 + 512);       // [ntiles*4 + 1][3][BN] block-boundary rows
   float* ybuf = side + (P.ntiles * 4 + 1) * 3 * BN;               // [ntiles*128][TLD]
   float* sred = ybuf + (P.ntiles * 128 + 2) * TLD;                // [epilogue warps][BN][2] + [BN] shifts
@@ -389,9 +389,21 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&tmem_empty[buf]);
+      // the threads of store row 0 (et < LPR) hold its residual in rv[0]: shared for the records' shift below (the
+      // previous unit's readers are past the barrier at the end of its read-out)
+      if (P.epi.stats_rec && et < LPR) *reinterpret_cast<float4*>(rrow0 + sub_c) = rv[0];
       asm volatile("bar.sync 1, 512;" ::: "memory");
       // coalesced read-out: RPP rows per pass, LPR lanes per row
-      float4 st1 = make_float4(0.f, 0.f, 0.f, 0.f), st2 = st1;   // GroupNorm partial sums of (v - cv)
+      // GroupNorm records: the sums are shifted by the unit's first value k0 (row 0 of the unit is never a pad column
+      // and needs no `side` rows), a sample of the data, so sum((v - k0)^2) - sum(v - k0)^2 / n does not cancel when
+      // the values share an offset far from the column constants (a residual stream with a DC component)
+      float4 k0 = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (P.epi.stats_rec) {
+        k0 = *reinterpret_cast<const float4*>(ybuf + sub_c);
+        const float4 rk = *reinterpret_cast<const float4*>(rrow0 + sub_c);
+        k0.x += rk.x; k0.y += rk.y; k0.z += rk.z; k0.w += rk.w;
+      }
+      float4 st1 = make_float4(0.f, 0.f, 0.f, 0.f), st2 = st1;   // GroupNorm partial sums of (v - cv - k0)
 #pragma unroll
       for (int j = 0; j < NJ; ++j) {
         if (mi[j] < 0) continue;
@@ -410,9 +422,12 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
           }
         }
         v.x += rv[j].x; v.y += rv[j].y; v.z += rv[j].z; v.w += rv[j].w;
-        st1.x += v.x; st1.y += v.y; st1.z += v.z; st1.w += v.w;
-        st2.x = fmaf(v.x, v.x, st2.x); st2.y = fmaf(v.y, v.y, st2.y);
-        st2.z = fmaf(v.z, v.z, st2.z); st2.w = fmaf(v.w, v.w, st2.w);
+        {
+          const float dx = v.x - k0.x, dy = v.y - k0.y, dz = v.z - k0.z, dw = v.w - k0.w;
+          st1.x += dx; st1.y += dy; st1.z += dz; st1.w += dw;
+          st2.x = fmaf(dx, dx, st2.x); st2.y = fmaf(dy, dy, st2.y);
+          st2.z = fmaf(dz, dz, st2.z); st2.w = fmaf(dw, dw, st2.w);
+        }
         v.x += cv.x; v.y += cv.y; v.z += cv.z; v.w += cv.w;
         const size_t m = static_cast<size_t>(mi[j]);
         if (P.epi.out32) *reinterpret_cast<float4*>(P.epi.out32 + m * P.epi.out_ld + nn0 + sub_c) = v;
@@ -446,7 +461,10 @@ conv_plane_kernel(const __grid_constant__ PlaneParams P) {
           d[0] = st1.x; d[1] = st2.x; d[2] = st1.y; d[3] = st2.y;
           d[4] = st1.z; d[5] = st2.z; d[6] = st1.w; d[7] = st2.w;
         }
-        if (et < LPR) *reinterpret_cast<float4*>(sred + (PL_EPI / 32) * BN * 2 + sub_c) = cv;
+        // the shift: cv + k0 == the stored value of the unit's first row, bit for bit
+        if (et < LPR)
+          *reinterpret_cast<float4*>(sred + (PL_EPI / 32) * BN * 2 + sub_c) =
+              make_float4(k0.x + cv.x, k0.y + cv.y, k0.z + cv.z, k0.w + cv.w);
       }
       asm volatile("bar.sync 1, 512;" ::: "memory");       // ybuf / side are rewritten by the next unit
       if (P.epi.stats_rec && et < BN) {

@@ -342,6 +342,7 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
       if (!cv_const) cv = load_cv(n);
       int mi[NJ];
       float4 rv[NJ];
+      float4 rk = make_float4(0.f, 0.f, 0.f, 0.f);   // residual of the unit's first row (GroupNorm record shift)
       {
         const int base = ((n * P.D + d) * P.H + h0) * P.W;
 #pragma unroll
@@ -351,11 +352,19 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
           if (mi[j] >= 0 && P.epi.resid)
             rv[j] = *reinterpret_cast<const float4*>(P.epi.resid + static_cast<size_t>(mi[j]) * C + sub_c);
         }
+        if (P.epi.stats_rec && P.epi.resid)
+          rk = *reinterpret_cast<const float4*>(P.epi.resid + static_cast<size_t>(base) * C + sub_c);
       }
       if (!mbar_wait(&ybuf_full[buf], (it >> 1) & 1, P.err_flag, 507)) break;
       const float* yb = ybuf + static_cast<size_t>(buf) * 128 * TLD;
       const float* sdb = side + static_cast<size_t>(buf) * 5 * 3 * C;
-      float4 st1 = make_float4(0.f, 0.f, 0.f, 0.f), st2 = st1;   // GroupNorm partial sums of (v - cv)
+      // GroupNorm records are shifted by the unit's first value k0, a sample of the data (see conv_plane_kernel)
+      float4 k0 = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (P.epi.stats_rec) {
+        k0 = *reinterpret_cast<const float4*>(yb + sub_c);
+        k0.x += rk.x; k0.y += rk.y; k0.z += rk.z; k0.w += rk.w;
+      }
+      float4 st1 = make_float4(0.f, 0.f, 0.f, 0.f), st2 = st1;   // GroupNorm partial sums of (v - cv - k0)
 #pragma unroll
       for (int j = 0; j < NJ; ++j) {
         if (mi[j] < 0) continue;
@@ -374,9 +383,12 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
           }
         }
         vv.x += rv[j].x; vv.y += rv[j].y; vv.z += rv[j].z; vv.w += rv[j].w;
-        st1.x += vv.x; st1.y += vv.y; st1.z += vv.z; st1.w += vv.w;
-        st2.x = fmaf(vv.x, vv.x, st2.x); st2.y = fmaf(vv.y, vv.y, st2.y);
-        st2.z = fmaf(vv.z, vv.z, st2.z); st2.w = fmaf(vv.w, vv.w, st2.w);
+        {
+          const float dx = vv.x - k0.x, dy = vv.y - k0.y, dz = vv.z - k0.z, dw = vv.w - k0.w;
+          st1.x += dx; st1.y += dy; st1.z += dz; st1.w += dw;
+          st2.x = fmaf(dx, dx, st2.x); st2.y = fmaf(dy, dy, st2.y);
+          st2.z = fmaf(dz, dz, st2.z); st2.w = fmaf(dw, dw, st2.w);
+        }
         vv.x += cv.x; vv.y += cv.y; vv.z += cv.z; vv.w += cv.w;
         const size_t m = static_cast<size_t>(mi[j]);
         if (P.epi.out32) *reinterpret_cast<float4*>(P.epi.out32 + m * C + sub_c) = vv;
@@ -406,7 +418,9 @@ __global__ void __launch_bounds__(R32_THREADS, 1) conv_res32_kernel(const __grid
           dd[0] = st1.x; dd[1] = st2.x; dd[2] = st1.y; dd[3] = st2.y;
           dd[4] = st1.z; dd[5] = st2.z; dd[6] = st1.w; dd[7] = st2.w;
         }
-        if (st < LPR) *reinterpret_cast<float4*>(cvs + buf * C + sub_c) = cv;
+        // the shift: cv + k0 == the stored value of the unit's first row, bit for bit
+        if (st < LPR)
+          *reinterpret_cast<float4*>(cvs + buf * C + sub_c) = make_float4(k0.x + cv.x, k0.y + cv.y, k0.z + cv.z, k0.w + cv.w);
         asm volatile("bar.sync 2, 256;" ::: "memory");
         if (st < C) {
           float a1 = 0.f, a2 = 0.f;

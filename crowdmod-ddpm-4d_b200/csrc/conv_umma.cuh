@@ -44,7 +44,8 @@ struct ConvEpilogue {
                             // fp16(v - hi) out16_lo elements further (hi|lo pair operand of the training forward)
   // GroupNorm statistics records of the values the launch writes (nullptr = none), plane and res32 kernels only: per
   // (sample, unit of the sample, output channel) a float4 {shift, sum(v - shift), sum((v - shift)^2), 0} over the unit's
-  // valid rows; units belong to ONE sample, so the consumer (gn_apply2_kernel) merges them in a fixed order ->
+  // valid rows, shift = the value the unit's first row stores (a sample of the data: no cancellation in the unit's
+  // variance when the values share a large offset); units belong to ONE sample, so the consumer (gn_apply2_kernel) merges them in a fixed order ->
   // bit-reproducible wherever the sample sits in the batch.
   float* stats_rec;
 };

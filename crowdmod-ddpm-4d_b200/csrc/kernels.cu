@@ -44,10 +44,10 @@ int pack_conv_weights(const float* w, const float* wx, __half* dst, int cout, in
 }
 
 int pack_conv_weights_padded(const float* w, __half* dst, int cout, int cin_src, int cin_packed, int terms,
-                             int perm, cudaStream_t st) {
-  const size_t total = (size_t)cout * 27 * cin_packed;
+                             int perm, cudaStream_t st, int dup) {
+  const size_t total = (size_t)cout * 27 * cin_packed * dup;
   const int blocks = (int)((total + 255) / 256 < 4096 ? (total + 255) / 256 : 4096);
-  pack_conv_weights_kernel<<<blocks, 256, 0, st>>>(w, nullptr, dst, cout, cin_packed, 0, 27, terms, perm, cin_src, 1);
+  pack_conv_weights_kernel<<<blocks, 256, 0, st>>>(w, nullptr, dst, cout, cin_packed, 0, 27, terms, perm, cin_src, dup);
   CM_CUDA(cudaGetLastError());
   return 0;
 }

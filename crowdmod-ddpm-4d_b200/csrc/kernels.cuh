@@ -15,8 +15,9 @@ int pack_conv_weights(const float* w, const float* wx, __half* dst, int cout, in
 // nearest-x2 + k3 conv folded into 8 phase convs with 2x2x2 combined taps
 // (layers.py:92-94).  dst: [terms*cout][64*cin], column = phase*8*cin + tap8*cin + ci.
 // k3 conv weights whose cin_src (< 32) input channels are zero-padded to cin_packed packed channels
+// (dup = 2: against hi|lo pair rows of 2 * cin_packed channels, as pack_conv_weights)
 int pack_conv_weights_padded(const float* w, __half* dst, int cout, int cin_src, int cin_packed, int terms,
-                             int perm, cudaStream_t st);
+                             int perm, cudaStream_t st, int dup = 1);
 // first-conv operand: API tensors -> channels 0..cin-1 of fp16 [B, P+F, H, W, 32] (other channels untouched)
 // dup = 2: rows of 64 (hi | lo halves of the 32 padded channels)
 int pack_first_input_enqueue(const float* x, const float* past, __half* out16, int B, int H, int W, int P, int F,

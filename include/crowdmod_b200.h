@@ -175,6 +175,61 @@ CM_API int cm_op_conv3d(int mode, const void* act16, int B, int D, int H, int W,
 CM_API int cm_op_gn_silu(const float* src0, int c0, const float* src1, int c1, const float* gamma,
                   const float* beta, int B, int pixels, float eps, int silu, void* out_norm16,
                   void* out_raw16, void* stream);
+/* Epilogue of a forward conv as the UNet plan fills it (every field optional, 0 / NULL = off):
+ * out = acc + bias + bias2 + temb row + resid, stored fp32 (out32 [M][cout]) and / or fp16 (out16, rows of out16_ld
+ * elements, 0 -> cout; out16_lo > 0: the lo half fp16(v - hi) out16_lo elements after the hi half).  temb: fp32 table
+ * of rows of temb_ld floats; temb_bstride == 0: the row *t_dev (device int32, NULL: row 0) for every sample
+ * (sampling), else row b * temb_bstride / temb_ld for sample b (training).  lo_from / lo_from_x > 0: channels from
+ * there on of the main / 1x1x1 source are the lo halves of hi|lo operand pairs.  stats_rec: GroupNorm records float4
+ * [B][units][cout] {shift, sum(v - shift), sum((v - shift)^2), 0} (plane / res32 kernels only). */
+typedef struct cm_conv_epilogue {
+  const float* bias;
+  const float* bias2;
+  const float* temb;
+  const int32_t* t_dev;
+  int32_t temb_ld, temb_bstride;
+  const float* resid;
+  float* out32;
+  void* out16;
+  int32_t out16_ld, out16_lo;
+  int32_t lo_from, lo_from_x;
+  float* stats_rec;
+} cm_conv_epilogue;
+/* cm_op_conv3d with the whole epilogue and hi|lo operand pairs: act16 rows hold dup * cin channels (dup = 2: [hi | lo]
+ * of every logical channel), extra16 rows dup * cin_extra; w / wx as cm_op_conv3d, packed for that layout.  impl as
+ * cm_op_conv3d (0 conv_umma, 2 conv_plane, 3 conv_res32; the kernel must cover the conv).  rec_geom (optional
+ * int32[4]) receives the records' geometry: {units per sample, rows per unit, planes per unit R, grid rows per unit
+ * HB}; unit u of a sample covers planes [(u / (H/HB)) * R, +R) and rows [(u % (H/HB)) * HB, +HB), all W columns
+ * ({0, 0, 0, 0} when the launch writes no records). */
+CM_API int cm_op_conv3d_epi(int mode, const void* act16, int B, int D, int H, int W, int cin, const void* extra16,
+                            int cin_extra, int dup, const float* w, const float* wx, int cout, int terms,
+                            const cm_conv_epilogue* epi, int impl, int32_t* rec_geom, void* stream);
+/* GroupNorm(8) (+SiLU) (+Dropout3d scale) -> fp16 operand as the UNet plan runs it (gn_silu_enqueue).  Sources as
+ * cm_op_gn_silu; drop_scale [B][drop_ld] (NULL: none) multiplies after the SiLU; dup = 2: out_norm16 / out_raw16 rows
+ * are [hi | lo] pairs of 2C; stats (NULL: none) [B][8][2] = (mean, rstd); rec0 / rec1 (NULL: none): the producing
+ * convs' records (cm_conv_epilogue::stats_rec, units and rows per unit) -- with records for every source no statistics
+ * pass runs.  *launches (optional): kernels enqueued. */
+typedef struct cm_gn_args {
+  const float* src0;
+  const float* src1;
+  int32_t c0, c1;
+  const float* gamma;
+  const float* beta;
+  int32_t B, pixels;
+  float eps;
+  int32_t silu;
+  const float* drop_scale;
+  int32_t drop_ld;
+  void* out_norm16;
+  void* out_raw16;
+  int32_t dup;
+  float* stats;
+  const float* rec0;
+  int32_t rec0_units, rec0_nvalid;
+  const float* rec1;
+  int32_t rec1_units, rec1_nvalid;
+} cm_gn_args;
+CM_API int cm_op_gn(const cm_gn_args* a, int32_t* launches, void* stream);
 /* attention core softmax(Q K^T / sqrt(dh)) V per (sample, head): qkv fp32 [B][S][3C] (q | k | v), ctx16 fp16 [B][S][C]
  * out.  Any S (S > 128 streams the keys with the online softmax); dh = C / heads even and <= 64. */
 CM_API int cm_op_attn_core(const float* qkv, void* ctx16, int B, int S, int C, int heads, void* stream);
@@ -195,8 +250,32 @@ CM_API int cm_op_attn_block(const float* x, const float* gamma, const float* bet
 CM_API int cm_op_first_conv(const float* x, const float* past, const float* w, const float* bias,
                      float* out, int B, int H, int W, int P, int F, int cin, int cout,
                      void* stream);
+/* The production first conv (unet.py:32,144): future / past (API layout) packed into the fp16 operand [B][P+F][H][W][32 *
+ * dup] (channels cin..31 zero; dup = 2: [hi | lo] rows), then the conv over the weights zero-padded to 32 input
+ * channels on the plane / res32 kernel (an error if neither covers the grid).  out32 [B][P+F][H][W][cout]; in16
+ * (optional) receives the packed operand; stats_rec / rec_geom as cm_op_conv3d_epi. */
+CM_API int cm_op_first_conv_packed(const float* x, const float* past, const float* w, const float* bias, int B, int H,
+                                   int W, int P, int F, int cin, int cout, int dup, float* out32, void* in16,
+                                   float* stats_rec, int32_t* rec_geom, void* stream);
 CM_API int cm_op_final_conv(const void* act16, const float* w, const float* bias, float* eps_out, int B,
                      int H, int W, int L, int P, int cin, int cout, void* stream);
+/* Final conv + reverse-step update (unet.py:121,165-167; ddpm.py:25-38,262-265; guidance.py:4-8) as the sampling chain
+ * runs it: cm_op_final_conv with act_ld (0 -> cin) / act_lo (> 0: hi|lo pair rows, lo at +act_lo); eps_out (NULL:
+ * none); x (NULL: no update), coef, nsteps, step, mode, noise, seed, sample_offset and history as
+ * cm_op_dit_unpatch_step; the step and {seed, sample_offset} are read from device memory, as in a captured chain step. */
+CM_API int cm_op_final_conv_step(const void* act16, int act_ld, int act_lo, const float* w, const float* bias,
+                                 float* eps_out, int B, int H, int W, int L, int P, int cin, int cout, float* x,
+                                 const float* coef, int nsteps, int step, int mode, const float* noise, uint64_t seed,
+                                 int64_t sample_offset, float* history, void* stream);
+/* Time-embedding MLP + every block's dense_1 (embeddings.py:22-34, layers.py:35,62) as temb_kernel runs it: row r of
+ * out [rows][ld] = dense_1 of SiLU(h2) per block (columns offs[k] .. + couts[k]), h2 = Linear(SiLU(h1)), h1 =
+ * Linear(table[t_r]) with t_r = t[r] (device int64, NULL: t_r = r, the sampling table).  table [T][base], w1 [E][base],
+ * w2 [E][E]; wd / bd / couts / offs are HOST arrays [nblocks] (wd / bd: device pointers).  save_e [rows][base] /
+ * save_h1 / save_h2 [rows][E] (NULL: none): the training forward's saves. */
+CM_API int cm_op_temb(const float* table, const float* w1, const float* b1, const float* w2, const float* b2,
+                      const void* const* wd, const void* const* bd, const int32_t* couts, const int32_t* offs,
+                      int nblocks, int base, int E, const int64_t* t, int rows, float* out, int ld, float* save_e,
+                      float* save_h1, float* save_h2, void* stream);
 
 /* Backward op-level entry points.  Geometry arguments describe the FORWARD conv (mode, input
  * grid B,D,H,W, cin, cout); dout16 is the fp16 gradient on the forward output grid.
