@@ -153,6 +153,7 @@ SIGNATURES = {
                                         C.c_int, C.c_void_p, C.c_void_p]),
     "cm_unet_backward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "cm_last_backward_launches": (C.c_int64, [C.c_void_p]),
+    "cm_unet_set_deterministic": (C.c_int, [C.c_void_p, C.c_int]),
     "cm_op_conv3d_dgrad": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                      C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "cm_op_conv3d_dgrad_f32": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
@@ -160,6 +161,9 @@ SIGNATURES = {
     "cm_op_conv3d_wgrad": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                      C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                      C.c_int, C.c_void_p]),
+    "cm_op_conv3d_wgrad_det": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                         C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
+                                         C.c_int, C.c_void_p]),
     "cm_op_conv3d": (C.c_int, [C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int,
                                C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
@@ -194,10 +198,15 @@ SIGNATURES = {
                                              C.c_int, C.c_void_p]),
     "cm_op_cast_colsum": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p,
                                     C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "cm_op_cast_colsum_det": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p,
+                                        C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "cm_op_rowsum_all": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64), C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "cm_op_final_conv_backward": (C.c_int, [C.c_void_p, C.c_float, C.c_void_p, C.c_int, C.c_int] + [C.c_void_p] * 4
                                   + [C.c_int] * 7 + [C.c_void_p, C.c_void_p]),
+    "cm_op_final_conv_backward_det": (C.c_int, [C.c_void_p, C.c_float, C.c_void_p, C.c_int, C.c_int]
+                                      + [C.c_void_p] * 4 + [C.c_int] * 7 + [C.c_void_p, C.c_void_p]),
     "cm_op_first_conv_wgrad": (C.c_int, [C.c_void_p] * 5 + [C.c_int] * 7 + [C.c_void_p]),
+    "cm_op_first_conv_wgrad_det": (C.c_int, [C.c_void_p] * 5 + [C.c_int] * 7 + [C.c_void_p]),
     "cm_op_temb_backward": (C.c_int, [C.c_void_p] * 4 + [C.c_int] * 4
                             + [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_int,
                                C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64)] + [C.c_void_p] * 7),

@@ -1,6 +1,7 @@
 // Library-level C ABI: error reporting, device error flag, op-level entry points used by the
 // unit tests (each wraps one kernel of the hot path; they allocate temporaries and synchronise,
 // the model-level calls in unet.cu do not).
+#include <algorithm>
 #include <cstring>
 #include <mutex>
 #include <string>
@@ -433,15 +434,16 @@ int cm_op_conv3d_dgrad_f32(int mode, const float* dout32, int B, int D, int H, i
   return 0;
 }
 
-int cm_op_conv3d_wgrad(int mode, const void* act16, int B, int D, int H, int W, int cin,
-                       const void* extra16, int cin_extra, const void* dout16, int cout, float* dw,
-                       float* dwx, int impl, void* stream) {
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
+static int conv3d_wgrad(int mode, const void* act16, int B, int D, int H, int W, int cin, const void* extra16,
+                        int cin_extra, const void* dout16, int cout, float* dw, float* dwx, int impl, bool det,
+                        cudaStream_t st) {
   if (int e = kernels_init()) return e;
   if (int e = backward_init()) return e;
   CM_CHECK(mode >= 0 && mode <= 3, "bad forward conv mode %d", mode);
+  CM_CHECK(!det || impl != 1, "the scalar restatement has no deterministic variant");
   const size_t gel = wgrad_g_elems(mode, cin, cin_extra, cout);
   float* G = nullptr;
+  float* part = nullptr;
   CM_CUDA(cudaMalloc(&G, gel * sizeof(float)));
   CM_CUDA(cudaMemsetAsync(G, 0, gel * sizeof(float), st));
   int rc = 0;
@@ -455,7 +457,8 @@ int cm_op_conv3d_wgrad(int mode, const void* act16, int B, int D, int H, int W, 
       cm::set_error("plane wgrad does not cover this shape");
       rc = 1;
     }
-    if (!rc) rc = wgrad_run_enqueue(R, st);
+    if (!rc && det) rc = cudaMalloc(&part, wgrad_run_partial_elems(R) * sizeof(float)) == cudaSuccess ? 0 : 1;
+    if (!rc) rc = wgrad_run_enqueue(R, st, part);
   } else {
     rc = wgrad_ref_enqueue(mode, static_cast<const __half*>(act16), static_cast<const __half*>(extra16),
                            static_cast<const __half*>(dout16), G, B, D, H, W, cin, cin_extra, cout, st);
@@ -463,9 +466,23 @@ int cm_op_conv3d_wgrad(int mode, const void* act16, int B, int D, int H, int W, 
   if (!rc) rc = unpack_wgrad_enqueue(mode, G, dw, dwx, cout, cin, cin_extra, 0, st);
   cudaError_t se = cudaStreamSynchronize(st);
   cudaFree(G);
+  cudaFree(part);
   if (rc) return rc;
   CM_CUDA(se);
   return 0;
+}
+
+int cm_op_conv3d_wgrad(int mode, const void* act16, int B, int D, int H, int W, int cin,
+                       const void* extra16, int cin_extra, const void* dout16, int cout, float* dw,
+                       float* dwx, int impl, void* stream) {
+  return conv3d_wgrad(mode, act16, B, D, H, W, cin, extra16, cin_extra, dout16, cout, dw, dwx, impl, false,
+                      static_cast<cudaStream_t>(stream));
+}
+int cm_op_conv3d_wgrad_det(int mode, const void* act16, int B, int D, int H, int W, int cin,
+                           const void* extra16, int cin_extra, const void* dout16, int cout, float* dw,
+                           float* dwx, int impl, void* stream) {
+  return conv3d_wgrad(mode, act16, B, D, H, W, cin, extra16, cin_extra, dout16, cout, dw, dwx, impl, true,
+                      static_cast<cudaStream_t>(stream));
 }
 
 // ---- fp32 kernels of the training backward (backward.cu), one enqueue function each ----
@@ -519,15 +536,27 @@ int cm_op_gn_backward(const float* src0, int c0, const float* src1, int c1, cons
   return 0;
 }
 
-int cm_op_cast_colsum(const float* src, void* dst16, int dup, float* acc_dst, int acc_init, float* colsum,
-                      int colsum_ld, int B, int pixels, int C, void* stream) {
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
+static int cast_colsum(const float* src, void* dst16, int dup, float* acc_dst, int acc_init, float* colsum,
+                       int colsum_ld, int B, int pixels, int C, bool det, cudaStream_t st) {
+  float* part = nullptr;
+  if (det) CM_CUDA(cudaMalloc(&part, cast_colsum_partial_elems(B, pixels, C) * sizeof(float)));
   const int rc = cast_colsum_enqueue(src, static_cast<__half*>(dst16), dup, acc_dst, acc_init, colsum, colsum_ld, B,
-                                     pixels, C, st);
+                                     pixels, C, st, part);
   cudaError_t se = cudaStreamSynchronize(st);
+  cudaFree(part);
   if (rc) return rc;
   CM_CUDA(se);
   return 0;
+}
+int cm_op_cast_colsum(const float* src, void* dst16, int dup, float* acc_dst, int acc_init, float* colsum,
+                      int colsum_ld, int B, int pixels, int C, void* stream) {
+  return cast_colsum(src, dst16, dup, acc_dst, acc_init, colsum, colsum_ld, B, pixels, C, false,
+                     static_cast<cudaStream_t>(stream));
+}
+int cm_op_cast_colsum_det(const float* src, void* dst16, int dup, float* acc_dst, int acc_init, float* colsum,
+                          int colsum_ld, int B, int pixels, int C, void* stream) {
+  return cast_colsum(src, dst16, dup, acc_dst, acc_init, colsum, colsum_ld, B, pixels, C, true,
+                     static_cast<cudaStream_t>(stream));
 }
 
 int cm_op_rowsum_all(const float* base, const int64_t* tab, int n, int B, float* grads, void* stream) {
@@ -544,10 +573,9 @@ int cm_op_rowsum_all(const float* base, const int64_t* tab, int n, int B, float*
   return 0;
 }
 
-int cm_op_final_conv_backward(const float* deps, float scale, const void* act16, int act_ld, int act_lo,
-                              const float* w, float* dact, float* dw, float* db, int B, int H, int W, int L, int P,
-                              int cin, int cout, void* dout16, void* stream) {
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
+static int final_conv_backward(const float* deps, float scale, const void* act16, int act_ld, int act_lo,
+                               const float* w, float* dact, float* dw, float* db, int B, int H, int W, int L, int P,
+                               int cin, int cout, void* dout16, bool det, cudaStream_t st) {
   if (int e = kernels_init()) return e;
   if (int e = backward_init()) return e;
   const __half* act = static_cast<const __half*>(act16);
@@ -574,29 +602,58 @@ int cm_op_final_conv_backward(const float* deps, float scale, const void* act16,
       rc = 2;
     }
   }
+  float* part = nullptr;
+  if (!rc && det) {
+    size_t n = final_conv_partial_elems(B, H, W, L, P, cin, cout, d16 != nullptr);
+    if (d16) n = std::max(n, wgrad_run_partial_elems(R));
+    rc = cudaMalloc(&part, n * sizeof(float)) == cudaSuccess ? 0 : 1;
+  }
   if (!rc)
     rc = final_conv_backward_enqueue(deps, scale_dev, act, act_ld, act_lo, w, dact, dw, db, B, H, W, L, P, cin, cout,
-                                     d16, st);
-  if (!rc && d16) rc = wgrad_run_enqueue(R, st);
+                                     d16, st, part);
+  if (!rc && d16) rc = wgrad_run_enqueue(R, st, part);
   if (!rc && d16) rc = unpack_wgrad_enqueue(0, G, dw, nullptr, cout | (32 << 16), cin, 0, 1, st);
   cudaError_t se = cudaStreamSynchronize(st);
   cudaFree(tmp);
+  cudaFree(part);
   if (rc) return rc;
   CM_CUDA(se);
   return 0;
 }
+int cm_op_final_conv_backward(const float* deps, float scale, const void* act16, int act_ld, int act_lo,
+                              const float* w, float* dact, float* dw, float* db, int B, int H, int W, int L, int P,
+                              int cin, int cout, void* dout16, void* stream) {
+  return final_conv_backward(deps, scale, act16, act_ld, act_lo, w, dact, dw, db, B, H, W, L, P, cin, cout, dout16,
+                             false, static_cast<cudaStream_t>(stream));
+}
+int cm_op_final_conv_backward_det(const float* deps, float scale, const void* act16, int act_ld, int act_lo,
+                                  const float* w, float* dact, float* dw, float* db, int B, int H, int W, int L, int P,
+                                  int cin, int cout, void* dout16, void* stream) {
+  return final_conv_backward(deps, scale, act16, act_ld, act_lo, w, dact, dw, db, B, H, W, L, P, cin, cout, dout16,
+                             true, static_cast<cudaStream_t>(stream));
+}
 
-int cm_op_first_conv_wgrad(const float* x, const float* past, const float* dout, float* dw, float* db, int B, int H,
-                           int W, int P, int F, int cin, int cout, void* stream) {
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
+static int first_conv_wgrad(const float* x, const float* past, const float* dout, float* dw, float* db, int B, int H,
+                            int W, int P, int F, int cin, int cout, bool det, cudaStream_t st) {
   if (int e = backward_init()) return e;
   CM_CUDA(cudaMemsetAsync(dw, 0, (size_t)cout * cin * 27 * sizeof(float), st));
   CM_CUDA(cudaMemsetAsync(db, 0, cout * sizeof(float), st));
-  const int rc = first_conv_wgrad_enqueue(x, past, dout, dw, db, B, H, W, P, F, cin, cout, st);
+  float* part = nullptr;
+  if (det) CM_CUDA(cudaMalloc(&part, first_conv_partial_elems(B, H, W, P, F, cin, cout) * sizeof(float)));
+  const int rc = first_conv_wgrad_enqueue(x, past, dout, dw, db, B, H, W, P, F, cin, cout, st, part);
   cudaError_t se = cudaStreamSynchronize(st);
+  cudaFree(part);
   if (rc) return rc;
   CM_CUDA(se);
   return 0;
+}
+int cm_op_first_conv_wgrad(const float* x, const float* past, const float* dout, float* dw, float* db, int B, int H,
+                           int W, int P, int F, int cin, int cout, void* stream) {
+  return first_conv_wgrad(x, past, dout, dw, db, B, H, W, P, F, cin, cout, false, static_cast<cudaStream_t>(stream));
+}
+int cm_op_first_conv_wgrad_det(const float* x, const float* past, const float* dout, float* dw, float* db, int B,
+                               int H, int W, int P, int F, int cin, int cout, void* stream) {
+  return first_conv_wgrad(x, past, dout, dw, db, B, H, W, P, F, cin, cout, true, static_cast<cudaStream_t>(stream));
 }
 
 int cm_op_temb_backward(const float* e, const float* h1, const float* h2, const float* dtemb, int ld, int B, int base,

@@ -104,6 +104,8 @@ int auto_scale_enqueue(const float* x, size_t n, float target, float* scale_dev,
 // =============================================================================================
 // dOut preparation: fp32 -> fp16 operand (+ residual fan-out, per-sample channel sums)
 // =============================================================================================
+// DET: colsum is the [chunks][B][C] partial table, one plain store per (CTA, channel)
+template <bool DET>
 __global__ void __launch_bounds__(1024)
 cast_colsum_kernel(const float* __restrict__ src, __half* __restrict__ dst16, int dup, float* __restrict__ acc_dst,
                    int acc_init, float* __restrict__ colsum, int colsum_ld, int pixels, int C, int chunks,
@@ -163,6 +165,10 @@ cast_colsum_kernel(const float* __restrict__ src, __half* __restrict__ dst16, in
       const float4 v = reinterpret_cast<float4*>(red)[r];
       a.x += v.x; a.y += v.y; a.z += v.z; a.w += v.w;
     }
+    if constexpr (DET) {
+      *reinterpret_cast<float4*>(colsum + ((size_t)chunk * gridDim.y + b) * C + tid * 4) = a;
+      return;
+    }
     float* cp = colsum + (size_t)b * colsum_ld + tid * 4;
     atomicAdd(cp + 0, a.x);
     atomicAdd(cp + 1, a.y);
@@ -171,19 +177,48 @@ cast_colsum_kernel(const float* __restrict__ src, __half* __restrict__ dst16, in
   }
 }
 
-int cast_colsum_enqueue(const float* src, __half* dst16, int dup, float* acc_dst, int acc_init, float* colsum,
-                        int colsum_ld, int B, int pixels, int C, cudaStream_t st) {
-  CM_CHECK(C % 4 == 0 && C / 4 <= 1024, "cast_colsum: bad channel count %d", C);
-  CM_CHECK(dup == 1 || dup == 2, "cast_colsum: dup must be 1 or 2");
-  const int Q = C / 4;
-  const int T = sweep_threads(Q);
+static int cast_colsum_chunks(int B, int pixels) {
   int chunks = 592 / B;
   if (chunks < 1) chunks = 1;
   if (chunks > (pixels + 7) / 8) chunks = (pixels + 7) / 8;
   if (chunks < 1) chunks = 1;
-  cast_colsum_kernel<<<dim3(chunks, B), T, (size_t)T * 16, st>>>(src, dst16, dup, acc_dst, acc_init, colsum,
-                                                                colsum_ld, pixels, C, chunks,
-                                                                device_error_flag());
+  return chunks;
+}
+
+size_t cast_colsum_partial_elems(int B, int pixels, int C) { return (size_t)cast_colsum_chunks(B, pixels) * B * C; }
+
+int cast_colsum_enqueue(const float* src, __half* dst16, int dup, float* acc_dst, int acc_init, float* colsum,
+                        int colsum_ld, int B, int pixels, int C, cudaStream_t st, float* part) {
+  CM_CHECK(C % 4 == 0 && C / 4 <= 1024, "cast_colsum: bad channel count %d", C);
+  CM_CHECK(dup == 1 || dup == 2, "cast_colsum: dup must be 1 or 2");
+  const int Q = C / 4;
+  const int T = sweep_threads(Q);
+  const int chunks = cast_colsum_chunks(B, pixels);
+  if (part && colsum) {
+    cast_colsum_kernel<true><<<dim3(chunks, B), T, (size_t)T * 16, st>>>(src, dst16, dup, acc_dst, acc_init, part, 0,
+                                                                        pixels, C, chunks, device_error_flag());
+    CM_CUDA(cudaGetLastError());
+    return sum_partials_enqueue(part, chunks, (size_t)B * C, (size_t)B * C, C, colsum_ld, colsum, 1, st);
+  }
+  cast_colsum_kernel<false><<<dim3(chunks, B), T, (size_t)T * 16, st>>>(src, dst16, dup, acc_dst, acc_init, colsum,
+                                                                       colsum_ld, pixels, C, chunks,
+                                                                       device_error_flag());
+  CM_CUDA(cudaGetLastError());
+  return 0;
+}
+
+__global__ void sum_partials_kernel(const float* __restrict__ part, int nsplit, size_t stride, size_t n, size_t seg,
+                                    size_t dst_ld, float* __restrict__ dst, int accumulate) {
+  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+    float a = 0.f;
+    for (int s = 0; s < nsplit; ++s) a += part[(size_t)s * stride + i];
+    float* d = dst + (i / seg) * dst_ld + i % seg;
+    *d = accumulate ? *d + a : a;
+  }
+}
+int sum_partials_enqueue(const float* part, int nsplit, size_t stride, size_t n, size_t seg, size_t dst_ld, float* dst,
+                         int accumulate, cudaStream_t st) {
+  sum_partials_kernel<<<grid_for(n, 256, 4096), 256, 0, st>>>(part, nsplit, stride, n, seg, dst_ld, dst, accumulate);
   CM_CUDA(cudaGetLastError());
   return 0;
 }
@@ -808,7 +843,8 @@ final_conv_dact_kernel(const float* __restrict__ deps, const float* __restrict__
   }
 }
 
-template <int COUT>
+// DET: dw is the per-CTA partial table [CTA][COUT * cin * 27 + COUT] (dw layout, then db), plain stores
+template <int COUT, bool DET>
 __global__ void __launch_bounds__(256)
 final_conv_wgrad_kernel(const float* __restrict__ deps, const float* __restrict__ scale_dev,
                         const __half* __restrict__ act, int ald, int alo, float* __restrict__ dw,
@@ -880,22 +916,35 @@ final_conv_wgrad_kernel(const float* __restrict__ deps, const float* __restrict_
       }
     }
   }
+  if constexpr (DET) {
+    dw += (size_t)blockIdx.x * (COUT * npairs + COUT);
+    db = dw + (size_t)COUT * npairs;
+  }
 #pragma unroll
   for (int k = 0; k < MAXP; ++k) {
     const int pr = threadIdx.x + k * 256;
     if (pr >= npairs) break;
     const int tap = pr / cin, ci = pr - tap * cin;
 #pragma unroll
-    for (int co = 0; co < COUT; ++co) atomicAdd(dw + ((size_t)co * cin + ci) * 27 + tap, acc[k][co]);
+    for (int co = 0; co < COUT; ++co) {
+      float* p = dw + ((size_t)co * cin + ci) * 27 + tap;
+      if constexpr (DET) *p = acc[k][co];
+      else atomicAdd(p, acc[k][co]);
+    }
   }
   if (threadIdx.x == 0) {
 #pragma unroll
-    for (int co = 0; co < COUT; ++co) atomicAdd(db + co, bacc[co]);
+    for (int co = 0; co < COUT; ++co) {
+      if constexpr (DET) db[co] = bacc[co];
+      else atomicAdd(db + co, bacc[co]);
+    }
   }
 }
 
 // d_eps * scale -> columns 0 .. cout-1 of the fp16 dOut operand [B][L][H][W][32] of the plane weight-gradient kernel (future
-// frames only; everything else in the buffer stays zero) and the bias gradient (block sums, one atomic per CTA and channel)
+// frames only; everything else in the buffer stays zero) and the bias gradient (block sums, one atomic per CTA and channel;
+// DET: db is the partial table [CTA][4], plain stores)
+template <bool DET>
 __global__ void __launch_bounds__(256)
 pack_final_dout_kernel(const float* __restrict__ deps, const float* __restrict__ scale_dev, __half* __restrict__ out,
                        float* __restrict__ db, int B, int H, int W, int L, int P, int cout) {
@@ -938,17 +987,33 @@ pack_final_dout_kernel(const float* __restrict__ deps, const float* __restrict__
   if (threadIdx.x < cout) {
     float a = 0.f;
     for (int k = 0; k < 8; ++k) a += red[k][threadIdx.x];
-    atomicAdd(db + threadIdx.x, a);
+    if constexpr (DET) db[blockIdx.x * 4 + threadIdx.x] = a;
+    else atomicAdd(db + threadIdx.x, a);
   }
 }
 
 constexpr int FCB_MAX_CIN = 256;   // the data-gradient kernel keeps all 27 * cin * cout weights in shared memory
+constexpr int FCB_PACK_CTAS = 592;  // pack_final_dout_kernel's grid
+
+static int final_wgrad_ppc(int B, int H, int W, int L, int P) {
+  const size_t opix = (size_t)B * H * W * (L - P);
+  return (int)((opix + 591) / 592);
+}
+static int final_wgrad_ctas(int B, int H, int W, int L, int P) {
+  const size_t opix = (size_t)B * H * W * (L - P);
+  const int ppc = final_wgrad_ppc(B, H, W, L, P);
+  return (int)((opix + ppc - 1) / ppc);
+}
+size_t final_conv_partial_elems(int B, int H, int W, int L, int P, int cin, int cout, bool packed) {
+  if (packed) return (size_t)FCB_PACK_CTAS * 4;
+  return (size_t)final_wgrad_ctas(B, H, W, L, P) * ((size_t)cout * cin * 27 + cout);
+}
 
 // dout16 != nullptr: the weight gradient is left to the caller's launch over dout16 (filled here, with the bias
 // gradient); nullptr: the SIMT weight-gradient kernel (cin <= 64)
 int final_conv_backward_enqueue(const float* deps, const float* scale_dev, const __half* act, int act_ld, int act_lo,
                                 const float* w, float* dact, float* dw, float* db, int B, int H, int W,
-                                int L, int P, int cin, int cout, __half* dout16, cudaStream_t st) {
+                                int L, int P, int cin, int cout, __half* dout16, cudaStream_t st, float* part) {
   const int ald = act_ld > 0 ? act_ld : cin;
   CM_CHECK(cout >= 1 && cout <= 4, "final conv supports 1..4 output channels (got %d)", cout);
   CM_CHECK(cin % 32 == 0 && cin <= FCB_MAX_CIN && (dout16 || 27 * cin <= 2048),
@@ -957,20 +1022,29 @@ int final_conv_backward_enqueue(const float* deps, const float* scale_dev, const
   const size_t total = (size_t)B * L * H * W * (cin / 8);
   const int blocks = grid_for(total, 256, 148 * 16);
   const size_t smem = (size_t)27 * cin * cout * sizeof(float);
-  const size_t opix = (size_t)B * H * W * (L - P);
-  const int ppc = (int)((opix + 591) / 592);
-  const int wblocks = (int)((opix + ppc - 1) / ppc);
+  const int ppc = final_wgrad_ppc(B, H, W, L, P);
+  const int wblocks = final_wgrad_ctas(B, H, W, L, P);
 #define CM_FB(CO)                                                                                   \
   case CO:                                                                                          \
     final_conv_dact_kernel<CO><<<blocks, 256, smem, st>>>(deps, scale_dev, w, dact, B, H, W, L, P, cin); \
-    if (dout16)                                                                                     \
-      pack_final_dout_kernel<<<592, 256, 0, st>>>(deps, scale_dev, dout16, db, B, H, W, L, P, cout); \
+    if (dout16 && part)                                                                             \
+      pack_final_dout_kernel<true><<<FCB_PACK_CTAS, 256, 0, st>>>(deps, scale_dev, dout16, part, B, H, W, L, P, cout); \
+    else if (dout16)                                                                                \
+      pack_final_dout_kernel<false><<<FCB_PACK_CTAS, 256, 0, st>>>(deps, scale_dev, dout16, db, B, H, W, L, P, cout); \
+    else if (part)                                                                                  \
+      final_conv_wgrad_kernel<CO, true><<<wblocks, 256, 0, st>>>(deps, scale_dev, act, ald, act_lo, part, nullptr, B, H, W, L, P, cin, ppc); \
     else                                                                                            \
-      final_conv_wgrad_kernel<CO><<<wblocks, 256, 0, st>>>(deps, scale_dev, act, ald, act_lo, dw, db, B, H, W, L, P, cin, ppc); \
+      final_conv_wgrad_kernel<CO, false><<<wblocks, 256, 0, st>>>(deps, scale_dev, act, ald, act_lo, dw, db, B, H, W, L, P, cin, ppc); \
     break;
   switch (cout) { CM_FB(1) CM_FB(2) CM_FB(3) CM_FB(4) }
 #undef CM_FB
   CM_CUDA(cudaGetLastError());
+  if (part && dout16) return sum_partials_enqueue(part, FCB_PACK_CTAS, 4, cout, cout, 0, db, 0, st);
+  if (part) {
+    const size_t nw = (size_t)cout * cin * 27;
+    if (int e = sum_partials_enqueue(part, wblocks, nw + cout, nw, nw, 0, dw, 0, st)) return e;
+    return sum_partials_enqueue(part + nw, wblocks, nw + cout, cout, cout, 0, db, 0, st);
+  }
   return 0;
 }
 
@@ -986,6 +1060,8 @@ constexpr int FW_PIX = 192;     // pixels per chunk
 constexpr int FW_THREADS = 288; // 9 warps x 12 k's
 constexpr int FW_KP = 108;      // padded K = 27 * 4 input channels
 
+// DET: dw is the per-CTA partial table [CTA][cout * K + cout] (dw layout, then db), plain stores
+template <bool DET>
 __global__ void __launch_bounds__(FW_THREADS)
 first_conv_wgrad_kernel(const float* __restrict__ x, const float* __restrict__ past,
                         const float* __restrict__ dout, float* __restrict__ dw, float* __restrict__ db,
@@ -1005,6 +1081,10 @@ first_conv_wgrad_kernel(const float* __restrict__ x, const float* __restrict__ p
 #pragma unroll
     for (int j = 0; j < 12; ++j) acc[g][j] = 0.f;
   const int ngrp = cout / 32;
+  if constexpr (DET) {
+    dw += (size_t)blockIdx.x * ((size_t)cout * K + cout);
+    db = dw + (size_t)cout * K;
+  }
   for (int chunk = blockIdx.x; chunk < nchunks; chunk += gridDim.x) {
     const size_t pix = (size_t)chunk * FW_PIX + tid;
     __syncthreads();                     // previous chunk fully consumed
@@ -1070,28 +1150,52 @@ first_conv_wgrad_kernel(const float* __restrict__ x, const float* __restrict__ p
 #pragma unroll
     for (int j = 0; j < 12; ++j) {
       const int k = warp * 12 + j;
-      if (k < K) atomicAdd(dw + (size_t)co * K + k, acc[g][j]);
+      if (k >= K) continue;
+      if constexpr (DET) dw[(size_t)co * K + k] = acc[g][j];
+      else atomicAdd(dw + (size_t)co * K + k, acc[g][j]);
     }
-    if (warp == 8) atomicAdd(db + co, bacc[g]);
+    if (warp == 8) {
+      if constexpr (DET) db[co] = bacc[g];
+      else atomicAdd(db + co, bacc[g]);
+    }
   }
 }
 
+static int first_wgrad_ctas(int B, int H, int W, int P, int F) {
+  const size_t total = (size_t)B * (P + F) * H * W;
+  const int nchunks = (int)((total + FW_PIX - 1) / FW_PIX);
+  return nchunks < 296 ? nchunks : 296;
+}
+size_t first_conv_partial_elems(int B, int H, int W, int P, int F, int cin, int cout) {
+  return (size_t)first_wgrad_ctas(B, H, W, P, F) * ((size_t)cout * 27 * cin + cout);
+}
+
 int first_conv_wgrad_enqueue(const float* x, const float* past, const float* dout, float* dw, float* db,
-                             int B, int H, int W, int P, int F, int cin, int cout, cudaStream_t st) {
+                             int B, int H, int W, int P, int F, int cin, int cout, cudaStream_t st, float* part) {
   CM_CHECK(cout == 32 || cout == 64, "first conv wgrad: cout must be 32 or 64 (got %d)", cout);
   CM_CHECK(27 * cin <= FW_KP, "first conv wgrad: at most 4 input channels (got %d)", cin);
   const size_t total = (size_t)B * (P + F) * H * W;
   const int nchunks = (int)((total + FW_PIX - 1) / FW_PIX);
-  const int blocks = nchunks < 296 ? nchunks : 296;
+  const int blocks = first_wgrad_ctas(B, H, W, P, F);
   const size_t smem = ((size_t)FW_PIX * FW_KP + (size_t)FW_PIX * (cout + 1)) * sizeof(float);
   static bool attr = false;
   if (!attr) {
-    CM_CUDA(cudaFuncSetAttribute(first_conv_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 180 * 1024));
+    CM_CUDA(cudaFuncSetAttribute(first_conv_wgrad_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 180 * 1024));
+    CM_CUDA(cudaFuncSetAttribute(first_conv_wgrad_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 180 * 1024));
     attr = true;
   }
-  first_conv_wgrad_kernel<<<blocks, FW_THREADS, smem, st>>>(x, past, dout, dw, db, B, H, W, P, F, cin, cout, nchunks);
+  if (!part) {
+    first_conv_wgrad_kernel<false><<<blocks, FW_THREADS, smem, st>>>(x, past, dout, dw, db, B, H, W, P, F, cin, cout,
+                                                                     nchunks);
+    CM_CUDA(cudaGetLastError());
+    return 0;
+  }
+  first_conv_wgrad_kernel<true><<<blocks, FW_THREADS, smem, st>>>(x, past, dout, part, nullptr, B, H, W, P, F, cin, cout,
+                                                                  nchunks);
   CM_CUDA(cudaGetLastError());
-  return 0;
+  const size_t nw = (size_t)cout * 27 * cin;
+  if (int e = sum_partials_enqueue(part, blocks, nw + cout, nw, nw, 0, dw, 0, st)) return e;
+  return sum_partials_enqueue(part + nw, blocks, nw + cout, cout, cout, 0, db, 0, st);
 }
 
 // =============================================================================================

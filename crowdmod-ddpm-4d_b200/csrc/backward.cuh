@@ -34,8 +34,15 @@ int auto_scale_enqueue(const float* x, size_t n, float target, float* scale_dev,
 //      residual fan-out (acc_dst (=|+=) src) and per-sample channel sums (bias / time-embedding
 //      projection gradients): colsum[b*colsum_ld + c] += sum_p src[b][p][c].  dup = 2: dst16 is the
 //      K-concatenated hi|lo pair [pixel][2C] (dgrad reads both halves, wgrad the hi half) ----
+// part != nullptr (deterministic): every CTA stores its channel sums into part [chunks][B][C] and one more launch adds
+// them to colsum in chunk order, instead of one atomicAdd per (CTA, channel); part holds cast_colsum_partial_elems.
 int cast_colsum_enqueue(const float* src, __half* dst16, int dup, float* acc_dst, int acc_init, float* colsum,
-                        int colsum_ld, int B, int pixels, int C, cudaStream_t st);
+                        int colsum_ld, int B, int pixels, int C, cudaStream_t st, float* part = nullptr);
+size_t cast_colsum_partial_elems(int B, int pixels, int C);
+// The ordered sum of deterministic reductions: for i < n, dst[(i / seg) * dst_ld + i % seg] (=, or += when
+// accumulate) sum over s = 0, 1, ..., nsplit - 1 of part[s * stride + i], added in that order.
+int sum_partials_enqueue(const float* part, int nsplit, size_t stride, size_t n, size_t seg, size_t dst_ld, float* dst,
+                         int accumulate, cudaStream_t st);
 // out[c] (+)= sum_b in[b*ld + c]
 int rowsum_enqueue(const float* in, float* out, int B, int C, int ld, int accumulate, cudaStream_t st);
 
@@ -91,13 +98,20 @@ int attn_long_backward_enqueue(const float* qkv, const float* dctx, const float*
 // act: fp16 [B][L][H][W][act_ld] (act_ld 0 -> cin); act_lo > 0: hi|lo pair rows, the lo half is added
 // dout16 != nullptr: dw is left to the caller, which runs a conv weight gradient over dout16 (fp16 [B][L][H][W][32],
 // d_eps * scale in columns 0 .. cout-1); cin <= 64 without it, <= 256 with it
+// part != nullptr (deterministic): per-CTA partial sums into part (final_conv_partial_elems), dw / db (=) their sums
+// in CTA order
 int final_conv_backward_enqueue(const float* deps, const float* scale_dev, const __half* act, int act_ld, int act_lo,
                                 const float* w, float* dact, float* dw, float* db, int B, int H, int W,
-                                int L, int P, int cin, int cout, __half* dout16, cudaStream_t st);
+                                int L, int P, int cin, int cout, __half* dout16, cudaStream_t st,
+                                float* part = nullptr);
+size_t final_conv_partial_elems(int B, int H, int W, int L, int P, int cin, int cout, bool packed);
 // ---- first conv weight / bias gradient (unet.py:32; inputs need no gradient) ----
-// dout fp32 [B][L][H][W][cout]; dw [cout][cin][27], db [cout] accumulated with atomics.
+// dout fp32 [B][L][H][W][cout]; dw [cout][cin][27], db [cout] accumulated with atomics, or with part != nullptr
+// (deterministic) (=) the CTA-ordered sums of per-CTA partials in part (first_conv_partial_elems).
 int first_conv_wgrad_enqueue(const float* x, const float* past, const float* dout, float* dw, float* db,
-                             int B, int H, int W, int P, int F, int cin, int cout, cudaStream_t st);
+                             int B, int H, int W, int P, int F, int cin, int cout, cudaStream_t st,
+                             float* part = nullptr);
+size_t first_conv_partial_elems(int B, int H, int W, int P, int F, int cin, int cout);
 
 // ---- time-embedding MLP backward helpers (embeddings.py:22-34; layers.py:35,62) ----
 // C[m][n] (=|+=) sum_k A(m,k) * B(k,n) with arbitrary element strides (tiny matrices only)

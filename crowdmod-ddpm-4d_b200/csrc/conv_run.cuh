@@ -44,7 +44,10 @@ struct WgradRun {
 int wgrad_run_prepare(WgradRun* R, unsigned kinds, int mode, const __half* act, int B, int D, int H, int W, int cin,
                       const __half* extra, int cin_extra, const __half* dout, int cout, float* G, int dout_ld = 0,
                       int act_ld = 0, int extra_ld = 0);
-int wgrad_run_enqueue(const WgradRun& R, cudaStream_t st);
+// part != nullptr: the deterministic variant (per-CTA / per-split partials in part, summed in a fixed order into G;
+// two launches per kernel launch); part holds wgrad_run_partial_elems(R) floats.
+int wgrad_run_enqueue(const WgradRun& R, cudaStream_t st, float* part = nullptr);
+size_t wgrad_run_partial_elems(const WgradRun& R);
 
 // Which kernels may take the weight gradient of the first conv (c = its cout) or the final conv (c = its cin) as a conv
 // weight gradient over the packed fp16 operands (wgrad_run).  0: the SIMT kernels of backward.cu, which cover 32 and 64

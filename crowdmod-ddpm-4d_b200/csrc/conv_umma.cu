@@ -4,6 +4,10 @@
 #include <cudaTypedefs.h>
 #include <string.h>
 
+#include <algorithm>
+
+#include "backward.cuh"
+
 namespace cm {
 
 namespace {
@@ -561,26 +565,31 @@ int res32_enqueue(const Res32Launch& L, cudaStream_t st) {
 // ================================ weight gradient (wgrad_umma.cuh) ================================
 namespace {
 
-template <int BKC, int BNC, int BN>
+template <int BKC, int BNC, int BN, bool DET>
 int wg_launch_t(const WgradLaunch& L, cudaStream_t st) {
-  wgrad_umma_kernel<BKC, BNC, BN><<<L.grid, WG_THREADS, L.smem, st>>>(L.p);
+  wgrad_umma_kernel<BKC, BNC, BN, DET><<<L.grid, WG_THREADS, L.smem, st>>>(L.p);
   CM_CUDA(cudaGetLastError());
   return 0;
 }
 template <int BKC, int BNC, int BN>
 int wg_attr_t() {
-  CM_CUDA(cudaFuncSetAttribute(wgrad_umma_kernel<BKC, BNC, BN>,
+  CM_CUDA(cudaFuncSetAttribute(wgrad_umma_kernel<BKC, BNC, BN, false>,
+                               cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+  CM_CUDA(cudaFuncSetAttribute(wgrad_umma_kernel<BKC, BNC, BN, true>,
                                cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
   return 0;
 }
-template <int BKC>
+template <int BKC, bool DET>
 int wg_dispatch(const WgradLaunch& L, cudaStream_t st) {
-  if (L.bnc == 32) return wg_launch_t<BKC, 32, 32>(L, st);
+  if (L.bnc == 32) return wg_launch_t<BKC, 32, 32, DET>(L, st);
   switch (L.bn) {
-    case 64: return wg_launch_t<BKC, 64, 64>(L, st);
-    case 128: return wg_launch_t<BKC, 64, 128>(L, st);
-    default: return wg_launch_t<BKC, 64, 256>(L, st);
+    case 64: return wg_launch_t<BKC, 64, 64, DET>(L, st);
+    case 128: return wg_launch_t<BKC, 64, 128, DET>(L, st);
+    default: return wg_launch_t<BKC, 64, 256, DET>(L, st);
   }
+}
+int wg_enqueue_det(const WgradLaunch& L, cudaStream_t st) {
+  return L.bkc == 64 ? wg_dispatch<64, true>(L, st) : wg_dispatch<32, true>(L, st);
 }
 
 }  // namespace
@@ -754,13 +763,14 @@ int wgrad_plane_prepare(WgradPlaneLaunch* L, const __half* act, int B, int D, in
   int n_sm = 148;
   cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, 0);
   L->grid = dim3(p.n_units < n_sm ? p.n_units : n_sm, 1, 1);
+  L->det_ctas = p.n_units < WP_DET_CTAS ? p.n_units : WP_DET_CTAS;
   L->smem = (size_t)stages * p.stage_bytes + 1024 + 256;
   L->ok = true;
   return 0;
 }
 
 int wgrad_plane_enqueue(const WgradPlaneLaunch& L, cudaStream_t st) {
-  wgrad_plane_kernel<32><<<L.grid, WP_THREADS, L.smem, st>>>(L.p);
+  wgrad_plane_kernel<32, false><<<L.grid, WP_THREADS, L.smem, st>>>(L.p);
   CM_CUDA(cudaGetLastError());
   return 0;
 }
@@ -768,14 +778,15 @@ int wgrad_plane_enqueue(const WgradPlaneLaunch& L, cudaStream_t st) {
 int wgrad_plane_init() {
   static bool done = false;
   if (done) return 0;
-  CM_CUDA(cudaFuncSetAttribute(wgrad_plane_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+  CM_CUDA(cudaFuncSetAttribute(wgrad_plane_kernel<32, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+  CM_CUDA(cudaFuncSetAttribute(wgrad_plane_kernel<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
   done = true;
   return 0;
 }
 
 int wgrad_enqueue(const WgradLaunch& L, cudaStream_t st) {
-  if (L.bkc == 64) return wg_dispatch<64>(L, st);
-  return wg_dispatch<32>(L, st);
+  if (L.bkc == 64) return wg_dispatch<64, false>(L, st);
+  return wg_dispatch<32, false>(L, st);
 }
 
 // ================================ kernel choice (conv_run.cuh) ================================
@@ -852,10 +863,37 @@ int wgrad_run_prepare(WgradRun* R, unsigned kinds, int mode, const __half* act, 
   return 0;
 }
 
-int wgrad_run_enqueue(const WgradRun& R, cudaStream_t st) {
-  for (int c = 0; c < R.n_plane; ++c)
-    if (int e = wgrad_plane_enqueue(R.plane[c], st)) return e;
-  return R.has_umma ? wgrad_enqueue(R.umma, st) : 0;
+int wgrad_run_enqueue(const WgradRun& R, cudaStream_t st, float* part) {
+  if (!part) {
+    for (int c = 0; c < R.n_plane; ++c)
+      if (int e = wgrad_plane_enqueue(R.plane[c], st)) return e;
+    return R.has_umma ? wgrad_enqueue(R.umma, st) : 0;
+  }
+  // deterministic: every launch stores its partials into `part`, then one launch adds them in CTA / split order into
+  // G's rows (each row of G belongs to exactly one of the launches, so the sums are plain stores)
+  for (int c = 0; c < R.n_plane; ++c) {
+    WgradPlaneParams p = R.plane[c].p;
+    p.part = part;
+    wgrad_plane_kernel<32, true><<<R.plane[c].det_ctas, WP_THREADS, R.plane[c].smem, st>>>(p);
+    CM_CUDA(cudaGetLastError());
+    // partial row (tap, ci) -> G row tap * cin + c0 + ci
+    if (int e = sum_partials_enqueue(part, R.plane[c].det_ctas, WP_PART, WP_PART, 32 * 32, (size_t)p.cin * 32,
+                                     p.G + (size_t)p.c0 * 32, 0, st))
+      return e;
+  }
+  if (!R.has_umma) return 0;
+  WgradLaunch L = R.umma;
+  L.p.part = part;
+  if (int e = wg_enqueue_det(L, st)) return e;
+  const size_t n = (size_t)L.p.nphase * L.p.krows * L.p.cout;
+  return sum_partials_enqueue(part, L.p.splits, n, n, n, 0, L.p.G, 0, st);
+}
+
+size_t wgrad_run_partial_elems(const WgradRun& R) {
+  size_t m = 0;
+  for (int c = 0; c < R.n_plane; ++c) m = std::max(m, (size_t)R.plane[c].det_ctas * WP_PART);
+  if (R.has_umma) m = std::max(m, (size_t)R.umma.p.splits * R.umma.p.nphase * R.umma.p.krows * R.umma.p.cout);
+  return m;
 }
 
 }  // namespace cm

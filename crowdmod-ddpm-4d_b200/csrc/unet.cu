@@ -9,6 +9,7 @@
 // epilogue of the last conv.
 #include <string.h>
 
+#include <algorithm>
 #include <map>
 #include <memory>
 #include <string>
@@ -191,6 +192,11 @@ struct cm_unet {
   const float* live_future = nullptr;
   const float* live_past = nullptr;
   const float* live_drop = nullptr;
+  // reproducible backward (cm_unet_set_deterministic): every weight-gradient and channel-sum reduction stores per-CTA
+  // partials into det_part and adds them in a fixed order; det_part is allocated by the first such backward
+  int deterministic = 0;
+  float* det_part = nullptr;
+  size_t det_part_elems = 0;
 
   int add_param(const std::string& name, std::vector<int64_t> shape) {
     ParamEntry e;
@@ -1013,12 +1019,47 @@ void fill_temb(cm_unet* u, TembParams& tp, const int64_t* t, int batch) {
 
 // Reverse walk of the plan.  Every gradient carries the loss scale S (u->loss_scale[0]); the flat
 // parameter-gradient buffer is multiplied by 1/S at the end.
+// Floats of partial-sum scratch the deterministic backward needs: the largest single reduction of the plan (every one
+// is summed out of the scratch by the launch that follows it, so one buffer serves them all in stream order).
+size_t det_partial_elems(const cm_unet* u, int B) {
+  const cm_unet_config& c = u->cfg;
+  const Level& l0 = u->levels[0];
+  size_t m = cast_colsum_partial_elems(B, l0.pps(), c.base_channels);
+  for (const Op& op : u->ops) {
+    if (op.type != OP_CONV) continue;
+    m = std::max(m, cast_colsum_partial_elems(B, u->levels[u->tens[op.out].level].pps(), op.cout));
+    m = std::max(m, wgrad_run_partial_elems(op.wgrad));
+  }
+  m = std::max(m, wgrad_run_partial_elems(u->first_wg));
+  m = std::max(m, wgrad_run_partial_elems(u->final_wg));
+  if (!u->first_wg.launches())
+    m = std::max(m, first_conv_partial_elems(B, l0.H, l0.W, c.past_len, c.future_len, c.in_channels, c.base_channels));
+  m = std::max(m, final_conv_partial_elems(B, l0.H, l0.W, l0.D, c.past_len, u->ops.back().cin, c.out_channels,
+                                           u->final_wg.launches() > 0));
+  return m;
+}
+
 int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, int64_t* launches) {
   const cm_unet_config& c = u->cfg;
   const int B = u->live_train_batch;
   const int E = c.base_channels * c.time_multiple;
   auto gp = [&](int pidx) { return grads + u->grad_off[pidx]; };
   int64_t nl = 0;
+  float* part = nullptr;
+  if (u->deterministic) {
+    const size_t need = det_partial_elems(u, B);
+    if (need > u->det_part_elems) {
+      CM_CUDA(cudaStreamSynchronize(st));
+      CM_CUDA(cudaFree(u->det_part));
+      u->det_part = nullptr;
+      u->det_part_elems = 0;
+      CM_CUDA(cudaMalloc(&u->det_part, need * sizeof(float)));
+      u->det_part_elems = need;
+    }
+    part = u->det_part;
+  }
+  // launches each deterministic reduction adds: the ordered sums of its partials
+  const int det_extra = part ? 1 : 0;
   CM_CUDA(cudaMemsetAsync(grads, 0, u->grad_total * sizeof(float), st));
   CM_CUDA(cudaMemsetAsync(u->zero_region, 0, u->zero_bytes, st));
   const Level& l0 = u->levels[0];
@@ -1036,10 +1077,13 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
         if (int e = final_conv_backward_enqueue(d_eps, u->loss_scale, u->tens[op.in].p16, u->live_dup * op.cin,
                                                 u->live_dup == 2 ? op.cin : 0, u->params[u->p_final_w].ptr, u->g32[op.in], gp(u->p_final_w),
                                                 gp(u->p_final_b), B, l0.H, l0.W, l0.D, c.past_len, op.cin,
-                                                c.out_channels, u->final_wg.launches() ? u->final_d16 : nullptr, st))
+                                                c.out_channels, u->final_wg.launches() ? u->final_d16 : nullptr, st,
+                                                part))
           return e;
+        nl += det_extra * (u->final_wg.launches() ? 1 : 2);
         if (u->final_wg.launches()) {
-          if (int e = wgrad_run_enqueue(u->final_wg, st)) return e;
+          if (int e = wgrad_run_enqueue(u->final_wg, st, part)) return e;
+          nl += det_extra * u->final_wg.launches();
           // G is (tap, cin) x 32 packed columns: G's cout in the upper half of the cout entry
           for (long long v : {0LL, (long long)u->final_g_off, (long long)u->grad_off[u->p_final_w], -1LL,
                               (long long)c.out_channels | (32LL << 16), (long long)op.cin, 0LL, 1LL})
@@ -1101,8 +1145,9 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
           written[op.resid] = 1;
         }
         if (int e = cast_colsum_enqueue(u->g32[op.out], u->g16[op.out], u->dgrad_dup, fan, fan_init, cs, cs_ld, B,
-                                        pix, op.cout, st))
+                                        pix, op.cout, st, part))
           return e;
+        nl += det_extra;
         // bias gradients = batch sums of the channel sums: all convs in one launch after the op loop
         for (int bidx : {op.bias, op.bias2}) {
           if (bidx < 0) continue;
@@ -1124,8 +1169,8 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
           if (int e = conv_run_enqueue(r, st)) return e;
           ++nl;
         }
-        if (int e = wgrad_run_enqueue(op.wgrad, st)) return e;
-        nl += op.wgrad.launches() - 1;
+        if (int e = wgrad_run_enqueue(op.wgrad, st, part)) return e;
+        nl += op.wgrad.launches() - 1 + det_extra * op.wgrad.launches();
         // packed-K scratch -> nn.Conv3d weight layout: all convs in one launch after the op loop
         for (long long v : {(long long)op.mode, (long long)op.g_off, (long long)u->grad_off[op.w],
                             op.wx >= 0 ? (long long)u->grad_off[op.wx] : -1LL, (long long)op.cout, (long long)op.cin,
@@ -1148,13 +1193,15 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
         if (u->first_wg.launches()) {
           float* cs = u->colsum + (size_t)B * u->first_colsum_off;
           if (int e = cast_colsum_enqueue(u->g32[op.out], u->g16[op.out], u->dgrad_dup, nullptr, 0, cs, c.base_channels, B,
-                                          l0.pps(), c.base_channels, st))
+                                          l0.pps(), c.base_channels, st, part))
             return e;
+          nl += det_extra;
           rs_tab.push_back((long long)(cs - reinterpret_cast<const float*>(u->tarena)));
           rs_tab.push_back((long long)c.base_channels);
           rs_tab.push_back((long long)c.base_channels);
           rs_tab.push_back((long long)u->grad_off[u->p_first_b]);
-          if (int e = wgrad_run_enqueue(u->first_wg, st)) return e;
+          if (int e = wgrad_run_enqueue(u->first_wg, st, part)) return e;
+          nl += det_extra * u->first_wg.launches();
           // G rows are (tap, 32 packed channels): cin of G in the upper half of the cin entry
           for (long long v : {0LL, (long long)u->first_g_off, (long long)u->grad_off[u->p_first_w], -1LL,
                               (long long)c.base_channels, (long long)c.in_channels | (32LL << 16), 0LL, 1LL})
@@ -1162,8 +1209,10 @@ int run_backward(cm_unet* u, const float* d_eps, float* grads, cudaStream_t st, 
           nl += u->first_wg.launches();
         } else if (int e = first_conv_wgrad_enqueue(u->live_future, u->live_past, u->g32[op.out], gp(u->p_first_w),
                                                     gp(u->p_first_b), B, l0.H, l0.W, c.past_len, c.future_len,
-                                                    c.in_channels, c.base_channels, st)) {
+                                                    c.in_channels, c.base_channels, st, part)) {
           return e;
+        } else {
+          nl += 2 * det_extra;
         }
         ++nl;
       } break;
@@ -1293,6 +1342,7 @@ int cm_unet_destroy(cm_unet* u) {
   cudaFree(u->d_coef);
   cudaFree(u->dpack);
   cudaFree(u->tarena);
+  cudaFree(u->det_part);
   delete u;
   return 0;
 }
@@ -1509,6 +1559,12 @@ int cm_unet_backward(cm_unet* u, const float* d_eps, float* grads, void* stream)
 }
 
 int64_t cm_last_backward_launches(const cm_unet* u) { return u ? u->last_backward_launches : -1; }
+
+int cm_unet_set_deterministic(cm_unet* u, int enabled) {
+  CM_CHECK(u, "null handle");
+  u->deterministic = enabled ? 1 : 0;
+  return 0;
+}
 
 int cm_unet_op_count(const cm_unet* u) { return u ? (int)u->ops.size() : -1; }
 

@@ -19,7 +19,9 @@
 //     below the box are zero (written once, never touched by TMA): ONE 128 x 96 x 16 MMA per (td, 16 pixels) -- an MN-major
 //     MMA costs ~160 cycles here whatever N is (measured with the N = 32 version: 131 us per launch);
 //   * three accumulators (td) of 96 columns live in TMEM for the whole launch: a persistent CTA adds all its units into
-//     them and writes them out once (fp32 atomics into the packed-K G, as wgrad_umma_kernel).
+//     them and writes them out once (fp32 atomics into the packed-K G, as wgrad_umma_kernel; deterministic (DET): plain
+//     stores of the CTA's 27 x 32 x 32 partial into `part`, summed in CTA order by wgrad_run_enqueue over a grid of
+//     WP_DET_CTAS that depends on the shape only).
 // One launch covers one 32-channel chunk of the source (c0); wider sources take one launch per chunk.
 #pragma once
 #include "common.cuh"
@@ -30,6 +32,8 @@ namespace cm {
 
 constexpr int WP_THREADS = 192;     // warp0 TMA, warp1 MMA, warps2-5 epilogue
 constexpr int WP_MAX_STAGES = 4;
+constexpr int WP_DET_CTAS = 148;    // deterministic grid: min(units, this), a constant rather than the device's SM count
+constexpr int WP_PART = 27 * 32 * 32;   // floats of one CTA's partial [tap][ci][co]
 
 struct WgradPlaneParams {
   CUtensorMap amap;      // activations, tiled 5-D (C, W, H, D, N), box {32, W+2, HB+3, 1, 1}
@@ -45,10 +49,11 @@ struct WgradPlaneParams {
   int g_slot_bytes;      // guard + box + guard
   int cin;               // channels of the whole main source: G row = tap * cin + c0 + ci
   float* G;              // [27 * cin (+ extra rows)][32] fp32, zeroed by the caller
+  float* part;           // DET only: [gridDim.x][27][32][32]
   int* err_flag;
 };
 
-template <int COUT>   // always 32 (a template keeps the definition in this header; instantiated in conv_umma.cu only)
+template <int COUT, bool DET>   // COUT always 32 (a template keeps the definition in this header; instantiated in conv_umma.cu)
 __global__ void __launch_bounds__(WP_THREADS, 1) wgrad_plane_kernel(const __grid_constant__ WgradPlaneParams P) {
   static_assert(COUT == 32, "one 32-column accumulator per (td, th)");
   constexpr uint32_t IDESC = make_idesc_f16_mn(128, 96);
@@ -161,7 +166,14 @@ __global__ void __launch_bounds__(WP_THREADS, 1) wgrad_plane_kernel(const __grid
         tmem_ld16_async(t_lane + a * 32, v0);
         tmem_ld16_async(t_lane + a * 32 + 16, v1);
         tmem_ld_wait();
-        if (tw < 3) {
+        if (DET && tw < 3) {
+          float4* gp = reinterpret_cast<float4*>(P.part + static_cast<size_t>(blockIdx.x) * WP_PART +
+                                                 (static_cast<size_t>((td * 3 + th) * 3 + tw) * 32 + lane) * 32);
+#pragma unroll
+          for (int i = 0; i < 16; i += 4) gp[i / 4] = make_float4(v0[i], v0[i + 1], v0[i + 2], v0[i + 3]);
+#pragma unroll
+          for (int i = 0; i < 16; i += 4) gp[4 + i / 4] = make_float4(v1[i], v1[i + 1], v1[i + 2], v1[i + 3]);
+        } else if (tw < 3) {
           float* gp = P.G + (static_cast<size_t>((td * 3 + th) * 3 + tw) * P.cin + P.c0 + lane) * 32;
 #pragma unroll
           for (int i = 0; i < 16; i += 4) red_add_v4(gp + i, v0[i], v0[i + 1], v0[i + 2], v0[i + 3]);
@@ -181,6 +193,7 @@ struct WgradPlaneLaunch {
   dim3 grid;
   size_t smem;
   bool ok;               // false: shape not covered, use wgrad_umma_kernel
+  int det_ctas;          // grid of the deterministic variant: min(units, WP_DET_CTAS)
 };
 
 // One 32-channel chunk (channels [c0, c0 + 32) of a source whose pixel rows hold act_ld elements) of a k3 s1 p1 conv with

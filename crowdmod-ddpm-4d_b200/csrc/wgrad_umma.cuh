@@ -18,7 +18,9 @@
 //                             match_input source.  One TMA im2col load per atom per k-block.
 //   N tile                  = BN output channels of dOut (BN/BNC loads of BNC channels).
 //   K                       = pixels, split across gridDim.y CTAs; partial sums are combined with
-//                             fp32 atomics into G (zeroed by the caller).
+//                             fp32 atomics into G (zeroed by the caller), or, deterministic (DET), stored
+//                             per split into `part` [split][phase][krows][cout] and summed in split order
+//                             by wgrad_run_enqueue.
 //
 // G is [phase][taps*cin + cin_extra][cout] fp32 ("packed-K" row order, identical to the
 // forward weight packing); unpack_wgrad_kernel (backward.cu) turns it into the nn.Conv3d
@@ -50,6 +52,7 @@ struct WgradParams {
   int krows;             // rows of G per phase
   int stages;
   float* G;
+  float* part;           // DET only: splits * nphase * krows * cout floats
   int* err_flag;
 };
 
@@ -64,7 +67,7 @@ __device__ __forceinline__ uint32_t mnmajor_desc_lo(uint32_t smem_addr, uint32_t
   return ((smem_addr >> 4) & 0x3FFFu) | (((lbo_bytes >> 4) & 0x3FFFu) << 16);
 }
 
-template <int BKC, int BNC, int BN>
+template <int BKC, int BNC, int BN, bool DET>
 __global__ void __launch_bounds__(WG_THREADS, 1)
 wgrad_umma_kernel(const __grid_constant__ WgradParams P) {
   constexpr int ROWA = BKC * 2, ROWB = BNC * 2;          // smem row bytes (swizzle span)
@@ -198,7 +201,8 @@ wgrad_umma_kernel(const __grid_constant__ WgradParams P) {
         krow = static_cast<size_t>(P.kd * P.kh * P.kw) * P.cin_main + (ga - P.atoms_main) * BKC + ch;
       }
     }
-    float* gp = P.G + (static_cast<size_t>(phase) * P.krows + krow) * P.cout + n_tile * BN;
+    float* gp = (DET ? P.part + static_cast<size_t>(split) * P.nphase * P.krows * P.cout : P.G) +
+                (static_cast<size_t>(phase) * P.krows + krow) * P.cout + n_tile * BN;
     mbar_wait(tmem_full, 0, P.err_flag, 203);
     tc_fence_after();
     const uint32_t t_lane = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16);
@@ -208,7 +212,10 @@ wgrad_umma_kernel(const __grid_constant__ WgradParams P) {
       tmem_ld16(t_lane + c * 16, v);
       if (!valid) continue;
 #pragma unroll
-      for (int i = 0; i < 16; i += 4) red_add_v4(gp + c * 16 + i, v[i], v[i + 1], v[i + 2], v[i + 3]);
+      for (int i = 0; i < 16; i += 4) {
+        if constexpr (DET) *reinterpret_cast<float4*>(gp + c * 16 + i) = make_float4(v[i], v[i + 1], v[i + 2], v[i + 3]);
+        else red_add_v4(gp + c * 16 + i, v[i], v[i + 1], v[i + 2], v[i + 3]);
+      }
     }
   }
   tc_fence_before();

@@ -89,6 +89,7 @@ class _NativePlan:
         self._grad_layout = None
         self._dropout_layout = None
         self.train_token = 0
+        self.deterministic = False    # the handle's cm_unet_set_deterministic mode
 
     def _query_names(self):
         lib = self.n.lib()

@@ -111,6 +111,12 @@ class _UNetFunction(torch.autograd.Function):
         offs, total = grad_layout(plan)
         flat = torch.empty(total, device=d_eps.device, dtype=torch.float32)
         d_eps = d_eps.contiguous().float()
+        # torch.use_deterministic_algorithms(True) makes the native backward reproducible bit for bit (fixed-order
+        # reductions instead of fp32 atomics); the handle keeps the mode, so it is set only when the flag changed
+        det = torch.are_deterministic_algorithms_enabled()
+        if plan.deterministic != det:
+            n.check(n.lib().cm_unet_set_deterministic(plan.handle, int(det)))
+            plan.deterministic = det
         n.check(n.lib().cm_unet_backward(plan.handle, n.ptr(d_eps), n.ptr(flat), n.current_stream()))
         _allreduce_mean(ctx.module, flat)
         ctx.module._last_flat_grad = flat

@@ -110,6 +110,11 @@ CM_API int cm_unet_train_forward(cm_unet* u, const float* future, const int64_t*
  * and unscaled before returning.  One backward per forward. */
 CM_API int cm_unet_backward(cm_unet* u, const float* d_eps, float* grads, void* stream);
 CM_API int64_t cm_last_backward_launches(const cm_unet* u);
+/* Reproducible backward (enabled != 0; default 0): every reduction of cm_unet_backward runs in a fixed order whose
+ * partition depends on the problem shape only, so identical inputs give a bitwise identical gradient buffer on every
+ * call, process and B200.  Weight gradients and channel sums store per-CTA partials (one scratch buffer, allocated
+ * by the first such backward) and add them in CTA order, one extra launch per reduction, instead of fp32 atomics. */
+CM_API int cm_unet_set_deterministic(cm_unet* u, int enabled);
 
 /* Measurement support for bench.py: the plan's ops (tag, kind: 0 first conv, 1 GroupNorm+SiLU,
  * 2 tcgen05 conv, 3 attention core, 4 final conv; algorithmic FLOPs per sample in the
@@ -291,6 +296,18 @@ CM_API int cm_op_conv3d_dgrad_f32(int mode, const float* dout32, int B, int D, i
 CM_API int cm_op_conv3d_wgrad(int mode, const void* act16, int B, int D, int H, int W, int cin,
                               const void* extra16, int cin_extra, const void* dout16, int cout,
                               float* dw, float* dwx, int impl, void* stream);
+/* The deterministic variants of the weight-gradient, channel-sum and first / final conv entries: the reductions of
+ * the training backward under cm_unet_set_deterministic (impl 0 / 2 as above; 1 is not accepted). */
+CM_API int cm_op_conv3d_wgrad_det(int mode, const void* act16, int B, int D, int H, int W, int cin,
+                                  const void* extra16, int cin_extra, const void* dout16, int cout,
+                                  float* dw, float* dwx, int impl, void* stream);
+CM_API int cm_op_cast_colsum_det(const float* src, void* dst16, int dup, float* acc_dst, int acc_init, float* colsum,
+                                 int colsum_ld, int B, int pixels, int C, void* stream);
+CM_API int cm_op_final_conv_backward_det(const float* deps, float scale, const void* act16, int act_ld, int act_lo,
+                                         const float* w, float* dact, float* dw, float* db, int B, int H, int W, int L,
+                                         int P, int cin, int cout, void* dout16, void* stream);
+CM_API int cm_op_first_conv_wgrad_det(const float* x, const float* past, const float* dout, float* dw, float* db,
+                                      int B, int H, int W, int P, int F, int cin, int cout, void* stream);
 
 /* fp32 kernels of the training backward, one enqueue function each (tests compare them with float64 autograd).
  * Channels-last fp32 tensors [B][pixels][C] unless stated.
