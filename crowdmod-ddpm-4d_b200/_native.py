@@ -290,6 +290,25 @@ def ptr(t):
     return None if t is None else C.c_void_p(t.data_ptr())
 
 
+def chain_args(past, x, tsteps, coef, mode, noise, seed, sample_offset, history, graph_mode):
+    """cm_chain_args of a reverse chain on ``x`` (both backbones' ``sample_chain``).  Returns (args, tsteps, coef):
+    the CPU int32 / fp32 copies of the schedule must stay alive until the C call returns."""
+    import torch
+    assert x.is_contiguous() and x.dtype == torch.float32
+    assert past.is_contiguous() and past.dtype == torch.float32
+    tsteps = tsteps.to(torch.int32).contiguous().cpu()
+    coef = coef.to(torch.float32).contiguous().cpu()
+    assert coef.shape == (tsteps.numel(), 8)
+    if noise is not None:
+        assert noise.is_cuda and noise.is_contiguous() and noise.dtype == torch.float32
+        assert noise.numel() == tsteps.numel() * x.numel()
+    a = ChainArgs(past=past.data_ptr(), x=x.data_ptr(), n=x.shape[0], nsteps=tsteps.numel(), tsteps=tsteps.data_ptr(),
+                  coef=coef.data_ptr(), mode=int(mode), noise=noise.data_ptr() if noise is not None else None,
+                  seed=int(seed) & 0xFFFFFFFFFFFFFFFF, sample_offset=int(sample_offset),
+                  history=history.data_ptr() if history is not None else None, use_graph=graph_mode)
+    return a, tsteps, coef
+
+
 def current_stream():
     import torch
     return C.c_void_p(torch.cuda.current_stream().cuda_stream)

@@ -349,23 +349,18 @@ int cm_op_final_conv_step(const void* act16, int act_ld, int act_lo, const float
   if (int e = kernels_init()) return e;
   CM_CHECK(!x || (nsteps >= 1 && step >= 0 && step < nsteps), "final conv: step %d outside [0, %d)", step, nsteps);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  // the step index and {seed, sample_offset} travel through device memory, as in cm_ddpm_sample
-  unsigned long long* dev = nullptr;
-  CM_CUDA(cudaMalloc(&dev, 3 * sizeof(unsigned long long)));
-  const unsigned long long h[3] = {seed, static_cast<unsigned long long>(sample_offset), static_cast<unsigned long long>(step)};
-  int rc = cudaMemcpyAsync(dev, h, sizeof(h), cudaMemcpyHostToDevice, st) == cudaSuccess ? 0 : 1;
   FinalParams f{};
   f.act = static_cast<const __half*>(act16);
   f.act_ld = act_ld; f.act_lo = act_lo;
   f.w = w; f.bias = bias; f.B = B; f.H = H; f.W = W; f.L = L; f.P = P; f.cin = cin; f.cout = cout;
   f.eps_out = eps_out;
-  f.x = x;
-  f.coef = coef;
-  f.step_dev = reinterpret_cast<const int*>(dev + 2);        // low word of a little-endian 64-bit slot
-  f.mode = mode;
-  f.noise = noise;
-  f.chain_dev = dev;
-  f.history = history;
+  f.rs.x = x;
+  f.rs.coef = coef;
+  f.rs.mode = mode;
+  f.rs.noise = noise;
+  f.rs.history = history;
+  unsigned long long* dev = nullptr;
+  int rc = stage_step_state(f.rs, &dev, seed, sample_offset, step, st);
   if (!rc) rc = final_conv_enqueue(f, st);
   cudaError_t se = cudaStreamSynchronize(st);
   cudaFree(dev);

@@ -13,12 +13,12 @@ FLAGS=(-gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo
 OBJ="${HERE}/build"
 mkdir -p "${OBJ}"
 pids=()
-for f in api conv_umma kernels unet backward feed_metrics dit attn_long; do
+for f in api conv_umma kernels chain unet backward feed_metrics dit attn_long; do
   if [[ ! -f "${OBJ}/${f}.o" || "${HERE}/${f}.cu" -nt "${OBJ}/${f}.o" || -n "$(find "${HERE}" -name '*.cuh' -newer "${OBJ}/${f}.o" 2>/dev/null)" || "${HERE}/../../include/crowdmod_b200.h" -nt "${OBJ}/${f}.o" ]]; then
     "${NVCC}" "${FLAGS[@]}" ${CM_PTXAS_V:+-Xptxas -v} -c "${HERE}/${f}.cu" -o "${OBJ}/${f}.o" &
     pids+=($!)
   fi
 done
 for p in "${pids[@]:-}"; do [[ -n "$p" ]] && wait "$p"; done
-"${NVCC}" "${FLAGS[@]}" -shared -o "${OUT}" "${OBJ}"/api.o "${OBJ}"/conv_umma.o "${OBJ}"/kernels.o "${OBJ}"/unet.o "${OBJ}"/backward.o "${OBJ}"/feed_metrics.o "${OBJ}"/dit.o "${OBJ}"/attn_long.o
+"${NVCC}" "${FLAGS[@]}" -shared -o "${OUT}" "${OBJ}"/api.o "${OBJ}"/conv_umma.o "${OBJ}"/kernels.o "${OBJ}"/chain.o "${OBJ}"/unet.o "${OBJ}"/backward.o "${OBJ}"/feed_metrics.o "${OBJ}"/dit.o "${OBJ}"/attn_long.o
 echo "built ${OUT}"

@@ -197,21 +197,10 @@ struct UnpatchParams {
   int ld;
   int B, C, H, W, P, F, p, pt, hp, wp, Tp;
   float* eps_out;        // optional [B][C][H][W][F]
-  // reverse-step update (as FinalParams of the UNet path): all optional
-  float* x;
-  const float* coef;     // device [nsteps][8]
-  int step;
-  const int* step_dev;   // device step index (graph replay): overrides `step` when set
-  int mode;
-  const float* noise;
-  unsigned long long seed;
-  long long sample_offset;
-  const unsigned long long* chain_dev;   // device {seed, sample_offset}: overrides the two fields above when set
-  float* history;
+  ReverseStep rs;        // reverse-step update (rs.x == nullptr -> eps only)
 };
-// un-patch + slice to the future frames (DiT4D_V4.py:80-102) + DDPM.step / DDIM update / Sparsity guidance / Philox
-// noise exactly as final_conv_kernel does for the UNet (ddpm.py:25-38, :262-265, guidance.py:4-8): one thread per
-// (b, y, x, f) handles the C <= 4 properties (one Philox draw).
+// un-patch + slice to the future frames (DiT4D_V4.py:80-102) + the reverse-step update final_conv_kernel fuses for the
+// UNet (chain.cuh): one thread per (b, y, x, f) handles the C <= 4 properties (one Philox draw).
 __global__ void dit_unpatch_step_kernel(UnpatchParams p) {
   const size_t total = (size_t)p.B * p.H * p.W * p.F;
   const size_t plane = (size_t)p.H * p.W * p.F;
@@ -226,46 +215,12 @@ __global__ void dit_unpatch_step_kernel(UnpatchParams p) {
     const size_t row = (((size_t)b * p.Tp + slot) * p.hp + ph) * p.wp + pw;
     float eps[4] = {0.f, 0.f, 0.f, 0.f};
     for (int c = 0; c < p.C; ++c) eps[c] = p.out[row * p.ld + ((dt * p.C + c) * p.p + dy) * p.p + dx];
-    const size_t e0 = ((size_t)b * p.C) * plane + ((size_t)y * p.W + xw) * p.F + f;
+    const size_t site = ((size_t)y * p.W + xw) * p.F + f;
+    const size_t e0 = ((size_t)b * p.C) * plane + site;
     if (p.eps_out)
       for (int c = 0; c < p.C; ++c) p.eps_out[e0 + c * plane] = eps[c];
-    if (!p.x) continue;
-    const int step = p.step_dev ? *p.step_dev : p.step;
-    const unsigned long long seed = p.chain_dev ? p.chain_dev[0] : p.seed;
-    const long long soff = p.chain_dev ? static_cast<long long>(p.chain_dev[1]) : p.sample_offset;
-    const float* cf = p.coef + (size_t)step * 8;
-    const size_t nelem = (size_t)p.B * p.C * plane;
-    float z[4] = {0.f, 0.f, 0.f, 0.f};
-    const float zc = (p.mode == 0) ? cf[2] : cf[4];
-    if (zc != 0.f) {
-      if (p.noise) {
-        for (int c = 0; c < p.C; ++c) z[c] = p.noise[(size_t)step * nelem + e0 + c * plane];
-      } else {
-        const unsigned long long gp = ((unsigned long long)(soff + b)) * (unsigned long long)plane +
-                                      ((size_t)y * p.W + xw) * p.F + f;
-        const uint4 rnd = philox4x32_10(make_uint4((uint32_t)gp, (uint32_t)(gp >> 32), (uint32_t)step, 0u),
-                                        make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
-        const float2 n0 = box_muller(rnd.x, rnd.y), n1 = box_muller(rnd.z, rnd.w);
-        z[0] = n0.x; z[1] = n0.y; z[2] = n1.x; z[3] = n1.y;
-      }
-    }
-    for (int c = 0; c < p.C; ++c) {
-      const size_t e = e0 + c * plane;
-      const float xv = p.x[e];
-      float xn;
-      if (p.mode == 0) {
-        xn = cf[0] * (xv - cf[1] * eps[c]) + cf[2] * z[c];
-      } else {
-        const float x0 = (xv - cf[0] * eps[c]) / cf[1];
-        xn = cf[2] * x0 + cf[3] * eps[c] + cf[4] * z[c];
-      }
-      if (c == 0 && cf[5] != 0.f) {
-        const float sg = (xn > 0.f) ? 1.f : ((xn < 0.f) ? -1.f : 0.f);
-        xn -= cf[5] * sg;
-      }
-      p.x[e] = xn;
-      if (p.history) p.history[(size_t)(step + 1) * nelem + e] = xn;
-    }
+    if (!p.rs.x) continue;
+    reverse_step_update(p.rs, eps, p.C, p.B, b, plane, site);
   }
 }
 
@@ -279,13 +234,12 @@ __global__ void dit_fill_t_range_kernel(long long* t, int n, int first) {
 }
 // sampling steps are batch-uniform: the step's (shift, scale, gate) vectors of every block are ONE row of the table
 // precomputed per weight load (the analogue of the UNet plan's time-embedding table); copied to mods row 0
-__global__ void dit_select_mods_kernel(float* __restrict__ mods, const float* __restrict__ table, const int* __restrict__ tsteps,
-                                       const int* __restrict__ step_dev, int J) {
-  const float* row = table + (size_t)tsteps[*step_dev] * J;
+__global__ void dit_select_mods_kernel(float* __restrict__ mods, const float* __restrict__ table, const int* __restrict__ t_dev,
+                                       int J) {
+  const float* row = table + (size_t)*t_dev * J;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < J / 4; i += gridDim.x * blockDim.x)
     reinterpret_cast<float4*>(mods)[i] = reinterpret_cast<const float4*>(row)[i];
 }
-__global__ void dit_advance_kernel(int* step_dev) { ++*step_dev; }
 
 int grid_for(size_t work_items, int block = 256) {
   size_t b = (work_items + block - 1) / block;
@@ -347,7 +301,7 @@ int unpatch_step_enqueue(const UnpatchParams& up, cudaStream_t st) {
                up.P + up.F == up.Tp * up.pt && up.F >= 1 && up.ld >= up.pt * up.C * up.p * up.p,
            "un-patch: bad geometry (C %d, %dx%d, P %d F %d, p %d, pt %d, ld %d)", up.C, up.H, up.W, up.P, up.F, up.p,
            up.pt, up.ld);
-  CM_CHECK(!up.x || (up.coef && (up.mode == 0 || up.mode == 1)), "un-patch: the update needs coefficients and mode 0 or 1");
+  CM_CHECK(!up.rs.x || (up.rs.coef && (up.rs.mode == 0 || up.rs.mode == 1)), "un-patch: the update needs coefficients and mode 0 or 1");
   dit_unpatch_step_kernel<<<grid_for((size_t)up.B * up.H * up.W * up.F), 256, 0, st>>>(up);
   DIT_LAUNCH_CHECK();
   return 0;
@@ -412,17 +366,11 @@ struct cm_dit {
   long long* t_dev = nullptr;
   __half *e16 = nullptr, *h16 = nullptr, *a16 = nullptr, *xm16 = nullptr, *ctx16 = nullptr, *g16 = nullptr;
   float *h32 = nullptr, *h2_32 = nullptr, *c32 = nullptr, *mods = nullptr, *x32 = nullptr, *qkv32 = nullptr, *out32 = nullptr,
-        *chain_x = nullptr, *chain_past = nullptr, *d_coef = nullptr;
-  int coef_cap = 0;
+        *chain_x = nullptr, *chain_past = nullptr;
   float* mods_table = nullptr;         // [table_steps][Jtot]: AdaLN vectors of every timestep (sampling, batch-uniform t)
   bool table_ready = false;
-  int* d_step = nullptr;
-  int* d_tsteps = nullptr;
-  unsigned long long* d_chain = nullptr;
-  cudaGraphExec_t graph_exec = nullptr;
-  cm_chain_args graph_key{};
-  int64_t graph_launches_per_step = 0;
-  int64_t last_launches = 0;
+  ChainDriver chain;
+  int64_t last_launches = 0;           // of the last cm_dit_forward / cm_dit_sample
   double flops_per_sample = 0.0;
 
   int add_param(const std::string& name, std::vector<int64_t> shape) {
@@ -600,10 +548,7 @@ int pack_all(cm_dit* u, cudaStream_t st) {
 
 int reserve(cm_dit* u, int batch) {
   if (batch <= u->reserved_batch) return 0;
-  if (u->graph_exec) {
-    cudaGraphExecDestroy(u->graph_exec);
-    u->graph_exec = nullptr;
-  }
+  chain_drop_graph(u->chain);
   if (u->arena) CM_CUDA(cudaFree(u->arena));
   u->arena = nullptr;
   u->prepared_batch = 0;
@@ -679,10 +624,7 @@ int prepare(cm_dit* u, int batch) {
     dit_epilogue(b.fc2.launch.p, 0, nullptr, u->mods, 0, 0, 0);
   }
   if (int e = prep_gemm(u, u->final_lin, u->xm16, batch, 1, Tp, Ns, u->out32)) return e;
-  if (u->graph_exec) {            // the captured step bakes the launches of the previous batch
-    cudaGraphExecDestroy(u->graph_exec);
-    u->graph_exec = nullptr;
-  }
+  chain_drop_graph(u->chain);     // the captured step bakes the launches of the previous batch
   u->prepared_batch = batch;
   return 0;
 }
@@ -811,12 +753,8 @@ int cm_dit_destroy(cm_dit* u) {
   if (u->adaln_wbuf) cudaFree(u->adaln_wbuf);
   if (u->adaln_bbuf) cudaFree(u->adaln_bbuf);
   if (u->patch_wbuf) cudaFree(u->patch_wbuf);
-  if (u->d_coef) cudaFree(u->d_coef);
-  if (u->d_tsteps) cudaFree(u->d_tsteps);
-  if (u->d_step) cudaFree(u->d_step);
-  if (u->d_chain) cudaFree(u->d_chain);
   if (u->mods_table) cudaFree(u->mods_table);
-  if (u->graph_exec) cudaGraphExecDestroy(u->graph_exec);
+  chain_free(u->chain);
   delete u;
   return 0;
 }
@@ -867,95 +805,28 @@ int cm_dit_forward(cm_dit* u, const float* future, const int64_t* t, const float
 }
 
 int cm_dit_sample(cm_dit* u, const cm_chain_args* a, void* stream) {
-  CM_CHECK(u && a && a->past && a->x && a->tsteps && a->coef, "null argument");
-  CM_CHECK(a->n >= 1 && a->nsteps >= 1, "n and nsteps must be >= 1");
-  CM_CHECK(a->mode == 0 || a->mode == 1, "mode must be 0 (DDPM) or 1 (DDIM)");
+  CM_CHECK(u && a, "null argument");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (int e = ensure_ready(u, a->n, st)) return e;
   if (int e = build_mods_table(u, st)) return e;
   const cm_dit_config& c = u->cfg;
-  for (int i = 0; i < a->nsteps; ++i)
-    CM_CHECK(a->tsteps[i] >= 0 && a->tsteps[i] < c.table_steps, "timestep %d outside the table", a->tsteps[i]);
-  if (a->nsteps > u->coef_cap) {
-    if (u->d_coef) CM_CUDA(cudaFree(u->d_coef));
-    if (u->d_tsteps) CM_CUDA(cudaFree(u->d_tsteps));
-    CM_CUDA(cudaMalloc(&u->d_coef, (size_t)a->nsteps * 8 * sizeof(float)));
-    CM_CUDA(cudaMalloc(&u->d_tsteps, (size_t)a->nsteps * sizeof(int)));
-    u->coef_cap = a->nsteps;
-    if (u->graph_exec) {
-      cudaGraphExecDestroy(u->graph_exec);
-      u->graph_exec = nullptr;
-    }
-  }
-  if (!u->d_step) CM_CUDA(cudaMalloc(&u->d_step, sizeof(int)));
-  if (!u->d_chain) CM_CUDA(cudaMalloc(&u->d_chain, 2 * sizeof(unsigned long long)));
-  // step index, timesteps, coefficients, Philox seed / shard offset, x and past all travel through buffers the handle
-  // owns: one captured step serves every chain of this (n, mode, noise, history)
-  const unsigned long long chain_host[2] = {a->seed, static_cast<unsigned long long>(a->sample_offset)};
-  CM_CUDA(cudaMemcpyAsync(u->d_coef, a->coef, (size_t)a->nsteps * 8 * sizeof(float), cudaMemcpyHostToDevice, st));
-  CM_CUDA(cudaMemcpyAsync(u->d_tsteps, a->tsteps, (size_t)a->nsteps * sizeof(int), cudaMemcpyHostToDevice, st));
-  CM_CUDA(cudaMemcpyAsync(u->d_chain, chain_host, sizeof(chain_host), cudaMemcpyHostToDevice, st));
-  CM_CUDA(cudaMemsetAsync(u->d_step, 0, sizeof(int), st));
-  const size_t xel = (size_t)a->n * c.out_channels * c.rows * c.cols * c.future_len;
-  const size_t pel = (size_t)a->n * c.in_channels * c.rows * c.cols * c.past_len;
-  CM_CUDA(cudaMemcpyAsync(u->chain_x, a->x, xel * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  CM_CUDA(cudaMemcpyAsync(u->chain_past, a->past, pel * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  UnpatchParams up{};
-  up.x = u->chain_x;
-  up.coef = u->d_coef;
-  up.step_dev = u->d_step;
-  up.mode = a->mode;
-  up.noise = a->noise;
-  up.chain_dev = u->d_chain;
-  up.history = a->history;
-  auto one_step = [&](cudaStream_t s2, int64_t* launches) -> int {
-    dit_select_mods_kernel<<<8, 256, 0, s2>>>(u->mods, u->mods_table, u->d_tsteps, u->d_step, u->Jtot);
-    CM_CUDA(cudaGetLastError());
-    // the denoiser reads the CURRENT x (the chain's staging copy) as its `future` input
-    if (int e = run_forward(u, a->n, u->chain_x, u->chain_past, up, 0, s2, launches)) return e;
-    dit_advance_kernel<<<1, 1, 0, s2>>>(u->d_step);
-    CM_CUDA(cudaGetLastError());
-    if (launches) *launches += 2;
-    return 0;
-  };
-  u->last_launches = 0;
-  if (!a->use_graph) {
-    for (int i = 0; i < a->nsteps; ++i)
-      if (int e = one_step(st, &u->last_launches)) return e;
-  } else {
-    const cm_chain_args& k = u->graph_key;
-    const bool reuse = u->graph_exec && k.n == a->n && k.mode == a->mode && k.noise == a->noise && k.history == a->history;
-    if (!reuse) {
-      if (u->graph_exec) {
-        cudaGraphExecDestroy(u->graph_exec);
-        u->graph_exec = nullptr;
-      }
-      cudaStream_t cs;
-      CM_CUDA(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
-      cudaGraph_t g = nullptr;
-      int64_t per_step = 0;
-      cudaError_t ce = cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal);
-      int e = 0;
-      if (ce == cudaSuccess) {
-        e = one_step(cs, &per_step);
-        ce = cudaStreamEndCapture(cs, &g);
-      }
-      cudaStreamDestroy(cs);
-      if (e || ce != cudaSuccess) {
-        if (g) cudaGraphDestroy(g);
-        if (e) return e;
-        CM_CUDA(ce);
-      }
-      CM_CUDA(cudaGraphInstantiate(&u->graph_exec, g, 0));
-      cudaGraphDestroy(g);
-      u->graph_key = *a;
-      u->graph_launches_per_step = per_step;
-    }
-    for (int i = 0; i < a->nsteps; ++i) CM_CUDA(cudaGraphLaunch(u->graph_exec, st));
-    u->last_launches = u->graph_launches_per_step * a->nsteps;
-  }
-  CM_CUDA(cudaMemcpyAsync(a->x, u->chain_x, xel * sizeof(float), cudaMemcpyDeviceToDevice, st));
-  return 0;
+  const size_t x_bytes = (size_t)a->n * c.out_channels * c.rows * c.cols * c.future_len * sizeof(float);
+  const size_t past_bytes = (size_t)a->n * c.in_channels * c.rows * c.cols * c.past_len * sizeof(float);
+  cm_chain_args args = *a;
+  args.use_graph = a->use_graph ? 1 : 0;   // any nonzero value: one captured step replayed nsteps times
+  const int e = chain_run(u->chain, args, c.table_steps, u->chain_x, x_bytes, u->chain_past, past_bytes,
+                          [u, n = a->n](const ReverseStep& rs, const int* t_dev, cudaStream_t s, int64_t* launches) {
+                            dit_select_mods_kernel<<<8, 256, 0, s>>>(u->mods, u->mods_table, t_dev, u->Jtot);
+                            CM_CUDA(cudaGetLastError());
+                            ++*launches;
+                            // the denoiser reads the CURRENT x (the chain's staging copy) as its `future` input
+                            UnpatchParams up{};
+                            up.rs = rs;
+                            return run_forward(u, n, u->chain_x, u->chain_past, up, 0, s, launches);
+                          },
+                          st);
+  u->last_launches = u->chain.launches;
+  return e;
 }
 
 // ---- op-level entry points: each launches through the enqueue function run_forward uses, then synchronises ----
@@ -1028,24 +899,19 @@ int cm_op_dit_unpatch_step(const float* out, int ld, int B, int C, int H, int W,
            "un-patch: %dx%d, P %d F %d not divisible by patch %d / t_patch %d (or more than 8 slots)", H, W, P, F, p, pt);
   CM_CHECK(!x || (nsteps >= 1 && step >= 0 && step < nsteps), "un-patch: step %d outside [0, %d)", step, nsteps);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  // the step index and {seed, sample_offset} travel through device memory, as in cm_dit_sample
-  unsigned long long* dev = nullptr;
-  CM_CUDA(cudaMalloc(&dev, 3 * sizeof(unsigned long long)));
-  const unsigned long long h[3] = {seed, static_cast<unsigned long long>(sample_offset), static_cast<unsigned long long>(step)};
-  int rc = cudaMemcpyAsync(dev, h, sizeof(h), cudaMemcpyHostToDevice, st) == cudaSuccess ? 0 : 1;
   UnpatchParams up{};
   up.out = out;
   up.ld = ld;
   up.B = B; up.C = C; up.H = H; up.W = W; up.P = P; up.F = F;
   up.p = p; up.pt = pt; up.hp = H / p; up.wp = W / p; up.Tp = (P + F) / pt;
   up.eps_out = eps_out;
-  up.x = x;
-  up.coef = coef;
-  up.step_dev = reinterpret_cast<const int*>(dev + 2);       // low word of a little-endian 64-bit slot
-  up.mode = mode;
-  up.noise = noise;
-  up.chain_dev = dev;
-  up.history = history;
+  up.rs.x = x;
+  up.rs.coef = coef;
+  up.rs.mode = mode;
+  up.rs.noise = noise;
+  up.rs.history = history;
+  unsigned long long* dev = nullptr;
+  int rc = stage_step_state(up.rs, &dev, seed, sample_offset, step, st);
   if (!rc) rc = unpatch_step_enqueue(up, st);
   rc = dit_op_sync(rc, st);
   cudaFree(dev);

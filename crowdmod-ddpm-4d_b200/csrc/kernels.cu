@@ -5,6 +5,7 @@
 #include "pack.cuh"
 
 #include <cooperative_groups.h>
+#include <type_traits>
 
 
 namespace cm {
@@ -1013,7 +1014,9 @@ __global__ void __launch_bounds__(256) final_conv_kernel(const FinalParams p) {
   for (int j = 0; j < FIN_FC; ++j)
 #pragma unroll
     for (int co = 0; co < COUT; ++co) acc3[j][co] = 0.f;
-  if (active) {
+  // the tap loop is instantiated with and without the lo half, so that the sampling path (single fp16 operands)
+  // never loads or converts one, independently of how the compiler treats the rest of the kernel
+  auto taps = [&](auto has_lo) {
     const int l0 = p.P + f0 - 1;                       // first of the FIN_FC + 2 input planes
     const int ald = p.act_ld > 0 ? p.act_ld : cin;     // pixel row stride (2*cin for hi|lo pair operands)
     const size_t pstride = (size_t)p.H * p.W * ald;    // elements per (b, l) plane
@@ -1033,7 +1036,7 @@ __global__ void __launch_bounds__(256) final_conv_kernel(const FinalParams p) {
             // planes past the chunk's last valid frame + 1 are never multiplied into a stored output
             if (ll >= 0 && ll < p.L) {
               u = *reinterpret_cast<const uint4*>(ap + (size_t)ll * pstride + c0);
-              if (p.act_lo > 0) ul = *reinterpret_cast<const uint4*>(ap + (size_t)ll * pstride + p.act_lo + c0);
+              if (decltype(has_lo)::value) ul = *reinterpret_cast<const uint4*>(ap + (size_t)ll * pstride + p.act_lo + c0);
             }
             const __half2* h2 = reinterpret_cast<const __half2*>(&u);
             const __half2* l2 = reinterpret_cast<const __half2*>(&ul);
@@ -1065,6 +1068,10 @@ __global__ void __launch_bounds__(256) final_conv_kernel(const FinalParams p) {
         }
       }
     }
+  };
+  if (active) {
+    if (p.act_lo > 0) taps(std::true_type{});
+    else taps(std::false_type{});
   }
   float acc[COUT];
 #pragma unroll
@@ -1082,7 +1089,8 @@ __global__ void __launch_bounds__(256) final_conv_kernel(const FinalParams p) {
   if (!active || sub >= FIN_FC || f >= F) continue;
 
   const size_t plane = (size_t)p.H * p.W * F;                       // elements per (b, c)
-  const size_t e0 = ((size_t)b * COUT) * plane + ((size_t)h * p.W + wc) * F + f;
+  const size_t site = ((size_t)h * p.W + wc) * F + f;
+  const size_t e0 = ((size_t)b * COUT) * plane + site;
   float eps[COUT];
 #pragma unroll
   for (int co = 0; co < COUT; ++co) eps[co] = acc[co] + p.bias[co];
@@ -1090,51 +1098,8 @@ __global__ void __launch_bounds__(256) final_conv_kernel(const FinalParams p) {
 #pragma unroll
     for (int co = 0; co < COUT; ++co) p.eps_out[e0 + co * plane] = eps[co];
   }
-  if (!p.x) continue;
-
-  const int step = *p.step_dev;
-  const float* cf = p.coef + (size_t)step * 8;
-  const size_t nelem = (size_t)p.B * COUT * plane;
-  float z[4] = {0.f, 0.f, 0.f, 0.f};
-  const float zc = (p.mode == 0) ? cf[2] : cf[4];
-  if (zc != 0.f) {
-    if (p.noise) {
-#pragma unroll
-      for (int co = 0; co < COUT; ++co) z[co] = p.noise[(size_t)step * nelem + e0 + co * plane];
-    } else {
-      const unsigned long long seed = p.chain_dev ? p.chain_dev[0] : p.seed;
-      const long long soff = p.chain_dev ? static_cast<long long>(p.chain_dev[1]) : p.sample_offset;
-      const unsigned long long gp =
-          ((unsigned long long)(soff + b)) * (unsigned long long)(p.H * p.W * F) +
-          ((size_t)h * p.W + wc) * F + f;
-      const uint4 rnd = philox4x32_10(
-          make_uint4((uint32_t)gp, (uint32_t)(gp >> 32), (uint32_t)step, 0u),
-          make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
-      const float2 n0 = box_muller(rnd.x, rnd.y), n1 = box_muller(rnd.z, rnd.w);
-      z[0] = n0.x; z[1] = n0.y; z[2] = n1.x; z[3] = n1.y;
-    }
-  }
-#pragma unroll
-  for (int co = 0; co < COUT; ++co) {
-    const size_t e = e0 + co * plane;
-    const float xv = p.x[e];
-    float xn;
-    if (p.mode == 0) {
-      // ddpm.py:33-37: one_by_sqrt_alpha * (x - (beta/sqrt(1-abar)) * eps) + sqrt(beta) * z
-      xn = cf[0] * (xv - cf[1] * eps[co]) + cf[2] * z[co];
-    } else {
-      // ddpm.py:262-265 (DDIM eq. 12)
-      const float x0 = (xv - cf[0] * eps[co]) / cf[1];
-      xn = cf[2] * x0 + cf[3] * eps[co] + cf[4] * z[co];
-    }
-    if (co == 0 && cf[5] != 0.f) {
-      // guidance.py:4-8 + ddpm.py:223-226: x[:,0] -= lambda*sigma*sign(x[:,0])
-      const float sg = (xn > 0.f) ? 1.f : ((xn < 0.f) ? -1.f : 0.f);
-      xn -= cf[5] * sg;
-    }
-    p.x[e] = xn;
-    if (p.history) p.history[(size_t)(step + 1) * nelem + e] = xn;
-  }
+  if (!p.rs.x) continue;
+  reverse_step_update(p.rs, eps, COUT, p.B, b, plane, site);
   }
 }
 
@@ -1886,46 +1851,6 @@ int kernels_init() {
   if (int rc = attn_long_init()) return rc;
   if (int rc = conv_init()) return rc;
   done = true;
-  return 0;
-}
-
-// =============================================================================================
-// chain bookkeeping
-// =============================================================================================
-__global__ void advance_step_kernel(int* step_dev, int* t_dev, const int* tsteps, int nsteps) {
-  const int s = *step_dev + 1;
-  *step_dev = s;
-  *t_dev = tsteps[s < nsteps ? s : nsteps - 1];
-}
-int advance_step_enqueue(int* step_dev, int* t_dev, const int* tsteps, int nsteps, cudaStream_t st) {
-  advance_step_kernel<<<1, 1, 0, st>>>(step_dev, t_dev, tsteps, nsteps);
-  CM_CUDA(cudaGetLastError());
-  return 0;
-}
-__global__ void advance_step_cond_kernel(int* step_dev, int* t_dev, const int* tsteps, int nsteps,
-                                         cudaGraphConditionalHandle h) {
-  const int s = *step_dev + 1;
-  *step_dev = s;
-  *t_dev = tsteps[s < nsteps ? s : nsteps - 1];
-  cudaGraphSetConditional(h, s < nsteps ? 1u : 0u);
-}
-int advance_step_cond_enqueue(int* step_dev, int* t_dev, const int* tsteps, int nsteps, cudaGraphConditionalHandle h,
-                              cudaStream_t st) {
-  advance_step_cond_kernel<<<1, 1, 0, st>>>(step_dev, t_dev, tsteps, nsteps, h);
-  CM_CUDA(cudaGetLastError());
-  return 0;
-}
-__global__ void chain_begin_kernel(int* step_dev, int* t_dev, const int* tsteps, unsigned long long* chain_dev,
-                                   unsigned long long seed, long long sample_offset) {
-  *step_dev = 0;
-  *t_dev = tsteps[0];
-  chain_dev[0] = seed;
-  chain_dev[1] = static_cast<unsigned long long>(sample_offset);
-}
-int chain_begin_enqueue(int* step_dev, int* t_dev, const int* tsteps, unsigned long long* chain_dev,
-                        unsigned long long seed, long long sample_offset, cudaStream_t st) {
-  chain_begin_kernel<<<1, 1, 0, st>>>(step_dev, t_dev, tsteps, chain_dev, seed, sample_offset);
-  CM_CUDA(cudaGetLastError());
   return 0;
 }
 

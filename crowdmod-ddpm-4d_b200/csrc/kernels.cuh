@@ -1,6 +1,7 @@
 // Bandwidth / small-op kernels of the UNet hot path (everything that is not the tcgen05 conv).
 // Each launcher cites the reference op it replaces.
 #pragma once
+#include "chain.cuh"
 #include "common.cuh"
 
 namespace cm {
@@ -73,17 +74,7 @@ struct FinalParams {
   int B, H, W, L, P;     // L = P + F; only frames l >= P are produced
   int cin, cout;
   float* eps_out;        // optional [B][cout][H][W][F]
-  // --- reverse-step update (all optional; x == nullptr -> eps only) ---
-  float* x;              // [B][cout][H][W][F] in/out
-  const float* coef;     // [nsteps][8] per-step coefficients
-  const int* step_dev;   // device step index
-  int mode;              // 0 = DDPM, 1 = DDIM
-  const float* noise;    // [nsteps][B*cout*H*W*F] or nullptr -> Philox
-  unsigned long long seed;
-  long long sample_offset;  // global index of sample 0 of this shard (Philox counter)
-  const unsigned long long* chain_dev;   // device {seed, sample_offset}: overrides the two fields above when set
-                                         // (a new seed / shard offset then needs no new CUDA graph)
-  float* history;        // optional [nsteps+1][B*cout*H*W*F]; slot step+1 written
+  ReverseStep rs;        // reverse-step update (rs.x == nullptr -> eps only)
 };
 int final_conv_enqueue(const FinalParams& p, cudaStream_t st);
 
@@ -129,16 +120,6 @@ bool attn_block_supported(int S, int C, int heads);
 int attn_block_enqueue(const float* x, const float* gamma, const float* beta, const __half* w_in, const float* b_in,
                        const __half* w_out, const float* b_out, float* out32, __half* out16, int B, int S, int C,
                        int heads, float eps, cudaStream_t st);
-
-// ---- chain bookkeeping: step += 1; t_dev = tsteps[step] ----
-int advance_step_enqueue(int* step_dev, int* t_dev, const int* tsteps, int nsteps, cudaStream_t st);
-// same, as the last node of a conditional WHILE body: also sets the loop condition (step < nsteps)
-int advance_step_cond_enqueue(int* step_dev, int* t_dev, const int* tsteps, int nsteps, cudaGraphConditionalHandle h,
-                              cudaStream_t st);
-// start of a chain: step = 0, t_dev = tsteps[0], chain_dev = {seed, sample_offset} (arguments travel as
-// kernel parameters: no host staging buffer, no synchronisation)
-int chain_begin_enqueue(int* step_dev, int* t_dev, const int* tsteps, unsigned long long* chain_dev,
-                        unsigned long long seed, long long sample_offset, cudaStream_t st);
 
 // ---- test-only: scalar restatement of exactly what conv_umma computes (same packed operands) ----
 struct ConvParams;

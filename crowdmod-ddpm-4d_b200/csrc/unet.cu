@@ -1,4 +1,4 @@
-// UNet execution plan + reverse-chain driver behind the C ABI (include/crowdmod_b200.h).
+// UNet execution plan behind the C ABI (include/crowdmod_b200.h); its reverse chain runs on the shared driver of chain.cu.
 //
 // The plan is a flat op list derived from the same constructor arguments the reference UNet
 // takes (models/backbones/unet.py:11-122) and executed in the order of UNet.forward
@@ -140,22 +140,9 @@ struct cm_unet {
   size_t arena_bytes = 0;
   float* temb_batch = nullptr;          // [batch][temb_ld]
   float* gn_partial = nullptr;          // [batch][GN chunks][8][2] slice statistics (reused by every GN)
-  int* d_step = nullptr;                // [0] step index, [1] current timestep
-  unsigned long long* d_chain = nullptr;   // [0] Philox seed, [1] sample offset (read by the step epilogue)
-  int* d_tsteps = nullptr;
-  float* d_coef = nullptr;
-  int chain_cap = 0;
-  std::vector<int> tsteps_host;         // what d_tsteps / d_coef currently hold (re-uploaded only on change)
-  std::vector<float> coef_host;
   float* chain_x = nullptr;             // staging copies of the caller's x / past: the graph bakes THESE pointers
   float* chain_past = nullptr;
-  // graph cache for the chain
-  cudaGraphExec_t graph_exec = nullptr;
-  cm_chain_args graph_key{};
-  int64_t last_chain_launches = 0;
-  int64_t graph_launches_per_step = 0;
-  int64_t last_chain_graph_launches = 0;
-  int last_chain_graph_rebuilt = 0;
+  ChainDriver chain;                    // chain state, graph cache and stats of cm_ddpm_sample
   int64_t last_backward_launches = 0;
   double flops_per_sample = 0.0;
   // ---- training state (cm_unet_train_forward / cm_unet_backward) ----
@@ -482,10 +469,7 @@ size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 int reserve(cm_unet* u, int batch) {
   if (batch <= u->reserved_batch) return 0;
-  if (u->graph_exec) {
-    cudaGraphExecDestroy(u->graph_exec);
-    u->graph_exec = nullptr;
-  }
+  chain_drop_graph(u->chain);
   if (u->arena) CM_CUDA(cudaFree(u->arena));
   u->arena = nullptr;
   u->train_prepared = 0;   // backward launches bake forward-arena pointers
@@ -526,8 +510,6 @@ int reserve(cm_unet* u, int batch) {
   u->gn_partial = reinterpret_cast<float*>(u->arena + gnp_off);
   u->chain_x = reinterpret_cast<float*>(u->arena + cx_off);
   u->chain_past = reinterpret_cast<float*>(u->arena + cp_off);
-  if (!u->d_step) CM_CUDA(cudaMalloc(&u->d_step, 2 * sizeof(int)));
-  if (!u->d_chain) CM_CUDA(cudaMalloc(&u->d_chain, 2 * sizeof(unsigned long long)));
   u->reserved_batch = batch;
   return 0;
 }
@@ -745,10 +727,7 @@ int ensure_ready(cm_unet* u, int batch, int dup, cudaStream_t st) {
   }
   if (int e = reserve(u, batch)) return e;
   if (u->live_batch != batch || u->live_dup != dup) {
-    if (u->graph_exec) {
-      cudaGraphExecDestroy(u->graph_exec);
-      u->graph_exec = nullptr;
-    }
+    chain_drop_graph(u->chain);
     u->train_prepared = 0;           // wgrad maps bake the activation row stride
     if (int e = prepare_convs(u, batch, dup)) return e;
   }
@@ -1321,7 +1300,7 @@ int cm_unet_create(const cm_unet_config* cfg, cm_unet** out) {
 
 int cm_unet_destroy(cm_unet* u) {
   if (!u) return 0;
-  if (u->graph_exec) cudaGraphExecDestroy(u->graph_exec);
+  chain_free(u->chain);
   cudaFree(u->arena);
   cudaFree(u->wpack);
   cudaFree(u->wpack2);
@@ -1334,12 +1313,8 @@ int cm_unet_destroy(cm_unet* u) {
   cudaFree(u->d_goff_b);
   cudaFree(u->d_couts);
   cudaFree(u->d_offs);
-  cudaFree(u->d_step);
-  cudaFree(u->d_chain);
   cudaFree(u->d_jobs);
   cudaFree(u->d_up_tab);
-  cudaFree(u->d_tsteps);
-  cudaFree(u->d_coef);
   cudaFree(u->dpack);
   cudaFree(u->tarena);
   cudaFree(u->det_part);
@@ -1372,10 +1347,7 @@ static int bind_one(cm_unet* u, int idx, const float* dev_ptr) {
     u->pack_called = false;
     u->jobs_dirty = true;
     u->train_prepared = 0;
-    if (u->graph_exec) {   // baked pointers are stale
-      cudaGraphExecDestroy(u->graph_exec);
-      u->graph_exec = nullptr;
-    }
+    chain_drop_graph(u->chain);   // baked pointers are stale
     u->live_batch = 0;   // force prepare_convs (bias pointers)
   }
   return 0;
@@ -1448,7 +1420,7 @@ int cm_unet_launches_per_forward(const cm_unet* u) {
   return n;
 }
 double cm_unet_flops_per_sample(const cm_unet* u) { return u ? u->flops_per_sample : 0.0; }
-int64_t cm_last_chain_launches(const cm_unet* u) { return u ? u->last_chain_launches : -1; }
+int64_t cm_last_chain_launches(const cm_unet* u) { return u ? u->chain.launches : -1; }
 
 int cm_unet_forward(cm_unet* u, const float* future, const int64_t* t, const float* past,
                     float* eps_out, int batch, void* stream) {
@@ -1662,164 +1634,29 @@ int cm_unet_profile_forward(cm_unet* u, const float* future, const int64_t* t, c
 }
 
 int cm_ddpm_sample(cm_unet* u, const cm_chain_args* a, void* stream) {
-  CM_CHECK(u && a && a->past && a->x && a->tsteps && a->coef, "null argument");
-  CM_CHECK(a->nsteps >= 1 && a->n >= 1, "nsteps and n must be >= 1");
-  CM_CHECK(a->mode == 0 || a->mode == 1, "mode must be 0 (DDPM) or 1 (DDIM)");
-  CM_CHECK(a->use_graph >= 0 && a->use_graph <= 2, "use_graph must be 0 (eager), 1 (per-step graph) or 2 (whole-chain graph)");
+  CM_CHECK(u && a, "null argument");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (int e = ensure_ready(u, a->n, 1, st)) return e;
   u->live_train_batch = 0;   // the arena is shared: a pending training backward can no longer run
-  for (int i = 0; i < a->nsteps; ++i)
-    CM_CHECK(a->tsteps[i] >= 0 && a->tsteps[i] < u->cfg.table_steps, "tsteps[%d]=%d out of range", i,
-             a->tsteps[i]);
-  if (a->nsteps > u->chain_cap) {
-    cudaFree(u->d_tsteps);
-    cudaFree(u->d_coef);
-    CM_CUDA(cudaMalloc(&u->d_tsteps, a->nsteps * sizeof(int)));
-    CM_CUDA(cudaMalloc(&u->d_coef, (size_t)a->nsteps * 8 * sizeof(float)));
-    u->chain_cap = a->nsteps;
-    u->tsteps_host.clear();
-    u->coef_host.clear();
-    if (u->graph_exec) {
-      cudaGraphExecDestroy(u->graph_exec);
-      u->graph_exec = nullptr;
-    }
-  }
-  // schedule tables: uploaded only when they differ from what the device already holds (the host
-  // vectors are the staging copies: the async copies read them, never the caller's arrays)
-  {
-    const bool same_t = (int)u->tsteps_host.size() == a->nsteps &&
-                        memcmp(u->tsteps_host.data(), a->tsteps, a->nsteps * sizeof(int)) == 0;
-    const bool same_c = (int)u->coef_host.size() == a->nsteps * 8 &&
-                        memcmp(u->coef_host.data(), a->coef, (size_t)a->nsteps * 8 * sizeof(float)) == 0;
-    if (!same_t || !same_c) {
-      // the previous chain may still be reading the device tables; the copy is stream-ordered behind it.
-      // The staging vectors are rewritten only here, after making sure the last upload has drained.
-      CM_CUDA(cudaStreamSynchronize(st));
-      u->tsteps_host.assign(a->tsteps, a->tsteps + a->nsteps);
-      u->coef_host.assign(a->coef, a->coef + (size_t)a->nsteps * 8);
-      CM_CUDA(cudaMemcpyAsync(u->d_tsteps, u->tsteps_host.data(), a->nsteps * sizeof(int), cudaMemcpyHostToDevice, st));
-      CM_CUDA(cudaMemcpyAsync(u->d_coef, u->coef_host.data(), (size_t)a->nsteps * 8 * sizeof(float),
-                              cudaMemcpyHostToDevice, st));
-      CM_CUDA(cudaStreamSynchronize(st));
-    }
-  }
   const cm_unet_config& c = u->cfg;
   const Level& l0 = u->levels[0];
   const size_t x_bytes = (size_t)a->n * c.out_channels * l0.H * l0.W * c.future_len * sizeof(float);
   const size_t past_bytes = (size_t)a->n * c.in_channels * l0.H * l0.W * c.past_len * sizeof(float);
-  CM_CUDA(cudaMemcpyAsync(u->chain_x, a->x, x_bytes, cudaMemcpyDeviceToDevice, st));
-  if (past_bytes) CM_CUDA(cudaMemcpyAsync(u->chain_past, a->past, past_bytes, cudaMemcpyDeviceToDevice, st));
-  if (int e = chain_begin_enqueue(u->d_step, u->d_step + 1, u->d_tsteps, u->d_chain, a->seed, a->sample_offset, st))
-    return e;
-
   RunCtx rc{};
   rc.batch = a->n;
-  rc.future = u->chain_x;
+  rc.future = u->chain_x;   // the denoiser reads the CURRENT x (the chain's staging copy)
   rc.past = u->chain_past;
   rc.temb = u->temb_table;
-  rc.t_dev = u->d_step + 1;
-  rc.temb_bstride = 0;
-  rc.fin = FinalParams{};
-  rc.fin.x = u->chain_x;
-  rc.fin.coef = u->d_coef;
-  rc.fin.step_dev = u->d_step;
-  rc.fin.mode = a->mode;
-  rc.fin.noise = a->noise;
-  rc.fin.chain_dev = u->d_chain;
-  rc.fin.history = a->history;
-
-  u->last_chain_launches = 0;
-  u->last_chain_graph_launches = 0;
-  u->last_chain_graph_rebuilt = 0;
-  if (!a->use_graph) {
-    for (int i = 0; i < a->nsteps; ++i) {
-      if (int e = run_ops(u, rc, st, &u->last_chain_launches)) return e;
-      if (int e = advance_step_enqueue(u->d_step, u->d_step + 1, u->d_tsteps, a->nsteps, st)) return e;
-      ++u->last_chain_launches;
-    }
-    CM_CUDA(cudaMemcpyAsync(a->x, u->chain_x, x_bytes, cudaMemcpyDeviceToDevice, st));
-    return 0;
-  }
-  // The captured work reads the step index, the timestep, the Philox seed / shard offset and x / past from
-  // buffers the handle owns, so one executable graph serves every chain of this (n, nsteps, mode, noise,
-  // history, kind).  kind 1: one denoiser step (+ update + step advance), replayed nsteps times.
-  // kind 2: the same step as the body of a conditional WHILE node whose condition the step-advance kernel
-  // sets from the device step counter -> the whole T-step loop is ONE graph launch (ddpm.py:214-231).
-  const cm_chain_args& k = u->graph_key;
-  const bool reuse = u->graph_exec && k.n == a->n && k.mode == a->mode && k.noise == a->noise &&
-                     k.history == a->history && k.nsteps == a->nsteps && k.use_graph == a->use_graph;
-  int64_t per_step = 0;
-  if (!reuse) {
-    if (u->graph_exec) {
-      cudaGraphExecDestroy(u->graph_exec);
-      u->graph_exec = nullptr;
-    }
-    cudaStream_t cs;
-    CM_CUDA(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
-    cudaGraph_t g = nullptr;
-    int e = 0;
-    cudaError_t ce = cudaSuccess;
-    if (a->use_graph == 1) {
-      ce = cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal);
-      if (ce == cudaSuccess) {
-        e = run_ops(u, rc, cs, &per_step);
-        if (!e) e = advance_step_enqueue(u->d_step, u->d_step + 1, u->d_tsteps, a->nsteps, cs);
-        ++per_step;
-        ce = cudaStreamEndCapture(cs, &g);
-      }
-    } else {
-      cudaGraphConditionalHandle h;
-      cudaGraph_t body = nullptr;
-      ce = cudaGraphCreate(&g, 0);
-      if (ce == cudaSuccess) ce = cudaGraphConditionalHandleCreate(&h, g, 1, cudaGraphCondAssignDefault);
-      if (ce == cudaSuccess) {
-        cudaGraphNodeParams np{};
-        np.type = cudaGraphNodeTypeConditional;
-        np.conditional.handle = h;
-        np.conditional.type = cudaGraphCondTypeWhile;
-        np.conditional.size = 1;
-        cudaGraphNode_t node;
-        ce = cudaGraphAddNode(&node, g, nullptr, 0, &np);
-        if (ce == cudaSuccess) body = np.conditional.phGraph_out[0];
-      }
-      if (ce == cudaSuccess)
-        ce = cudaStreamBeginCaptureToGraph(cs, body, nullptr, nullptr, 0, cudaStreamCaptureModeThreadLocal);
-      if (ce == cudaSuccess) {
-        e = run_ops(u, rc, cs, &per_step);
-        if (!e) e = advance_step_cond_enqueue(u->d_step, u->d_step + 1, u->d_tsteps, a->nsteps, h, cs);
-        ++per_step;
-        cudaGraph_t done = nullptr;
-        ce = cudaStreamEndCapture(cs, &done);
-      }
-    }
-    cudaStreamDestroy(cs);
-    if (e || ce != cudaSuccess) {
-      if (g) cudaGraphDestroy(g);
-      if (e) return e;
-      CM_CUDA(ce);
-    }
-    CM_CUDA(cudaGraphInstantiate(&u->graph_exec, g, 0));
-    cudaGraphDestroy(g);
-    u->graph_key = *a;
-    u->graph_launches_per_step = per_step;
-    u->last_chain_graph_rebuilt = 1;
-  } else {
-    per_step = u->graph_launches_per_step;
-  }
-  if (a->use_graph == 1) {
-    for (int i = 0; i < a->nsteps; ++i) CM_CUDA(cudaGraphLaunch(u->graph_exec, st));
-    u->last_chain_graph_launches = a->nsteps;
-  } else {
-    CM_CUDA(cudaGraphLaunch(u->graph_exec, st));
-    u->last_chain_graph_launches = 1;
-  }
-  u->last_chain_launches = per_step * a->nsteps;
-  CM_CUDA(cudaMemcpyAsync(a->x, u->chain_x, x_bytes, cudaMemcpyDeviceToDevice, st));
-  return 0;
+  return chain_run(u->chain, *a, c.table_steps, u->chain_x, x_bytes, u->chain_past, past_bytes,
+                   [u, &rc](const ReverseStep& rs, const int* t_dev, cudaStream_t s, int64_t* launches) {
+                     rc.t_dev = t_dev;
+                     rc.fin.rs = rs;
+                     return run_ops(u, rc, s, launches);
+                   },
+                   st);
 }
 
-int64_t cm_last_chain_graph_launches(const cm_unet* u) { return u ? u->last_chain_graph_launches : -1; }
-int cm_last_chain_graph_rebuilt(const cm_unet* u) { return u ? u->last_chain_graph_rebuilt : -1; }
+int64_t cm_last_chain_graph_launches(const cm_unet* u) { return u ? u->chain.graph_launches : -1; }
+int cm_last_chain_graph_rebuilt(const cm_unet* u) { return u ? u->chain.graph_rebuilt : -1; }
 
 }  // extern "C"

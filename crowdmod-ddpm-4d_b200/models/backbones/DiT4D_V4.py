@@ -256,21 +256,8 @@ class DiT4D_V4(nn.Module):
         n = _native()
         plan = self._plan()
         plan.sync(self)
-        assert x.is_contiguous() and x.dtype == torch.float32 and past.is_contiguous() and past.dtype == torch.float32
-        tsteps = tsteps.to(torch.int32).contiguous().cpu()
-        coef = coef.to(torch.float32).contiguous().cpu()
-        assert coef.shape == (tsteps.numel(), 8)
-        if noise is not None:
-            assert noise.is_cuda and noise.is_contiguous() and noise.dtype == torch.float32
-            assert noise.numel() == tsteps.numel() * x.numel()
-        a = n.ChainArgs()
-        a.past, a.x, a.n, a.nsteps = past.data_ptr(), x.data_ptr(), x.shape[0], tsteps.numel()
-        a.tsteps, a.coef, a.mode = tsteps.data_ptr(), coef.data_ptr(), int(mode)
-        a.noise = noise.data_ptr() if noise is not None else None
-        a.seed = int(seed) & 0xFFFFFFFFFFFFFFFF
-        a.sample_offset = int(sample_offset)
-        a.history = history.data_ptr() if history is not None else None
-        a.use_graph = 0 if use_graph in (False, 0, "eager") else 1     # one captured step, replayed nsteps times
+        graph_mode = 0 if use_graph in (False, 0, "eager") else 1     # one captured step, replayed nsteps times
+        a, tsteps, coef = n.chain_args(past, x, tsteps, coef, mode, noise, seed, sample_offset, history, graph_mode)
         n.check(n.lib().cm_dit_sample(plan.handle, C.byref(a), n.current_stream()))
         return x
 

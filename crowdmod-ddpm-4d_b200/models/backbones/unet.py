@@ -291,27 +291,8 @@ class UNet(nn.Module):
         plan = self._plan(rows, cols, past_len, future_len)
         plan.sync(self, need_table=True)
         plan.train_token += 1
-        assert x.is_contiguous() and x.dtype == torch.float32
-        assert past.is_contiguous() and past.dtype == torch.float32
-        tsteps = tsteps.to(torch.int32).contiguous().cpu()
-        coef = coef.to(torch.float32).contiguous().cpu()
-        assert coef.shape == (tsteps.numel(), 8)
-        if noise is not None:
-            assert noise.is_contiguous() and noise.dtype == torch.float32
-            assert noise.numel() == tsteps.numel() * x.numel()
-        a = n.ChainArgs()
-        a.past = past.data_ptr()
-        a.x = x.data_ptr()
-        a.n = x.shape[0]
-        a.nsteps = tsteps.numel()
-        a.tsteps = tsteps.data_ptr()
-        a.coef = coef.data_ptr()
-        a.mode = int(mode)
-        a.noise = noise.data_ptr() if noise is not None else None
-        a.seed = int(seed) & 0xFFFFFFFFFFFFFFFF
-        a.sample_offset = int(sample_offset)
-        a.history = history.data_ptr() if history is not None else None
-        a.use_graph = _graph_mode(use_graph)
+        a, tsteps, coef = n.chain_args(past, x, tsteps, coef, mode, noise, seed, sample_offset, history,
+                                       _graph_mode(use_graph))
         n.check(n.lib().cm_ddpm_sample(plan.handle, C.byref(a), n.current_stream()))
         return x
 

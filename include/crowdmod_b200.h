@@ -382,7 +382,9 @@ CM_API int cm_dit_forward(cm_dit* d, const float* future, const int64_t* t, cons
                    void* stream);
 /* _generate_ddpm / _generate_ddim with this backbone (ddpm.py:206-282): the update is fused into the un-patch kernel;
  * the AdaLN vectors of all timesteps come from a table built once per weight load; use_graph = 0 eager launches,
- * != 0 one captured step replayed nsteps times (seed / offset / x / past go through buffers the handle owns) */
+ * != 0 one captured step replayed nsteps times (seed / offset / x / past go through buffers the handle owns).  The
+ * schedule (tsteps / coef) is uploaded only when it differs from the last chain's; the captured step is re-captured
+ * when n, nsteps, mode, noise or history change. */
 CM_API int cm_dit_sample(cm_dit* d, const cm_chain_args* args, void* stream);
 CM_API double cm_dit_flops_per_sample(const cm_dit* d);
 CM_API int64_t cm_dit_last_launches(const cm_dit* d);

@@ -161,7 +161,7 @@ def main():
             if not (own <= 1e-6 and d <= (1e-3 if "PSNR" in k else 1e-4)):
                 fails.append(f"generate_metrics: {k} differs by {own:.3e} from its own pairs, {d:.3e} from one GPU")
 
-    # the DiT backbone has the same sample_chain contract (cm_dit_sample, whole-chain graph by default)
+    # the DiT backbone has the same sample_chain contract (cm_dit_sample, per-step graph by default)
     single, sharded = pair(dit_cfg(), "DDPM-DiT")
     from oracle import dit_oracle as dto             # the zero-initialised projections get seeded noise: eps != 0
     sd = dto.randomize_zero_init({k: v.detach().clone() for k, v in single.denoiser.state_dict().items()}, 5)

@@ -114,6 +114,54 @@ def test_dit_philox_chain_is_deterministic_and_shard_invariant():
     assert not torch.equal(run(past, x_T, 1), a)
 
 
+def _dit_chain_inputs(meta, n=3):
+    kw = meta["kw"]
+    shape = (n, 3, kw["grid_rows"], kw["grid_cols"], kw["future_len"])
+    past = do.synthetic_macroprops(n, 3, kw["grid_rows"], kw["grid_cols"], kw["past_len"], 4).cuda().contiguous()
+    return past, torch.randn(shape, generator=torch.Generator().manual_seed(2)).cuda()
+
+
+def test_dit_eager_equals_step_graph_with_history():
+    """The eager chain and the captured step replayed nsteps times enqueue the same kernels: bitwise-equal x_0 and
+    history (Philox noise, Sparsity guidance), and the same launch count."""
+    from crowdmod_ddpm_4d_b200.models.diffusion.ddpm import DDPM, ddpm_coefficients
+    meta, _ = load_golden("dit_small_b3")
+    net, _ = build_dit(meta)
+    net = net.cuda().eval()
+    ts, coef = ddpm_coefficients(DDPM(timesteps=8, scale=0.5), "Sparsity", 0.1)
+    past, x_T = _dit_chain_inputs(meta)
+    runs = []
+    for use_graph in ("eager", True):
+        x = x_T.clone()
+        hist = torch.zeros((ts.numel() + 1,) + tuple(x.shape), device="cuda")
+        net.sample_chain(past, x, ts, coef, mode=0, seed=9, history=hist, use_graph=use_graph)
+        runs.append((x, hist, net.native_stats()[0]))
+    (xe, he, le), (xg, hg, lg) = runs
+    assert torch.equal(xe, xg) and torch.equal(he[1:], hg[1:]) and torch.equal(hg[-1], xg)
+    assert le == lg > 0
+
+
+def test_dit_same_length_schedules_back_to_back_equal_a_fresh_handle():
+    """As for the UNet: a second schedule of the same length on the same handle (new tsteps / coef, same graph shape)
+    equals the same chain on a fresh handle."""
+    from crowdmod_ddpm_4d_b200.models.diffusion.ddpm import DDPM, ddpm_coefficients
+    meta, _ = load_golden("dit_small_b3")
+    ts_a, coef_a = ddpm_coefficients(DDPM(timesteps=6, scale=0.5))
+    ts_b, coef_b = (v[:6] for v in ddpm_coefficients(DDPM(timesteps=8, scale=0.5)))
+    past, x_T = _dit_chain_inputs(meta)
+
+    def run(net, ts, coef):
+        x = x_T.clone()
+        net.sample_chain(past, x, ts, coef, mode=0, seed=5)
+        return x
+
+    net = build_dit(meta)[0].cuda().eval()
+    first = run(net, ts_a, coef_a)
+    second = run(net, ts_b, coef_b)
+    assert torch.equal(second, run(build_dit(meta)[0].cuda().eval(), ts_b, coef_b))
+    assert not torch.equal(first, second)
+
+
 def test_dit_driver_and_training_guard():
     """DDPM_model(arch='DDPM-DiT') builds the backbone from the reference's config keys (ddpm.py:88-104) and samples;
     a training forward raises instead of silently running something else."""

@@ -256,6 +256,29 @@ def test_whole_chain_is_one_graph_launch_and_survives_new_seeds_and_buffers():
     assert torch.equal(x, outs[0])
 
 
+def test_same_length_schedules_back_to_back_equal_a_fresh_handle():
+    """One handle runs two different schedules of the same length back to back: the schedule tables are uploaded only
+    when they change, so the second chain must see the new tsteps / coef and equal the same chain on a fresh handle."""
+    from crowdmod_ddpm_4d_b200.models.diffusion.ddpm import DDPM, ddpm_coefficients
+    meta, _ = load_golden("unet_small_b3")
+    ts_a, coef_a = ddpm_coefficients(DDPM(timesteps=6, scale=0.5))
+    ts_b, coef_b = (v[:6] for v in ddpm_coefficients(DDPM(timesteps=8, scale=0.5)))
+    g = torch.Generator(device="cuda").manual_seed(8)
+    past = torch.randn(3, 3, 4, 4, 2, device="cuda", generator=g)
+    xT = torch.randn(3, 3, 4, 4, 2, device="cuda", generator=g)
+
+    def run(net, ts, coef):
+        x = xT.clone()
+        net.sample_chain(past, x, ts, coef, mode=0, seed=5)
+        return x
+
+    net = build_unet(meta).cuda().eval()
+    first = run(net, ts_a, coef_a)
+    second = run(net, ts_b, coef_b)
+    assert torch.equal(second, run(build_unet(meta).cuda().eval(), ts_b, coef_b))
+    assert not torch.equal(first, second)
+
+
 def test_philox_noise_is_standard_normal_and_shard_invariant():
     """One chain step with coefficients {A=0, C=1} returns exactly the injected z: checks the
     in-kernel Philox/Box-Muller stream and that it depends on the GLOBAL sample index only."""
